@@ -22,6 +22,9 @@ lm_iter   = seconds per full LM iteration (linearize + Schur + reduction over ra
 multi_gpu_parity (N>1) = N-rank vs 1-rank reduced system S, b and LM step on a small scene, run in this process;
             lm_iter.step_check = cost, model decrease, step norm and candidate cost of one LM step of the benchmarked
             problem: the problem is the same for every N, so these numbers must be too.
+
+  python bench.py --dump-outputs bench_outputs/    (N = 1) also writes what the last timed step computed, see
+                                                   dump_outputs(); the seeded workload makes two builds comparable
 """
 from __future__ import annotations
 
@@ -37,6 +40,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True        # the benchmark writes nothing into the tree (it may be read-only)
 
 METRIC = "BA corner observations/s (residual+Jacobian+normal equations)"
 UNIT = "observations/s"
@@ -379,9 +383,30 @@ def multi_gpu_parity(torch, dist, rank, world, local):
     return out
 
 
-def measure(torch, dist, gp, scene, stream, args, rank, world, local, full=True):
+DUMP_BUDGET_BYTES = 60_000_000           # array data; the .npy headers stay well inside 64 MB on top
+
+
+def dump_outputs(gp, out_dir, seed=0):
+    """What a caller of the timed step (rcc_ba_linearize) reads back, left on the device by the last timed step: the
+    normal-equation blocks of rcc_ba_get_normal_blocks, FP64, as out_dir/<name>.npy.  W holds one 6 x 6 block per
+    observation (3.4 GB on cfg4), so it is written as W_sample: the blocks of a fixed sorted sample of observations,
+    drawn with default_rng(seed), as many as fit in DUMP_BUDGET_BYTES beside the other arrays."""
+    nb = gp.normal_blocks(want_W=True)
+    W = nb.pop("W")
+    used = sum(a.nbytes for a in nb.values())
+    if used > DUMP_BUDGET_BYTES:
+        raise SystemExit(f"--dump-outputs: the normal-equation blocks alone take {used} bytes")
+    n = min(len(W), (DUMP_BUDGET_BYTES - used) // (36 * 8))
+    nb["W_sample"] = W[np.sort(np.random.default_rng(seed).choice(len(W), n, replace=False))]
+    del W
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in nb.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
+def measure(torch, dist, gp, scene, stream, args, rank, world, local, full=True, dump_dir=None):
     """All device-side and end-to-end measurements of one resident problem.  Returns a dict of per-rank numbers
-    (not yet reduced over ranks)."""
+    (not yet reduced over ranks).  With dump_dir, the outputs of the last timed step are written there (untimed)."""
     def barrier():
         if world > 1:
             dist.barrier()
@@ -414,6 +439,8 @@ def measure(torch, dist, gp, scene, stream, args, rank, world, local, full=True)
     r["total_ms"] = float(sum(a.elapsed_time(b) for a, b in pairs))
     r["prof"] = gp.profile()
     gp.profile_enable(False)
+    if dump_dir is not None:
+        dump_outputs(gp, dump_dir)
 
     # ---------------- materialised evaluation K1 (HBM-write-bound kernel) ----------------
     if full:
@@ -557,7 +584,7 @@ def run_ours(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    m = measure(torch, dist, gp, scene, stream, args, rank, world, local)
+    m = measure(torch, dist, gp, scene, stream, args, rank, world, local, dump_dir=args.dump_outputs)
     clocks = sampler.stop() if rank == 0 else None
     d = gp.dims
     n_red, n_pairs_local = int(d.n_reduced), int(d.n_pairs)
@@ -716,7 +743,13 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=10.0, help="timed CPU work of the cpu_baseline leg")
     ap.add_argument("--no-cfg2", action="store_true", help="skip the cfg2 line at N=1")
     ap.add_argument("--no-cpu-lm", action="store_true", help="skip the CPU seconds per LM iteration (lm_iter.cpu, N=1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy "
+                                                          "(N=1, --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "ours" or args.gpus != 1):
+        ap.error("--dump-outputs needs --impl ours and --gpus 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -4,8 +4,6 @@ import ctypes
 import os
 import re
 
-import pytest
-
 from robot_camera_calibration_b200 import _lib
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -43,15 +41,22 @@ def test_bad_arguments_are_rejected_without_a_device():
 
 def test_no_cpu_fallback():
     """Without a CUDA device creating a problem must fail loudly (RCC_CUDA_ERROR),
-    never fall back to a CPU path."""
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    from robot_camera_calibration_b200.problem import BAProblem
-    with pytest.raises(_lib.RccError) as e:
-        BAProblem(4, 4, 1, 0)
-    assert e.value.status == _lib.RCC_CUDA_ERROR
-    assert "no CPU fallback" in str(e.value)
+    never fall back to a CPU path.  Checked in a child process that sees no device,
+    so that it holds on a GPU machine as well."""
+    import subprocess
+    import sys
+    child = ("from robot_camera_calibration_b200 import _lib\n"
+             "from robot_camera_calibration_b200.problem import BAProblem\n"
+             "try:\n"
+             "    BAProblem(4, 4, 1, 0)\n"
+             "except _lib.RccError as e:\n"
+             "    assert e.status == _lib.RCC_CUDA_ERROR, e\n"
+             "    assert 'no CPU fallback' in str(e), e\n"
+             "else:\n"
+             "    raise SystemExit('a problem was created without a device')\n")
+    r = subprocess.run([sys.executable, "-c", child], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True)
+    assert r.returncode == 0, r.stdout + r.stderr
 
 
 def test_product_never_imports_the_oracle():
