@@ -186,22 +186,24 @@ struct SchurPrepArgs {
 };
 void launch_schur_prep(const SchurPrepArgs& a, cudaStream_t s);
 
+// Column tiling of the block-sparse SYRK: the kept blocks are cut into sub-tiles of SYRK_SUBTILE consecutive
+// blocks (the granularity of tile_ptr; one warp each), and one CTA of schur_syrk_kernel covers a column tile of
+// SYRK_CTA_SUBTILES neighbouring sub-tiles.
+constexpr int SYRK_SUBTILE = 32;
+constexpr int SYRK_CTA_SUBTILES = 2;
+
 struct SchurSyrkArgs {
   int32_t n_f, n_e;
   int32_t n_shared, n_bb;
-  int32_t tile_w;                // kept blocks per column sub-tile of tile_ptr (32)
-  int32_t n_tiles;               // ceil(n_f / tile_w) sub-tiles
+  int32_t n_tiles;               // ceil(n_f / SYRK_SUBTILE) sub-tiles
   int32_t ld;                    // row stride of S
+  int32_t n_ctas;                // entries of cta_list
   const int32_t* col_ptr;        // [n_f+1]
   const int32_t* col_pair;       // pair ids of column f, ascending e
   const int32_t* pair_e;         // [n_pairs]
   const int32_t* pair_f;         // [n_pairs]
   const int32_t* tile_ptr;       // [n_e*(n_tiles+1)]
-  const uint32_t* tile_mask;     // [n_e*n_tiles] bit b of [e][J]: row e has a pair with f = 32 J + b
-  int32_t variant;               // 0: v2 (accumulators in shared memory), 1: v3 (accumulators in registers), 2: v4 (v2 with a tensor-core product)
-  int32_t n_pairs36_fits_u32;    // 36 n_pairs < 2^32 (v3 indexes Y with 32-bit offsets)
   const int32_t* cta_list;       // [n_ctas][2] (f, column tile) of schur_syrk_kernel, heaviest first
-  int32_t n_ctas;
   const double* Y;
   const double* Yb;
   const double* Hff;             // [n_f*36]
@@ -211,7 +213,6 @@ struct SchurSyrkArgs {
 };
 void launch_schur_syrk(const SchurSyrkArgs& a, cudaStream_t s);     // kept x kept blocks (upper triangle)
 void launch_schur_border(const SchurSyrkArgs& a, cudaStream_t s);   // kept x [shared | rhs] strip
-int schur_cta_subtiles();        // tile_ptr sub-tiles covered by one schur_syrk CTA column tile
 
 struct SchurSharedArgs {
   int32_t n_e, n_f, n_shared, n_bb, ld;

@@ -229,9 +229,6 @@ static void cam_lists(const std::vector<Chunk>& chunks, int n_cam, std::vector<i
   for (size_t i = 0; i < chunks.size(); ++i) list[cur[chunks[i].cam]++] = (int32_t)i;
 }
 
-// SYRK variant for dense rows (>= 10 % of the kept blocks seen per eliminated block): 0 = v2, 1 = v3
-constexpr int SYRK_DEFAULT_DENSE = 0;
-
 static int env_int(const char* name, int dflt) {
   const char* v = getenv(name);
   return (v && *v) ? atoi(v) : dflt;
@@ -431,9 +428,8 @@ static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker
     P->col_pair.upload(col_pair, s);
     RCC_CUDA(cudaStreamSynchronize(s));
   }
-  // ---- 32-block column sub-tiles of the Schur SYRK: tile_ptr[e][J] = first pair of row e with f >= 32 J
-  P->tile_w = 32;
-  P->n_tiles = (P->n_f + P->tile_w - 1) / P->tile_w;
+  // ---- column sub-tiles of the Schur SYRK: tile_ptr[e][J] = first pair of row e with f >= SYRK_SUBTILE J
+  P->n_tiles = (P->n_f + SYRK_SUBTILE - 1) / SYRK_SUBTILE;
   {
     const int nt = P->n_tiles;
     std::vector<int32_t> tile_ptr((size_t)P->n_e * (nt + 1));
@@ -442,38 +438,20 @@ static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker
       int p = row_ptr[e];
       const int end = row_ptr[e + 1];
       for (int J = 0; J <= nt; ++J) {
-        const int fmin = J * P->tile_w;
+        const int fmin = J * SYRK_SUBTILE;
         while (p < end && pair_f[p] < fmin) ++p;
         tile_ptr[(size_t)e * (nt + 1) + J] = (J == nt) ? end : p;
       }
     }
     P->tile_ptr.upload(tile_ptr, s);
-    // presence masks of the register-accumulator SYRK: bit b of [e][J] <=> row e has the pair (e, 32 J + b)
-    std::vector<uint32_t> tile_mask((size_t)P->n_e * nt, 0u);
-#pragma omp parallel for schedule(static)
-    for (int e = 0; e < P->n_e; ++e)
-      for (int p = row_ptr[e]; p < row_ptr[e + 1]; ++p)
-        tile_mask[(size_t)e * nt + pair_f[p] / 32] |= 1u << (pair_f[p] % 32);
-    P->tile_mask.upload(tile_mask, s);
-    {
-      // which SYRK: v3 spends FP64 issue slots on absent partners (a lane per output column, whether or not its
-      // block is seen from the row) and saves v2's accumulator traffic through shared memory -- it wins when the
-      // rows are dense.  Density = mean share of the kept blocks that a row sees.
-      const double density = (P->n_e > 0 && P->n_f > 0) ? (double)P->n_pairs / ((double)P->n_e * P->n_f) : 0.0;
-      P->syrk_variant = density >= 0.10 ? SYRK_DEFAULT_DENSE : 0;
-      const char* v = getenv("RCC_SYRK");
-      if (v && !strcmp(v, "v2")) P->syrk_variant = 0;
-      if (v && !strcmp(v, "v3")) P->syrk_variant = 1;
-      if (v && !strcmp(v, "v4")) P->syrk_variant = 2;
-    }
     // work list of the SYRK: one CTA per (block row f, column tile J on or right of the diagonal),
     // column tile major so that co-resident CTAs read the same columns of Y (L2 locality; a
     // heaviest-first order was measured slower on cfg4 for that reason)
-    const int cs = schur_cta_subtiles();
-    const int nct = (nt + cs - 1) / cs;
+    const int ctw = SYRK_SUBTILE * SYRK_CTA_SUBTILES;   // kept blocks per column tile
+    const int nct = (nt + SYRK_CTA_SUBTILES - 1) / SYRK_CTA_SUBTILES;
     std::vector<int64_t> order;
     for (int J = 0; J < nct; ++J)
-      for (int f = 0; f < std::min(P->n_f, (J + 1) * 32 * cs); ++f) order.push_back((int64_t)f * nct + J);
+      for (int f = 0; f < std::min(P->n_f, (J + 1) * ctw); ++f) order.push_back((int64_t)f * nct + J);
     std::vector<int32_t> cta_list(2 * order.size());
     for (size_t i = 0; i < order.size(); ++i) {
       cta_list[2 * i] = (int32_t)(order[i] / nct);
@@ -493,10 +471,10 @@ static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker
       int64_t cum = 0;
       int g = 1;
       for (int J = 0; J < nct && g < G; ++J) {
-        cum += std::min(P->n_f, (J + 1) * 32 * cs);
+        cum += std::min(P->n_f, (J + 1) * ctw);
         if (cum * G >= (int64_t)order.size() * g) {
           P->syrk_grp_cta[g] = (int)cum;
-          P->syrk_grp_col[g] = std::min(6 * P->n_f, (J + 1) * 32 * cs * 6);
+          P->syrk_grp_col[g] = std::min(6 * P->n_f, (J + 1) * ctw * 6);
           ++g;
         }
       }
@@ -662,12 +640,9 @@ static void do_schur(P_t* P, double radius) {
     Scoped t(P, ST_SCHUR_SYRK, 5);
     SchurSyrkArgs a{};
     a.n_f = P->n_f; a.n_e = P->n_e; a.n_shared = P->n_shared; a.n_bb = P->n_bb;
-    a.tile_w = P->tile_w; a.n_tiles = P->n_tiles; a.ld = P->ld;
+    a.n_tiles = P->n_tiles; a.ld = P->ld;
     a.col_ptr = P->col_ptr.p; a.col_pair = P->col_pair.p; a.pair_e = P->pair_e.p; a.pair_f = P->pair_f.p;
     a.cta_list = P->syrk_ctas.p; a.n_ctas = P->n_syrk_ctas;
-    a.tile_mask = P->tile_mask.p;
-    a.n_pairs36_fits_u32 = (uint64_t)P->n_pairs * 36 < ((uint64_t)1 << 32);
-    a.variant = (P->syrk_variant == 1 && !(P->tile_mask.p && a.n_pairs36_fits_u32)) ? 0 : P->syrk_variant;
     a.tile_ptr = P->tile_ptr.p; a.Y = P->Y.p; a.Yb = P->Yb.p; a.Hff = P->Hff.p; a.gf = P->gf.p; a.Hfs = P->Hfs.p;
     a.S = P->S.p;
     RCC_CUDA(cudaEventRecord(P->ev_fork, P->stream));

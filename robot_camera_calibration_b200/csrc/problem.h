@@ -46,7 +46,7 @@ struct rcc_ba_problem {
   int n_views = 0, n_markers = 0, n_e = 0, n_f = 0;
   int n_bb = 2, n_red = 0, ld = 0;
   int64_t n_obs = 0, n_pairs = 0;
-  int tile_w = 32, n_tiles = 1, n_syrk_ctas = 0;
+  int n_tiles = 1, n_syrk_ctas = 0;
   // overlapped reduction (multi-rank): the SYRK work list is cut into groups of column tiles; group g covers the
   // CTAs [syrk_grp_cta[g], syrk_grp_cta[g+1]) and the columns [syrk_grp_col[g], syrk_grp_col[g+1]) of S
   static constexpr int SYRK_GROUPS = 8;
@@ -90,8 +90,6 @@ struct rcc_ba_problem {
   rcc::DBuf<int32_t> f_piece_list;   // F-pass chunk ids grouped by upload piece
   int f_piece_ptr[PIX_PIECES + 1] = {0};
   rcc::DBuf<int32_t> row_ptr, pair_e, pair_f, pair_mptr, pair_members, row_pos0, col_ptr, col_pair, tile_ptr, syrk_ctas, e_count;
-  rcc::DBuf<uint32_t> tile_mask;   // [n_e][n_tiles] presence bits of row e inside a 32-block column sub-tile (SYRK v3)
-  int syrk_variant = 0;            // 0: v2 (shared-memory accumulators), 1: v3 (register accumulators), 2: v4 (v2 + DMMA product); RCC_SYRK=v2|v3|v4
   rcc::DBuf<uint8_t> e_const;
 
   // linearisation products

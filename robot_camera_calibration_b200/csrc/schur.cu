@@ -183,8 +183,8 @@ void launch_schur_prep(const SchurPrepArgs& a, cudaStream_t s) {
 }
 
 // ---------------------------------------------------------------------------
-// schur_syrk (v2): CTA (f, J) owns the 6 x (6 * SY_WARPS * 32) strip of S in
-// block row f and column tile J; warp w of the CTA owns the 32 kept blocks of
+// schur_syrk: CTA (f, J) owns the 6 x (6 * SY_WARPS * SY_SUB) strip of S in
+// block row f and column tile J; warp w of the CTA owns the SY_SUB kept blocks of
 // sub-tile J * SY_WARPS + w and keeps their 6 x 6 output blocks in its private
 // slice of shared memory.  The CTA walks the pairs (e, f) of column f in
 // batches (Y_ef staged by cp.async, double buffered, one barrier per batch);
@@ -194,34 +194,11 @@ void launch_schur_prep(const SchurPrepArgs& a, cudaStream_t s) {
 // warp's slice.  No barrier per pair, no cross-warp traffic, fixed summation
 // order (ascending e) -> bitwise reproducible.
 // ---------------------------------------------------------------------------
-#ifndef RCC_SY_WARPS
-#define RCC_SY_WARPS 2
-#endif
-#ifndef RCC_SY_SUB
-#define RCC_SY_SUB 32
-#endif
-#ifndef RCC_SY_CTAS
-#define RCC_SY_CTAS 6
-#endif
-constexpr int SY_WARPS = RCC_SY_WARPS;
-constexpr int SY_SUB = RCC_SY_SUB;   // kept blocks per warp sub-tile: a multiple of SchurSyrkArgs::tile_w (32)
-constexpr int SY_G = SY_SUB / 32;    // tile_ptr entries per warp sub-tile
-#ifndef RCC_SY_BATCH
-#define RCC_SY_BATCH 32
-#endif
-#ifndef RCC_SY_PF
-#define RCC_SY_PF 1      // prefetch depth of the partner-column loads, in 32-item steps
-#endif
-#ifndef RCC_SY_COLS
-#define RCC_SY_COLS 1    // columns of a partner block per lane item (1, 2 or 3): fatter items = fewer 32-item steps per pair
-#endif
-constexpr int SY_COLS = RCC_SY_COLS;
-constexpr int SY_IPB = 6 / SY_COLS;      // items per partner block
-static_assert(6 % SY_COLS == 0, "items must tile the six columns of a block");
-constexpr int SY_BATCH = RCC_SY_BATCH;   // pairs of column f staged per round (<= 32: one lane per pair holds its range)
+constexpr int SY_WARPS = SYRK_CTA_SUBTILES;   // one warp per sub-tile
+constexpr int SY_SUB = SYRK_SUBTILE;          // kept blocks per warp sub-tile = tile_ptr granularity
+constexpr int SY_IPB = 6;                     // items (columns) per partner block
+constexpr int SY_BATCH = 32;                  // pairs of column f staged per round (<= 32: one lane per pair holds its range)
 static_assert(SY_BATCH <= 32, "a batch must fit the lanes of a warp");
-static_assert(SY_SUB % 32 == 0, "warp sub-tile must be a multiple of the tile_ptr granularity");
-int schur_cta_subtiles() { return SY_WARPS * SY_G; }
 
 __device__ __forceinline__ void sy_cp_async16(void* smem_dst, const void* gmem_src) {
   const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
@@ -242,23 +219,26 @@ __device__ __forceinline__ bool sy_advance(SyCursor& c, int nb, int lo_lane, int
   return true;
 }
 // one lane's item of a step: column c of partner block Y_ef' and its slot in the warp's output slice
-struct SyItem { double2 y[3 * SY_COLS]; int pf, col; };   // pf < 0: idle lane.  (raw loads only: nothing here waits on memory)
+struct SyItem { double2 y[3]; int pf, col; };   // pf < 0: idle lane.  (raw loads only: nothing here waits on memory)
 __device__ __forceinline__ void sy_load(const SchurSyrkArgs& a, const SyCursor& c, int lane, int subbase, SyItem& it) {
   const int idx = c.base + lane;
   it.pf = -1;
   it.col = 0;
   if (idx < c.n_items) {
-    const int jj = idx / SY_IPB, col = (idx - jj * SY_IPB) * SY_COLS;
+    const int jj = idx / SY_IPB, col = idx - jj * SY_IPB;
     const int j = c.lo + jj;
     const double2* yp = reinterpret_cast<const double2*>(a.Y + (size_t)j * 36 + col * 6);
 #pragma unroll
-    for (int i = 0; i < 3 * SY_COLS; ++i) it.y[i] = yp[i];
+    for (int i = 0; i < 3; ++i) it.y[i] = yp[i];
     it.pf = a.pair_f[j];
     it.col = col;
   }
 }
 
-__global__ void __launch_bounds__(SY_WARPS * 32, RCC_SY_CTAS) schur_syrk_kernel(const SchurSyrkArgs a) {
+// SchurSyrkArgs stays in the parameter bank (__grid_constant__) and its fields are read where they are used.
+// Without it the compiler loads a by-value struct of up to 128 bytes into registers at entry, which costs
+// schur_border_kernel 24 registers.
+__global__ void __launch_bounds__(SY_WARPS * 32, 6) schur_syrk_kernel(const __grid_constant__ SchurSyrkArgs a) {
   extern __shared__ __align__(16) double sm[];
   // work list: (block row f, column tile J >= tile of f), largest estimated work first
   const int f = a.cta_list[2 * blockIdx.x];
@@ -270,7 +250,7 @@ __global__ void __launch_bounds__(SY_WARPS * 32, RCC_SY_CTAS) schur_syrk_kernel(
   for (int k = lane; k < SY_SUB * 36; k += 32) acc[k] = 0.0;
 
   const int js = J * SY_WARPS + warp;                 // this warp's sub-tile
-  const bool active = (js >= sub_of_f) && (js * SY_G < a.n_tiles);
+  const bool active = (js >= sub_of_f) && (js < a.n_tiles);
   const int subbase = js * SY_SUB;
   const int c0 = a.col_ptr[f], c1 = a.col_ptr[f + 1];
   const int tps = a.n_tiles + 1;
@@ -292,8 +272,8 @@ __global__ void __launch_bounds__(SY_WARPS * 32, RCC_SY_CTAS) schur_syrk_kernel(
     if (active && cb + lane < c1) {
       const int p = a.col_pair[cb + lane];
       const int* tp = a.tile_ptr + (size_t)a.pair_e[p] * tps;
-      lo = (js == sub_of_f) ? p : tp[js * SY_G];
-      hi = tp[min((js + 1) * SY_G, a.n_tiles)];
+      lo = (js == sub_of_f) ? p : tp[js];
+      hi = tp[min(js + 1, a.n_tiles)];
     }
   };
 
@@ -317,26 +297,12 @@ __global__ void __launch_bounds__(SY_WARPS * 32, RCC_SY_CTAS) schur_syrk_kernel(
       SyItem it_c, it_n;
       bool have = sy_advance(cur, nb, lo_cur, hi_cur);
       if (have) sy_load(a, cur, lane, subbase, it_c);
-#if RCC_SY_PF >= 2
-      // second prefetch stage: the partner columns come from L2 (~600 cycles) and one step lasts ~200
-      SyCursor nn2;
-      SyItem it_nn;
-      nxt = cur;
-      bool have_n = have && sy_advance(nxt, nb, lo_cur, hi_cur);
-      if (have_n) sy_load(a, nxt, lane, subbase, it_n);
-#endif
       int q_loaded = -1;
       double Yi[36];   // Y_ef, column-major: Yi[r * 6 + k] = Y_ef[k][r]
       while (have) {
-#if RCC_SY_PF >= 2
-        nn2 = nxt;
-        const bool have_nn = have_n && sy_advance(nn2, nb, lo_cur, hi_cur);
-        if (have_nn) sy_load(a, nn2, lane, subbase, it_nn);
-#else
         nxt = cur;
         const bool have_n = sy_advance(nxt, nb, lo_cur, hi_cur);
         if (have_n) sy_load(a, nxt, lane, subbase, it_n);
-#endif
         if (cur.q != q_loaded) {
           const double2* src = reinterpret_cast<const double2*>(ybuf + cur.q * 36);
 #pragma unroll
@@ -349,36 +315,28 @@ __global__ void __launch_bounds__(SY_WARPS * 32, RCC_SY_CTAS) schur_syrk_kernel(
         }
         if (it_c.pf >= 0) {
           double2* ap = reinterpret_cast<double2*>(acc + (it_c.pf - subbase) * 36 + it_c.col * 6);
+          const double2 y0 = it_c.y[0], y1 = it_c.y[1], y2 = it_c.y[2];
+          double v[6];
 #pragma unroll
-          for (int cc = 0; cc < SY_COLS; ++cc) {
-            const double2 y0 = it_c.y[3 * cc], y1 = it_c.y[3 * cc + 1], y2 = it_c.y[3 * cc + 2];
-            double v[6];
-#pragma unroll
-            for (int r = 0; r < 6; ++r) {
-              double t = Yi[r * 6] * y0.x;
-              t = fma(Yi[r * 6 + 1], y0.y, t);
-              t = fma(Yi[r * 6 + 2], y1.x, t);
-              t = fma(Yi[r * 6 + 3], y1.y, t);
-              t = fma(Yi[r * 6 + 4], y2.x, t);
-              t = fma(Yi[r * 6 + 5], y2.y, t);
-              v[r] = t;
-            }
-            double2 a0 = ap[3 * cc], a1 = ap[3 * cc + 1], a2 = ap[3 * cc + 2];
-            a0.x += v[0]; a0.y += v[1];
-            a1.x += v[2]; a1.y += v[3];
-            a2.x += v[4]; a2.y += v[5];
-            ap[3 * cc] = a0; ap[3 * cc + 1] = a1; ap[3 * cc + 2] = a2;
+          for (int r = 0; r < 6; ++r) {
+            double t = Yi[r * 6] * y0.x;
+            t = fma(Yi[r * 6 + 1], y0.y, t);
+            t = fma(Yi[r * 6 + 2], y1.x, t);
+            t = fma(Yi[r * 6 + 3], y1.y, t);
+            t = fma(Yi[r * 6 + 4], y2.x, t);
+            t = fma(Yi[r * 6 + 5], y2.y, t);
+            v[r] = t;
           }
+          double2 a0 = ap[0], a1 = ap[1], a2 = ap[2];
+          a0.x += v[0]; a0.y += v[1];
+          a1.x += v[2]; a1.y += v[3];
+          a2.x += v[4]; a2.y += v[5];
+          ap[0] = a0; ap[1] = a1; ap[2] = a2;
         }
         __syncwarp();   // the next pair may touch the same output columns from other lanes
         cur = nxt;
         it_c = it_n;
         have = have_n;
-#if RCC_SY_PF >= 2
-        nxt = nn2;
-        it_n = it_nn;
-        have_n = have_nn;
-#endif
       }
     }
     lo_cur = lo_nxt;
@@ -401,346 +359,13 @@ __global__ void __launch_bounds__(SY_WARPS * 32, RCC_SY_CTAS) schur_syrk_kernel(
   }
 }
 
-// ---------------------------------------------------------------------------
-// schur_syrk (v3, register accumulators): same CTA = (block row f, column tile J) and the same staging of the
-// pairs (e, f) of column f as v2, but the warp's 6 x 192 strip of S lives in REGISTERS: lane l owns the columns
-// l, l + 32, ..., l + 160 of the warp's 32-block sub-tile (6 columns x 6 rows = 36 accumulators).  For a pair
-// (e, f) a 32-bit presence mask of row e over the sub-tile (tile_mask) tells every lane whether the block its
-// column sits in is a partner, and tile_ptr + popcount of the mask below it is that partner's pair index: the lane
-// loads its 48-byte column of Y_ef' (a zero column when the block is absent) -- all six columns of a visit are in
-// flight together -- and adds Y_ef^T y to its accumulators.  No shared-memory read-modify-write, no ordering
-// between lanes, one store of the strip at the end; a 32-column window none of whose blocks is present is skipped.
-// Lanes whose block is absent do no useful work (the price: FP64 issue slots at the density of the rows), which
-// pays off when rows are dense enough that v2's accumulator traffic through shared memory is the limit.
-// Fixed summation order (ascending e) -> bitwise reproducible.
-// ---------------------------------------------------------------------------
-constexpr int SR_WARPS = SY_WARPS * SY_G;   // one 32-block sub-tile per warp, the CTA covers the same column tile as v2
-constexpr int SR_BATCH = 32;
-#ifndef RCC_SR_PASS
-#define RCC_SR_PASS 3    // columns of a lane whose partner loads are in flight together: 6 (one pass, ~250 registers) or 3
-#endif
-#ifndef RCC_SR_CTAS
-#define RCC_SR_CTAS (RCC_SR_PASS == 6 ? 4 : 6)
-#endif
-constexpr int SR_PASS = RCC_SR_PASS;
-static_assert(6 % SR_PASS == 0, "passes must tile the six columns of a lane");
-__device__ __align__(16) double sr_zero_column[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
-// blocks of the sub-tile that the 32 columns 32 j .. 32 j + 31 touch
-__host__ __device__ constexpr unsigned sr_window(int j) {
-  const int b0 = (32 * j) / 6, b1 = (32 * j + 31) / 6;
-  return (b1 >= 31 ? 0xffffffffu : ((1u << (b1 + 1)) - 1u)) & ~((1u << b0) - 1u);
-}
-
-__global__ void __launch_bounds__(SR_WARPS * 32, RCC_SR_CTAS) schur_syrk_reg_kernel(const SchurSyrkArgs a) {
-  __shared__ __align__(16) double yi[2][SR_BATCH * 36];   // staged Y_ef of the batch, double buffered
-  const int f = a.cta_list[2 * blockIdx.x];
-  const int J = a.cta_list[2 * blockIdx.x + 1];
-  const int sub_of_f = f >> 5;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int js = J * SR_WARPS + warp;                 // this warp's sub-tile
-  const bool active = (js >= sub_of_f) && (js < a.n_tiles);
-  const int subbase = js * 32;
-  const int c0 = a.col_ptr[f], c1 = a.col_ptr[f + 1];
-  const int tps = a.n_tiles + 1;
-  // the diagonal sub-tile only takes partners f' >= f
-  const unsigned keep = (js == sub_of_f) ? ~((1u << (f & 31)) - 1u) : 0xffffffffu;
-  int blk[6], colo[6];                                // block (0..31) and column in the block of this lane's columns
-  unsigned below[6];                                  // bits of the blocks before it
-#pragma unroll
-  for (int j = 0; j < 6; ++j) {
-    const int c = lane + 32 * j;
-    blk[j] = c / 6;
-    colo[j] = (c - blk[j] * 6) * 6;                   // offset of the column inside a 36-double block
-    below[j] = (1u << blk[j]) - 1u;
-  }
-  double acc[6][6];
-#pragma unroll
-  for (int j = 0; j < 6; ++j)
-#pragma unroll
-    for (int r = 0; r < 6; ++r) acc[j][r] = 0.0;
-
-  auto stage = [&](int cb, int buf) {
-    const int nb = min(SR_BATCH, c1 - cb);
-    double2* dst = reinterpret_cast<double2*>(yi[buf]);
-    for (int k = tid; k < nb * 18; k += SR_WARPS * 32) {
-      const int q = k / 18, piece = k - q * 18;
-      const int p = a.col_pair[cb + q];
-      sy_cp_async16(dst + k, reinterpret_cast<const double2*>(a.Y + (size_t)p * 36) + piece);
-    }
-    asm volatile("cp.async.commit_group;" ::: "memory");
-  };
-  // lane q of every warp: presence mask and first pair of row e_q inside the warp's sub-tile
-  auto meta = [&](int cb, unsigned& mask, int& base) {
-    mask = 0u;
-    base = 0;
-    if (active && cb + lane < c1) {
-      const int e = a.pair_e[a.col_pair[cb + lane]];
-      mask = a.tile_mask[(size_t)e * a.n_tiles + js];
-      base = a.tile_ptr[(size_t)e * tps + js];
-    }
-  };
-
-  unsigned mask_cur, mask_nxt = 0u;
-  int base_cur, base_nxt = 0;
-  if (c0 < c1) stage(c0, 0);
-  meta(c0, mask_cur, base_cur);
-  int buf = 0;
-  for (int cb = c0; cb < c1; cb += SR_BATCH, buf ^= 1) {
-    const int nb = min(SR_BATCH, c1 - cb);
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
-    __syncthreads();   // batch `cb` staged by everyone; batch `cb - SR_BATCH` consumed by everyone
-    if (cb + SR_BATCH < c1) {
-      stage(cb + SR_BATCH, buf ^ 1);
-      meta(cb + SR_BATCH, mask_nxt, base_nxt);
-    }
-    if (active) {
-      for (int q = 0; q < nb; ++q) {
-        const unsigned mfull = __shfl_sync(0xffffffffu, mask_cur, q);
-        const unsigned m = mfull & keep;
-        if (m == 0u) continue;                         // warp-uniform
-        const int base = __shfl_sync(0xffffffffu, base_cur, q);
-        const double2* yq = reinterpret_cast<const double2*>(yi[buf] + q * 36);   // Y_ef: yq[3 r + i] = rows 2i, 2i+1 of column r
-        // SR_PASS columns of the lane per pass: their partner columns (or the zero column) are in flight together,
-        // then Y_ef^T y is added row by row (Y_ef comes from the staged copy, broadcast)
-#pragma unroll
-        for (int j0 = 0; j0 < 6; j0 += SR_PASS) {
-          unsigned win = 0u;
-#pragma unroll
-          for (int j = j0; j < j0 + SR_PASS; ++j) win |= sr_window(j);
-          if (!(m & win)) continue;                      // warp-uniform
-          double2 y[SR_PASS][3];
-#pragma unroll
-          for (int jj = 0; jj < SR_PASS; ++jj) {
-            const int j = j0 + jj;
-            // pair index of the lane's block in row e = first pair of the sub-tile + partners below it (32-bit
-            // offsets: the launcher checks 36 n_pairs < 2^32); absent block -> the zero column
-            const unsigned off = (unsigned)(base + __popc(mfull & below[j])) * 36u + (unsigned)colo[j];
-            const double2* yp = ((m >> blk[j]) & 1u) ? reinterpret_cast<const double2*>(a.Y + off)
-                                                     : reinterpret_cast<const double2*>(sr_zero_column);
-            y[jj][0] = yp[0];
-            y[jj][1] = yp[1];
-            y[jj][2] = yp[2];
-          }
-#pragma unroll
-          for (int r = 0; r < 6; ++r) {
-            const double2 a0 = yq[3 * r], a1 = yq[3 * r + 1], a2 = yq[3 * r + 2];
-#pragma unroll
-            for (int jj = 0; jj < SR_PASS; ++jj) {
-              const int j = j0 + jj;
-              if (m & sr_window(j)) {                    // warp-uniform
-                double t = acc[j][r];
-                t = fma(a0.x, y[jj][0].x, t);
-                t = fma(a0.y, y[jj][0].y, t);
-                t = fma(a1.x, y[jj][1].x, t);
-                t = fma(a1.y, y[jj][1].y, t);
-                t = fma(a2.x, y[jj][2].x, t);
-                t = fma(a2.y, y[jj][2].y, t);
-                acc[j][r] = t;
-              }
-            }
-          }
-        }
-      }
-    }
-    mask_cur = mask_nxt;
-    base_cur = base_nxt;
-  }
-  // S strip = base - acc   (upper triangle in block granularity); a warp-wide store is 32 consecutive columns
-  if (!active) return;
-  const size_t row0 = (size_t)6 * f;
-#pragma unroll
-  for (int j = 0; j < 6; ++j) {
-    const int fp = subbase + blk[j];
-    if (fp >= a.n_f || fp < f) continue;
-#pragma unroll
-    for (int r = 0; r < 6; ++r) {
-      double base = 0.0;
-      if (fp == f) base = a.Hff[(size_t)f * 36 + r * 6 + colo[j] / 6];
-      a.S[(row0 + r) * a.ld + (size_t)6 * subbase + lane + 32 * j] = base - acc[j][r];
-    }
-  }
-}
-
-// ---------------------------------------------------------------------------
-// schur_syrk (v4, tensor-core product): same CTA = (block row f, column tile J), same staging of the pairs (e, f) of
-// column f and the same per-warp accumulator slice in shared memory as v2, but the product of a visit is formed by the
-// FP64 tensor cores.  The partner blocks of row e inside the warp's sub-tile are CONSECUTIVE pairs, i.e. their
-// column-major 6 x 6 records are one contiguous 6 x (6 n_p) panel P of Y; O = Y_ef^T P is computed 8 columns at a
-// time with mma.m8n8k4 (A = Y_ef^T padded to 8 x 8: one register per lane and k-step instead of v2's 36 broadcast
-// registers, B = 8 columns of P read straight from global memory, two k-steps for the 6 rows) and the 6 x 8 result
-// fragment is added to the slice (layout [block][row][column]: a lane's two results are one 16-byte access).
-// What this saves over v2 is shared-memory traffic -- no re-read of Y_ef per (pair, sub-tile), which is 36 of v2's
-// ~95 wavefronts per visit -- and instructions; what it costs is FP64 pipe time (8 x 8 x 8 executed for 6 x 8 x 6).
-// Fixed order (ascending e, column groups in order) -> bitwise reproducible.
-// ---------------------------------------------------------------------------
-constexpr int SM_WARPS = SY_WARPS * SY_G;   // one 32-block sub-tile per warp; the CTA covers the same column tile as v2
-constexpr int SM_BATCH = 32;
-constexpr int SM_CHUNK = 6;                 // column groups of a visit whose B fragments are loaded together
-
-// D(8x8) += A(8x4) B(4x8), FP64.  Lane l holds A[l/4][l%4], B[l%4][l/4], D[l/4][2(l%4)], D[l/4][2(l%4)+1].
-__device__ __forceinline__ void sm_dmma(double (&c)[2], double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-               : "+d"(c[0]), "+d"(c[1])
-               : "d"(a), "d"(b));
-}
-
-struct SmVisit {
-  const double* Yp;   // panel of the partner blocks: column col of the panel at Yp + 6 col
-  int ncol;           // 6 x partners (0: nothing to do)
-  int ngrp;           // column groups of 8
-  int pf_lane;        // lane i < partners: position of partner i in the warp's slice
-  double a0, a1;      // A fragments (Y_ef^T) of the two k-steps
-};
-// B fragments of the column groups cg0 .. cg0 + SM_CHUNK - 1: lane (g = l/4, t = l%4) holds P[t][8 cg + g] and P[4 + t][..]
-__device__ __forceinline__ void sm_load(const SmVisit& v, int cg0, int g, int t, double (&b0)[SM_CHUNK], double (&b1)[SM_CHUNK]) {
-#pragma unroll
-  for (int i = 0; i < SM_CHUNK; ++i) {
-    const int col = 8 * (cg0 + i) + g;
-    const bool ok = col < v.ncol;
-    b0[i] = ok ? v.Yp[col * 6 + t] : 0.0;
-    b1[i] = (ok && t < 2) ? v.Yp[col * 6 + 4 + t] : 0.0;
-  }
-}
-__device__ __forceinline__ void sm_compute(const SmVisit& v, int cg0, int g, int t, const double (&b0)[SM_CHUNK],
-                                           const double (&b1)[SM_CHUNK], double* acc) {
-#pragma unroll
-  for (int i = 0; i < SM_CHUNK; ++i) {
-    const int cg = cg0 + i;
-    if (cg < v.ngrp) {                                   // warp-uniform
-      double d[2] = {0.0, 0.0};
-      sm_dmma(d, v.a0, b0[i]);
-      sm_dmma(d, v.a1, b1[i]);
-      const int col = 8 * cg + 2 * t;                    // the lane holds O[g][col], O[g][col + 1]: same partner block
-      const int jj = col / 6, c = col - 6 * jj;
-      const int pfl = __shfl_sync(0xffffffffu, v.pf_lane, jj & 31);
-      if (g < 6 && col < v.ncol) {
-        double2* ap = reinterpret_cast<double2*>(acc + pfl * 36 + g * 6 + c);
-        double2 w = *ap;
-        w.x += d[0];
-        w.y += d[1];
-        *ap = w;
-      }
-    }
-  }
-}
-
-__global__ void __launch_bounds__(SM_WARPS * 32, 6) schur_syrk_mma_kernel(const SchurSyrkArgs a) {
-  extern __shared__ __align__(16) double sm[];
-  const int f = a.cta_list[2 * blockIdx.x];
-  const int J = a.cta_list[2 * blockIdx.x + 1];
-  const int sub_of_f = f >> 5;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int g = lane >> 2, t = lane & 3;
-  double* acc = sm + warp * (32 * 36);                // [32 blocks][6 rows][6 columns]
-  double* yi = sm + SM_WARPS * 32 * 36;               // [2][SM_BATCH][36] staged Y_ef
-  for (int k = lane; k < 32 * 36; k += 32) acc[k] = 0.0;
-
-  const int js = J * SM_WARPS + warp;                 // this warp's sub-tile
-  const bool active = (js >= sub_of_f) && (js < a.n_tiles);
-  const int subbase = js * 32;
-  const int c0 = a.col_ptr[f], c1 = a.col_ptr[f + 1];
-  const int tps = a.n_tiles + 1;
-
-  auto stage = [&](int cb, int buf) {
-    const int nb = min(SM_BATCH, c1 - cb);
-    double2* dst = reinterpret_cast<double2*>(yi + buf * SM_BATCH * 36);
-    for (int k = tid; k < nb * 18; k += SM_WARPS * 32) {
-      const int q = k / 18, piece = k - q * 18;
-      const int p = a.col_pair[cb + q];
-      sy_cp_async16(dst + k, reinterpret_cast<const double2*>(a.Y + (size_t)p * 36) + piece);
-    }
-    asm volatile("cp.async.commit_group;" ::: "memory");
-  };
-  // lane q of every warp: partner range of pair q of the batch inside the warp's sub-tile
-  auto meta = [&](int cb, int& lo, int& hi) {
-    lo = 0;
-    hi = 0;
-    if (active && cb + lane < c1) {
-      const int p = a.col_pair[cb + lane];
-      const int* tp = a.tile_ptr + (size_t)a.pair_e[p] * tps;
-      lo = (js == sub_of_f) ? p : tp[js];
-      hi = tp[js + 1];
-    }
-  };
-  // everything a visit needs except the B fragments (q >= nb or no partner: ncol = 0)
-  auto setup = [&](int q, int nb, int lo_lane, int hi_lane, const double* ybuf, SmVisit& v) {
-    const int qq = min(q, nb - 1);
-    const int lo = __shfl_sync(0xffffffffu, lo_lane, qq);
-    const int hi = __shfl_sync(0xffffffffu, hi_lane, qq);
-    const int np = (q < nb) ? max(hi - lo, 0) : 0;
-    v.ncol = 6 * np;
-    v.ngrp = (v.ncol + 7) >> 3;
-    v.Yp = a.Y + (size_t)lo * 36;
-    v.pf_lane = (lane < np) ? a.pair_f[lo + lane] - subbase : 0;
-    const double* yb = ybuf + qq * 36;                  // Y_ef: element (k, r) at yb[6 r + k]
-    v.a0 = (g < 6) ? yb[g * 6 + t] : 0.0;
-    v.a1 = (g < 6 && t < 2) ? yb[g * 6 + 4 + t] : 0.0;
-  };
-  auto rest = [&](const SmVisit& v) {                  // column groups beyond the first chunk (rows with > 8 partners)
-    for (int cg0 = SM_CHUNK; cg0 < v.ngrp; cg0 += SM_CHUNK) {
-      double b0[SM_CHUNK], b1[SM_CHUNK];
-      sm_load(v, cg0, g, t, b0, b1);
-      sm_compute(v, cg0, g, t, b0, b1, acc);
-    }
-  };
-
-  int lo_cur, hi_cur, lo_nxt = 0, hi_nxt = 0;
-  if (c0 < c1) stage(c0, 0);
-  meta(c0, lo_cur, hi_cur);
-  int buf = 0;
-  for (int cb = c0; cb < c1; cb += SM_BATCH, buf ^= 1) {
-    const int nb = min(SM_BATCH, c1 - cb);
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
-    __syncthreads();   // batch `cb` staged by everyone; batch `cb - SM_BATCH` consumed by everyone
-    if (cb + SM_BATCH < c1) {
-      stage(cb + SM_BATCH, buf ^ 1);
-      meta(cb + SM_BATCH, lo_nxt, hi_nxt);
-    }
-    if (active) {
-      const double* ybuf = yi + buf * SM_BATCH * 36;
-      // two pairs per round: the loads of both are issued before the first is computed
-      for (int q = 0; q < nb; q += 2) {
-        SmVisit v0, v1;
-        setup(q, nb, lo_cur, hi_cur, ybuf, v0);
-        setup(q + 1, nb, lo_cur, hi_cur, ybuf, v1);
-        double b00[SM_CHUNK], b01[SM_CHUNK], b10[SM_CHUNK], b11[SM_CHUNK];
-        sm_load(v0, 0, g, t, b00, b01);
-        sm_load(v1, 0, g, t, b10, b11);
-        sm_compute(v0, 0, g, t, b00, b01, acc);
-        rest(v0);
-        __syncwarp();   // the next pair may touch the same outputs from other lanes
-        sm_compute(v1, 0, g, t, b10, b11, acc);
-        rest(v1);
-        __syncwarp();
-      }
-    }
-    lo_cur = lo_nxt;
-    hi_cur = hi_nxt;
-  }
-  // S strip = base - acc   (upper triangle in block granularity), rows written as contiguous runs
-  if (!active) return;
-  __syncwarp();
-  const int nblk = min(32, a.n_f - subbase);
-  const size_t row0 = (size_t)6 * f;
-  for (int r = 0; r < 6; ++r) {
-    for (int cl = lane; cl < nblk * 6; cl += 32) {
-      const int fl = cl / 6, c = cl - fl * 6;
-      const int fp = subbase + fl;
-      if (fp < f) continue;
-      double base = 0.0;
-      if (fp == f) base = a.Hff[(size_t)f * 36 + r * 6 + c];
-      a.S[(row0 + r) * a.ld + (size_t)6 * subbase + cl] = base - acc[fl * 36 + r * 6 + c];
-    }
-  }
-}
-
 // border strip of block row f:  [H_fs | g_f] - sum_e Y_ef^T Yb_e.  Every pair of column f meets every
 // border block, so a lane owns fixed border columns and keeps their 6-row outputs in registers:
 // lane = (slot u, column); the (warp, slot) slices stride over the staged pairs and are summed in a
 // fixed order at the end.  Y_ef and e are staged per batch exactly as in schur_syrk_kernel.
 constexpr int SB_WARPS = 4;
 constexpr int SB_MAXPASS = 4;   // up to 128 border columns (n_shared <= 125)
-__global__ void __launch_bounds__(SB_WARPS * 32) schur_border_kernel(const SchurSyrkArgs a) {
+__global__ void __launch_bounds__(SB_WARPS * 32) schur_border_kernel(const __grid_constant__ SchurSyrkArgs a) {
   __shared__ __align__(16) double yi[2][SY_BATCH * 36];
   __shared__ int se[2][SY_BATCH];
   __shared__ double red[SB_WARPS * 32 * 6];
@@ -834,24 +459,10 @@ __global__ void __launch_bounds__(SB_WARPS * 32) schur_border_kernel(const Schur
 
 void launch_schur_syrk(const SchurSyrkArgs& a, cudaStream_t s) {
   if (a.n_f == 0) return;
-  RCC_REQUIRE(a.tile_w == 32, RCC_BAD_ARG, "schur_syrk: tile_ptr granularity must be 32");
   const size_t smem = (size_t)(SY_WARPS * SY_SUB * 36 + 2 * SY_BATCH * 36) * sizeof(double);
   static SmemOptIn optin;
   optin.ensure(schur_syrk_kernel, smem);
-  if (a.n_ctas > 0) {
-    if (a.variant == 2) {
-      const size_t smem4 = (size_t)(SM_WARPS * 32 * 36 + 2 * SM_BATCH * 36) * sizeof(double);
-      static SmemOptIn optin4;
-      optin4.ensure(schur_syrk_mma_kernel, smem4);
-      schur_syrk_mma_kernel<<<a.n_ctas, SM_WARPS * 32, smem4, s>>>(a);
-    } else if (a.variant == 1) {
-      RCC_REQUIRE(a.tile_mask != nullptr, RCC_BAD_ARG, "schur_syrk: the register variant needs the presence masks");
-      RCC_REQUIRE(a.n_pairs36_fits_u32, RCC_BAD_ARG, "schur_syrk: the register variant indexes Y with 32-bit offsets");
-      schur_syrk_reg_kernel<<<a.n_ctas, SR_WARPS * 32, 0, s>>>(a);
-    } else {
-      schur_syrk_kernel<<<a.n_ctas, SY_WARPS * 32, smem, s>>>(a);
-    }
-  }
+  if (a.n_ctas > 0) schur_syrk_kernel<<<a.n_ctas, SY_WARPS * 32, smem, s>>>(a);
   RCC_CUDA(cudaGetLastError());
 }
 

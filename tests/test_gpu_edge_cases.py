@@ -333,13 +333,10 @@ def test_integer_pixel_entry_points_are_bit_identical_to_fp64(shuffled):
                     assert np.array_equal(np.asarray(a), np.asarray(b))
 
 
-@pytest.mark.parametrize("variant", ["v3", "v4"])
 @pytest.mark.parametrize("model,elim", [("single", "views"), ("single", "markers"), ("rig", "views")])
-def test_alternative_syrk_kernels_match_the_oracle(model, elim, variant, monkeypatch):
-    """RCC_SYRK=v3 (strip of S in registers, presence masks per 32-block sub-tile) and v4 (tensor-core product into
-    the shared-memory slice) -- the measured-and-not-chosen variants in schur.cu -- stay correct: ragged rows over
-    several sub-tiles, both elimination directions."""
-    monkeypatch.setenv("RCC_SYRK", variant)              # read when the observations are set
+def test_syrk_ragged_rows_over_several_subtiles_match_the_oracle(model, elim):
+    """The block-sparse Schur SYRK on ragged rows that span several 32-block column sub-tiles, in both elimination
+    directions and for the rig model."""
     s = make_scene(70, 90, 0.35, n_cam=2 if model == "rig" else 1, model=model, seed=77, round_pixels=True)
     rng = np.random.default_rng(5)
     _keep(s, rng.random(s.n_blocks) < 0.8)               # ragged rows

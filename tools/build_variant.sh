@@ -1,5 +1,5 @@
 #!/bin/bash
-# builds a kernel-variant library: tools/build_variant.sh NAME "-DRCC_SY_SUB=64 ..."  -> robot_camera_calibration_b200/build/variants/librcc_ba_NAME.so
+# builds a kernel-variant library: tools/build_variant.sh NAME "-DRCC_K2_MIN_CTAS=2 ..."  -> robot_camera_calibration_b200/build/variants/librcc_ba_NAME.so
 set -e
 cd "$(dirname "$0")/.."
 name=$1; defs=$2
