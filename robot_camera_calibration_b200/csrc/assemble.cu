@@ -205,35 +205,40 @@ assemble_kernel(const AssembleArgs a) {
     }
     __syncwarp();
     // ---- phase 2: tile products over the 8 residual rows of every block ----
-    const int nblk = min(BPW, ch.count - it);
-#pragma unroll
-    for (int bb = 0; bb < BPW; ++bb) {
-      if (bb < nblk) {
-        const double* f0 = frag + bb * BS;
-        const double* f1 = f0 + 4 * RS;
-        const double a0 = f0[0], a1 = f1[0];
-        const double b0 = f0[PG::COL_B], b1 = f1[PG::COL_B];
-        dmma(cAA, a0, a0); dmma(cAA, a1, a1);
-        dmma(cAB, a0, b0); dmma(cAB, a1, b1);
-        if (EPASS) { dmma(cBB, b0, b0); dmma(cBB, b1, b1); }
-        if (RIG) {
-          const double x0 = f0[PG::COL_X], x1 = f1[PG::COL_X];
-          dmma(cAX, a0, x0); dmma(cAX, a1, x1);
-          if (EPASS) {
-            dmma(cBX, b0, x0); dmma(cBX, b1, x1);
-            dmma(cXX, x0, x0); dmma(cXX, x1, x1);
-          }
-        }
+    auto block_products = [&](int bb) {
+      const double* f0 = frag + bb * BS;
+      const double* f1 = f0 + 4 * RS;
+      const double a0 = f0[0], a1 = f1[0];
+      const double b0 = f0[PG::COL_B], b1 = f1[PG::COL_B];
+      dmma(cAA, a0, a0); dmma(cAA, a1, a1);
+      dmma(cAB, a0, b0); dmma(cAB, a1, b1);
+      if (EPASS) { dmma(cBB, b0, b0); dmma(cBB, b1, b1); }
+      if (RIG) {
+        const double x0 = f0[PG::COL_X], x1 = f1[PG::COL_X];
+        dmma(cAX, a0, x0); dmma(cAX, a1, x1);
         if (EPASS) {
-          // cross block W = J_own^T J_other of this observation block (rows own, columns other)
-          const double t0 = f0[PG::COL_C], t1 = f1[PG::COL_C];
-          double cW[2] = {0.0, 0.0};
-          dmma(cW, a0, t0); dmma(cW, a1, t1);
-          if (lane < 24 && (lane & 3) < 3)
-            *reinterpret_cast<double2*>(a.W + ((int64_t)ch.start + it + bb) * 36 + (lane >> 2) * 6 + 2 * (lane & 3)) =
-                make_double2(cW[0], cW[1]);
+          dmma(cBX, b0, x0); dmma(cBX, b1, x1);
+          dmma(cXX, x0, x0); dmma(cXX, x1, x1);
         }
       }
+      if (EPASS) {
+        // cross block W = J_own^T J_other of this observation block (rows own, columns other)
+        const double t0 = f0[PG::COL_C], t1 = f1[PG::COL_C];
+        double cW[2] = {0.0, 0.0};
+        dmma(cW, a0, t0); dmma(cW, a1, t1);
+        if (lane < 24 && (lane & 3) < 3)
+          *reinterpret_cast<double2*>(a.W + ((int64_t)ch.start + it + bb) * 36 + (lane >> 2) * 6 + 2 * (lane & 3)) =
+              make_double2(cW[0], cW[1]);
+      }
+    };
+    // a full group (every group of a chunk but its last) runs as straight-line code, so that the fragment
+    // loads of the next blocks can be issued ahead of the current block's MMAs
+    if (ch.count - it >= BPW) {
+#pragma unroll
+      for (int bb = 0; bb < BPW; ++bb) block_products(bb);
+    } else {
+#pragma unroll 1
+      for (int bb = 0; bb < ch.count - it; ++bb) block_products(bb);
     }
     __syncwarp();
   }
@@ -365,7 +370,7 @@ __device__ __forceinline__ void finalize_side_body(const FinalizeSideArgs& a, in
 // finalize_shared: shared x shared block, gradient and cost per camera, all from
 // the E-pass partials.  Stage 1: CTA (slice, camera) sums its share of the
 // camera's chunk list for every partial element (fixed order).  Stage 2: the
-// last stage-1 CTA of a camera to finish sums the FIN_SLICES partials in slice
+// last stage-1 CTA of a camera to finish sums the n_slices partials in slice
 // order and scatters them into H_ss / g_s / cost.
 // ---------------------------------------------------------------------------
 template <bool RIG>
@@ -381,7 +386,7 @@ __device__ __forceinline__ void finalize_shared_partial_body(const FinalizeShare
   const int32_t* __restrict__ list = a.cam_chunks_e + a.cam_ptr_e[cam];
   const double* __restrict__ part = a.part_e;
   const int n = a.cam_ptr_e[cam + 1] - a.cam_ptr_e[cam];
-  const int per = (n + FIN_SLICES - 1) / FIN_SLICES;
+  const int per = (n + a.n_slices - 1) / a.n_slices;
   const int lo = slice * per, hi = min(n, lo + per);
   double acc[NR];
 #pragma unroll
@@ -407,7 +412,7 @@ __device__ __forceinline__ void finalize_shared_partial_body(const FinalizeShare
     double s = 0.0;
 #pragma unroll
     for (int w = 0; w < 8; ++w) s += red[w][k];
-    a.scratch[((size_t)cam * FIN_SLICES + slice) * PART + k] = s;
+    a.scratch[((size_t)cam * a.n_slices + slice) * PART + k] = s;
   }
   // the last slice of the camera to arrive runs the second stage (fixed summation order: slice 0, 1, ...)
   __shared__ int is_last;
@@ -415,7 +420,7 @@ __device__ __forceinline__ void finalize_shared_partial_body(const FinalizeShare
   __syncthreads();
   if (threadIdx.x == 0) {
     const int done = atomicAdd(a.done_count + cam, 1);
-    is_last = (done == FIN_SLICES - 1);
+    is_last = (done == a.n_slices - 1);
     if (is_last) a.done_count[cam] = 0;   // ready for the next launch
   }
   __syncthreads();
@@ -455,8 +460,9 @@ __device__ __forceinline__ void finalize_shared_final_body(const FinalizeSharedA
   for (int k = tid; k < SP * ns; k += blockDim.x) H[(size_t)base * ns + k] = 0.0;
   for (int k = tid; k < PART; k += blockDim.x) {
     double s = 0.0;
-#pragma unroll 16
-    for (int sl = 0; sl < FIN_SLICES; ++sl) s += __ldcg(a.scratch + ((size_t)cam * FIN_SLICES + sl) * PART + k);
+    const double* src = a.scratch + (size_t)cam * a.n_slices * PART + k;
+#pragma unroll 32
+    for (int sl = 0; sl < a.n_slices; ++sl) s += __ldcg(src + (size_t)sl * PART);
     tot[k] = s;
   }
   __syncthreads();
@@ -480,11 +486,11 @@ __global__ void __launch_bounds__(256) finalize_fused_kernel(const FinalizeSideA
                                                              const FinalizeSharedArgs sh) {
   int i = blockIdx.x;
   const int warp = threadIdx.x >> 5;
-  if (i < FIN_SLICES * sh.n_cam) {
-    finalize_shared_partial_body<RIG>(sh, i % FIN_SLICES, i / FIN_SLICES);
+  if (i < sh.n_slices * sh.n_cam) {
+    finalize_shared_partial_body<RIG>(sh, i % sh.n_slices, i / sh.n_slices);
     return;
   }
-  i -= FIN_SLICES * sh.n_cam;
+  i -= sh.n_slices * sh.n_cam;
   const int f_ctas = (f.n_own + FIN_OWN_PER_CTA - 1) / FIN_OWN_PER_CTA;
   if (i < f_ctas) {
     finalize_side_body<RIG, false>(f, i * FIN_OWN_PER_CTA + warp);
@@ -495,7 +501,7 @@ __global__ void __launch_bounds__(256) finalize_fused_kernel(const FinalizeSideA
 
 void launch_finalize(bool rig, const FinalizeSideArgs& e, const FinalizeSideArgs& f, const FinalizeSharedArgs& sh,
                      cudaStream_t s) {
-  const int grid = ceil_div(e.n_own, FIN_OWN_PER_CTA) + ceil_div(f.n_own, FIN_OWN_PER_CTA) + FIN_SLICES * sh.n_cam;
+  const int grid = ceil_div(e.n_own, FIN_OWN_PER_CTA) + ceil_div(f.n_own, FIN_OWN_PER_CTA) + sh.n_slices * sh.n_cam;
   if (rig) finalize_fused_kernel<true><<<grid, 256, 0, s>>>(e, f, sh);
   else finalize_fused_kernel<false><<<grid, 256, 0, s>>>(e, f, sh);
   RCC_CUDA(cudaGetLastError());

@@ -98,11 +98,18 @@ struct FinalizeSharedArgs {
   double* Hss;                  // [n_shared*n_shared] block diagonal (zeroed by the kernel)
   double* gs;                   // [n_shared]
   double* cost2_cam;            // [n_cam] sum r^2 per camera
-  double* scratch;              // [n_cam * FIN_SLICES * PART_E] first-stage partial tiles
+  double* scratch;              // [n_cam * n_slices * PART_E] first-stage partial tiles
   int32_t* done_count;          // [n_cam] first-stage CTAs finished (zero between launches)
   int32_t robust;               // 1: cost = tail slot (sum rho), else BB[7][7] (sum r^2)
+  int32_t n_slices;             // first-stage CTAs per camera (fin_slices)
 };
-constexpr int FIN_SLICES = 64;  // CTAs per camera in the first stage of finalize_shared
+// First-stage CTAs per camera of finalize_shared: enough that the first stage of all cameras together puts two
+// CTAs on every SM (one camera would otherwise read its E-pass partials through a fraction of the GPU), and at
+// least 64.
+inline int fin_slices(int n_sm, int n_cam) {
+  const int per_cam = (2 * n_sm + n_cam - 1) / n_cam;
+  return per_cam > 64 ? per_cam : 64;
+}
 // E side, F side and both stages of the shared reduction in one launch
 void launch_finalize(bool rig, const FinalizeSideArgs& e, const FinalizeSideArgs& f, const FinalizeSharedArgs& sh,
                      cudaStream_t s);

@@ -611,7 +611,7 @@ static void do_linearize(P_t* P) {
     FinalizeSideArgs fe{P->part_e.p, P->e_chunks.p, P->e_chunk_ptr.p, P->n_e, P->n_shared, P->Hee.p, P->ge.p, P->Hes.p};
     FinalizeSideArgs ff{P->part_f.p, P->f_chunks.p, P->f_chunk_ptr.p, P->n_f, P->n_shared, P->Hff.p, P->gf.p, P->Hfs.p};
     FinalizeSharedArgs fs{P->part_e.p, P->cam_chunks_e.p, P->cam_ptr_e.p, P->n_cam, P->n_shared, P->Hss.p, P->gs.p,
-                          P->cost2_cam.p, P->fin_scratch.p, P->fin_done.p, P->loss != 0 ? 1 : 0};
+                          P->cost2_cam.p, P->fin_scratch.p, P->fin_done.p, P->loss != 0 ? 1 : 0, P->fin_slices};
     launch_finalize(P->rig, fe, ff, fs, P->stream);
   }
   P->linearized = true;
@@ -1105,6 +1105,7 @@ int rcc_ba_create(const rcc_ba_options* opt, rcc_ba_problem** out) {
     P->sp = P->rig ? 15 : 9;
     P->n_cam = opt->n_cameras;
     P->n_shared = P->n_cam * P->sp;
+    P->fin_slices = fin_slices(prop.multiProcessorCount, P->n_cam);
     P->n_views = opt->n_views;
     P->n_markers = opt->n_markers;
     P->n_obs = opt->n_obs_blocks;
@@ -1140,7 +1141,7 @@ int rcc_ba_create(const rcc_ba_options* opt, rcc_ba_problem** out) {
     P->c_intr.assign(P->n_cam, 0); P->c_dist.assign(P->n_cam, 0); P->c_ext.assign(P->n_cam, 0);
     P->Hee.alloc((size_t)P->n_e * 36); P->ge.alloc((size_t)P->n_e * 6); P->Hes.alloc((size_t)P->n_e * 6 * P->n_shared);
     P->Hff.alloc((size_t)P->n_f * 36); P->gf.alloc((size_t)P->n_f * 6); P->Hfs.alloc((size_t)P->n_f * 6 * P->n_shared);
-    P->fin_scratch.alloc((size_t)P->n_cam * FIN_SLICES * PassGeom<true>::PART_E);
+    P->fin_scratch.alloc((size_t)P->n_cam * P->fin_slices * PassGeom<true>::PART_E);
     P->fin_done.alloc((size_t)P->n_cam); P->fin_done.zero(s);
     P->Hss.alloc((size_t)P->n_shared * P->n_shared); P->gs.alloc((size_t)P->n_shared); P->cost2_cam.alloc(P->n_cam);
     P->Linv.alloc((size_t)P->n_e * 36); P->Yb.alloc((size_t)P->n_e * P->n_bb * 36); P->d2e.alloc((size_t)P->n_e * 6);

@@ -42,6 +42,7 @@ struct rcc_ba_problem {
   rcc_ba_options opt{};
   bool rig = false;
   int sp = 9, n_cam = 1, n_shared = 9;
+  int fin_slices = 64;   // first-stage CTAs per camera of the shared-parameter finalize (kernels.h: fin_slices)
   bool elim_view = true;
   int n_views = 0, n_markers = 0, n_e = 0, n_f = 0;
   int n_bb = 2, n_red = 0, ld = 0;
