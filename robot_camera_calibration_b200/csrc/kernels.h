@@ -290,14 +290,13 @@ void launch_pack_band(double* S, int32_t ld, int32_t n_rows, int32_t c0, int32_t
 void launch_apply(const double* x, const double* d, double* out, int64_t n, cudaStream_t s);
 // make a symmetric full matrix out of the upper triangle (parity read-back only)
 void launch_symmetrize(double* S, int32_t n, int32_t ld, cudaStream_t s);
-// gather pixels from caller order into a sorted order
-void launch_permute_pixels(const double* src, const int32_t* orig, double* dst, int64_t n, cudaStream_t s);
-// one piece of an upload in sorted order: e_pix[g] = (double) src16[g] (src16 == nullptr: e_pix already holds the
-// piece) and f_pix[f_inv[g]] = e_pix[g], so that the F-sorted copy is complete when the last piece has landed
-void launch_scatter_pixels(const int16_t* src16, double* e_pix, const int32_t* f_inv, double* f_pix, int64_t n,
-                           cudaStream_t s);
-// integer pixels -> FP64: dst[g] = (double) src[orig ? orig[g] : g]  for blocks g in [0, n)
-void launch_convert_pixels_i16(const int16_t* src, const int32_t* orig, double* dst, int64_t n, cudaStream_t s);
+// caller's pixel blocks (T = double, int32_t or int16_t) -> both sorted FP64 layouts, for sorted blocks g in [0, n):
+// e_pix[g] = (double) src[orig ? orig[g] : g] and f_pix[f_inv[g]] = e_pix[g].  src == nullptr: e_pix already holds
+// the blocks (an FP64 upload copied straight into it) and is only read, never written again.  src must not alias
+// e_pix or f_pix otherwise.  Called on a piece of the sorted order, e_pix and f_inv point at the piece's first block.
+template <typename T>
+void launch_load_pixels(const T* src, const int32_t* orig, double* e_pix, const int32_t* f_inv, double* f_pix,
+                        int64_t n, cudaStream_t s);
 // write a scratch buffer (L2 flush)
 void launch_fill(double* p, int64_t n, double v, cudaStream_t s);
 // FP64 FMA throughput microbenchmark kernel; returns number of FMAs issued

@@ -16,6 +16,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <numeric>
+#include <type_traits>
 
 using namespace rcc;
 
@@ -234,8 +235,7 @@ static int env_int(const char* name, int dflt) {
   return (v && *v) ? atoi(v) : dflt;
 }
 
-static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker_idx, const int32_t* cam_idx,
-                          const double* pixels) {
+static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker_idx, const int32_t* cam_idx) {
   const int64_t n = P->n_obs;
   RCC_REQUIRE(n < (int64_t)2000000000 / 36 * 8, RCC_BAD_ARG, "too many observation blocks for 32-bit indexing");
   RCC_CUDA(cudaStreamSynchronize(P->side_stream));   // a piecewise pixel upload may still target the old buffers
@@ -271,20 +271,17 @@ static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker
   P->cam_ptr_e.upload(ptr, s);
   {
     std::vector<int32_t> own((size_t)n), oth((size_t)n), cam((size_t)n);
-    std::vector<double> pix((size_t)n * 8);
 #pragma omp parallel for
     for (int64_t i = 0; i < n; ++i) {
       const int32_t o = perm_e[i];
       own[i] = e_of[o];
       oth[i] = f_of[o];
       cam[i] = cam_idx[o];
-      memcpy(&pix[(size_t)i * 8], pixels + (size_t)o * 8, 64);
     }
     P->e_own.upload(own, s);
     P->e_oth.upload(oth, s);
     P->e_cam.upload(cam, s);
     P->e_orig.upload(perm_e, s);
-    P->e_pix.upload(pix, s);
     RCC_CUDA(cudaStreamSynchronize(s));
   }
   {
@@ -296,7 +293,7 @@ static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker
     P->pix_pending = false;
     // pieces are cut at eliminated-block boundaries: 8 for large uploads (what is left after the copy is the work
     // of the last piece: keep it short), 4 for small ones, where a piece must still be worth a launch
-    const int np = n >= 4000000 ? rcc_ba_problem::PIX_PIECES : 4;
+    const int np = n >= rcc_ba_problem::LARGE_UPLOAD_BLOCKS ? rcc_ba_problem::PIX_PIECES : 4;
     P->piece_chunk[0] = 0;
     P->piece_block[0] = 0;
     int e_cut = 0;
@@ -347,26 +344,16 @@ static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker
   P->cam_ptr_f.upload(ptr, s);
   {
     std::vector<int32_t> oth((size_t)n);
-    std::vector<double> pix((size_t)n * 8);
 #pragma omp parallel for
-    for (int64_t i = 0; i < n; ++i) {
-      const int32_t o = perm_f[i];
-      oth[i] = e_of[o];
-      memcpy(&pix[(size_t)i * 8], pixels + (size_t)o * 8, 64);
-    }
+    for (int64_t i = 0; i < n; ++i) oth[i] = e_of[perm_f[i]];
     P->f_oth.upload(oth, s);
-    P->f_orig.upload(perm_f, s);
-    {
-      // E-sorted position -> F-sorted position (the piecewise uploads scatter every piece into f_pix as it lands)
-      std::vector<int32_t> e_pos_of_caller((size_t)n), f_inv((size_t)n);
+    // E-sorted position -> F-sorted position (the pixel loader scatters every E-sorted block into f_pix)
+    std::vector<int32_t> e_pos_of_caller((size_t)n), f_inv((size_t)n);
 #pragma omp parallel for
-      for (int64_t i = 0; i < n; ++i) e_pos_of_caller[perm_e[i]] = (int32_t)i;
+    for (int64_t i = 0; i < n; ++i) e_pos_of_caller[perm_e[i]] = (int32_t)i;
 #pragma omp parallel for
-      for (int64_t i = 0; i < n; ++i) f_inv[e_pos_of_caller[perm_f[i]]] = (int32_t)i;
-      P->f_inv.upload(f_inv, s);
-      RCC_CUDA(cudaStreamSynchronize(s));
-    }
-    P->f_pix.upload(pix, s);
+    for (int64_t i = 0; i < n; ++i) f_inv[e_pos_of_caller[perm_f[i]]] = (int32_t)i;
+    P->f_inv.upload(f_inv, s);
     RCC_CUDA(cudaStreamSynchronize(s));
   }
 
@@ -489,6 +476,8 @@ static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker
   }
 
   // ---- buffers that scale with the observations
+  P->e_pix.alloc((size_t)n * 8);
+  P->f_pix.alloc((size_t)n * 8);
   P->part_e.alloc((size_t)P->n_chunks_e * (P->rig ? PassGeom<true>::PART_E : PassGeom<false>::PART_E));
   P->part_f.alloc((size_t)P->n_chunks_f * (P->rig ? PassGeom<true>::PART_F : PassGeom<false>::PART_F));
   P->W.alloc((size_t)n * 36);
@@ -553,7 +542,7 @@ static void do_linearize(P_t* P) {
   a.loss = P->loss;
   a.loss_a2 = P->loss_scale * P->loss_scale;
   {
-    Scoped t(P, ST_ASSEMBLE_E, 1);
+    Scoped t(P, ST_ASSEMBLE_E, P->pix_pending ? 0 : 1);
     a.oth = P->e_oth.p;
     a.pix = P->e_pix.p;
     a.chunks = P->e_chunks.p;
@@ -561,8 +550,11 @@ static void do_linearize(P_t* P) {
     a.partials = P->part_e.p;
     a.W = P->W.p;
     if (P->pix_pending) {
-      // pixels are still arriving on the side stream: the E pass of a piece starts when the piece has landed
+      // pixels are still arriving on the side stream: the E pass of a piece starts when the piece has landed,
+      // and so does its F pass on large uploads (the piece scattered itself into f_pix, and no F chunk straddles
+      // pieces)
       const int part = P->rig ? PassGeom<true>::PART_E : PassGeom<false>::PART_E;
+      f_done = P->n_obs >= rcc_ba_problem::LARGE_UPLOAD_BLOCKS;
       for (int k = 0; k < rcc_ba_problem::PIX_PIECES; ++k) {
         const int c0 = P->piece_chunk[k], c1 = P->piece_chunk[k + 1];
         RCC_CUDA(cudaStreamWaitEvent(P->stream, P->ev_piece[k], 0));
@@ -572,12 +564,8 @@ static void do_linearize(P_t* P) {
         ak.n_chunks = c1 - c0;
         ak.partials = P->part_e.p + (size_t)c0 * part;
         launch_assemble(P->rig, true, P->elim_view, ak, P->stream);
-        // ... and so does its F pass: the piece scattered itself into f_pix, and no F chunk straddles pieces
-        // (large uploads only: on cfg2-sized problems four more launches cost more than they hide)
-        if (P->n_obs < 4000000) {
-          P->launch_count += 1;
-          continue;
-        }
+        P->launch_count += 1;
+        if (!f_done) continue;
         AssembleArgs af = a;
         af.oth = P->f_oth.p;
         af.pix = P->f_pix.p;
@@ -587,10 +575,8 @@ static void do_linearize(P_t* P) {
         af.partials = P->part_f.p;
         af.W = nullptr;
         launch_assemble(P->rig, false, !P->elim_view, af, P->stream);
-        P->launch_count += 2;
+        P->launch_count += 1;
       }
-      P->launch_count -= 1;   // Scoped already counted one E-pass launch
-      f_done = P->n_obs >= 4000000;
     } else {
       launch_assemble(P->rig, true, P->elim_view, a, P->stream);
     }
@@ -1033,14 +1019,59 @@ static void do_solve(P_t* P, const rcc_lm_options& o, rcc_lm_summary& sum) {
 // ---------------------------------------------------------------------------
 // extern "C" boundary
 // ---------------------------------------------------------------------------
+// caller's pixels (FP64 or integer, caller order) -> e_pix and f_pix
 template <typename T>
-static void set_observations_int(P_t* P, const int32_t* view_idx, const int32_t* marker_idx, const int32_t* cam_idx,
-                                 const T* pixels) {
+static void load_pixels(P_t* P, const T* pixels, bool piecewise) {
+  if (piecewise) {
+    // caller order is the E-sorted order: copy on the side streams in pieces cut at chunk boundaries, FP64 straight
+    // into e_pix; linearize overlaps its E pass with the pieces still in flight
+    constexpr bool f64 = std::is_same<T, double>::value;
+    if (!f64) P->staging.ensure((size_t)P->n_obs * 8 * sizeof(T));
+    T* dst = f64 ? reinterpret_cast<T*>(P->e_pix.p) : reinterpret_cast<T*>(P->staging.p);
+    Scoped t(P, ST_H2D, 0);
+    RCC_CUDA(cudaEventRecord(P->ev_fork, P->stream));          // earlier readers of e_pix on the main stream
+    RCC_CUDA(cudaStreamWaitEvent(P->side_stream, P->ev_fork, 0));
+    RCC_CUDA(cudaStreamWaitEvent(P->side_stream2, P->ev_fork, 0));
+    for (int k = 0; k < rcc_ba_problem::PIX_PIECES; ++k) {
+      // pieces alternate between two streams: two copy engines in flight keep the link busier (48 -> 52 GB/s)
+      cudaStream_t cs = (k & 1) ? P->side_stream2 : P->side_stream;
+      const int64_t b0 = P->piece_block[k], b1 = P->piece_block[k + 1];
+      if (b1 > b0) {
+        RCC_CUDA(cudaMemcpyAsync(dst + b0 * 8, pixels + b0 * 8, (size_t)(b1 - b0) * 8 * sizeof(T),
+                                 cudaMemcpyHostToDevice, cs));
+        launch_load_pixels<T>(f64 ? nullptr : dst + b0 * 8, nullptr, P->e_pix.p + b0 * 8, P->f_inv.p + b0, P->f_pix.p,
+                              b1 - b0, cs);
+        P->launch_count += 1;
+      }
+      RCC_CUDA(cudaEventRecord(P->ev_piece[k], cs));
+    }
+    P->pix_pending = true;
+  } else {
+    const size_t bytes = (size_t)P->n_obs * 8 * sizeof(T);
+    Scoped t(P, ST_H2D, P->n_obs > 0 ? 1 : 0);
+    P->staging.ensure(bytes);
+    if (bytes) RCC_CUDA(cudaMemcpyAsync(P->staging.p, pixels, bytes, cudaMemcpyHostToDevice, P->stream));
+    launch_load_pixels<T>(reinterpret_cast<const T*>(P->staging.p), P->e_orig.p, P->e_pix.p, P->f_inv.p, P->f_pix.p,
+                          P->n_obs, P->stream);
+  }
+}
+
+template <typename T>
+static void set_observations(P_t* P, const int32_t* view_idx, const int32_t* marker_idx, const int32_t* cam_idx,
+                             const T* pixels) {
   RCC_REQUIRE(view_idx && marker_idx && pixels, RCC_BAD_ARG, "null pointer");
-  std::vector<double> px((size_t)P->n_obs * 8);     // one-time setup: widen on the host
-#pragma omp parallel for
-  for (int64_t i = 0; i < P->n_obs * 8; ++i) px[i] = (double)pixels[i];
-  build_indices(P, view_idx, marker_idx, cam_idx, px.data());
+  build_indices(P, view_idx, marker_idx, cam_idx);
+  load_pixels(P, pixels, false);
+  RCC_CUDA(cudaStreamSynchronize(P->stream));
+  P->staging.release();   // only needed again by a later update_pixels that goes through it
+}
+
+template <typename T>
+static void update_pixels(P_t* P, const T* pixels) {
+  RCC_REQUIRE(pixels, RCC_BAD_ARG, "null pointer");
+  RCC_REQUIRE(P->have_obs, RCC_NOT_READY, "set_observations has not been called");
+  load_pixels(P, pixels, P->pix_identity);
+  P->linearized = P->schur_done = P->step_ready = P->cand_ready = false;
 }
 
 static thread_local std::string g_create_error;
@@ -1264,89 +1295,33 @@ int rcc_ba_set_marker_sizes(rcc_ba_problem* P, const double* sizes) {
 int rcc_ba_set_observations(rcc_ba_problem* P, const int32_t* view_idx, const int32_t* marker_idx,
                             const int32_t* cam_idx, const double* pixels) {
   API_BEGIN(P)
-  RCC_REQUIRE(view_idx && marker_idx && pixels, RCC_BAD_ARG, "null pointer");
-  build_indices(P, view_idx, marker_idx, cam_idx, pixels);
+  set_observations(P, view_idx, marker_idx, cam_idx, pixels);
   API_END(P)
 }
 
 int rcc_ba_update_pixels(rcc_ba_problem* P, const double* pixels) {
   API_BEGIN(P)
-  RCC_REQUIRE(pixels, RCC_BAD_ARG, "null pointer");
-  RCC_REQUIRE(P->have_obs, RCC_NOT_READY, "set_observations has not been called");
-  if (P->pix_identity) {
-    // caller order is the E-sorted order: copy straight into e_pix on the side stream, in pieces cut at
-    // chunk boundaries; linearize overlaps its E pass with the pieces still in flight
-    Scoped t(P, ST_H2D, 0);
-    RCC_CUDA(cudaEventRecord(P->ev_fork, P->stream));          // earlier readers of e_pix on the main stream
-    RCC_CUDA(cudaStreamWaitEvent(P->side_stream, P->ev_fork, 0));
-    RCC_CUDA(cudaStreamWaitEvent(P->side_stream2, P->ev_fork, 0));
-    for (int k = 0; k < rcc_ba_problem::PIX_PIECES; ++k) {
-      // pieces alternate between two streams: two copy engines in flight keep the link busier (48 -> 52 GB/s)
-      cudaStream_t cs = (k & 1) ? P->side_stream2 : P->side_stream;
-      const int64_t b0 = P->piece_block[k], b1 = P->piece_block[k + 1];
-      if (b1 > b0) {
-        RCC_CUDA(cudaMemcpyAsync(P->e_pix.p + b0 * 8, pixels + b0 * 8, (size_t)(b1 - b0) * 8 * sizeof(double),
-                                 cudaMemcpyHostToDevice, cs));
-        launch_scatter_pixels(nullptr, P->e_pix.p + b0 * 8, P->f_inv.p + b0, P->f_pix.p, b1 - b0, cs);
-        P->launch_count += 1;
-      }
-      RCC_CUDA(cudaEventRecord(P->ev_piece[k], cs));
-    }
-    P->pix_pending = true;
-  } else {
-    Scoped t(P, ST_H2D, 2);
-    P->pix_staging.upload(pixels, (size_t)P->n_obs * 8, P->stream);
-    launch_permute_pixels(P->pix_staging.p, P->e_orig.p, P->e_pix.p, P->n_obs, P->stream);
-    launch_permute_pixels(P->pix_staging.p, P->f_orig.p, P->f_pix.p, P->n_obs, P->stream);
-  }
-  P->linearized = P->schur_done = P->step_ready = P->cand_ready = false;
+  update_pixels(P, pixels);
   API_END(P)
 }
 
 int rcc_ba_set_observations_i16(rcc_ba_problem* P, const int32_t* view_idx, const int32_t* marker_idx,
                                 const int32_t* cam_idx, const int16_t* pixels) {
   API_BEGIN(P)
-  set_observations_int(P, view_idx, marker_idx, cam_idx, pixels);
+  set_observations(P, view_idx, marker_idx, cam_idx, pixels);
   API_END(P)
 }
 
 int rcc_ba_set_observations_i32(rcc_ba_problem* P, const int32_t* view_idx, const int32_t* marker_idx,
                                 const int32_t* cam_idx, const int32_t* pixels) {
   API_BEGIN(P)
-  set_observations_int(P, view_idx, marker_idx, cam_idx, pixels);
+  set_observations(P, view_idx, marker_idx, cam_idx, pixels);
   API_END(P)
 }
 
 int rcc_ba_update_pixels_i16(rcc_ba_problem* P, const int16_t* pixels) {
   API_BEGIN(P)
-  RCC_REQUIRE(pixels, RCC_BAD_ARG, "null pointer");
-  RCC_REQUIRE(P->have_obs, RCC_NOT_READY, "set_observations has not been called");
-  P->pix_i16.ensure((size_t)P->n_obs * 8);
-  if (P->pix_identity) {
-    // same piecewise scheme as rcc_ba_update_pixels with a quarter of the bytes on the link: each piece is
-    // copied and widened to FP64 on its copy stream; the E pass of the piece starts when its event fires
-    Scoped t(P, ST_H2D, rcc_ba_problem::PIX_PIECES);
-    RCC_CUDA(cudaEventRecord(P->ev_fork, P->stream));
-    RCC_CUDA(cudaStreamWaitEvent(P->side_stream, P->ev_fork, 0));
-    RCC_CUDA(cudaStreamWaitEvent(P->side_stream2, P->ev_fork, 0));
-    for (int k = 0; k < rcc_ba_problem::PIX_PIECES; ++k) {
-      cudaStream_t cs = (k & 1) ? P->side_stream2 : P->side_stream;
-      const int64_t b0 = P->piece_block[k], b1 = P->piece_block[k + 1];
-      if (b1 > b0) {
-        RCC_CUDA(cudaMemcpyAsync(P->pix_i16.p + b0 * 8, pixels + b0 * 8, (size_t)(b1 - b0) * 8 * sizeof(int16_t),
-                                 cudaMemcpyHostToDevice, cs));
-        launch_scatter_pixels(P->pix_i16.p + b0 * 8, P->e_pix.p + b0 * 8, P->f_inv.p + b0, P->f_pix.p, b1 - b0, cs);
-      }
-      RCC_CUDA(cudaEventRecord(P->ev_piece[k], cs));
-    }
-    P->pix_pending = true;
-  } else {
-    Scoped t(P, ST_H2D, 2);
-    P->pix_i16.upload(pixels, (size_t)P->n_obs * 8, P->stream);
-    launch_convert_pixels_i16(P->pix_i16.p, P->e_orig.p, P->e_pix.p, P->n_obs, P->stream);
-    launch_convert_pixels_i16(P->pix_i16.p, P->f_orig.p, P->f_pix.p, P->n_obs, P->stream);
-  }
-  P->linearized = P->schur_done = P->step_ready = P->cand_ready = false;
+  update_pixels(P, pixels);
   API_END(P)
 }
 

@@ -67,6 +67,9 @@ struct rcc_ba_problem {
   // copy runs on the side stream in PIX_PIECES pieces cut at chunk boundaries, and the next linearize
   // starts the E pass of a piece as soon as that piece has landed
   static constexpr int PIX_PIECES = 8;
+  // from this many observation blocks on, an upload is cut into PIX_PIECES pieces (below: 4) and linearize runs the
+  // F pass of each piece as it lands; below it, four more launches cost more than they hide
+  static constexpr int64_t LARGE_UPLOAD_BLOCKS = 4000000;
   bool pix_identity = false;         // e_orig is the identity permutation
   bool pix_pending = false;          // pieces in flight on the copy streams (each piece also scatters itself into f_pix)
   int piece_chunk[PIX_PIECES + 1] = {0};
@@ -83,9 +86,9 @@ struct rcc_ba_problem {
   bool const_dirty = true;
 
   // observation blocks, E-sorted and F-sorted
-  rcc::DBuf<int32_t> e_own, e_oth, e_cam, e_orig, f_oth, f_orig, f_inv, e_chunk_ptr, f_chunk_ptr;   // f_inv: E-sorted -> F-sorted position
-  rcc::DBuf<double> e_pix, f_pix, pix_staging;
-  rcc::DBuf<int16_t> pix_i16;        // device staging of rcc_ba_update_pixels_i16
+  rcc::DBuf<int32_t> e_own, e_oth, e_cam, e_orig, f_oth, f_inv, e_chunk_ptr, f_chunk_ptr;   // f_inv: E-sorted -> F-sorted position
+  rcc::DBuf<double> e_pix, f_pix;
+  rcc::DBuf<char> staging;           // caller's pixels on the device, of any element type, before launch_load_pixels
   rcc::DBuf<rcc::Chunk> e_chunks, f_chunks;
   rcc::DBuf<int32_t> cam_chunks_e, cam_ptr_e, cam_chunks_f, cam_ptr_f;
   rcc::DBuf<int32_t> f_piece_list;   // F-pass chunk ids grouped by upload piece

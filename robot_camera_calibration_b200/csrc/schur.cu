@@ -780,61 +780,46 @@ void launch_symmetrize(double* S, int32_t n, int32_t ld, cudaStream_t s) {
   RCC_CUDA(cudaGetLastError());
 }
 
-__global__ void permute_pixels_kernel(const double* __restrict__ src, const int32_t* __restrict__ orig,
-                                      double* __restrict__ dst, int64_t n) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;  // one double2 per thread
-  if (i >= n * 4) return;
-  const int64_t g = i >> 2;
-  const int q = (int)(i & 3);
-  const double2 v = reinterpret_cast<const double2*>(src + (size_t)orig[g] * 8)[q];
-  reinterpret_cast<double2*>(dst + g * 8)[q] = v;
+// one corner (x, y) of a caller's pixel block, widened to FP64: one 16-, 8- or 4-byte load
+__device__ __forceinline__ double2 load_corner(const double* p) { return *reinterpret_cast<const double2*>(p); }
+__device__ __forceinline__ double2 load_corner(const int32_t* p) {
+  const int2 v = *reinterpret_cast<const int2*>(p);
+  return make_double2((double)v.x, (double)v.y);
 }
-void launch_permute_pixels(const double* src, const int32_t* orig, double* dst, int64_t n, cudaStream_t s) {
-  if (n == 0) return;
-  permute_pixels_kernel<<<ceil_div(n * 4, 256), 256, 0, s>>>(src, orig, dst, n);
-  RCC_CUDA(cudaGetLastError());
-}
-
-// one thread per corner (2 x int16 = one 32-bit load, one 16-byte store): both sides coalesced
-__global__ void convert_pixels_i16_kernel(const int16_t* __restrict__ src, const int32_t* __restrict__ orig,
-                                          double* __restrict__ dst, int64_t n) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n * 4) return;
-  const int64_t g = i >> 2;
-  const int q = (int)(i & 3);
-  const int64_t sg = orig ? (int64_t)orig[g] : g;
-  const short2 v = reinterpret_cast<const short2*>(src + sg * 8)[q];
-  reinterpret_cast<double2*>(dst + g * 8)[q] = make_double2((double)v.x, (double)v.y);
-}
-void launch_convert_pixels_i16(const int16_t* src, const int32_t* orig, double* dst, int64_t n, cudaStream_t s) {
-  if (n == 0) return;
-  convert_pixels_i16_kernel<<<ceil_div(n * 4, 256), 256, 0, s>>>(src, orig, dst, n);
-  RCC_CUDA(cudaGetLastError());
+__device__ __forceinline__ double2 load_corner(const int16_t* p) {
+  const short2 v = *reinterpret_cast<const short2*>(p);
+  return make_double2((double)v.x, (double)v.y);
 }
 
 // one thread per corner: 16-byte records on both sides; the F-sorted side is a scatter of whole 64-byte blocks
-__global__ void scatter_pixels_kernel(const int16_t* __restrict__ src16, double* __restrict__ e_pix,
-                                      const int32_t* __restrict__ f_inv, double* __restrict__ f_pix, int64_t n) {
+template <typename T>
+__global__ void load_pixels_kernel(const T* __restrict__ src, const int32_t* __restrict__ orig,
+                                   double* __restrict__ e_pix, const int32_t* __restrict__ f_inv,
+                                   double* __restrict__ f_pix, int64_t n) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n * 4) return;
   const int64_t g = i >> 2;
   const int q = (int)(i & 3);
   double2 v;
-  if (src16) {
-    const short2 s = reinterpret_cast<const short2*>(src16 + g * 8)[q];
-    v = make_double2((double)s.x, (double)s.y);
+  if (src) {
+    const int64_t sg = orig ? (int64_t)orig[g] : g;
+    v = load_corner(src + sg * 8 + q * 2);
     reinterpret_cast<double2*>(e_pix + g * 8)[q] = v;
   } else {
     v = reinterpret_cast<const double2*>(e_pix + g * 8)[q];
   }
   reinterpret_cast<double2*>(f_pix + (int64_t)f_inv[g] * 8)[q] = v;
 }
-void launch_scatter_pixels(const int16_t* src16, double* e_pix, const int32_t* f_inv, double* f_pix, int64_t n,
-                           cudaStream_t s) {
+template <typename T>
+void launch_load_pixels(const T* src, const int32_t* orig, double* e_pix, const int32_t* f_inv, double* f_pix,
+                        int64_t n, cudaStream_t s) {
   if (n == 0) return;
-  scatter_pixels_kernel<<<ceil_div(n * 4, 256), 256, 0, s>>>(src16, e_pix, f_inv, f_pix, n);
+  load_pixels_kernel<T><<<ceil_div(n * 4, 256), 256, 0, s>>>(src, orig, e_pix, f_inv, f_pix, n);
   RCC_CUDA(cudaGetLastError());
 }
+template void launch_load_pixels(const double*, const int32_t*, double*, const int32_t*, double*, int64_t, cudaStream_t);
+template void launch_load_pixels(const int32_t*, const int32_t*, double*, const int32_t*, double*, int64_t, cudaStream_t);
+template void launch_load_pixels(const int16_t*, const int32_t*, double*, const int32_t*, double*, int64_t, cudaStream_t);
 
 __global__ void fill_kernel(double* p, int64_t n, double v) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) p[i] = v;

@@ -225,6 +225,31 @@ def test_update_pixels_matches_a_fresh_problem(shuffled):
                 assert np.array_equal(gq.evaluate(want_jacobians=False)["residuals"], e2["residuals"])
 
 
+def test_update_pixels_in_pieces_at_size_matches_a_fresh_problem():
+    """From LARGE_UPLOAD_BLOCKS (problem.h) on, a piecewise update_pixels is cut into 8 pieces and linearize runs the
+    F pass of each piece as soon as it has landed.  FP64 and int16 updates on such a scene must give exactly what a
+    problem built from those pixels gives: the F chunks are cut at the same piece boundaries in both."""
+    s = make_scene(5000, 4000, 0.25, blocked=True, chunk_views=250, round_pixels=True, seed=65)
+    assert s.n_blocks >= 4_000_000
+    key = s.view_idx.astype(np.int64) * len(s.markers) + s.marker_idx
+    assert np.all(np.diff(key) >= 0)                 # caller order == E-sorted order: the piecewise path
+    rng = np.random.default_rng(10)
+    new_pixels = [s.pixels + rng.integers(-2, 3, s.pixels.shape) for _ in range(2)]
+    with BAProblem.from_scene(s, eliminate="views") as gp:
+        gp.linearize()
+        for pix, dt in zip(new_pixels, (np.float64, np.int16)):
+            gp.update_pixels(pix.astype(dt))
+            cost = gp.linearize()
+            nb = gp.normal_blocks()
+            s.pixels = pix
+            with BAProblem.from_scene(s, eliminate="views") as gq:
+                assert gq.linearize() == cost
+                nq = gq.normal_blocks()
+            for k in ("Hee", "Hff", "W", "ge", "gf", "Hes", "Hfs", "Hss", "gs"):
+                assert np.array_equal(nq[k], nb[k]), k
+            del nb, nq
+
+
 @pytest.mark.parametrize("model", ["single", "rig"])
 def test_bitwise_repeatability_stress(model):
     """compute-sanitizer's racecheck is closed on the pool, so the hand-rolled last-CTA protocol of the
