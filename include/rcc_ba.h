@@ -177,6 +177,23 @@ int rcc_ba_accept_step(rcc_ba_problem* p);
 /* whole Levenberg-Marquardt loop */
 int rcc_ba_solve(rcc_ba_problem* p, const rcc_lm_options* opt, rcc_lm_summary* summary);
 
+/* Parameter covariance at the current parameters (ceres::Covariance semantics):
+ *   C = (J^T J)^-1 of the UNDAMPED Gauss-Newton system, J the same loss-weighted Jacobian the LM step uses (Huber /
+ *   Cauchy applied: Ceres's apply_loss_function = true).  C is not scaled by a residual variance: a caller whose
+ *   pixel noise has standard deviation sigma multiplies by sigma^2.  Rows and columns of constant blocks (the gauge,
+ *   rcc_ba_set_constant) are exactly zero; every other entry is the entry of the inverse of J^T J restricted to the
+ *   free parameters.  Marginal blocks only, row-major, in the caller's block index order whichever set is
+ *   eliminated; any pointer may be NULL:
+ *     cov_shared  n_shared x n_shared   per camera fx fy cx cy k1 k2 p1 p2 k3 [ext 6], cross-camera terms included
+ *     cov_views   n_views x 6 x 6
+ *     cov_markers n_markers x 6 x 6
+ * Returns RCC_NOT_SPD when J^T J restricted to the free parameters is not positive definite (an unobserved block, no
+ * gauge held constant): a non-positive pivot of an eliminated block's H_ee or of the reduced system, or a reduced-
+ * system pivot below 1e-10 of its diagonal entry.  Single rank only: with a communicator of several ranks attached
+ * it returns RCC_BAD_ARG.  Afterwards the handle is linearised at the current point and the reduced system has been
+ * consumed: call rcc_ba_schur again before rcc_ba_solve_step (rcc_ba_solve does). */
+int rcc_ba_covariance(rcc_ba_problem* p, double* cov_shared, double* cov_views, double* cov_markers);
+
 /* ---- read-backs for parity tests (host buffers; any may be NULL) -------- */
 typedef struct {
   int32_t eliminated_is_view; /* 1: E = views, F = markers ; 0: E = markers, F = views */
@@ -213,7 +230,8 @@ int rcc_ba_comm_init(rcc_ba_problem* p, const char id[RCC_COMM_ID_BYTES], int32_
 /* ---- measurement -------------------------------------------------------- */
 /* per-stage device time (CUDA events on the handle's stream) accumulated since
  * the last reset.  names: "expand","assemble_e","assemble_f","finalize","schur_prep",
- * "schur_syrk","schur_shared","allreduce","mask","cholesky","backsub","cost","evaluate" */
+ * "schur_syrk","schur_shared","allreduce","mask","cholesky","backsub","cost","evaluate","h2d",
+ * "inverse","covariance","cov_extract" (the last three: rcc_ba_covariance) */
 int rcc_ba_profile_enable(rcc_ba_problem* p, int32_t on);
 int rcc_ba_profile_reset(rcc_ba_problem* p);
 int rcc_ba_profile_get(rcc_ba_problem* p, const char* stage, double* total_ms, int64_t* launches);

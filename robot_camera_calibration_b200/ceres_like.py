@@ -18,6 +18,7 @@ from __future__ import annotations
 
 import numpy as np
 
+from . import _lib as L
 from .problem import BAProblem
 
 
@@ -240,3 +241,70 @@ def Solve(options, problem):
         if rig:
             ea[:] = ext[i]
     return Summary(s)
+
+
+class CovarianceOptions:
+    """ceres::Covariance::Options.  apply_loss_function=False evaluates J without the robust loss."""
+
+    def __init__(self, apply_loss_function=True):
+        self.apply_loss_function = bool(apply_loss_function)
+
+
+class Covariance:
+    """ceres::Covariance: blocks of (J^T J)^-1 at the problem's current parameters (rcc_ba_covariance; not scaled by
+    a residual variance).  Supported pairs: (x, x) for any parameter block, and any pair of intrinsics, distortion
+    or extrinsics arrays, of one camera or of two.  A constant block gives zeros."""
+
+    def __init__(self, options=None):
+        self.options = options if options is not None else CovarianceOptions()
+        self._blocks = {}
+
+    def Compute(self, covariance_blocks, problem):
+        """bool Compute(covariance_blocks, problem): False when J^T J is not positive definite (rank deficient)."""
+        pairs = [(a, b) for a, b in covariance_blocks]
+        gp, (vlist, mlist, clist, rig) = problem._build()
+        where = {}          # id(array) -> ("views" | "markers", index) or ("shared", first column)
+        for i, a in enumerate(vlist):
+            where[id(a)] = ("views", i)
+        for i, a in enumerate(mlist):
+            where[id(a)] = ("markers", i)
+        sp = 15 if rig else 9
+        for c, (_, intr, dist, ext) in enumerate(clist):
+            where[id(intr)] = ("shared", sp * c)
+            where[id(dist)] = ("shared", sp * c + 4)
+            if rig:
+                where[id(ext)] = ("shared", sp * c + 9)
+        for a, b in pairs:
+            for x in (a, b):
+                if id(x) not in where:
+                    raise ValueError("parameter block not found in the problem")      # Ceres aborts here
+            if a is not b and (where[id(a)][0] != "shared" or where[id(b)][0] != "shared"):
+                raise NotImplementedError("covariance between two different pose blocks, or a pose and a camera "
+                                          "block, is not computed on this path")
+        with gp:
+            if not self.options.apply_loss_function:
+                gp.set_loss("trivial")
+            try:
+                cov = gp.covariance()
+            except L.RccError as e:
+                if e.status == L.RCC_NOT_SPD:
+                    return False
+                raise
+        self._blocks = {}
+        for a, b in pairs:
+            (ka, ia), (kb, ib) = where[id(a)], where[id(b)]
+            if ka == "shared":
+                blk = cov["shared"][ia:ia + a.size, ib:ib + b.size]
+            else:
+                blk = cov[ka][ia]
+            self._blocks[(id(a), id(b))] = blk.copy()
+            self._blocks[(id(b), id(a))] = blk.T.copy()
+        return True
+
+    def GetCovarianceBlock(self, a, b, out):
+        """bool GetCovarianceBlock(a, b, out): out (row-major size(a) x size(b)); False for a pair Compute did not get."""
+        blk = self._blocks.get((id(a), id(b)))
+        if blk is None:
+            return False
+        np.asarray(out).reshape(-1)[:] = blk.reshape(-1)
+        return True

@@ -190,6 +190,8 @@ struct SchurPrepArgs {
   double* Y;                     // [n_pairs*36] column-major 6x6 blocks  L^-1 W
   double* Yb;                    // [n_e*n_bb*36] column-major blocks L^-1 [Hes | ge | 0]
   double* d2e;                   // [n_e*6] damping actually applied
+  int32_t* pivot_fail;           // nullable: set to 1 when a free block's pivot of chol(Hee + D) is not positive
+                                 // (the factorisation clamps it to 1e-300 and carries on)
 };
 void launch_schur_prep(const SchurPrepArgs& a, cudaStream_t s);
 
@@ -274,6 +276,28 @@ struct BacksubArgs {
   double* partials;       // [n_e*4]: mcc, |d|^2, |x|^2, 0 per E block
 };
 void launch_backsub(const BacksubArgs& a, cudaStream_t s);
+
+// Parameter covariance from the inverse of the undamped reduced system.  Sinv: S^-1 in the row-major upper triangle
+// of the reduced buffer (rows and columns of constants zero).  Partner k of row e is pair row_ptr[e] + k (its kept
+// block f, record Y) for k < m_e, and border block k - m_e (shared columns 6 (k - m_e) ..., record Yb, the g_e and
+// pad columns left out) after it.
+struct CovArgs {
+  int32_t n_e, n_f, n_shared, n_bb;
+  int32_t n, ld;                 // reduced size 6 n_f + n_shared, row stride of the buffer
+  const int32_t* row_ptr;
+  const int32_t* pair_f;
+  const double* Y;               // undamped schur_prep outputs
+  const double* Yb;
+  const double* Linv;
+  const double* Sinv;
+  double* cov_e;                 // [n_e*36] row-major
+  double* cov_f;                 // [n_f*36] row-major
+  double* cov_s;                 // [n_shared*n_shared] row-major
+};
+// Cov(e) = L_e^-T (I + Y_e S^-1 Y_e^T) L_e^-1 for every eliminated block (Y_e = the 6 x n row of partners)
+void launch_cov_eliminated(const CovArgs& a, cudaStream_t s);
+// the kept 6 x 6 diagonal blocks and the shared block of S^-1, both triangles filled
+void launch_cov_kept(const CovArgs& a, cudaStream_t s);
 
 // F-side model-cost-change / norms: out[0..2] = mcc_F, |dF|^2, |xF|^2
 void launch_f_stats(const double* gF, const double* d2f, const double* delta_F, const double* x_f, const double* x_s,

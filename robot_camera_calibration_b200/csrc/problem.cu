@@ -27,7 +27,8 @@ namespace rcc {
 
 static const char* kStageNames[ST_COUNT] = {"expand", "assemble_e", "assemble_f", "finalize", "schur_prep",
                                             "schur_syrk", "schur_shared", "allreduce", "mask", "cholesky",
-                                            "backsub", "cost", "evaluate", "h2d"};
+                                            "backsub", "cost", "evaluate", "h2d", "inverse", "covariance",
+                                            "cov_extract"};
 const char* stage_name(int s) { return (s >= 0 && s < ST_COUNT) ? kStageNames[s] : "?"; }
 
 cudaEvent_t StageTimer::get() {
@@ -604,7 +605,8 @@ static void do_linearize(P_t* P) {
   P->schur_done = P->step_ready = P->cand_ready = false;
 }
 
-static void do_schur(P_t* P, double radius) {
+// pivot_fail (device, nullable): set when a free eliminated block's pivot of chol(H_ee + D_e) is not positive
+static void do_schur(P_t* P, double radius, int32_t* pivot_fail = nullptr) {
   RCC_REQUIRE(P->linearized, RCC_NOT_READY, "linearize has not been called");
   bool eager = false;
   RCC_REQUIRE(radius > 0, RCC_BAD_ARG, "radius must be positive");
@@ -618,6 +620,7 @@ static void do_schur(P_t* P, double radius) {
     a.row_ptr = P->row_ptr.p; a.pair_mptr = P->pair_mptr.p; a.pair_members = P->pair_members.p; a.row_pos0 = P->row_pos0.p; a.W = P->W.p;
     a.radius = radius; a.min_diag = P->min_diag; a.max_diag = P->max_diag; a.jacobi = P->jacobi;
     a.Linv = P->Linv.p; a.Y = P->Y.p; a.Yb = P->Yb.p; a.d2e = P->d2e.p;
+    a.pivot_fail = pivot_fail;
     launch_schur_prep(a, P->stream);
   }
   {
@@ -760,6 +763,27 @@ static int cholesky_mode(P_t* P) {
   return mode;
 }
 
+// Cholesky of the reduced system in place, by the method cholesky_mode() picks; dev_info[0] receives 0 or the first
+// column with a non-positive pivot.  with_rhs: the (n+1) x (n+1) bordered matrix [[S, b], [b^T, big]], whose last row
+// comes out as L^-1 b (see do_step); otherwise S alone.
+static void factor_reduced(P_t* P, bool with_rhs) {
+  const int n = P->n_red;
+  const int mode = cholesky_mode(P);
+  if (mode == 0) {
+    if (with_rhs) set_border_pivot_kernel<<<1, 1, 0, P->stream>>>(P->S.p + (size_t)n * P->ld + n);
+    RCC_SOLVER(cusolverDnDpotrf(P->solver, CUBLAS_FILL_MODE_LOWER, with_rhs ? n + 1 : n, P->S.p, P->ld,
+                                P->potrf_work.p, P->potrf_lwork, P->dev_info.p));
+  } else {
+    // dense.cu: the right-hand side is row n of every panel (never a column), so no border pivot is needed.
+    // mode 2: block column J is factored and updated by rank J % n_ranks, finished panels are broadcast in place.
+    const int64_t before = P->chol.launches;
+    chol_factor(P->S.p, n, P->ld, with_rhs ? n + 1 : n, P->rank, mode == 2 ? P->n_ranks : 1,
+                mode == 2 ? P->comm : nullptr, P->stream, P->chol);
+    P->launch_count += P->chol.launches - before;
+    RCC_CUDA(cudaMemcpyAsync(P->dev_info.p, P->chol.info, sizeof(int), cudaMemcpyDeviceToDevice, P->stream));
+  }
+}
+
 // all-reduce + damping/mask + Cholesky + back-substitution + candidate parameters
 static void do_step(P_t* P) {
   RCC_REQUIRE(P->schur_done, RCC_NOT_READY, "schur has not been called");
@@ -779,20 +803,7 @@ static void do_step(P_t* P) {
     // leaves y = L^-1 b in that row -- the forward substitution comes out of potrf for free -- and one
     // triangular solve L^T x = -y remains (cusolverDnDpotrs would run two).
     Scoped t(P, ST_CHOLESKY, 4);
-    const int mode = cholesky_mode(P);
-    if (mode == 0) {
-      set_border_pivot_kernel<<<1, 1, 0, P->stream>>>(P->S.p + (size_t)n * P->ld + n);
-      RCC_SOLVER(cusolverDnDpotrf(P->solver, CUBLAS_FILL_MODE_LOWER, n + 1, P->S.p, P->ld, P->potrf_work.p,
-                                  P->potrf_lwork, P->dev_info.p));
-    } else {
-      // dense.cu: the right-hand side is row n of every panel (never a column), so no border pivot is needed.
-      // mode 2: block column J is factored and updated by rank J % n_ranks, finished panels are broadcast in place.
-      const int64_t before = P->chol.launches;
-      chol_factor(P->S.p, n, P->ld, n + 1, P->rank, mode == 2 ? P->n_ranks : 1, mode == 2 ? P->comm : nullptr,
-                  P->stream, P->chol);
-      P->launch_count += P->chol.launches - before;
-      RCC_CUDA(cudaMemcpyAsync(P->dev_info.p, P->chol.info, sizeof(int), cudaMemcpyDeviceToDevice, P->stream));
-    }
+    factor_reduced(P, true);
     extract_rhs_kernel<<<ceil_div(n, 256), 256, 0, P->stream>>>(P->S.p, n, P->ld, P->rhs.p);
     RCC_CUDA(cudaGetLastError());
     // hand-written back-substitution (dense.cu K5d) where it is the faster one: 0.49 / 0.98 / 2.63 ms against
@@ -834,6 +845,105 @@ static void do_step(P_t* P) {
   P->schur_done = false;  // S now holds the Cholesky factor
   P->step_ready = true;
   P->cand_ready = false;
+}
+
+// ---------------------------------------------------------------------------
+// parameter covariance (rcc_ba_covariance)
+// ---------------------------------------------------------------------------
+// A free parameter whose Cholesky pivot keeps less than this fraction of its diagonal entry is taken as undetermined:
+// J^T J without a gauge held constant factors in FP64 with pivots of about +-1e-11 of their diagonal there instead of
+// an exact zero, while the determined problems of the test scenes keep 1e-4 or more.
+constexpr double COV_MIN_PIVOT = 1e-10;
+
+__global__ void save_diag_kernel(const double* __restrict__ S, int n, int ld, double* __restrict__ d) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) d[i] = S[(size_t)i * ld + i];
+}
+__global__ void pivot_check_kernel(const double* __restrict__ L, int n, int ld, const double* __restrict__ d,
+                                   int32_t* flag) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const double l = L[(size_t)i * ld + i];
+  if (!(l * l >= COV_MIN_PIVOT * d[i])) *flag = 1;
+}
+// the mask left a unit diagonal on every constant parameter, which the inverse keeps: zero it
+__global__ void zero_const_diag_kernel(double* S, int ld, const int32_t* __restrict__ idx, int n_const) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n_const) S[(size_t)idx[i] * ld + idx[i]] = 0.0;
+}
+
+enum { CI_POTRF = 0, CI_POTRI, CI_HEE_PIVOT, CI_S_PIVOT, CI_N };
+
+static void do_covariance(P_t* P, double* cov_shared, double* cov_views, double* cov_markers) {
+  RCC_REQUIRE(!(P->comm && P->n_ranks > 1), RCC_BAD_ARG,
+              "covariance is computed on a single rank only; this handle has a communicator of several ranks");
+  const int n = P->n_red;
+  cudaStream_t s = P->stream;
+  P->cov_info.ensure(CI_N);
+  RCC_CUDA(cudaMemsetAsync(P->cov_info.p, 0, CI_N * sizeof(int32_t), s));
+  do_linearize(P);
+  // an infinite radius makes every LM diagonal exactly zero (lm_diagonal divides by it): the undamped system
+  do_schur(P, INFINITY, P->cov_info.p + CI_HEE_PIVOT);
+  {
+    Scoped t(P, ST_MASK, P->n_const > 0 ? 2 : 1);
+    MaskArgs m{n, P->ld, INFINITY, P->min_diag, P->max_diag, P->jacobi, P->const_idx.p, P->n_const, P->S.p, P->rhs.p,
+               P->d2f.p, P->gFm.p};
+    launch_mask_damp(m, s);
+  }
+  P->schur_done = P->step_ready = P->cand_ready = false;   // S is about to become the factor, then the inverse
+  P->cov_diag.ensure((size_t)n);
+  {
+    Scoped t(P, ST_CHOLESKY, 4);
+    save_diag_kernel<<<ceil_div(n, 256), 256, 0, s>>>(P->S.p, n, P->ld, P->cov_diag.p);
+    factor_reduced(P, false);
+    pivot_check_kernel<<<ceil_div(n, 256), 256, 0, s>>>(P->S.p, n, P->ld, P->cov_diag.p, P->cov_info.p + CI_S_PIVOT);
+    RCC_CUDA(cudaMemcpyAsync(P->cov_info.p + CI_POTRF, P->dev_info.p, sizeof(int), cudaMemcpyDeviceToDevice, s));
+    RCC_CUDA(cudaGetLastError());
+  }
+  int32_t* hi = reinterpret_cast<int32_t*>(P->h_pinned + 32);
+  RCC_CUDA(cudaMemcpyAsync(hi, P->cov_info.p, CI_N * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+  RCC_CUDA(cudaMemcpyAsync(hi + CI_N, P->fail_flag.p, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+  sync(P);
+  if (hi[CI_N]) throw Error(RCC_EVAL_FAILED, "evaluation failed: corner behind the camera or non-finite residual");
+  if (hi[CI_HEE_PIVOT])
+    throw Error(RCC_NOT_SPD, "J^T J is not positive definite: an eliminated block's H_ee has a non-positive pivot");
+  if (hi[CI_POTRF] != 0 || hi[CI_S_PIVOT])
+    throw Error(RCC_NOT_SPD, "J^T J is not positive definite: the reduced system has a non-positive or vanishing pivot"
+                             " (potrf info " + std::to_string(hi[CI_POTRF]) + ")");
+  {
+    Scoped t(P, ST_INVERSE, 1);
+    int lwork = 0;
+    RCC_SOLVER(cusolverDnDpotri_bufferSize(P->solver, CUBLAS_FILL_MODE_LOWER, n, P->S.p, P->ld, &lwork));
+    P->potrf_work.ensure((size_t)std::max(lwork, P->potrf_lwork));
+    RCC_SOLVER(cusolverDnDpotri(P->solver, CUBLAS_FILL_MODE_LOWER, n, P->S.p, P->ld, P->potrf_work.p, lwork,
+                                P->cov_info.p + CI_POTRI));
+  }
+  P->cov_e.ensure((size_t)P->n_e * 36);
+  P->cov_f.ensure((size_t)P->n_f * 36);
+  P->cov_s.ensure((size_t)P->n_shared * P->n_shared);
+  CovArgs c{};
+  c.n_e = P->n_e; c.n_f = P->n_f; c.n_shared = P->n_shared; c.n_bb = P->n_bb; c.n = n; c.ld = P->ld;
+  c.row_ptr = P->row_ptr.p; c.pair_f = P->pair_f.p; c.Y = P->Y.p; c.Yb = P->Yb.p; c.Linv = P->Linv.p; c.Sinv = P->S.p;
+  c.cov_e = P->cov_e.p; c.cov_f = P->cov_f.p; c.cov_s = P->cov_s.p;
+  {
+    Scoped t(P, ST_COVARIANCE, P->n_const > 0 ? 2 : 1);
+    if (P->n_const > 0) zero_const_diag_kernel<<<ceil_div(P->n_const, 256), 256, 0, s>>>(P->S.p, P->ld, P->const_idx.p,
+                                                                                        P->n_const);
+    launch_cov_eliminated(c, s);
+  }
+  {
+    Scoped t(P, ST_COV_EXTRACT, 1);
+    launch_cov_kept(c, s);
+  }
+  double* ce = P->elim_view ? cov_views : cov_markers;
+  double* cf = P->elim_view ? cov_markers : cov_views;
+  if (ce) P->cov_e.download(ce, (size_t)P->n_e * 36, s);
+  if (cf) P->cov_f.download(cf, (size_t)P->n_f * 36, s);
+  if (cov_shared) P->cov_s.download(cov_shared, (size_t)P->n_shared * P->n_shared, s);
+  RCC_CUDA(cudaMemcpyAsync(hi, P->cov_info.p, CI_N * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+  sync(P);
+  if (hi[CI_POTRI] != 0)
+    throw Error(RCC_NOT_SPD, "inverse of the reduced system: potri info " + std::to_string(hi[CI_POTRI]));
 }
 
 static EvalArgs eval_args(P_t* P, bool cand) {
@@ -1530,6 +1640,12 @@ int rcc_ba_solve(rcc_ba_problem* P, const rcc_lm_options* opt, rcc_lm_summary* s
   rcc_lm_summary s;
   do_solve(P, o, s);
   if (summary) *summary = s;
+  API_END(P)
+}
+
+int rcc_ba_covariance(rcc_ba_problem* P, double* cov_shared, double* cov_views, double* cov_markers) {
+  API_BEGIN(P)
+  do_covariance(P, cov_shared, cov_views, cov_markers);
   API_END(P)
 }
 

@@ -17,7 +17,8 @@ namespace rcc {
 
 enum Stage : int {
   ST_EXPAND = 0, ST_ASSEMBLE_E, ST_ASSEMBLE_F, ST_FINALIZE, ST_SCHUR_PREP, ST_SCHUR_SYRK, ST_SCHUR_SHARED,
-  ST_ALLREDUCE, ST_MASK, ST_CHOLESKY, ST_BACKSUB, ST_COST, ST_EVALUATE, ST_H2D, ST_COUNT
+  ST_ALLREDUCE, ST_MASK, ST_CHOLESKY, ST_BACKSUB, ST_COST, ST_EVALUATE, ST_H2D, ST_INVERSE, ST_COVARIANCE,
+  ST_COV_EXTRACT, ST_COUNT
 };
 const char* stage_name(int s);
 
@@ -111,6 +112,10 @@ struct rcc_ba_problem {
   rcc::DBuf<double> potrf_work, packed_S;   // packed_S: the packed column bands of the overlapped reduction (multi-rank)
   rcc::DBuf<int> dev_info;
   int potrf_lwork = 0;
+  // rcc_ba_covariance: the eliminated / kept / shared blocks, diag(S) before the factorisation, and the status words
+  // [potrf info, potri info, H_ee pivot, S pivot]
+  rcc::DBuf<double> cov_e, cov_f, cov_s, cov_diag;
+  rcc::DBuf<int32_t> cov_info;
 
   // reduced solve: 0 = cusolverDnDpotrf replicated on every rank, 1 = dense.cu on this rank, 2 = dense.cu with the
   // block columns distributed over the ranks (RCC_CHOLESKY = cusolver | own | dist | auto)

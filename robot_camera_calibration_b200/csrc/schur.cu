@@ -47,6 +47,7 @@ __global__ void __launch_bounds__(128, 3) schur_prep_kernel(const SchurPrepArgs 
     double s = H[j * 6 + j] + d2[j];
 #pragma unroll
     for (int k = 0; k < j; ++k) s -= L[j][k] * L[j][k];
+    if (a.pivot_fail && !is_const && !(s > 1e-300) && lane == 0) *a.pivot_fail = 1;
     s = fmax(s, 1e-300);
     const double ljj = sqrt(s);
     L[j][j] = ljj;
@@ -666,6 +667,192 @@ __global__ void __launch_bounds__(128) backsub_kernel(const BacksubArgs a) {
 void launch_backsub(const BacksubArgs& a, cudaStream_t s) {
   if (a.n_e == 0) return;
   backsub_kernel<<<ceil_div((int64_t)a.n_e * 32, 128), 128, 0, s>>>(a);
+  RCC_CUDA(cudaGetLastError());
+}
+
+// ---------------------------------------------------------------------------
+// covariance of the eliminated blocks: one warp per eliminated block e, the matrix analogue of backsub_kernel.
+// The inverse of [[H_EE, B], [B^T, C]] has the diagonal blocks H_ee^-1 + H_ee^-1 B_e S^-1 B_e^T H_ee^-1, i.e.
+//     Cov(e) = L^-T (I + G) L^-1,   G = Y_e S^-1 Y_e^T = sum_{k,l} Y_k S^-1[k, l] Y_l^T
+// over the partners k, l of row e.  With U_l = sum_{k<l} Y_k S^-1[k, l] + 1/2 Y_l S^-1[l, l] and T = sum_l U_l Y_l^T,
+// G = T + T^T: only the upper triangle of S^-1 is read, each unordered pair once.  Lane j of the warp owns partner
+// l = 32 lt + j of partner tile lt and keeps U_l in registers; the partner tiles kt <= lt stream their Y records
+// through the warp's shared slice, and every lane multiplies the broadcast Y_k with its own 6 x 6 block of S^-1.
+// Each warp owns its e: no atomics, and every sum runs in a fixed order (bitwise reproducible).
+// ---------------------------------------------------------------------------
+constexpr int COV_WARPS = 4;
+constexpr int COV_TILE = 32;   // partners per tile = lanes
+
+// partner k of row e: its record (column-major 6 x 6, Y_k[a][b] at b * 6 + a) and first reduced index
+struct CovRow {
+  int p0, m;
+  __device__ const double* rec(const CovArgs& a, int e, int k) const {
+    return k < m ? a.Y + (size_t)(p0 + k) * 36 : a.Yb + ((size_t)e * a.n_bb + (k - m)) * 36;
+  }
+  __device__ int gidx(const CovArgs& a, int k) const {
+    return k < m ? 6 * a.pair_f[p0 + k] : 6 * a.n_f + 6 * (k - m);
+  }
+};
+
+__global__ void __launch_bounds__(COV_WARPS * 32) cov_eliminated_kernel(const __grid_constant__ CovArgs a) {
+  __shared__ __align__(16) double rec_all[COV_WARPS][COV_TILE * 36];
+  __shared__ int gi_all[COV_WARPS][COV_TILE];
+  const int e = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  if (e >= a.n_e) return;
+  double* rec = rec_all[warp];
+  int* gi = gi_all[warp];
+  CovRow row{a.row_ptr[e], a.row_ptr[e + 1] - a.row_ptr[e]};
+  const int K = row.m + a.n_bb;
+  const int n_tiles = (K + COV_TILE - 1) / COV_TILE;
+  const int n = a.n, ld = a.ld;
+  double T[36];
+#pragma unroll
+  for (int i = 0; i < 36; ++i) T[i] = 0.0;
+
+  for (int lt = 0; lt < n_tiles; ++lt) {
+    const int l = lt * COV_TILE + lane;
+    const bool l_on = l < K;
+    const int gl = l_on ? row.gidx(a, l) : 0;
+    double U[36];   // U[a * 6 + c]
+#pragma unroll
+    for (int i = 0; i < 36; ++i) U[i] = 0.0;
+    for (int kt = 0; kt <= lt; ++kt) {
+      const int nk = min(COV_TILE, K - kt * COV_TILE);
+      __syncwarp();
+      // stage the tile's records; border records keep only their shared columns (not g_e, not the pad)
+      for (int idx = lane; idx < nk * 18; idx += 32) {
+        const int q = idx / 18, piece = idx - q * 18;
+        const int k = kt * COV_TILE + q;
+        double2 v = reinterpret_cast<const double2*>(row.rec(a, e, k))[piece];
+        if (k >= row.m && 6 * (k - row.m) + piece / 3 >= a.n_shared) v = make_double2(0.0, 0.0);
+        reinterpret_cast<double2*>(rec + q * 36)[piece] = v;
+      }
+      if (lane < nk) gi[lane] = row.gidx(a, kt * COV_TILE + lane);
+      __syncwarp();
+      if (!l_on) continue;
+      const int kend = (kt == lt) ? lane + 1 : nk;   // k <= l
+      for (int kk = 0; kk < kend; ++kk) {
+        const int gk = gi[kk];
+        const bool diag = kt == lt && kk == lane;
+        double Sb[36];   // S^-1[gk + b][gl + c] at b * 6 + c
+        if (!diag && gk + 6 <= n && gl + 6 <= n) {
+          // k < l: the block lies strictly in the upper triangle (kept blocks and border blocks ascend with k)
+#pragma unroll
+          for (int b = 0; b < 6; ++b) {
+            const double2* sp = reinterpret_cast<const double2*>(a.Sinv + (size_t)(gk + b) * ld + gl);
+#pragma unroll
+            for (int i = 0; i < 3; ++i) {
+              const double2 v = sp[i];
+              Sb[b * 6 + 2 * i] = v.x;
+              Sb[b * 6 + 2 * i + 1] = v.y;
+            }
+          }
+        } else {
+          // the diagonal block (half of it, mirrored from the upper triangle) or a block that reaches past the
+          // last shared parameter (those rows / columns are zero)
+#pragma unroll
+          for (int b = 0; b < 6; ++b)
+#pragma unroll
+            for (int c = 0; c < 6; ++c) {
+              int r = gk + b, cc = gl + c;
+              if (diag && b > c) {
+                r = gk + c;
+                cc = gl + b;
+              }
+              const double v = (r < n && cc < n) ? a.Sinv[(size_t)r * ld + cc] : 0.0;
+              Sb[b * 6 + c] = diag ? 0.5 * v : v;
+            }
+        }
+        const double* y = rec + kk * 36;
+#pragma unroll
+        for (int b = 0; b < 6; ++b)
+#pragma unroll
+          for (int r = 0; r < 6; ++r) {
+            const double ykb = y[b * 6 + r];
+#pragma unroll
+            for (int c = 0; c < 6; ++c) U[r * 6 + c] = fma(ykb, Sb[b * 6 + c], U[r * 6 + c]);
+          }
+      }
+    }
+    // T += U_l Y_l^T; the last staged tile is lt itself, so Y_l is this lane's record
+    if (l_on) {
+      const double* yl = rec + lane * 36;
+#pragma unroll
+      for (int r = 0; r < 6; ++r)
+#pragma unroll
+        for (int s = 0; s < 6; ++s) {
+          double t = T[r * 6 + s];
+#pragma unroll
+          for (int c = 0; c < 6; ++c) t = fma(U[r * 6 + c], yl[c * 6 + s], t);
+          T[r * 6 + s] = t;
+        }
+    }
+  }
+#pragma unroll
+  for (int i = 0; i < 36; ++i)
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) T[i] += __shfl_xor_sync(0xffffffffu, T[i], o);
+  if (lane != 0) return;
+  // M = I + T + T^T (exactly symmetric);  Cov = L^-T M L^-1, upper triangle computed, lower mirrored
+  const double* Li = a.Linv + (size_t)e * 36;   // row-major lower triangular
+  double X[36];                                 // X = M L^-1
+#pragma unroll
+  for (int r = 0; r < 6; ++r)
+#pragma unroll
+    for (int j = 0; j < 6; ++j) {
+      double v = 0.0;
+#pragma unroll
+      for (int k = j; k < 6; ++k) v = fma(T[r * 6 + k] + T[k * 6 + r] + (r == k ? 1.0 : 0.0), Li[k * 6 + j], v);
+      X[r * 6 + j] = v;
+    }
+  double* out = a.cov_e + (size_t)e * 36;
+#pragma unroll
+  for (int i = 0; i < 6; ++i)
+#pragma unroll
+    for (int j = i; j < 6; ++j) {
+      double v = 0.0;
+#pragma unroll
+      for (int r = i; r < 6; ++r) v = fma(Li[r * 6 + i], X[r * 6 + j], v);
+      out[i * 6 + j] = v;
+      out[j * 6 + i] = v;
+    }
+}
+
+void launch_cov_eliminated(const CovArgs& a, cudaStream_t s) {
+  if (a.n_e == 0) return;
+  cov_eliminated_kernel<<<ceil_div((int64_t)a.n_e * 32, COV_WARPS * 32), COV_WARPS * 32, 0, s>>>(a);
+  RCC_CUDA(cudaGetLastError());
+}
+
+// one thread per output element: the kept diagonal blocks, then the shared block
+__global__ void cov_kept_kernel(const __grid_constant__ CovArgs a) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t nf = (int64_t)a.n_f * 36;
+  int g0, r, c;
+  double* out;
+  if (i < nf) {
+    const int f = (int)(i / 36), j = (int)(i - (int64_t)f * 36);
+    g0 = 6 * f;
+    r = j / 6;
+    c = j - 6 * r;
+    out = a.cov_f + i;
+  } else if (i < nf + (int64_t)a.n_shared * a.n_shared) {
+    const int j = (int)(i - nf);
+    g0 = 6 * a.n_f;
+    r = j / a.n_shared;
+    c = j - r * a.n_shared;
+    out = a.cov_s + j;
+  } else {
+    return;
+  }
+  const int lo = min(r, c), hi = max(r, c);
+  *out = a.Sinv[(size_t)(g0 + lo) * a.ld + g0 + hi];
+}
+
+void launch_cov_kept(const CovArgs& a, cudaStream_t s) {
+  const int64_t total = (int64_t)a.n_f * 36 + (int64_t)a.n_shared * a.n_shared;
+  cov_kept_kernel<<<ceil_div(total, 256), 256, 0, s>>>(a);
   RCC_CUDA(cudaGetLastError());
 }
 

@@ -267,6 +267,18 @@ class BAProblem:
         self._check(self.lib.rcc_ba_solve(self.h, C.byref(o), C.byref(s)))
         return {f: getattr(s, f) for f, _ in L.LMSummary._fields_}
 
+    def covariance(self):
+        """Parameter covariance at the current parameters, ceres::Covariance semantics: the marginal blocks of
+        (J^T J)^-1 of the undamped Gauss-Newton system, J the loss-weighted Jacobian the LM step uses.  Not scaled by
+        a residual variance: with pixel noise of standard deviation sigma, multiply by sigma**2.  Rows and columns of
+        constant blocks are exactly zero.  Returns {"shared": (n_shared, n_shared), "views": (n_views, 6, 6),
+        "markers": (n_markers, 6, 6)}; raises RccError(RCC_NOT_SPD) when J^T J restricted to the free parameters is
+        not positive definite.  Leaves the handle linearised at the current point (rcc_ba_covariance)."""
+        out = {"shared": np.empty((self.dims.n_shared, self.dims.n_shared)), "views": np.empty((self.n_views, 6, 6)),
+               "markers": np.empty((self.n_markers, 6, 6))}
+        self._check(self.lib.rcc_ba_covariance(self.h, _dp(out["shared"]), _dp(out["views"]), _dp(out["markers"])))
+        return out
+
     # ------------------------------------------------------------------ multi-GPU
     @staticmethod
     def comm_unique_id():
@@ -292,7 +304,7 @@ class BAProblem:
         return ms.value, n.value
 
     STAGES = ("expand", "assemble_e", "assemble_f", "finalize", "schur_prep", "schur_syrk", "schur_shared",
-              "allreduce", "mask", "cholesky", "backsub", "cost", "evaluate", "h2d")
+              "allreduce", "mask", "cholesky", "backsub", "cost", "evaluate", "h2d", "inverse", "covariance", "cov_extract")
 
     def profile(self):
         return {s: self.profile_get(s) for s in self.STAGES}
