@@ -182,8 +182,8 @@ int rcc_ba_solve(rcc_ba_problem* p, const rcc_lm_options* opt, rcc_lm_summary* s
  *   Cauchy applied: Ceres's apply_loss_function = true).  C is not scaled by a residual variance: a caller whose
  *   pixel noise has standard deviation sigma multiplies by sigma^2.  Rows and columns of constant blocks (the gauge,
  *   rcc_ba_set_constant) are exactly zero; every other entry is the entry of the inverse of J^T J restricted to the
- *   free parameters.  Marginal blocks only, row-major, in the caller's block index order whichever set is
- *   eliminated; any pointer may be NULL:
+ *   free parameters.  Marginal blocks (rcc_ba_covariance_blocks gives any pair of blocks), row-major, in the
+ *   caller's block index order whichever set is eliminated; any pointer may be NULL:
  *     cov_shared  n_shared x n_shared   per camera fx fy cx cy k1 k2 p1 p2 k3 [ext 6], cross-camera terms included
  *     cov_views   n_views x 6 x 6
  *     cov_markers n_markers x 6 x 6
@@ -193,6 +193,19 @@ int rcc_ba_solve(rcc_ba_problem* p, const rcc_lm_options* opt, rcc_lm_summary* s
  * it returns RCC_BAD_ARG.  Afterwards the handle is linearised at the current point and the reduced system has been
  * consumed: call rcc_ba_schur again before rcc_ba_solve_step (rcc_ba_solve does). */
 int rcc_ba_covariance(rcc_ba_problem* p, double* cov_shared, double* cov_views, double* cov_markers);
+
+/* Cross-covariance blocks of (J^T J)^-1 for any pairs of parameter blocks (ceres::Covariance::Compute with a list of
+ * block pairs), same semantics, conditions and after-state as rcc_ba_covariance: the undamped, loss-weighted system,
+ * not scaled by a residual variance, exactly zero wherever a constant block is involved.
+ *   pairs  n_pairs x 4 int32: kind_a, index_a, kind_b, index_b  (rcc_block_kind; index = view, marker or camera)
+ *   out    n_pairs x 36: Cov(a, b) row-major size(a) x size(b) (Ceres GetCovarianceBlock layout) at the start of
+ *          its 36-double slot, the rest of the slot zero.  size: view/marker/ext 6, intr 4, dist 5.
+ * Cov(b, a) is exactly the transpose of Cov(a, b), and a pair's block does not depend on the other pairs of the request
+ * or on its position there; two calls give bitwise equal results.  RCC_BAD_ARG (checked before any device work) for an
+ * unknown kind, an index out of range, RCC_BLOCK_EXT on the single-camera model, n_pairs < 0, a NULL pairs or out
+ * with n_pairs > 0, or a communicator of several ranks; n_pairs == 0 returns RCC_OK at once.  RCC_NOT_SPD and
+ * RCC_EVAL_FAILED as for rcc_ba_covariance. */
+int rcc_ba_covariance_blocks(rcc_ba_problem* p, int64_t n_pairs, const int32_t* pairs, double* out);
 
 /* ---- read-backs for parity tests (host buffers; any may be NULL) -------- */
 typedef struct {

@@ -88,6 +88,7 @@ SIGNATURES = {
     "rcc_ba_accept_step": (C.c_int, [_H]),
     "rcc_ba_solve": (C.c_int, [_H, C.POINTER(LMOptions), C.POINTER(LMSummary)]),
     "rcc_ba_covariance": (C.c_int, [_H, c_double_p, c_double_p, c_double_p]),
+    "rcc_ba_covariance_blocks": (C.c_int, [_H, C.c_int64, c_int32_p, c_double_p]),
     "rcc_ba_get_dims": (C.c_int, [_H, C.POINTER(Dims)]),
     "rcc_ba_get_normal_blocks": (C.c_int, [_H] + [c_double_p] * 9),
     "rcc_ba_get_reduced_system": (C.c_int, [_H, c_double_p, c_double_p]),

@@ -299,6 +299,33 @@ void launch_cov_eliminated(const CovArgs& a, cudaStream_t s);
 // the kept 6 x 6 diagonal blocks and the shared block of S^-1, both triangles filled
 void launch_cov_kept(const CovArgs& a, cudaStream_t s);
 
+// Cross-covariance blocks (rcc_ba_covariance_blocks).  A side of a pair is an eliminated block e, whose items are its
+// K_e = m_e + n_bb partners (records as in CovArgs), or a kept or shared block: one item, the identity record on its
+// reduced columns [g, g + w).  Each pair is canonicalised on the host so that side b has at least as many items as
+// side a, and the kernel computes X = sum_{k in a} sum_{l in b} C_ak S^-1[k, l] C_bl^T; then
+//     Cov(a, b) = delta_ab L_a^-T L_a^-1 + P_a X P_b^T,   P = -L_e^-T for an eliminated side, I otherwise.
+struct CovPairDesc {
+  int32_t e_a, e_b;              // eliminated block of side a / b, or -1 for a kept or shared block
+  int32_t g_a, w_a, g_b, w_b;    // kept or shared side: first reduced index and width (4, 5 or 6)
+  int32_t item0, n_items;        // its work items [item0, item0 + n_items) of its launch, in summation order
+  int32_t rows, cols;            // Cov(a, b) is rows x cols (6 for an eliminated side)
+  int32_t transpose;             // 1: the request was (b, a), written as the cols x rows transpose
+  int32_t pad;
+};
+// one work item: items [k0, k0 + COV_PAIR_CHUNK) of side a against the tile [l0, l0 + 32) of side b
+struct CovPairItem { int32_t pair, k0, l0; };
+constexpr int COV_PAIR_CHUNK = 256;
+struct CovPairsArgs {
+  CovArgs m;                     // sizes, partner lists, Y / Yb / Linv and S^-1 (its outputs unused)
+  const CovPairDesc* pairs;      // every requested pair; this launch covers [pair_begin, pair_begin + n_pairs)
+  const CovPairItem* items;      // the items of those pairs (item0 counts from here)
+  int32_t pair_begin, n_pairs, n_items;
+  double* partial;               // [n_items*36]: X of each item, row-major 6 x 6
+  double* out;                   // [all pairs*36]: Cov of each request at the start of its 36-double slot
+};
+// partials of every item, then each pair's sum over its items in item order and the output (no atomics)
+void launch_cov_pairs(const CovPairsArgs& a, cudaStream_t s);
+
 // F-side model-cost-change / norms: out[0..2] = mcc_F, |dF|^2, |xF|^2
 void launch_f_stats(const double* gF, const double* d2f, const double* delta_F, const double* x_f, const double* x_s,
                     int32_t n_f, int32_t n_shared, double* out3, cudaStream_t s);

@@ -16,6 +16,7 @@
 #include <cmath>
 #include <cstdlib>
 #include <numeric>
+#include <tuple>
 #include <type_traits>
 
 using namespace rcc;
@@ -400,6 +401,7 @@ static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker
     P->row_pos0.upload(row_pos0, s);
   }
   P->row_ptr.upload(row_ptr, s);
+  P->row_ptr_h = row_ptr;
   P->pair_e.upload(pair_e, s);
   P->pair_f.upload(pair_f, s);
   P->pair_mptr.upload(pair_mptr, s);
@@ -874,9 +876,15 @@ __global__ void zero_const_diag_kernel(double* S, int ld, const int32_t* __restr
 
 enum { CI_POTRF = 0, CI_POTRI, CI_HEE_PIVOT, CI_S_PIVOT, CI_N };
 
-static void do_covariance(P_t* P, double* cov_shared, double* cov_views, double* cov_markers) {
+static void require_single_rank(P_t* P) {
   RCC_REQUIRE(!(P->comm && P->n_ranks > 1), RCC_BAD_ARG,
               "covariance is computed on a single rank only; this handle has a communicator of several ranks");
+}
+
+// The part every covariance call shares: linearise, the undamped reduced system with the constants masked, its
+// factorisation with the pivot checks, and potri.  Leaves S^-1 in the upper triangle of P->S, with a unit diagonal
+// still on the constant parameters (zero_const_diag clears it).
+static void covariance_inverse(P_t* P) {
   const int n = P->n_red;
   cudaStream_t s = P->stream;
   P->cov_info.ensure(CI_N);
@@ -918,17 +926,43 @@ static void do_covariance(P_t* P, double* cov_shared, double* cov_views, double*
     RCC_SOLVER(cusolverDnDpotri(P->solver, CUBLAS_FILL_MODE_LOWER, n, P->S.p, P->ld, P->potrf_work.p, lwork,
                                 P->cov_info.p + CI_POTRI));
   }
+}
+
+// one launch when there are constants (counted by the caller's Scoped)
+static void zero_const_diag(P_t* P) {
+  if (P->n_const > 0)
+    zero_const_diag_kernel<<<ceil_div(P->n_const, 256), 256, 0, P->stream>>>(P->S.p, P->ld, P->const_idx.p,
+                                                                              P->n_const);
+}
+
+static CovArgs cov_args(P_t* P) {
+  CovArgs c{};
+  c.n_e = P->n_e; c.n_f = P->n_f; c.n_shared = P->n_shared; c.n_bb = P->n_bb; c.n = P->n_red; c.ld = P->ld;
+  c.row_ptr = P->row_ptr.p; c.pair_f = P->pair_f.p; c.Y = P->Y.p; c.Yb = P->Yb.p; c.Linv = P->Linv.p; c.Sinv = P->S.p;
+  c.cov_e = P->cov_e.p; c.cov_f = P->cov_f.p; c.cov_s = P->cov_s.p;
+  return c;
+}
+
+// after the caller's downloads: wait for them and report a failed potri
+static void covariance_finish(P_t* P) {
+  int32_t* hi = reinterpret_cast<int32_t*>(P->h_pinned + 32);
+  RCC_CUDA(cudaMemcpyAsync(hi, P->cov_info.p, CI_N * sizeof(int32_t), cudaMemcpyDeviceToHost, P->stream));
+  sync(P);
+  if (hi[CI_POTRI] != 0)
+    throw Error(RCC_NOT_SPD, "inverse of the reduced system: potri info " + std::to_string(hi[CI_POTRI]));
+}
+
+static void do_covariance(P_t* P, double* cov_shared, double* cov_views, double* cov_markers) {
+  require_single_rank(P);
+  cudaStream_t s = P->stream;
+  covariance_inverse(P);
   P->cov_e.ensure((size_t)P->n_e * 36);
   P->cov_f.ensure((size_t)P->n_f * 36);
   P->cov_s.ensure((size_t)P->n_shared * P->n_shared);
-  CovArgs c{};
-  c.n_e = P->n_e; c.n_f = P->n_f; c.n_shared = P->n_shared; c.n_bb = P->n_bb; c.n = n; c.ld = P->ld;
-  c.row_ptr = P->row_ptr.p; c.pair_f = P->pair_f.p; c.Y = P->Y.p; c.Yb = P->Yb.p; c.Linv = P->Linv.p; c.Sinv = P->S.p;
-  c.cov_e = P->cov_e.p; c.cov_f = P->cov_f.p; c.cov_s = P->cov_s.p;
+  const CovArgs c = cov_args(P);
   {
     Scoped t(P, ST_COVARIANCE, P->n_const > 0 ? 2 : 1);
-    if (P->n_const > 0) zero_const_diag_kernel<<<ceil_div(P->n_const, 256), 256, 0, s>>>(P->S.p, P->ld, P->const_idx.p,
-                                                                                        P->n_const);
+    zero_const_diag(P);
     launch_cov_eliminated(c, s);
   }
   {
@@ -940,10 +974,106 @@ static void do_covariance(P_t* P, double* cov_shared, double* cov_views, double*
   if (ce) P->cov_e.download(ce, (size_t)P->n_e * 36, s);
   if (cf) P->cov_f.download(cf, (size_t)P->n_f * 36, s);
   if (cov_shared) P->cov_s.download(cov_shared, (size_t)P->n_shared * P->n_shared, s);
-  RCC_CUDA(cudaMemcpyAsync(hi, P->cov_info.p, CI_N * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-  sync(P);
-  if (hi[CI_POTRI] != 0)
-    throw Error(RCC_NOT_SPD, "inverse of the reduced system: potri info " + std::to_string(hi[CI_POTRI]));
+  covariance_finish(P);
+}
+
+// A launch of the pair kernels covers whole pairs and at most about this many work items (36 doubles of partials
+// each), so that the scratch stays bounded however many pairs one call requests.
+constexpr int64_t COV_PAIR_BATCH_ITEMS = 1 << 20;
+
+static void do_covariance_blocks(P_t* P, int64_t n_pairs, const int32_t* pairs, double* out) {
+  RCC_REQUIRE(n_pairs >= 0 && n_pairs <= INT32_MAX / 36, RCC_BAD_ARG, "n_pairs out of range");
+  RCC_REQUIRE(n_pairs == 0 || (pairs && out), RCC_BAD_ARG, "null pointer");
+  require_single_rank(P);
+  // a side of a pair: an eliminated block (e >= 0, K partners) or a kept or shared block (reduced columns [g, g + w))
+  struct Side { int e, g, w, K; };
+  auto side = [&](int32_t kind, int32_t index) -> Side {
+    int count = 0;
+    switch (kind) {
+      case RCC_BLOCK_VIEW: count = P->n_views; break;
+      case RCC_BLOCK_MARKER: count = P->n_markers; break;
+      case RCC_BLOCK_INTR: case RCC_BLOCK_DIST: count = P->n_cam; break;
+      case RCC_BLOCK_EXT:
+        RCC_REQUIRE(P->rig, RCC_BAD_ARG, "RCC_BLOCK_EXT needs the rig model");
+        count = P->n_cam;
+        break;
+      default: throw Error(RCC_BAD_ARG, "unknown block kind " + std::to_string(kind));
+    }
+    RCC_REQUIRE(index >= 0 && index < count, RCC_BAD_ARG, "block index out of range");
+    if (kind == RCC_BLOCK_VIEW || kind == RCC_BLOCK_MARKER) {
+      if ((kind == RCC_BLOCK_VIEW) == P->elim_view) return Side{index, 0, 6, 0};
+      return Side{-1, 6 * index, 6, 1};
+    }
+    const int g = 6 * P->n_f + P->sp * index;
+    if (kind == RCC_BLOCK_INTR) return Side{-1, g, 4, 1};
+    if (kind == RCC_BLOCK_DIST) return Side{-1, g + 4, 5, 1};
+    return Side{-1, g + 9, 6, 1};
+  };
+  std::vector<Side> sa((size_t)n_pairs), sb((size_t)n_pairs);
+  for (int64_t p = 0; p < n_pairs; ++p) {
+    sa[p] = side(pairs[4 * p], pairs[4 * p + 1]);
+    sb[p] = side(pairs[4 * p + 2], pairs[4 * p + 3]);
+  }
+  if (n_pairs == 0) return;
+  RCC_REQUIRE(P->have_obs && (int64_t)P->row_ptr_h.size() == (int64_t)P->n_e + 1, RCC_NOT_READY,
+              "observations have not been set");
+  for (int64_t p = 0; p < n_pairs; ++p)
+    for (Side* x : {&sa[p], &sb[p]})
+      if (x->e >= 0) x->K = P->row_ptr_h[x->e + 1] - P->row_ptr_h[x->e] + P->n_bb;
+
+  // canonical order: side b has the more items (ties: the larger block), so that the lanes of an item run over the
+  // long side; the request (b, a) is then written as the transpose of Cov(a, b)
+  std::vector<CovPairDesc> desc((size_t)n_pairs);
+  std::vector<CovPairItem> items;
+  std::vector<int64_t> batch_pair{0}, batch_item{0};
+  auto key = [](const Side& x) { return std::make_tuple(x.K, x.e >= 0, x.e >= 0 ? x.e : x.g); };
+  for (int64_t p = 0; p < n_pairs; ++p) {
+    Side a = sa[p], b = sb[p];
+    const bool swap = key(a) > key(b);
+    if (swap) std::swap(a, b);
+    const int64_t n_items = (int64_t)ceil_div(a.K, COV_PAIR_CHUNK) * ceil_div(b.K, 32);
+    if ((int64_t)items.size() - batch_item.back() + n_items > COV_PAIR_BATCH_ITEMS && p > batch_pair.back()) {
+      batch_pair.push_back(p);
+      batch_item.push_back((int64_t)items.size());
+    }
+    CovPairDesc& d = desc[p];
+    d.e_a = a.e; d.e_b = b.e; d.g_a = a.g; d.w_a = a.w; d.g_b = b.g; d.w_b = b.w;
+    d.item0 = (int32_t)((int64_t)items.size() - batch_item.back());
+    d.n_items = (int32_t)n_items;
+    d.rows = a.w; d.cols = b.w; d.transpose = swap ? 1 : 0;
+    for (int k0 = 0; k0 < a.K; k0 += COV_PAIR_CHUNK)
+      for (int l0 = 0; l0 < b.K; l0 += 32) items.push_back(CovPairItem{(int32_t)p, k0, l0});
+  }
+  batch_pair.push_back(n_pairs);
+  batch_item.push_back((int64_t)items.size());
+  const int n_batches = (int)batch_pair.size() - 1;
+
+  cudaStream_t s = P->stream;
+  covariance_inverse(P);
+  int64_t max_items = 0;
+  for (int b = 0; b < n_batches; ++b) max_items = std::max(max_items, batch_item[b + 1] - batch_item[b]);
+  P->cov_desc.upload(desc.data(), desc.size(), s);
+  P->cov_items.upload(items.data(), items.size(), s);
+  P->cov_partial.ensure((size_t)max_items * 36);
+  P->cov_out.ensure((size_t)n_pairs * 36);
+  CovPairsArgs c{};
+  c.m = cov_args(P);
+  c.pairs = P->cov_desc.p;
+  c.partial = P->cov_partial.p;
+  c.out = P->cov_out.p;
+  {
+    Scoped t(P, ST_COVARIANCE, (P->n_const > 0 ? 1 : 0) + 2 * n_batches);
+    zero_const_diag(P);
+    for (int b = 0; b < n_batches; ++b) {
+      c.items = P->cov_items.p + batch_item[b];
+      c.pair_begin = (int32_t)batch_pair[b];
+      c.n_pairs = (int32_t)(batch_pair[b + 1] - batch_pair[b]);
+      c.n_items = (int32_t)(batch_item[b + 1] - batch_item[b]);
+      launch_cov_pairs(c, s);
+    }
+  }
+  P->cov_out.download(out, (size_t)n_pairs * 36, s);
+  covariance_finish(P);
 }
 
 static EvalArgs eval_args(P_t* P, bool cand) {
@@ -1646,6 +1776,12 @@ int rcc_ba_solve(rcc_ba_problem* P, const rcc_lm_options* opt, rcc_lm_summary* s
 int rcc_ba_covariance(rcc_ba_problem* P, double* cov_shared, double* cov_views, double* cov_markers) {
   API_BEGIN(P)
   do_covariance(P, cov_shared, cov_views, cov_markers);
+  API_END(P)
+}
+
+int rcc_ba_covariance_blocks(rcc_ba_problem* P, int64_t n_pairs, const int32_t* pairs, double* out) {
+  API_BEGIN(P)
+  do_covariance_blocks(P, n_pairs, pairs, out);
   API_END(P)
 }
 

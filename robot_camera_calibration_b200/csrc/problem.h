@@ -94,6 +94,7 @@ struct rcc_ba_problem {
   rcc::DBuf<int32_t> cam_chunks_e, cam_ptr_e, cam_chunks_f, cam_ptr_f;
   rcc::DBuf<int32_t> f_piece_list;   // F-pass chunk ids grouped by upload piece
   int f_piece_ptr[PIX_PIECES + 1] = {0};
+  std::vector<int32_t> row_ptr_h;    // row_ptr on the host (rcc_ba_covariance_blocks plans its work from it)
   rcc::DBuf<int32_t> row_ptr, pair_e, pair_f, pair_mptr, pair_members, row_pos0, col_ptr, col_pair, tile_ptr, syrk_ctas, e_count;
   rcc::DBuf<uint8_t> e_const;
 
@@ -116,6 +117,10 @@ struct rcc_ba_problem {
   // [potrf info, potri info, H_ee pivot, S pivot]
   rcc::DBuf<double> cov_e, cov_f, cov_s, cov_diag;
   rcc::DBuf<int32_t> cov_info;
+  // rcc_ba_covariance_blocks: the canonical pairs, their work items, the items' partials and the outputs
+  rcc::DBuf<rcc::CovPairDesc> cov_desc;
+  rcc::DBuf<rcc::CovPairItem> cov_items;
+  rcc::DBuf<double> cov_partial, cov_out;
 
   // reduced solve: 0 = cusolverDnDpotrf replicated on every rank, 1 = dense.cu on this rank, 2 = dense.cu with the
   // block columns distributed over the ranks (RCC_CHOLESKY = cusolver | own | dist | auto)

@@ -694,6 +694,20 @@ struct CovRow {
   }
 };
 
+// stage the records of partners [k0, k0 + nk) of row e into rec and their first reduced indices into gi; border
+// records keep only their shared columns (not g_e, not the pad)
+__device__ __forceinline__ void cov_stage(const CovArgs& a, const CovRow& row, int e, int k0, int nk, int lane,
+                                          double* rec, int* gi) {
+  for (int idx = lane; idx < nk * 18; idx += 32) {
+    const int q = idx / 18, piece = idx - q * 18;
+    const int k = k0 + q;
+    double2 v = reinterpret_cast<const double2*>(row.rec(a, e, k))[piece];
+    if (k >= row.m && 6 * (k - row.m) + piece / 3 >= a.n_shared) v = make_double2(0.0, 0.0);
+    reinterpret_cast<double2*>(rec + q * 36)[piece] = v;
+  }
+  if (lane < nk) gi[lane] = row.gidx(a, k0 + lane);
+}
+
 __global__ void __launch_bounds__(COV_WARPS * 32) cov_eliminated_kernel(const __grid_constant__ CovArgs a) {
   __shared__ __align__(16) double rec_all[COV_WARPS][COV_TILE * 36];
   __shared__ int gi_all[COV_WARPS][COV_TILE];
@@ -720,15 +734,7 @@ __global__ void __launch_bounds__(COV_WARPS * 32) cov_eliminated_kernel(const __
     for (int kt = 0; kt <= lt; ++kt) {
       const int nk = min(COV_TILE, K - kt * COV_TILE);
       __syncwarp();
-      // stage the tile's records; border records keep only their shared columns (not g_e, not the pad)
-      for (int idx = lane; idx < nk * 18; idx += 32) {
-        const int q = idx / 18, piece = idx - q * 18;
-        const int k = kt * COV_TILE + q;
-        double2 v = reinterpret_cast<const double2*>(row.rec(a, e, k))[piece];
-        if (k >= row.m && 6 * (k - row.m) + piece / 3 >= a.n_shared) v = make_double2(0.0, 0.0);
-        reinterpret_cast<double2*>(rec + q * 36)[piece] = v;
-      }
-      if (lane < nk) gi[lane] = row.gidx(a, kt * COV_TILE + lane);
+      cov_stage(a, row, e, kt * COV_TILE, nk, lane, rec, gi);
       __syncwarp();
       if (!l_on) continue;
       const int kend = (kt == lt) ? lane + 1 : nk;   // k <= l
@@ -853,6 +859,195 @@ __global__ void cov_kept_kernel(const __grid_constant__ CovArgs a) {
 void launch_cov_kept(const CovArgs& a, cudaStream_t s) {
   const int64_t total = (int64_t)a.n_f * 36 + (int64_t)a.n_shared * a.n_shared;
   cov_kept_kernel<<<ceil_div(total, 256), 256, 0, s>>>(a);
+  RCC_CUDA(cudaGetLastError());
+}
+
+// ---------------------------------------------------------------------------
+// cross-covariance blocks (kernels.h CovPairDesc): one warp per work item (pair, chunk of side a, tile of side b).
+// Lane j owns item l = l0 + j of side b and accumulates U_l = sum_k C_ak S^-1[k, l] over the chunk, whose records
+// stream through the warp's shared slice as in cov_eliminated_kernel; then X = sum_l U_l C_bl^T over the tile is
+// summed across the lanes and stored as the item's partial.  cov_pairs_combine_kernel adds a pair's partials in item
+// order and applies P_a, P_b and the diagonal term.  Every sum has a fixed order that depends on the pair alone.
+// ---------------------------------------------------------------------------
+
+// Sb[b * 6 + c] = S^-1[gk + b][gl + c] for b < wk, c < wl (zero elsewhere and past n), read from the upper triangle
+__device__ __forceinline__ void cov_load_block(const double* __restrict__ S, int n, int ld, int gk, int wk, int gl,
+                                               int wl, double* Sb) {
+  const bool whole = wk == 6 && wl == 6 && gk + 6 <= n && gl + 6 <= n && ((gk | gl) & 1) == 0;
+  if (whole && gk + 5 <= gl) {
+#pragma unroll
+    for (int b = 0; b < 6; ++b) {
+      const double2* sp = reinterpret_cast<const double2*>(S + (size_t)(gk + b) * ld + gl);
+#pragma unroll
+      for (int i = 0; i < 3; ++i) {
+        const double2 v = sp[i];
+        Sb[b * 6 + 2 * i] = v.x;
+        Sb[b * 6 + 2 * i + 1] = v.y;
+      }
+    }
+  } else if (whole && gl + 5 <= gk) {
+#pragma unroll
+    for (int c = 0; c < 6; ++c) {
+      const double2* sp = reinterpret_cast<const double2*>(S + (size_t)(gl + c) * ld + gk);
+#pragma unroll
+      for (int i = 0; i < 3; ++i) {
+        const double2 v = sp[i];
+        Sb[2 * i * 6 + c] = v.x;
+        Sb[(2 * i + 1) * 6 + c] = v.y;
+      }
+    }
+  } else {
+    // a window that straddles the diagonal, is narrower than 6, or reaches past the last shared parameter
+#pragma unroll
+    for (int b = 0; b < 6; ++b)
+#pragma unroll
+      for (int c = 0; c < 6; ++c) {
+        const int r = gk + b, cc = gl + c, lo = min(r, cc), hi = max(r, cc);
+        Sb[b * 6 + c] = (b < wk && c < wl && hi < n) ? S[(size_t)lo * ld + hi] : 0.0;
+      }
+  }
+}
+
+__global__ void __launch_bounds__(COV_WARPS * 32) cov_pairs_kernel(const __grid_constant__ CovPairsArgs a) {
+  __shared__ __align__(16) double rec_all[COV_WARPS][COV_TILE * 36];
+  __shared__ int gi_all[COV_WARPS][COV_TILE];
+  const int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  if (w >= a.n_items) return;
+  double* rec = rec_all[warp];
+  int* gi = gi_all[warp];
+  const CovArgs& m = a.m;
+  const CovPairItem it = a.items[w];
+  const CovPairDesc pd = a.pairs[it.pair];
+  CovRow ra{0, 0}, rb{0, 0};
+  int Ka = 1, Kb = 1;
+  if (pd.e_a >= 0) {
+    ra = CovRow{m.row_ptr[pd.e_a], m.row_ptr[pd.e_a + 1] - m.row_ptr[pd.e_a]};
+    Ka = ra.m + m.n_bb;
+  }
+  if (pd.e_b >= 0) {
+    rb = CovRow{m.row_ptr[pd.e_b], m.row_ptr[pd.e_b + 1] - m.row_ptr[pd.e_b]};
+    Kb = rb.m + m.n_bb;
+  }
+  const int na = min(COV_PAIR_CHUNK, Ka - it.k0);
+  const int l = it.l0 + lane;
+  const bool l_on = l < Kb;
+  const int gl = pd.e_b >= 0 ? (l_on ? rb.gidx(m, l) : 0) : pd.g_b;
+  const int wl = pd.e_b >= 0 ? 6 : pd.w_b, wk = pd.e_a >= 0 ? 6 : pd.w_a;
+  double U[36];   // U[r * 6 + c]: row r of side a, column c of item l
+#pragma unroll
+  for (int i = 0; i < 36; ++i) U[i] = 0.0;
+  for (int kt = 0; kt < na; kt += COV_TILE) {
+    const int nk = min(COV_TILE, na - kt);
+    __syncwarp();
+    if (pd.e_a >= 0) {
+      cov_stage(m, ra, pd.e_a, it.k0 + kt, nk, lane, rec, gi);
+    } else {
+      for (int i = lane; i < 36; i += 32) rec[i] = (i % 7 == 0) ? 1.0 : 0.0;   // the identity record
+      if (lane == 0) gi[0] = pd.g_a;
+    }
+    __syncwarp();
+    if (!l_on) continue;
+    for (int kk = 0; kk < nk; ++kk) {
+      double Sb[36];
+      cov_load_block(m.Sinv, m.n, m.ld, gi[kk], wk, gl, wl, Sb);
+      const double* y = rec + kk * 36;
+#pragma unroll
+      for (int b = 0; b < 6; ++b)
+#pragma unroll
+        for (int r = 0; r < 6; ++r) {
+          const double ykb = y[b * 6 + r];
+#pragma unroll
+          for (int c = 0; c < 6; ++c) U[r * 6 + c] = fma(ykb, Sb[b * 6 + c], U[r * 6 + c]);
+        }
+    }
+  }
+  // X = U_l C_bl^T (C_bl = I on a kept or shared side); the border records lose their g_e and pad columns
+  if (l_on && pd.e_b >= 0) {
+    const double* yl = rb.rec(m, pd.e_b, l);
+    const int ncol = l < rb.m ? 6 : min(6, m.n_shared - 6 * (l - rb.m));
+    double X[36];
+#pragma unroll
+    for (int r = 0; r < 6; ++r)
+#pragma unroll
+      for (int s = 0; s < 6; ++s) {
+        double t = 0.0;
+#pragma unroll
+        for (int c = 0; c < 6; ++c) t = fma(U[r * 6 + c], c < ncol ? yl[c * 6 + s] : 0.0, t);
+        X[r * 6 + s] = t;
+      }
+#pragma unroll
+    for (int i = 0; i < 36; ++i) U[i] = X[i];
+  } else if (!l_on) {
+#pragma unroll
+    for (int i = 0; i < 36; ++i) U[i] = 0.0;
+  }
+#pragma unroll
+  for (int i = 0; i < 36; ++i)
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) U[i] += __shfl_xor_sync(0xffffffffu, U[i], o);
+  if (lane == 0) {
+    double* out = a.partial + (size_t)w * 36;
+#pragma unroll
+    for (int i = 0; i < 36; ++i) out[i] = U[i];
+  }
+}
+
+// one 64-thread block per pair: X = the pair's partials summed in item order, M = X (or I + (X + X^T) / 2 for
+// (e, e), exactly symmetric), Cov = +-L_a^-T M L_b^-1 with the L^-1 of the eliminated sides only
+__global__ void __launch_bounds__(64) cov_pairs_combine_kernel(const __grid_constant__ CovPairsArgs a) {
+  __shared__ double M[36], Z[36], O[36];
+  const int t = threadIdx.x;
+  const int p = a.pair_begin + blockIdx.x;
+  const CovPairDesc pd = a.pairs[p];
+  const bool same = pd.e_a >= 0 && pd.e_a == pd.e_b;
+  if (t < 36) {
+    const double* src = a.partial + (size_t)pd.item0 * 36 + t;
+    double v = 0.0;
+    for (int i = 0; i < pd.n_items; ++i) v += src[(size_t)i * 36];
+    M[t] = v;
+    O[t] = 0.0;
+  }
+  __syncthreads();
+  const int r = t / 6, c = t - 6 * (t / 6);
+  double sym = 0.0;
+  if (same && t < 36) sym = 0.5 * (M[r * 6 + c] + M[c * 6 + r]) + (r == c ? 1.0 : 0.0);
+  __syncthreads();
+  if (same && t < 36) M[t] = sym;
+  __syncthreads();
+  // Z = M L_b^-1 (Linv row-major lower triangular)
+  if (t < 36) {
+    double v = M[t];
+    if (pd.e_b >= 0) {
+      const double* Lb = a.m.Linv + (size_t)pd.e_b * 36;
+      v = 0.0;
+      for (int j = c; j < 6; ++j) v = fma(M[r * 6 + j], Lb[j * 6 + c], v);
+    }
+    Z[t] = v;
+  }
+  __syncthreads();
+  // Cov = L_a^-T Z, negated when exactly one side is eliminated; (e, e): the upper triangle, mirrored
+  if (t < 36 && !(same && r > c)) {
+    double v = Z[t];
+    if (pd.e_a >= 0) {
+      const double* La = a.m.Linv + (size_t)pd.e_a * 36;
+      v = 0.0;
+      for (int i = r; i < 6; ++i) v = fma(La[i * 6 + r], Z[i * 6 + c], v);
+    }
+    if ((pd.e_a >= 0) != (pd.e_b >= 0)) v = -v;
+    if (r < pd.rows && c < pd.cols) {
+      O[pd.transpose ? c * pd.rows + r : r * pd.cols + c] = v;
+      if (same) O[c * pd.cols + r] = v;
+    }
+  }
+  __syncthreads();
+  if (t < 36) a.out[(size_t)p * 36 + t] = O[t];
+}
+
+void launch_cov_pairs(const CovPairsArgs& a, cudaStream_t s) {
+  cov_pairs_kernel<<<ceil_div((int64_t)a.n_items * 32, COV_WARPS * 32), COV_WARPS * 32, 0, s>>>(a);
+  RCC_CUDA(cudaGetLastError());
+  cov_pairs_combine_kernel<<<a.n_pairs, 64, 0, s>>>(a);
   RCC_CUDA(cudaGetLastError());
 }
 

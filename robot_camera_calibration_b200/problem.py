@@ -21,6 +21,11 @@ def _ip(a):
     return a.ctypes.data_as(L.c_int32_p) if a is not None else None
 
 
+_BLOCK_KINDS = {"view": L.BLOCK_VIEW, "marker": L.BLOCK_MARKER, "intr": L.BLOCK_INTR, "dist": L.BLOCK_DIST,
+                "ext": L.BLOCK_EXT}
+_BLOCK_SIZES = {L.BLOCK_VIEW: 6, L.BLOCK_MARKER: 6, L.BLOCK_INTR: 4, L.BLOCK_DIST: 5, L.BLOCK_EXT: 6}
+
+
 def _f64(a, shape=None):
     a = np.ascontiguousarray(a, dtype=np.float64)
     if shape is not None:
@@ -147,9 +152,7 @@ class BAProblem:
         self._check(self.lib.rcc_ba_update_pixels(self.h, _dp(px)))
 
     def set_constant(self, kind, index, is_constant=True):
-        if isinstance(kind, str):
-            kind = {"view": L.BLOCK_VIEW, "marker": L.BLOCK_MARKER, "intr": L.BLOCK_INTR,
-                    "dist": L.BLOCK_DIST, "ext": L.BLOCK_EXT}[kind]
+        kind = _BLOCK_KINDS[kind] if isinstance(kind, str) else kind
         self._check(self.lib.rcc_ba_set_constant(self.h, kind, index, int(bool(is_constant))))
 
     def set_loss(self, loss, scale=1.0):
@@ -278,6 +281,19 @@ class BAProblem:
                "markers": np.empty((self.n_markers, 6, 6))}
         self._check(self.lib.rcc_ba_covariance(self.h, _dp(out["shared"]), _dp(out["views"]), _dp(out["markers"])))
         return out
+
+    def covariance_blocks(self, pairs):
+        """Cross-covariance blocks of (J^T J)^-1, the same semantics as covariance(): pairs is an iterable of
+        ((kind, index), (kind, index)), kind "view" | "marker" | "intr" | "dist" | "ext" (or the integer codes) and
+        index the view, marker or camera.  Returns one (size_a, size_b) array per pair, size 6 for a pose or rig
+        extrinsic, 4 for intrinsics, 5 for distortion; Cov(b, a) is exactly Cov(a, b).T.  With pixel noise of
+        standard deviation sigma, multiply by sigma**2 (rcc_ba_covariance_blocks)."""
+        req = np.array([[_BLOCK_KINDS[k] if isinstance(k, str) else int(k), int(i)] for pair in pairs
+                        for k, i in pair], dtype=np.int32).reshape(-1, 4)
+        out = np.zeros((len(req), 36))
+        self._check(self.lib.rcc_ba_covariance_blocks(self.h, len(req), _ip(req), _dp(out)))
+        return [out[p, :_BLOCK_SIZES[ka] * _BLOCK_SIZES[kb]].reshape(_BLOCK_SIZES[ka], _BLOCK_SIZES[kb])
+                for p, (ka, _, kb, _) in enumerate(req.tolist())]
 
     # ------------------------------------------------------------------ multi-GPU
     @staticmethod
