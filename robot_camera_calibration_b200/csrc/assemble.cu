@@ -23,6 +23,7 @@
 // as coalesced 16-byte stores; the per-block cross tile J_own^T J_other (the
 // Schur off-diagonal block W) is written straight to HBM.  finalize_* reduce the
 // chunk partials in a fixed order (deterministic, no FP64 atomics).
+#include "chunk.cuh"
 #include "common.cuh"
 #include "kernels.h"
 #include "model.cuh"
@@ -60,13 +61,6 @@ struct RowSink {
   __device__ __forceinline__ void ext(int i, const double* jx) { put6(i, PG::COL_X, jx); }
 };
 
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gmem_src) {
-  const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gmem_src) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
-
 // D(8x8) += A(8x4) B(4x8), FP64.  Lane l holds A[l/4][l%4], B[l%4][l/4], D[l/4][2(l%4)], D[l/4][2(l%4)+1].
 __device__ __forceinline__ void dmma(double (&c)[2], double a, double b) {
   asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
@@ -81,15 +75,14 @@ __device__ __forceinline__ void dmma(double (&c)[2], double a, double b) {
 #define RCC_K2_MIN_CTAS_F 3   // single-camera F pass: 56 KB smem per CTA would allow 4, measured below
 #endif
 
-// per-warp shared memory (doubles): staged rows | 2 x BPW other-pose records | own pose, ext pose, shared params
+// per-warp shared memory (doubles): staged rows | pose region (chunk.cuh)
 template <bool RIG, bool EPASS>
 struct WarpSmem {
   using PG = PassGeom<RIG>;
   static constexpr int RS = EPASS ? PG::RS_E : PG::RS_F;
   static constexpr int BS = 8 * RS + 2;   // block stride: +16 B so the corner lanes of two blocks interleave over the banks
   static constexpr int STAGE = PG::BPW * BS;
-  static constexpr int CONSTS = STAGE + 2 * PG::BPW * POSEX;
-  static constexpr int TOTAL = CONSTS + 2 * POSEX + 16;
+  static constexpr int TOTAL = STAGE + CHUNK_POSE_SMEM<RIG>;
 };
 
 template <bool RIG, bool EPASS, bool OWN_IS_VIEW, bool LOSS>
@@ -107,47 +100,16 @@ assemble_kernel(const AssembleArgs a) {
   const int chunk_id = a.chunk_list ? a.chunk_list[launch_pos] : launch_pos;
   double* wsm = smem + warp * WS::TOTAL;
   double* rows = wsm;                 // [BPW][8 rows][RS]
-  double* stage = wsm + WS::STAGE;    // [2][BPW][POSEX] expanded pose of the other block, double buffered
-  double* own_x = wsm + WS::CONSTS;   // [POSEX] expanded pose of the own block
-  double* ext_x = own_x + POSEX;      // [POSEX] body_T_cam (rig)
-  double* sh = ext_x + POSEX;         // [SP] shared parameters of the chunk's camera
 
   const Chunk ch = a.chunks[chunk_id];
   const int b = lane >> 2;            // block of the warp iteration this lane evaluates a corner of
   const int t = lane & 3;             // corner
-  const double* oth_table = OWN_IS_VIEW ? a.marker_x : a.view_x;
 
-  // chunk constants -> shared memory; pad columns of the staged rows (never read back as results,
-  // but they do enter the MMAs) are cleared once
-  {
-    const double* src = (OWN_IS_VIEW ? a.view_x : a.marker_x) + (size_t)ch.own * POSEX;
-    if (lane < POSEX) own_x[lane] = src[lane];
-    if (RIG && lane < POSEX) ext_x[lane] = a.ext_x[(size_t)ch.cam * POSEX + lane];
-    if (lane < PG::SP) sh[lane] = a.shared[ch.cam * PG::SP + lane];
-    for (int k = lane; k < BPW * BS; k += 32) rows[k] = 0.0;
-  }
-  // software pipeline: other-block indices two iterations ahead (lane q holds block q),
-  // other-block pose records one iteration ahead (cp.async into stage[buf])
-  auto load_oth = [&](int it) -> int {
-    return (lane < BPW && it + lane < ch.count) ? a.oth[(int64_t)ch.start + it + lane] : 0;
-  };
-  auto issue_stage = [&](int it, int buf, int oth_reg) {
-    constexpr int PIECES = BPW * (POSEX / 2);   // 8 records x 12 16-byte pieces = 3 per lane
-#pragma unroll
-    for (int r = 0; r < PIECES / 32; ++r) {
-      const int idx = lane + 32 * r;
-      const int q = idx / (POSEX / 2), c = idx - q * (POSEX / 2);
-      const int o = __shfl_sync(0xffffffffu, oth_reg, q);
-      if (it + q < ch.count)
-        cp_async16(stage + (buf * BPW + q) * POSEX + 2 * c, oth_table + (size_t)o * POSEX + 2 * c);
-    }
-    cp_async_commit();
-  };
-  int oth_cur = load_oth(0);
-  int oth_nxt = load_oth(BPW);
-  issue_stage(0, 0, oth_cur);
-  double2 px_nxt = make_double2(0.0, 0.0);
-  if (b < ch.count) px_nxt = *reinterpret_cast<const double2*>(a.pix + ((int64_t)ch.start + b) * 8 + 2 * t);
+  // chunk constants -> shared memory; pad columns of the staged rows (never read back as results, but they do enter
+  // the MMAs) are cleared once; then the first group's poses and pixels are set in flight
+  ChunkPoses<RIG, OWN_IS_VIEW, AssembleArgs> poses(a, ch, wsm + WS::STAGE, lane);
+  for (int k = lane; k < BPW * BS; k += 32) rows[k] = 0.0;
+  poses.start();
 
   // chunk accumulators: 8x8 tiles in MMA fragment layout
   double cAA[2] = {0.0, 0.0}, cAB[2] = {0.0, 0.0}, cBB[2] = {0.0, 0.0};
@@ -159,27 +121,11 @@ assemble_kernel(const AssembleArgs a) {
   int buf = 0;
 
   for (int it = 0; it < ch.count; it += BPW, buf ^= 1) {
-    const bool valid = (it + b) < ch.count;
-    const int64_t g = (int64_t)ch.start + it + b;
-    cp_async_wait_all();
-    __syncwarp();
-    // prefetch for the next iterations (overlaps with this iteration's arithmetic)
-    const double2 px = px_nxt;
-    if (it + BPW < ch.count) {
-      issue_stage(it + BPW, buf ^ 1, oth_nxt);
-      oth_nxt = load_oth(it + 2 * BPW);
-      if (it + BPW + b < ch.count) px_nxt = *reinterpret_cast<const double2*>(a.pix + (g + BPW) * 8 + 2 * t);
-    }
     // ---- phase 1: corner evaluation ---------------------------------------
-    const double* ox_rec = stage + (buf * BPW + b) * POSEX;
-    const double* vx = OWN_IS_VIEW ? own_x : ox_rec;
-    const double* mx = OWN_IS_VIEW ? ox_rec : own_x;
+    double2 px;
     BlockGeom<RIG> geo;
-    double ox = 0.0, oy = 0.0;
-    if (valid) {
-      block_geometry<RIG>(vx, mx, RIG ? ext_x : nullptr, geo);
-      corner_xy(t, mx[PX_HS], ox, oy);
-    }
+    double ox, oy;
+    const bool valid = poses.group(it, buf, px, geo, ox, oy);
     double w = 1.0;
     if (LOSS) {
       // s = sum of the 8 squared residuals of the block: residual-only evaluation, then a
@@ -187,7 +133,7 @@ assemble_kernel(const AssembleArgs a) {
       double s_blk = 0.0;
       if (valid) {
         CornerRows<RIG> c;
-        eval_corner<RIG, false>(geo, sh, ox, oy, px.x, px.y, c);
+        eval_corner<RIG, false>(geo, poses.sh, ox, oy, px.x, px.y, c);
         s_blk = c.r[0] * c.r[0] + c.r[1] * c.r[1];
       }
       s_blk += __shfl_xor_sync(0xffffffffu, s_blk, 1);
@@ -200,7 +146,7 @@ assemble_kernel(const AssembleArgs a) {
     if (valid) {
       RowSink<RIG, EPASS, OWN_IS_VIEW> sink{{my_rows, my_rows + 4 * RS}, w};
       double r0, r1;
-      const double depth = eval_corner_emit<RIG>(geo, sh, ox, oy, px.x, px.y, sink, r0, r1);
+      const double depth = eval_corner<RIG, true>(geo, poses.sh, ox, oy, px.x, px.y, sink, r0, r1);
       if (!(depth > 0.0) || !isfinite(r0) || !isfinite(r1)) *a.fail_flag = 1;
     }
     __syncwarp();

@@ -3,6 +3,7 @@
 // K6's cost-only evaluation used for the LM gain ratio (evaluate_kernel).
 //
 // K1 is HBM-write-bound: 1 408 B out per 72 B in per observation block.
+#include "chunk.cuh"
 #include "common.cuh"
 #include "kernels.h"
 #include "model.cuh"
@@ -138,11 +139,10 @@ static void launch_evaluate_t(const EvalArgs& a, cudaStream_t s) {
 }
 
 // ---------------------------------------------------------------------------
-// materialise_kernel: K1 proper.  Same chunk pipeline as the fused kernel K2 (one warp per
-// (own block, camera) chunk, own pose in shared memory, other-pose records prefetched by
-// cp.async one iteration ahead, lane 4b+t evaluates corner t of block b and streams its
-// rows to shared memory as soon as a column group is complete), but the staged rows are
-// the Ceres layout and leave the SM as TMA bulk copies instead of feeding MMAs.
+// materialise_kernel: K1 proper.  The chunk pose pipeline of the fused kernel K2 (chunk.cuh: one
+// warp per (own block, camera) chunk, lane 4b+t evaluates corner t of block b and streams its
+// rows to shared memory as soon as a column group is complete), but the staged rows are the
+// Ceres layout and leave the SM as TMA bulk copies instead of feeding MMAs.
 // ---------------------------------------------------------------------------
 template <bool RIG, bool OWN_IS_VIEW>
 struct CeresSink {
@@ -178,90 +178,40 @@ struct CeresSink {
   __device__ __forceinline__ void ext(int i, const double* jx) { put6(ER::JX, i, jx); }
 };
 
-__device__ __forceinline__ void ev_cp_async16(void* smem_dst, const void* gmem_src) {
-  const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gmem_src) : "memory");
-}
-
 constexpr int MAT_WARPS = 4;
 template <bool RIG>
-struct MatSmem {   // per warp, doubles
-  static constexpr int STAGE = EvalRec<RIG>::SIZE;          // other-pose records [2][8][POSEX]
-  static constexpr int CONSTS = STAGE + 2 * 8 * POSEX;      // own pose, ext pose, shared parameters
-  static constexpr int TOTAL = CONSTS + 2 * POSEX + 16;
+struct MatSmem {   // per warp, doubles: Ceres-layout rows | pose region (chunk.cuh)
+  static constexpr int TOTAL = EvalRec<RIG>::SIZE + CHUNK_POSE_SMEM<RIG>;
 };
 
 template <bool RIG, bool OWN_IS_VIEW>
 __global__ void __launch_bounds__(MAT_WARPS * 32, 3) materialise_kernel(const EvalArgs a) {
   using ER = EvalRec<RIG>;
   using MS = MatSmem<RIG>;
-  constexpr int SP = RIG ? 15 : 9, BPW = 8;
+  constexpr int BPW = PassGeom<RIG>::BPW;
   extern __shared__ __align__(128) double smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int chunk_id = blockIdx.x * MAT_WARPS + warp;
   if (chunk_id >= a.n_chunks) return;
   double* wsm = smem + (size_t)warp * MS::TOTAL;
   double* wrec = wsm;                 // Ceres-layout rows of the current group of 8 blocks
-  double* stage = wsm + MS::STAGE;
-  double* own_x = wsm + MS::CONSTS;
-  double* ext_x = own_x + POSEX;
-  double* sh = ext_x + POSEX;
   const Chunk ch = a.chunks[chunk_id];
   const int b = lane >> 2, t = lane & 3;
-  const double* oth_table = OWN_IS_VIEW ? a.marker_x : a.view_x;
-  {
-    const double* src = (OWN_IS_VIEW ? a.view_x : a.marker_x) + (size_t)ch.own * POSEX;
-    if (lane < POSEX) own_x[lane] = src[lane];
-    if (RIG && lane < POSEX) ext_x[lane] = a.ext_x[(size_t)ch.cam * POSEX + lane];
-    if (lane < SP) sh[lane] = a.shared[ch.cam * SP + lane];
-  }
-  auto load_oth = [&](int it) -> int {
-    return (lane < BPW && it + lane < ch.count) ? a.oth[(int64_t)ch.start + it + lane] : 0;
-  };
+  ChunkPoses<RIG, OWN_IS_VIEW, EvalArgs> poses(a, ch, wsm + ER::SIZE, lane);
+  poses.start();
   auto load_pos = [&](int it) -> int {   // caller position of the lane's block
     return (it + b < ch.count) ? (a.orig ? a.orig[(int64_t)ch.start + it + b] : ch.start + it + b) : 0;
   };
-  auto issue_stage = [&](int it, int buf, int oth_reg) {
-#pragma unroll
-    for (int r = 0; r < 3; ++r) {   // 8 records x 12 16-byte pieces
-      const int idx = lane + 32 * r;
-      const int q = idx / (POSEX / 2), c = idx - q * (POSEX / 2);
-      const int o = __shfl_sync(0xffffffffu, oth_reg, q);
-      if (it + q < ch.count)
-        ev_cp_async16(stage + (buf * BPW + q) * POSEX + 2 * c, oth_table + (size_t)o * POSEX + 2 * c);
-    }
-    asm volatile("cp.async.commit_group;" ::: "memory");
-  };
-  int oth_cur = load_oth(0);
-  int oth_nxt = load_oth(BPW);
-  issue_stage(0, 0, oth_cur);
   int pos_nxt = load_pos(0);
-  double2 px_nxt = make_double2(0.0, 0.0);
-  if (b < ch.count) px_nxt = *reinterpret_cast<const double2*>(a.pix + ((int64_t)ch.start + b) * 8 + 2 * t);
   double cost = 0.0;
   int buf = 0;
   for (int it = 0; it < ch.count; it += BPW, buf ^= 1) {
-    const bool valid = (it + b) < ch.count;
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
-    __syncwarp();
-    const double2 px = px_nxt;
-    const int pos = pos_nxt;
-    if (it + BPW < ch.count) {
-      issue_stage(it + BPW, buf ^ 1, oth_nxt);
-      oth_nxt = load_oth(it + 2 * BPW);
-      pos_nxt = load_pos(it + BPW);
-      if (it + BPW + b < ch.count)
-        px_nxt = *reinterpret_cast<const double2*>(a.pix + ((int64_t)ch.start + it + BPW + b) * 8 + 2 * t);
-    }
-    const double* ox_rec = stage + (buf * BPW + b) * POSEX;
-    const double* vx = OWN_IS_VIEW ? own_x : ox_rec;
-    const double* mx = OWN_IS_VIEW ? ox_rec : own_x;
+    double2 px;
     BlockGeom<RIG> geo;
-    double ox = 0.0, oy = 0.0;
-    if (valid) {
-      block_geometry<RIG>(vx, mx, RIG ? ext_x : nullptr, geo);
-      corner_xy(t, mx[PX_HS], ox, oy);
-    }
+    double ox, oy;
+    const int pos = pos_nxt;
+    if (it + BPW < ch.count) pos_nxt = load_pos(it + BPW);
+    const bool valid = poses.group(it, buf, px, geo, ox, oy);
     // the previous group's bulk copies must have read the staging rows before they are rewritten
     asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
     __syncwarp();
@@ -269,7 +219,7 @@ __global__ void __launch_bounds__(MAT_WARPS * 32, 3) materialise_kernel(const Ev
     if (valid) {
       CeresSink<RIG, OWN_IS_VIEW> sink{wrec, b, t, {0, 0, 0, 0, 0}};
       double r0, r1;
-      const double depth = eval_corner_emit<RIG>(geo, sh, ox, oy, px.x, px.y, sink, r0, r1);
+      const double depth = eval_corner<RIG, true>(geo, poses.sh, ox, oy, px.x, px.y, sink, r0, r1);
       if (!(depth > 0.0) || !isfinite(r0) || !isfinite(r1)) *a.fail_flag = 1;
       r2 = r0 * r0 + r1 * r1;
     }

@@ -194,7 +194,8 @@ RCC_HD void block_geometry(const double* __restrict__ vx, const double* __restri
   }
 }
 
-// Two Jacobian rows (u, v) of one corner.
+// Two residual rows (u, v) of one corner and their Jacobian rows; the Jacobian rows are written as an eval_corner
+// sink.
 //   jv : d/d view  (rvec 0:3, t 3:6)   [world_T_camera | world_T_body]
 //   jm : d/d marker
 //   js : d/d (fx fy cx cy k1 k2 p1 p2 k3)
@@ -207,104 +208,33 @@ struct CornerRows {
   double js[2][9];
   double jx[2][6];
   double depth;
+  RCC_HD void shared(int i, const double* v, double) {
+#pragma unroll
+    for (int k = 0; k < 9; ++k) js[i][k] = v[k];
+  }
+  RCC_HD void marker(int i, const double* v) {
+#pragma unroll
+    for (int k = 0; k < 6; ++k) jm[i][k] = v[k];
+  }
+  RCC_HD void view(int i, const double* v) {
+#pragma unroll
+    for (int k = 0; k < 6; ++k) jv[i][k] = v[k];
+  }
+  RCC_HD void ext(int i, const double* v) {
+#pragma unroll
+    for (int k = 0; k < 6; ++k) jx[i][k] = v[k];
+  }
 };
 
-// shared = fx fy cx cy k1 k2 p1 p2 k3 ; (ox, oy) = corner in the tag frame ;
-// (pu, pv) = observed pixel.  WANT_J = false computes the residual only.
-template <bool RIG, bool WANT_J>
-RCC_HD void eval_corner(const BlockGeom<RIG>& g, const double* __restrict__ sh, double ox, double oy,
-                        double pu, double pv, CornerRows<RIG>& out) {
-  const double fx = sh[0], fy = sh[1], cx = sh[2], cy = sh[3];
-  const double k1 = sh[4], k2 = sh[5], p1 = sh[6], p2 = sh[7], k3 = sh[8];
-  double d[3], P[3];
-#pragma unroll
-  for (int i = 0; i < 3; ++i) {
-    d[i] = g.Rcm[3 * i] * ox + g.Rcm[3 * i + 1] * oy;
-    P[i] = d[i] + g.c0[i];
-  }
-  out.depth = P[2];
-  const double iz = 1.0 / P[2];
-  const double x = P[0] * iz, y = P[1] * iz;
-  const double xx = x * x, yy = y * y, xy = x * y;
-  const double r2 = xx + yy;
-  const double r4 = r2 * r2, r6 = r4 * r2;
-  const double rad = 1.0 + k1 * r2 + k2 * r4 + k3 * r6;
-  const double tx = 2.0 * xy, ax = r2 + 2.0 * xx, ay = r2 + 2.0 * yy;
-  const double xd = x * rad + p1 * tx + p2 * ax;
-  const double yd = y * rad + p1 * ay + p2 * tx;
-  out.r[0] = fx * xd + cx - pu;
-  out.r[1] = fy * yd + cy - pv;
-  if (!WANT_J) return;
-
-  // d(xd,yd)/d(x,y)
-  const double drad = k1 + 2.0 * k2 * r2 + 3.0 * k3 * r4;  // d rad / d r2
-  const double dxx = rad + 2.0 * xx * drad + 2.0 * p1 * y + 6.0 * p2 * x;
-  const double dxy = 2.0 * xy * drad + 2.0 * p1 * x + 2.0 * p2 * y;
-  const double dyy = rad + 2.0 * yy * drad + 6.0 * p1 * y + 2.0 * p2 * x;
-  // A = d(u,v)/dPc  (2x3)
-  double A[2][3];
-  A[0][0] = fx * dxx * iz;
-  A[0][1] = fx * dxy * iz;
-  A[0][2] = -(A[0][0] * x + A[0][1] * y);
-  A[1][0] = fy * dxy * iz;
-  A[1][1] = fy * dyy * iz;
-  A[1][2] = -(A[1][0] * x + A[1][1] * y);
-
-  // intrinsics / distortion
-  out.js[0][0] = xd;  out.js[0][1] = 0.0; out.js[0][2] = 1.0; out.js[0][3] = 0.0;
-  out.js[1][0] = 0.0; out.js[1][1] = yd;  out.js[1][2] = 0.0; out.js[1][3] = 1.0;
-  const double fxx = fx * x, fyy = fy * y;
-  out.js[0][4] = fxx * r2; out.js[0][5] = fxx * r4; out.js[0][6] = fx * tx; out.js[0][7] = fx * ax; out.js[0][8] = fxx * r6;
-  out.js[1][4] = fyy * r2; out.js[1][5] = fyy * r4; out.js[1][6] = fy * ay; out.js[1][7] = fy * tx; out.js[1][8] = fyy * r6;
-
-  // J = A [p]x M is formed as (A [p]x) M: 12 + 18 operations instead of 27 + 18
-  double B[2][3];
-  // marker rotation: dPc/drm = -[d]x Km ; marker translation: dPc/dtm = Mt
-  a_cross(A, d, -1.0, B);
-#pragma unroll
-  for (int i = 0; i < 2; ++i) {
-    row_mat(B[i], g.Km, out.jm[i]);
-#pragma unroll
-    for (int j = 0; j < 3; ++j) {
-      const double mt = A[i][0] * g.Mt[j] + A[i][1] * g.Mt[3 + j] + A[i][2] * g.Mt[6 + j];
-      out.jm[i][3 + j] = mt;
-      out.jv[i][3 + j] = -mt;  // dPc/dt_view = -Mt
-    }
-  }
-  if (!RIG) {
-    // view rotation: dPc/drv = [Pc]x Jr(rv)
-    a_cross(A, P, 1.0, B);
-#pragma unroll
-    for (int i = 0; i < 2; ++i) row_mat(B[i], g.Jrv, out.jv[i]);
-  } else {
-    // A' = A Rx^T ; body rotation: dPc/drb = Rx^T [qb]x Jr(rb) ; extrinsic translation: dPc/dtx = -Rx^T
-    double qb[3], Ax[2][3];
-#pragma unroll
-    for (int i = 0; i < 3; ++i) qb[i] = g.Rbm[3 * i] * ox + g.Rbm[3 * i + 1] * oy + g.qb0[i];
-#pragma unroll
-    for (int i = 0; i < 2; ++i) {
-      row_mat(A[i], g.RxT, Ax[i]);
-#pragma unroll
-      for (int j = 0; j < 3; ++j) out.jx[i][3 + j] = -Ax[i][j];
-    }
-    a_cross(Ax, qb, 1.0, B);
-#pragma unroll
-    for (int i = 0; i < 2; ++i) row_mat(B[i], g.Jrv, out.jv[i]);
-    // extrinsic rotation: dPc/drx = [Pc]x Jr(rx)
-    a_cross(A, P, 1.0, B);
-#pragma unroll
-    for (int i = 0; i < 2; ++i) row_mat(B[i], g.Jrx, out.jx[i]);
-  }
-}
-
-// Same arithmetic as eval_corner<RIG,true>, but every column group of the two
-// residual rows is handed to `sink` as soon as it is complete, so that a kernel
-// can store it (shared memory) immediately and keep register live ranges short.
+// Residuals (r0, r1) = (u, v) of one corner and, with WANT_J, their analytic Jacobian rows.
+// shared = fx fy cx cy k1 k2 p1 p2 k3 ; (ox, oy) = corner in the tag frame ; (pu, pv) = observed pixel.
+// Every column group of the two rows is handed to `sink` as soon as it is complete, so that a kernel can store
+// it (shared memory) immediately and keep register live ranges short:
 //   sink.shared(i, js[9], r)   sink.marker(i, jm[6])   sink.view(i, jv[6])   sink.ext(i, jx[6])
-// with i = 0 (u row), 1 (v row).  Returns the corner's depth.
-template <bool RIG, class Geo, class Sink>
-RCC_HD double eval_corner_emit(const Geo& g, const double* __restrict__ sh, double ox, double oy,
-                               double pu, double pv, Sink& sink, double& r0, double& r1) {
+// with i = 0 (u row), 1 (v row).  WANT_J = false returns before the first sink call.  Returns the corner's depth.
+template <bool RIG, bool WANT_J, class Sink>
+RCC_HD double eval_corner(const BlockGeom<RIG>& g, const double* __restrict__ sh, double ox, double oy, double pu,
+                          double pv, Sink& sink, double& r0, double& r1) {
   const double fx = sh[0], fy = sh[1], cx = sh[2], cy = sh[3];
   const double k1 = sh[4], k2 = sh[5], p1 = sh[6], p2 = sh[7], k3 = sh[8];
   double d[3], P[3];
@@ -324,17 +254,20 @@ RCC_HD double eval_corner_emit(const Geo& g, const double* __restrict__ sh, doub
   const double yd = y * rad + p1 * ay + p2 * tx;
   r0 = fx * xd + cx - pu;
   r1 = fy * yd + cy - pv;
-  {
+  if (!WANT_J) return P[2];
+  {  // intrinsics / distortion
     const double fxx = fx * x, fyy = fy * y;
     const double js0[9] = {xd, 0.0, 1.0, 0.0, fxx * r2, fxx * r4, fx * tx, fx * ax, fxx * r6};
     sink.shared(0, js0, r0);
     const double js1[9] = {0.0, yd, 0.0, 1.0, fyy * r2, fyy * r4, fy * ay, fy * tx, fyy * r6};
     sink.shared(1, js1, r1);
   }
-  const double drad = k1 + 2.0 * k2 * r2 + 3.0 * k3 * r4;
+  // d(xd,yd)/d(x,y)
+  const double drad = k1 + 2.0 * k2 * r2 + 3.0 * k3 * r4;  // d rad / d r2
   const double dxx = rad + 2.0 * xx * drad + 2.0 * p1 * y + 6.0 * p2 * x;
   const double dxy = 2.0 * xy * drad + 2.0 * p1 * x + 2.0 * p2 * y;
   const double dyy = rad + 2.0 * yy * drad + 6.0 * p1 * y + 2.0 * p2 * x;
+  // A = d(u,v)/dPc  (2x3)
   double A[2][3];
   A[0][0] = fx * dxx * iz;
   A[0][1] = fx * dxy * iz;
@@ -343,6 +276,7 @@ RCC_HD double eval_corner_emit(const Geo& g, const double* __restrict__ sh, doub
   A[1][1] = fy * dyy * iz;
   A[1][2] = -(A[1][0] * x + A[1][1] * y);
 
+  // J = A [p]x M is formed as (A [p]x) M: 12 + 18 operations instead of 27 + 18
   double jvt[2][3];  // d/d t_view = -A Mt (kept until the rotation part is ready)
   double B[2][3];
   a_cross(A, d, -1.0, B);   // marker rotation: -A [d]x Km
@@ -394,6 +328,13 @@ RCC_HD double eval_corner_emit(const Geo& g, const double* __restrict__ sh, doub
     }
   }
   return P[2];
+}
+
+// eval_corner into a CornerRows (residuals, depth and, with WANT_J, the Jacobian rows)
+template <bool RIG, bool WANT_J>
+RCC_HD void eval_corner(const BlockGeom<RIG>& g, const double* __restrict__ sh, double ox, double oy, double pu,
+                        double pv, CornerRows<RIG>& out) {
+  out.depth = eval_corner<RIG, WANT_J>(g, sh, ox, oy, pu, pv, out, out.r[0], out.r[1]);
 }
 
 // Robust loss rho(s) on s = ||r_block||^2 (all 8 residuals of a tag), Ceres semantics:
