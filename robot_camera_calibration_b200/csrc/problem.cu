@@ -1316,6 +1316,10 @@ static void update_pixels(P_t* P, const T* pixels) {
 
 static thread_local std::string g_create_error;
 
+// 6-wide column blocks of the dense border of the reduced system: the shared parameters and the right-hand side.
+// The border kernels hold at most 128 columns (schur_border_kernel: SB_MAXPASS passes of 32).
+static int64_t border_blocks(int64_t n_shared) { return (n_shared + 1 + 5) / 6; }
+
 #define API_BEGIN(P)                                     \
   if (!(P)) return RCC_BAD_ARG;                          \
   try {                                                  \
@@ -1357,6 +1361,12 @@ int rcc_ba_create(const rcc_ba_options* opt, rcc_ba_problem** out) {
   if (opt->n_views <= 0 || opt->n_markers <= 0 || opt->n_cameras <= 0 || opt->n_obs_blocks < 0 ||
       (opt->model != RCC_MODEL_SINGLE && opt->model != RCC_MODEL_RIG))
     return RCC_BAD_ARG;
+  const int sp = opt->model == RCC_MODEL_RIG ? 15 : 9;
+  if (border_blocks((int64_t)opt->n_cameras * sp) * 6 > 128) {
+    g_create_error = "too many cameras: the shared border holds at most 125 parameters (8 rig or 13 single-model cameras)";
+    fprintf(stderr, "[rcc_ba] create failed: %s\n", g_create_error.c_str());
+    return RCC_BAD_ARG;
+  }
   P_t* P = new P_t();
   try {
     int ndev = 0;
@@ -1373,7 +1383,7 @@ int rcc_ba_create(const rcc_ba_options* opt, rcc_ba_problem** out) {
                     "; this library carries sm_100a code only");
     P->opt = *opt;
     P->rig = opt->model == RCC_MODEL_RIG;
-    P->sp = P->rig ? 15 : 9;
+    P->sp = sp;
     P->n_cam = opt->n_cameras;
     P->n_shared = P->n_cam * P->sp;
     P->fin_slices = fin_slices(prop.multiProcessorCount, P->n_cam);
@@ -1383,12 +1393,10 @@ int rcc_ba_create(const rcc_ba_options* opt, rcc_ba_problem** out) {
     P->elim_view = opt->eliminate == RCC_ELIM_VIEWS || (opt->eliminate == RCC_ELIM_AUTO && opt->n_views >= opt->n_markers);
     P->n_e = P->elim_view ? P->n_views : P->n_markers;
     P->n_f = P->elim_view ? P->n_markers : P->n_views;
-    P->n_bb = (P->n_shared + 1 + 5) / 6;
+    P->n_bb = (int)border_blocks(P->n_shared);
     P->n_red = 6 * P->n_f + P->n_shared;
     P->ld = 6 * P->n_f + 6 * P->n_bb;
     RCC_REQUIRE((int64_t)P->n_red * P->ld < (int64_t)1 << 40, RCC_BAD_ARG, "reduced system too large");
-    RCC_REQUIRE(P->n_bb * 6 <= 128, RCC_BAD_ARG,
-                "too many cameras: the shared border holds at most 125 parameters (8 rig or 13 single-model cameras)");
     RCC_CUDA(cudaStreamCreateWithFlags(&P->stream, cudaStreamNonBlocking));
     P->own_stream = true;
     RCC_CUDA(cudaStreamCreateWithFlags(&P->side_stream, cudaStreamNonBlocking));
