@@ -21,7 +21,8 @@
  *
  * Parameter blocks (FP64), conventions cited to camera_pose.cpp:
  *   intr[4] = fx fy cx cy   (K[0] K[4] K[2] K[5], :61-62)
- *   dist[5] = k1 k2 p1 p2 k3 (:39,63-64)
+ *   dist[5] = k1 k2 p1 p2 k3 (:39,63-64)        [radial-tangential lens, the default]
+ *           = k1 k2 k3 k4 -                       [equidistant lens, rcc_ba_set_lens]
  *   view[6] = Rodrigues rvec, t of world_T_camera (:88-98)   [rig: world_T_body]
  *   marker[6] = rvec, t of world_T_target (:111-121)
  *   ext[6]  = rvec, t of body_T_cam   (rig model only; not in the reference)
@@ -54,6 +55,19 @@ enum rcc_model { RCC_MODEL_SINGLE = 0, RCC_MODEL_RIG = 1 };
 enum rcc_eliminate { RCC_ELIM_AUTO = 0, RCC_ELIM_VIEWS = 1, RCC_ELIM_MARKERS = 2 };
 enum rcc_loss { RCC_LOSS_TRIVIAL = 0, RCC_LOSS_HUBER = 1, RCC_LOSS_CAUCHY = 2 };
 enum rcc_block_kind { RCC_BLOCK_VIEW = 0, RCC_BLOCK_MARKER = 1, RCC_BLOCK_INTR = 2, RCC_BLOCK_DIST = 3, RCC_BLOCK_EXT = 4 };
+/* Lens model of every camera of a handle.  For the corner Pc = (X, Y, Z) in the camera frame:
+ *   RCC_LENS_RADTAN       pinhole + radial-tangential (cv::projectPoints): x = X/Z, y = Y/Z, r2 = x^2 + y^2,
+ *                         x' = x (1 + k1 r2 + k2 r2^2 + k3 r2^3) + 2 p1 x y + p2 (r2 + 2 x^2), y' likewise
+ *   RCC_LENS_EQUIDISTANT  equidistant fisheye, Kannala-Brandt with 4 coefficients (cv::fisheye with skew 0, ROS
+ *                         camera_info "equidistant", Kalibr "equidistant"):
+ *                         rho = sqrt(X^2 + Y^2), th = atan2(rho, Z), th_d = th (1 + k1 th^2 + k2 th^4 + k3 th^6 + k4 th^8),
+ *                         (x', y') = th_d (X, Y) / rho   (-> (X, Y) / Z on the optical axis)
+ * then u = fx x' + cx, v = fy y' + cy for both.  Under the equidistant lens dist[5] = k1 k2 k3 k4 and a reserved
+ * slot 4: the projection ignores it, its jac_dist column is exactly 0, the library always holds it constant (whatever
+ * rcc_ba_set_constant says), so its step and its covariance rows and columns are exactly 0 and
+ * rcc_ba_get_intrinsics returns it as it was set.  A corner with Z <= 0 fails the evaluation (RCC_EVAL_FAILED) under
+ * either lens: the equidistant field of view is below 180 degrees. */
+enum rcc_lens { RCC_LENS_RADTAN = 0, RCC_LENS_EQUIDISTANT = 1 };
 
 typedef struct {
   int32_t model;      /* rcc_model */
@@ -139,6 +153,10 @@ int rcc_ba_set_constant(rcc_ba_problem* p, int32_t block_kind, int32_t index, in
  * HuberLoss(scale) / CauchyLoss(scale), scale in pixels); the reported cost becomes 0.5 * sum rho(s) */
 int rcc_ba_set_loss(rcc_ba_problem* p, int32_t loss, double scale);
 
+/* lens model of every camera (rcc_lens; default RCC_LENS_RADTAN).  May be called at any time; like rcc_ba_set_loss it
+ * invalidates the linearisation.  RCC_BAD_ARG for an unknown lens. */
+int rcc_ba_set_lens(rcc_ba_problem* p, int32_t lens);
+
 int rcc_ba_get_intrinsics(rcc_ba_problem* p, double* intr, double* dist);
 int rcc_ba_get_rig_extrinsics(rcc_ba_problem* p, double* ext);
 int rcc_ba_get_view_poses(rcc_ba_problem* p, double* views);
@@ -148,7 +166,7 @@ int rcc_ba_get_marker_poses(rcc_ba_problem* p, double* markers);
  * Outputs are in the caller's observation order.  Any pointer may be NULL.
  *   residuals   : n_obs_blocks x 8
  *   jac_intr    : n_obs_blocks x 8 x 4   row-major per block  (= jacobians[0])
- *   jac_dist    : n_obs_blocks x 8 x 5                        (= jacobians[1])
+ *   jac_dist    : n_obs_blocks x 8 x 5                        (= jacobians[1]; column 4 is 0 under the equidistant lens)
  *   jac_view    : n_obs_blocks x 8 x 6                        (= jacobians[2])
  *   jac_marker  : n_obs_blocks x 8 x 6                        (= jacobians[3])
  *   jac_ext     : n_obs_blocks x 8 x 6   (rig only)           (= jacobians[4])
@@ -275,6 +293,11 @@ int rcc_fp64_peak_tflops(int32_t device, double* tflops);
  *   initialisation), refined pose out ; final_cost n (may be NULL; -1 = failed) */
 int rcc_pnp_batch(int32_t device, int64_t n, const double* shared9, const double* sizes, const double* pixels,
                   double* cam_T_tag, double* final_cost, int32_t max_iterations);
+/* the same for a lens (rcc_lens): shared9 = fx fy cx cy followed by that lens's dist[5].  The equidistant homography
+ * start undistorts each corner by solving th_d(th) for th with Newton's method (cv::fisheye::undistortPoints) and
+ * takes tan(th) along the distorted direction.  RCC_BAD_ARG for an unknown lens. */
+int rcc_pnp_batch_lens(int32_t device, int32_t lens, int64_t n, const double* shared9, const double* sizes,
+                       const double* pixels, double* cam_T_tag, double* final_cost, int32_t max_iterations);
 
 #ifdef __cplusplus
 }

@@ -22,6 +22,8 @@ STATUS_NAMES = ["RCC_OK", "RCC_BAD_ARG", "RCC_CUDA_ERROR", "RCC_NCCL_ERROR", "RC
 MODEL_SINGLE, MODEL_RIG = 0, 1
 ELIM_AUTO, ELIM_VIEWS, ELIM_MARKERS = 0, 1, 2
 BLOCK_VIEW, BLOCK_MARKER, BLOCK_INTR, BLOCK_DIST, BLOCK_EXT = range(5)
+LENS_RADTAN, LENS_EQUIDISTANT = 0, 1
+LENSES = {"radtan": LENS_RADTAN, "equidistant": LENS_EQUIDISTANT}
 COMM_ID_BYTES = 128
 
 
@@ -74,6 +76,7 @@ SIGNATURES = {
     "rcc_ba_update_pixels_i16": (C.c_int, [_H, c_int16_p]),
     "rcc_ba_set_constant": (C.c_int, [_H, C.c_int32, C.c_int32, C.c_int32]),
     "rcc_ba_set_loss": (C.c_int, [_H, C.c_int32, C.c_double]),
+    "rcc_ba_set_lens": (C.c_int, [_H, C.c_int32]),
     "rcc_ba_get_intrinsics": (C.c_int, [_H, c_double_p, c_double_p]),
     "rcc_ba_get_rig_extrinsics": (C.c_int, [_H, c_double_p]),
     "rcc_ba_get_view_poses": (C.c_int, [_H, c_double_p]),
@@ -108,6 +111,8 @@ SIGNATURES = {
     "rcc_fp64_peak_tflops": (C.c_int, [C.c_int32, c_double_p]),
     "rcc_pnp_batch": (C.c_int, [C.c_int32, C.c_int64, c_double_p, c_double_p, c_double_p, c_double_p, c_double_p,
                                 C.c_int32]),
+    "rcc_pnp_batch_lens": (C.c_int, [C.c_int32, C.c_int32, C.c_int64, c_double_p, c_double_p, c_double_p, c_double_p,
+                                     c_double_p, C.c_int32]),
 }
 
 _lib = None

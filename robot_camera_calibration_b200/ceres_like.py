@@ -24,12 +24,16 @@ from .problem import BAProblem
 
 class TagReprojectionCost:
     """CostFunction of one detected tag: 8 residuals (4 corners x (u,v)), parameter
-    blocks intr[4], dist[5], view[6], marker[6] (+ ext[6] in a rig)."""
+    blocks intr[4], dist[5], view[6], marker[6] (+ ext[6] in a rig).  lens "radtan" (dist = k1 k2 p1 p2 k3) or
+    "equidistant" (dist = k1 k2 k3 k4 + a reserved slot that is held constant)."""
 
-    def __init__(self, pixels, tag_size, rig=False):
+    def __init__(self, pixels, tag_size, rig=False, lens="radtan"):
+        if lens not in L.LENSES:
+            raise ValueError(f"unknown lens {lens!r}: expected one of {sorted(L.LENSES)}")
         self.pixels = np.ascontiguousarray(pixels, dtype=np.float64).reshape(8)
         self.tag_size = float(tag_size)
         self.rig = bool(rig)
+        self.lens = lens
 
     def num_residuals(self):
         return 8
@@ -43,7 +47,7 @@ class TagReprojectionCost:
         row-major (8 x block_size_i).  Returns False on evaluation failure."""
         intr, dist, view, marker = parameters[:4]
         ext = parameters[4] if self.rig else None
-        with BAProblem(1, 1, 1, 1, model="rig" if self.rig else "single") as p:
+        with BAProblem(1, 1, 1, 1, model="rig" if self.rig else "single", lens=self.lens) as p:
             p.set_intrinsics(intr, dist)
             if self.rig:
                 p.set_rig_extrinsics(ext)
@@ -168,12 +172,16 @@ class Problem:
         if not self._blocks:
             raise ValueError("problem has no residual blocks")
         rig = self._blocks[0][0].rig
+        lens = self._blocks[0][0].lens
         views, markers, cams = {}, {}, {}
         vi, mi, ci, px, sizes = [], [], [], [], {}
         seen = {}     # id(array) -> camera key: one Ceres parameter block must belong to exactly one GPU camera
         for cost, intr, dist, view, marker, ext in self._blocks:
             if cost.rig != rig:
                 raise NotImplementedError("rig and single-camera cost functions cannot be mixed in one problem")
+            if cost.lens != lens:
+                raise NotImplementedError("cost functions of different lenses cannot be mixed in one problem: the "
+                                          "lens applies to every camera of the GPU problem")
             v = views.setdefault(id(view), (len(views), view))[0]
             m = markers.setdefault(id(marker), (len(markers), marker))[0]
             key = (id(intr), id(dist), id(ext) if ext is not None else 0)
@@ -191,7 +199,7 @@ class Problem:
         mlist = [a for _, a in sorted(markers.values(), key=lambda t: t[0])]
         clist = sorted(cams.values(), key=lambda t: t[0])
         gp = BAProblem(len(vlist), len(mlist), len(clist), len(vi), model="rig" if rig else "single",
-                       device=self.device, eliminate=self.eliminate)
+                       device=self.device, eliminate=self.eliminate, lens=lens)
         gp.set_intrinsics(np.stack([c[1] for c in clist]), np.stack([c[2] for c in clist]))
         if rig:
             gp.set_rig_extrinsics(np.stack([c[3] for c in clist]))

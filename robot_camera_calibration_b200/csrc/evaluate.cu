@@ -55,7 +55,7 @@ struct EvalIdx {      // raw loads only: nothing here may wait on memory when th
 
 // K6: residual / cost evaluation without Jacobians (LM gain ratio, Evaluate() without jacobians).
 // Persistent warps, a group of 8 blocks per warp iteration, the next group's indices and pixels in flight.
-template <bool RIG>
+template <bool RIG, Lens L>
 __global__ void __launch_bounds__(EVAL_THREADS, EVAL_CTAS_PER_SM) evaluate_kernel(const EvalArgs a) {
   constexpr int SP = RIG ? 15 : 9;
   constexpr int WPC = EVAL_THREADS / 32;
@@ -112,7 +112,7 @@ __global__ void __launch_bounds__(EVAL_THREADS, EVAL_CTAS_PER_SM) evaluate_kerne
       double ox, oy;
       corner_xy(t, mx[PX_HS], ox, oy);
       CornerRows<RIG> c;
-      eval_corner<RIG, false>(geo, a.shared + (size_t)cur.cam * SP, ox, oy, cur.px.x, cur.px.y, c);
+      eval_corner<RIG, false, L>(geo, a.shared + (size_t)cur.cam * SP, ox, oy, cur.px.x, cur.px.y, c);
       if (!(c.depth > 0.0) || !isfinite(c.r[0]) || !isfinite(c.r[1])) *a.fail_flag = 1;
       r2 = c.r[0] * c.r[0] + c.r[1] * c.r[1];
       if (a.residuals)
@@ -132,9 +132,9 @@ __global__ void __launch_bounds__(EVAL_THREADS, EVAL_CTAS_PER_SM) evaluate_kerne
   if (threadIdx.x == 0 && a.cost2_partials) a.cost2_partials[blockIdx.x] = s;
 }
 
-template <bool RIG>
+template <bool RIG, Lens L>
 static void launch_evaluate_t(const EvalArgs& a, cudaStream_t s) {
-  evaluate_kernel<RIG><<<eval_grid(a.n), EVAL_THREADS, 0, s>>>(a);
+  evaluate_kernel<RIG, L><<<eval_grid(a.n), EVAL_THREADS, 0, s>>>(a);
   RCC_CUDA(cudaGetLastError());
 }
 
@@ -184,7 +184,7 @@ struct MatSmem {   // per warp, doubles: Ceres-layout rows | pose region (chunk.
   static constexpr int TOTAL = EvalRec<RIG>::SIZE + CHUNK_POSE_SMEM<RIG>;
 };
 
-template <bool RIG, bool OWN_IS_VIEW>
+template <bool RIG, bool OWN_IS_VIEW, Lens L>
 __global__ void __launch_bounds__(MAT_WARPS * 32, 3) materialise_kernel(const EvalArgs a) {
   using ER = EvalRec<RIG>;
   using MS = MatSmem<RIG>;
@@ -219,7 +219,7 @@ __global__ void __launch_bounds__(MAT_WARPS * 32, 3) materialise_kernel(const Ev
     if (valid) {
       CeresSink<RIG, OWN_IS_VIEW> sink{wrec, b, t, {0, 0, 0, 0, 0}};
       double r0, r1;
-      const double depth = eval_corner<RIG, true>(geo, poses.sh, ox, oy, px.x, px.y, sink, r0, r1);
+      const double depth = eval_corner<RIG, true, L>(geo, poses.sh, ox, oy, px.x, px.y, sink, r0, r1);
       if (!(depth > 0.0) || !isfinite(r0) || !isfinite(r1)) *a.fail_flag = 1;
       r2 = r0 * r0 + r1 * r1;
     }
@@ -263,10 +263,10 @@ __global__ void __launch_bounds__(MAT_WARPS * 32, 3) materialise_kernel(const Ev
   if (lane == 0 && a.cost2_partials) a.cost2_partials[chunk_id] = cost;
 }
 
-template <bool RIG, bool OWN_IS_VIEW>
+template <bool RIG, bool OWN_IS_VIEW, Lens L>
 static void launch_materialise_t(const EvalArgs& a, cudaStream_t s) {
   const size_t smem = (size_t)MAT_WARPS * MatSmem<RIG>::TOTAL * sizeof(double);
-  auto k = materialise_kernel<RIG, OWN_IS_VIEW>;
+  auto k = materialise_kernel<RIG, OWN_IS_VIEW, L>;
   static SmemOptIn optin;
   optin.ensure(k, smem);
   k<<<ceil_div(a.n_chunks, MAT_WARPS), MAT_WARPS * 32, smem, s>>>(a);
@@ -275,27 +275,33 @@ static void launch_materialise_t(const EvalArgs& a, cudaStream_t s) {
 
 int eval_partials(bool want_jac, const EvalArgs& a) { return want_jac ? a.n_chunks : eval_grid(a.n); }
 
-void launch_evaluate(bool rig, bool want_jac, const EvalArgs& a, cudaStream_t s) {
-  if (a.n == 0) return;
+template <Lens L>
+static void launch_evaluate_l(bool rig, bool want_jac, const EvalArgs& a, cudaStream_t s) {
   if (want_jac) {
     if (rig) {
-      if (a.own_is_view) launch_materialise_t<true, true>(a, s);
-      else launch_materialise_t<true, false>(a, s);
+      if (a.own_is_view) launch_materialise_t<true, true, L>(a, s);
+      else launch_materialise_t<true, false, L>(a, s);
     } else {
-      if (a.own_is_view) launch_materialise_t<false, true>(a, s);
-      else launch_materialise_t<false, false>(a, s);
+      if (a.own_is_view) launch_materialise_t<false, true, L>(a, s);
+      else launch_materialise_t<false, false, L>(a, s);
     }
     return;
   }
-  if (rig) launch_evaluate_t<true>(a, s);
-  else launch_evaluate_t<false>(a, s);
+  if (rig) launch_evaluate_t<true, L>(a, s);
+  else launch_evaluate_t<false, L>(a, s);
 }
 
-void launch_cost(bool rig, const EvalArgs& a, cudaStream_t s) {
+void launch_evaluate(bool rig, bool want_jac, int lens, const EvalArgs& a, cudaStream_t s) {
+  if (a.n == 0) return;
+  if (lens == LENS_EQUIDISTANT) launch_evaluate_l<LENS_EQUIDISTANT>(rig, want_jac, a, s);
+  else launch_evaluate_l<LENS_RADTAN>(rig, want_jac, a, s);
+}
+
+void launch_cost(bool rig, int lens, const EvalArgs& a, cudaStream_t s) {
   EvalArgs b = a;
   b.residuals = nullptr;
   b.jac_intr = b.jac_dist = b.jac_view = b.jac_marker = b.jac_ext = nullptr;
-  launch_evaluate(rig, false, b, s);
+  launch_evaluate(rig, false, lens, b, s);
 }
 
 // deterministic single-CTA sum

@@ -73,8 +73,11 @@ struct AssembleArgs {
 };
 
 // K2: fused residual + Jacobian + J^T J tiles.  own_is_view tells which pose
-// table the segment owner indexes.
-void launch_assemble(bool rig, bool epass, bool own_is_view, const AssembleArgs& a, cudaStream_t s);
+// table the segment owner indexes; lens is a Lens (model.cuh).  Under the equidistant lens tile B holds
+// [cx cy k1 k2 k3 k4 0 | r]: the reserved slot's column is zero.
+void launch_assemble(bool rig, bool epass, bool own_is_view, int lens, const AssembleArgs& a, cudaStream_t s);
+// the equidistant instantiations (assemble_equidistant.cu)
+void launch_assemble_equidistant(bool rig, bool epass, bool own_is_view, const AssembleArgs& a, cudaStream_t s);
 
 // per-own-block reduction of the chunk partials
 struct FinalizeSideArgs {
@@ -151,10 +154,10 @@ struct EvalArgs {
   int32_t own_is_view;
 };
 int eval_grid(int64_t n);   // CTAs launch_evaluate / launch_cost will use
-void launch_evaluate(bool rig, bool want_jac, const EvalArgs& a, cudaStream_t s);
+void launch_evaluate(bool rig, bool want_jac, int lens, const EvalArgs& a, cudaStream_t s);
 // number of cost partials launch_evaluate writes (want_jac: one per chunk; else one per CTA)
 int eval_partials(bool want_jac, const EvalArgs& a);
-void launch_cost(bool rig, const EvalArgs& a, cudaStream_t s);
+void launch_cost(bool rig, int lens, const EvalArgs& a, cudaStream_t s);
 // deterministic sum of n doubles -> out[0] (single CTA)
 void launch_sum(const double* in, int64_t n, double* out, double scale, cudaStream_t s);
 

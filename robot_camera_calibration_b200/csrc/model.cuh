@@ -1,5 +1,5 @@
-// Reprojection cost functor: pinhole + radial-tangential camera observing the
-// four corners of a square fiducial tag through Rodrigues poses.
+// Reprojection cost functor: pinhole + radial-tangential (or equidistant fisheye)
+// camera observing the four corners of a square fiducial tag through Rodrigues poses.
 //
 // Conventions (all from /root/reference/real_preprocessing/src/camera_pose.cpp):
 //   intrinsics fx fy cx cy = K[0] K[4] K[2] K[5]                     :61-62
@@ -31,10 +31,30 @@ constexpr int PX_R = 0, PX_JR = 9, PX_T = 18;
 constexpr int PX_RJ = PX_JR;   // marker records
 constexpr int PX_HS = 21;  // marker records: half tag size (filled by expand_poses_kernel)
 
+// Lens model of a camera (the same for every camera of a problem):
+//   LENS_RADTAN       pinhole + radial-tangential, dist = k1 k2 p1 p2 k3 (cv::projectPoints)
+//   LENS_EQUIDISTANT  equidistant fisheye (Kannala-Brandt), dist = k1 k2 k3 k4 + one reserved slot that the
+//                     projection ignores (cv::fisheye::projectPoints with skew 0)
+enum Lens : int { LENS_RADTAN = 0, LENS_EQUIDISTANT = 1 };
+
 // sin(t)/t, accurate for all t >= 0
 RCC_HD double sinc_d(double t2, double t) {
   if (t2 < 1e-6) return 1.0 - t2 * (1.0 / 6.0) + t2 * t2 * (1.0 / 120.0);
   return sin(t) / t;
+}
+
+// atan2 as a template, so that code instantiating only the radial-tangential lens never needs atan2 for its scalar
+// type (tests/host_harness/flop_count.cpp counts operations through a scalar class)
+template <class T>
+RCC_HD T atan2_t(T y, T x) {
+  return atan2(y, x);
+}
+
+// (t - sin t cos t) / t^3 given sc = sin t cos t, accurate for all t >= 0 (series below t = 0.1: no cancellation)
+RCC_HD double tsc3_d(double t2, double t, double sc) {
+  if (t2 < 1e-2)
+    return 2.0 / 3.0 + t2 * (-2.0 / 15.0 + t2 * (4.0 / 315.0 + t2 * (-2.0 / 2835.0 + t2 * (4.0 / 155925.0))));
+  return (t - sc) / (t * t2);
 }
 
 // rvec,t (6 doubles) -> R, Jr, t.   R = I + A K + B K^2,  Jr = I - B K + C K^2,
@@ -198,7 +218,7 @@ RCC_HD void block_geometry(const double* __restrict__ vx, const double* __restri
 // sink.
 //   jv : d/d view  (rvec 0:3, t 3:6)   [world_T_camera | world_T_body]
 //   jm : d/d marker
-//   js : d/d (fx fy cx cy k1 k2 p1 p2 k3)
+//   js : d/d (fx fy cx cy k1 k2 p1 p2 k3)   [equidistant: fx fy cx cy k1 k2 k3 k4, reserved slot 0]
 //   jx : d/d body_T_cam (rig only)
 template <bool RIG>
 struct CornerRows {
@@ -227,12 +247,14 @@ struct CornerRows {
 };
 
 // Residuals (r0, r1) = (u, v) of one corner and, with WANT_J, their analytic Jacobian rows.
-// shared = fx fy cx cy k1 k2 p1 p2 k3 ; (ox, oy) = corner in the tag frame ; (pu, pv) = observed pixel.
+// shared = fx fy cx cy k1 k2 p1 p2 k3 (LENS_RADTAN) | fx fy cx cy k1 k2 k3 k4 - (LENS_EQUIDISTANT);
+// (ox, oy) = corner in the tag frame ; (pu, pv) = observed pixel.
 // Every column group of the two rows is handed to `sink` as soon as it is complete, so that a kernel can store
 // it (shared memory) immediately and keep register live ranges short:
 //   sink.shared(i, js[9], r)   sink.marker(i, jm[6])   sink.view(i, jv[6])   sink.ext(i, jx[6])
 // with i = 0 (u row), 1 (v row).  WANT_J = false returns before the first sink call.  Returns the corner's depth.
-template <bool RIG, bool WANT_J, class Sink>
+// The lenses differ only in the residual, js and A = d(u,v)/dPc; the pose column groups are formed from A.
+template <bool RIG, bool WANT_J, Lens L = LENS_RADTAN, class Sink>
 RCC_HD double eval_corner(const BlockGeom<RIG>& g, const double* __restrict__ sh, double ox, double oy, double pu,
                           double pv, Sink& sink, double& r0, double& r1) {
   const double fx = sh[0], fy = sh[1], cx = sh[2], cy = sh[3];
@@ -243,38 +265,79 @@ RCC_HD double eval_corner(const BlockGeom<RIG>& g, const double* __restrict__ sh
     d[i] = g.Rcm[3 * i] * ox + g.Rcm[3 * i + 1] * oy;
     P[i] = d[i] + g.c0[i];
   }
-  const double iz = 1.0 / P[2];
-  const double x = P[0] * iz, y = P[1] * iz;
-  const double xx = x * x, yy = y * y, xy = x * y;
-  const double r2 = xx + yy;
-  const double r4 = r2 * r2, r6 = r4 * r2;
-  const double rad = 1.0 + k1 * r2 + k2 * r4 + k3 * r6;
-  const double tx = 2.0 * xy, ax = r2 + 2.0 * xx, ay = r2 + 2.0 * yy;
-  const double xd = x * rad + p1 * tx + p2 * ax;
-  const double yd = y * rad + p1 * ay + p2 * tx;
-  r0 = fx * xd + cx - pu;
-  r1 = fy * yd + cy - pv;
-  if (!WANT_J) return P[2];
-  {  // intrinsics / distortion
-    const double fxx = fx * x, fyy = fy * y;
-    const double js0[9] = {xd, 0.0, 1.0, 0.0, fxx * r2, fxx * r4, fx * tx, fx * ax, fxx * r6};
-    sink.shared(0, js0, r0);
-    const double js1[9] = {0.0, yd, 0.0, 1.0, fyy * r2, fyy * r4, fy * ay, fy * tx, fyy * r6};
-    sink.shared(1, js1, r1);
+  double A[2][3];   // A = d(u,v)/dPc  (2x3)
+  if constexpr (L == LENS_RADTAN) {
+    const double iz = 1.0 / P[2];
+    const double x = P[0] * iz, y = P[1] * iz;
+    const double xx = x * x, yy = y * y, xy = x * y;
+    const double r2 = xx + yy;
+    const double r4 = r2 * r2, r6 = r4 * r2;
+    const double rad = 1.0 + k1 * r2 + k2 * r4 + k3 * r6;
+    const double tx = 2.0 * xy, ax = r2 + 2.0 * xx, ay = r2 + 2.0 * yy;
+    const double xd = x * rad + p1 * tx + p2 * ax;
+    const double yd = y * rad + p1 * ay + p2 * tx;
+    r0 = fx * xd + cx - pu;
+    r1 = fy * yd + cy - pv;
+    if (!WANT_J) return P[2];
+    {  // intrinsics / distortion
+      const double fxx = fx * x, fyy = fy * y;
+      const double js0[9] = {xd, 0.0, 1.0, 0.0, fxx * r2, fxx * r4, fx * tx, fx * ax, fxx * r6};
+      sink.shared(0, js0, r0);
+      const double js1[9] = {0.0, yd, 0.0, 1.0, fyy * r2, fyy * r4, fy * ay, fy * tx, fyy * r6};
+      sink.shared(1, js1, r1);
+    }
+    // d(xd,yd)/d(x,y)
+    const double drad = k1 + 2.0 * k2 * r2 + 3.0 * k3 * r4;  // d rad / d r2
+    const double dxx = rad + 2.0 * xx * drad + 2.0 * p1 * y + 6.0 * p2 * x;
+    const double dxy = 2.0 * xy * drad + 2.0 * p1 * x + 2.0 * p2 * y;
+    const double dyy = rad + 2.0 * yy * drad + 6.0 * p1 * y + 2.0 * p2 * x;
+    A[0][0] = fx * dxx * iz;
+    A[0][1] = fx * dxy * iz;
+    A[0][2] = -(A[0][0] * x + A[0][1] * y);
+    A[1][0] = fy * dxy * iz;
+    A[1][1] = fy * dyy * iz;
+    A[1][2] = -(A[1][0] * x + A[1][1] * y);
+  } else {
+    // equidistant: rho = |(X, Y)|, th = atan2(rho, Z), th_d = th f(th^2), f = 1 + k1 th^2 + .. + k4 th^8,
+    // (x', y') = s (X, Y) with s = th_d / rho = f c, c = th / rho = 1 / (R sinc th), R = |Pc|.
+    // sin th = rho / R and cos th = Z / R, so no trigonometric function is evaluated besides atan2.
+    // Nothing divides by a small rho: c (series of 1 / sinc near the axis), and q = (1/rho) ds/drho below, stay
+    // finite on the optical axis.
+    const double e1 = sh[4], e2 = sh[5], e3 = sh[6], e4 = sh[7];
+    const double rho2 = P[0] * P[0] + P[1] * P[1];
+    const double R2 = rho2 + P[2] * P[2], iR2 = 1.0 / R2;
+    const double rho = sqrt(rho2);
+    const double th = atan2_t(rho, P[2]);
+    const double t2 = th * th;
+    const double c = t2 < 1e-6 ? 1.0 / (sqrt(R2) * (1.0 - t2 * (1.0 / 6.0) + t2 * t2 * (1.0 / 120.0))) : th / rho;
+    const double f = 1.0 + t2 * (e1 + t2 * (e2 + t2 * (e3 + t2 * e4)));
+    const double s = f * c;
+    const double xd = s * P[0], yd = s * P[1];
+    r0 = fx * xd + cx - pu;
+    r1 = fy * yd + cy - pv;
+    if (!WANT_J) return P[2];
+    {  // intrinsics / distortion: d x' / d k_i = th^(2i) c X; the reserved slot has a zero column
+      const double t4 = t2 * t2, t6 = t4 * t2, t8 = t4 * t4;
+      const double fxc = fx * c * P[0], fyc = fy * c * P[1];
+      const double js0[9] = {xd, 0.0, 1.0, 0.0, fxc * t2, fxc * t4, fxc * t6, fxc * t8, 0.0};
+      sink.shared(0, js0, r0);
+      const double js1[9] = {0.0, yd, 0.0, 1.0, fyc * t2, fyc * t4, fyc * t6, fyc * t8, 0.0};
+      sink.shared(1, js1, r1);
+    }
+    // d th_d / d th = 1 + 3 k1 th^2 + .. + 9 k4 th^8 ;  f'(th) / th = 2 k1 + 4 k2 th^2 + .. + 8 k4 th^6
+    const double fd = 1.0 + t2 * (3.0 * e1 + t2 * (5.0 * e2 + t2 * (7.0 * e3 + t2 * (9.0 * e4))));
+    const double fp = 2.0 * e1 + t2 * (4.0 * e2 + t2 * (6.0 * e3 + t2 * (8.0 * e4)));
+    // dx'/dX = s + X^2 q, dx'/dY = X Y q, dx'/dZ = -X fd / R^2, with q = (fp - fd (th - sin th cos th) / th^3) c^3
+    const double q = (fp - fd * tsc3_d(t2, th, rho * P[2] * iR2)) * (c * c * c);
+    const double gz = -fd * iR2;
+    const double qxy = q * P[0] * P[1];
+    A[0][0] = fx * (s + q * P[0] * P[0]);
+    A[0][1] = fx * qxy;
+    A[0][2] = fx * gz * P[0];
+    A[1][0] = fy * qxy;
+    A[1][1] = fy * (s + q * P[1] * P[1]);
+    A[1][2] = fy * gz * P[1];
   }
-  // d(xd,yd)/d(x,y)
-  const double drad = k1 + 2.0 * k2 * r2 + 3.0 * k3 * r4;  // d rad / d r2
-  const double dxx = rad + 2.0 * xx * drad + 2.0 * p1 * y + 6.0 * p2 * x;
-  const double dxy = 2.0 * xy * drad + 2.0 * p1 * x + 2.0 * p2 * y;
-  const double dyy = rad + 2.0 * yy * drad + 6.0 * p1 * y + 2.0 * p2 * x;
-  // A = d(u,v)/dPc  (2x3)
-  double A[2][3];
-  A[0][0] = fx * dxx * iz;
-  A[0][1] = fx * dxy * iz;
-  A[0][2] = -(A[0][0] * x + A[0][1] * y);
-  A[1][0] = fy * dxy * iz;
-  A[1][1] = fy * dyy * iz;
-  A[1][2] = -(A[1][0] * x + A[1][1] * y);
 
   // J = A [p]x M is formed as (A [p]x) M: 12 + 18 operations instead of 27 + 18
   double jvt[2][3];  // d/d t_view = -A Mt (kept until the rotation part is ready)
@@ -331,10 +394,10 @@ RCC_HD double eval_corner(const BlockGeom<RIG>& g, const double* __restrict__ sh
 }
 
 // eval_corner into a CornerRows (residuals, depth and, with WANT_J, the Jacobian rows)
-template <bool RIG, bool WANT_J>
+template <bool RIG, bool WANT_J, Lens L = LENS_RADTAN>
 RCC_HD void eval_corner(const BlockGeom<RIG>& g, const double* __restrict__ sh, double ox, double oy, double pu,
                         double pv, CornerRows<RIG>& out) {
-  out.depth = eval_corner<RIG, WANT_J>(g, sh, ox, oy, pu, pv, out, out.r[0], out.r[1]);
+  out.depth = eval_corner<RIG, WANT_J, L>(g, sh, ox, oy, pu, pv, out, out.r[0], out.r[1]);
 }
 
 // Robust loss rho(s) on s = ||r_block||^2 (all 8 residuals of a tag), Ceres semantics:

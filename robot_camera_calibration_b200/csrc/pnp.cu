@@ -7,7 +7,7 @@
 // starts from the homography between the tag plane and the undistorted
 // normalised image points and refines with Levenberg-Marquardt; the cost and
 // its analytic Jacobian are the same model.cuh functions the bundle adjustment
-// uses (view = identity, marker = cam_T_tag).
+// uses (view = identity, marker = cam_T_tag), for either lens.
 #include "common.cuh"
 #include "kernels.h"
 #include "model.cuh"
@@ -67,7 +67,7 @@ __device__ void rot_to_rvec(const double* R, double* r) {
 }
 
 // cost and (optionally) J^T J, J^T r of the 8 residuals wrt pose p (rvec,t)
-template <bool WANT_J>
+template <bool WANT_J, Lens L>
 __device__ double pnp_cost(const double* p, const double* sh, double hs, const double* pix, double* H, double* g,
                            bool* ok) {
   double idx[POSEX], px[POSEX];
@@ -86,7 +86,7 @@ __device__ double pnp_cost(const double* p, const double* sh, double hs, const d
     double ox, oy;
     corner_xy(k, hs, ox, oy);
     CornerRows<false> c;
-    eval_corner<false, WANT_J>(geo, sh, ox, oy, pix[2 * k], pix[2 * k + 1], c);
+    eval_corner<false, WANT_J, L>(geo, sh, ox, oy, pix[2 * k], pix[2 * k + 1], c);
     if (!(c.depth > 0.0) || !isfinite(c.r[0]) || !isfinite(c.r[1])) *ok = false;
     cost += c.r[0] * c.r[0] + c.r[1] * c.r[1];
     if (WANT_J) {
@@ -100,6 +100,7 @@ __device__ double pnp_cost(const double* p, const double* sh, double hs, const d
   return 0.5 * cost;
 }
 
+template <Lens L>
 __global__ void __launch_bounds__(128) pnp_kernel(int64_t n, const double* __restrict__ shared9,
                                                   const double* __restrict__ sizes, const double* __restrict__ pixels,
                                                   double* __restrict__ poses, double* __restrict__ final_cost,
@@ -115,18 +116,40 @@ __global__ void __launch_bounds__(128) pnp_kernel(int64_t n, const double* __res
   for (int k = 0; k < 6; ++k) have_guess |= (p[k] != 0.0);
 
   if (!have_guess) {
-    // ---- undistorted normalised image points (fixed-point iteration, like cv::undistortPoints)
+    // ---- undistorted normalised image points
     double xn[4], yn[4];
     for (int k = 0; k < 4; ++k) {
       const double x0 = (pix[2 * k] - sh[2]) / sh[0], y0 = (pix[2 * k + 1] - sh[3]) / sh[1];
       double x = x0, y = y0;
-      for (int it = 0; it < 20; ++it) {
-        const double r2 = x * x + y * y;
-        const double rad = 1.0 + r2 * (sh[4] + r2 * (sh[5] + r2 * sh[8]));
-        const double dx = 2.0 * sh[6] * x * y + sh[7] * (r2 + 2.0 * x * x);
-        const double dy = sh[6] * (r2 + 2.0 * y * y) + 2.0 * sh[7] * x * y;
-        x = (x0 - dx) / rad;
-        y = (y0 - dy) / rad;
+      if (L == LENS_RADTAN) {
+        // fixed-point iteration, like cv::undistortPoints
+        for (int it = 0; it < 20; ++it) {
+          const double r2 = x * x + y * y;
+          const double rad = 1.0 + r2 * (sh[4] + r2 * (sh[5] + r2 * sh[8]));
+          const double dx = 2.0 * sh[6] * x * y + sh[7] * (r2 + 2.0 * x * x);
+          const double dy = sh[6] * (r2 + 2.0 * y * y) + 2.0 * sh[7] * x * y;
+          x = (x0 - dx) / rad;
+          y = (y0 - dy) / rad;
+        }
+      } else {
+        // th_d = |(x0, y0)|: solve th (1 + k1 th^2 + .. + k4 th^8) = th_d for th by Newton's method (as
+        // cv::fisheye::undistortPoints does), then the pinhole point tan(th) along the distorted direction
+        const double thd = sqrt(x0 * x0 + y0 * y0);
+        double th = thd;
+        for (int it = 0; it < 20; ++it) {
+          const double t2 = th * th;
+          const double f = th * (1.0 + t2 * (sh[4] + t2 * (sh[5] + t2 * (sh[6] + t2 * sh[7])))) - thd;
+          const double df = 1.0 + t2 * (3.0 * sh[4] + t2 * (5.0 * sh[5] + t2 * (7.0 * sh[6] + t2 * 9.0 * sh[7])));
+          if (!(fabs(df) > 1e-12)) break;
+          th -= f / df;
+        }
+        // a point at or beyond 90 degrees has no pinhole image: clamp just short of it
+        th = fmin(fmax(th, 0.0), 1.5);
+        if (thd > 1e-300) {
+          const double sc = tan(th) / thd;
+          x = x0 * sc;
+          y = y0 * sc;
+        }
       }
       xn[k] = x; yn[k] = y;
     }
@@ -167,7 +190,7 @@ __global__ void __launch_bounds__(128) pnp_kernel(int64_t n, const double* __res
   // ---- Levenberg-Marquardt on the 8 residuals
   double H[36], g[6];
   bool ok;
-  double cost = pnp_cost<true>(p, sh, hs, pix, H, g, &ok);
+  double cost = pnp_cost<true, L>(p, sh, hs, pix, H, g, &ok);
   double lambda = 1e-3;
   for (int it = 0; it < max_iter; ++it) {
     double A6[6][6], rhs[6];
@@ -181,7 +204,7 @@ __global__ void __launch_bounds__(128) pnp_kernel(int64_t n, const double* __res
     double dn = 0.0, pn = 0.0;
     for (int a = 0; a < 6; ++a) { q[a] = p[a] + rhs[a]; dn += rhs[a] * rhs[a]; pn += p[a] * p[a]; }
     bool ok2;
-    const double c2 = pnp_cost<false>(q, sh, hs, pix, nullptr, nullptr, &ok2);
+    const double c2 = pnp_cost<false, L>(q, sh, hs, pix, nullptr, nullptr, &ok2);
     // Accept on "not worse up to rounding": along the weakly determined depth direction of a small tag the cost is
     // flat to 1e-16 relative while the step is still 1e-8, so convergence is declared on the step alone.
     // Below a relative step of 1e-5 the Gauss-Newton model is exact to rounding while the cost comparison is pure
@@ -189,7 +212,7 @@ __global__ void __launch_bounds__(128) pnp_kernel(int64_t n, const double* __res
     const bool tiny = dn <= 1e-10 * (pn + 1e-10);
     if (ok2 && (tiny || c2 <= cost * (1.0 + 4e-16))) {
       for (int a = 0; a < 6; ++a) p[a] = q[a];
-      cost = pnp_cost<true>(p, sh, hs, pix, H, g, &ok);
+      cost = pnp_cost<true, L>(p, sh, hs, pix, H, g, &ok);
       lambda = fmax(lambda * 0.1, 1e-12);
       if (dn <= 1e-26 * (pn + 1e-26)) break;
     } else {
@@ -203,9 +226,10 @@ __global__ void __launch_bounds__(128) pnp_kernel(int64_t n, const double* __res
 
 }  // namespace rcc
 
-extern "C" int rcc_pnp_batch(int32_t device, int64_t n, const double* shared9, const double* sizes,
-                             const double* pixels, double* cam_T_tag, double* final_cost, int32_t max_iterations) {
+extern "C" int rcc_pnp_batch_lens(int32_t device, int32_t lens, int64_t n, const double* shared9, const double* sizes,
+                                  const double* pixels, double* cam_T_tag, double* final_cost, int32_t max_iterations) {
   using namespace rcc;
+  if (lens != LENS_RADTAN && lens != LENS_EQUIDISTANT) return RCC_BAD_ARG;
   if (n < 0 || !shared9 || (n > 0 && (!sizes || !pixels || !cam_T_tag))) return RCC_BAD_ARG;
   if (n == 0) return RCC_OK;
   try {
@@ -221,8 +245,11 @@ extern "C" int rcc_pnp_batch(int32_t device, int64_t n, const double* shared9, c
     dpx.upload(pixels, (size_t)n * 8, s);
     dpose.upload(cam_T_tag, (size_t)n * 6, s);
     dcost.alloc((size_t)n);
-    pnp_kernel<<<ceil_div(n, 128), 128, 0, s>>>(n, dsh.p, dsz.p, dpx.p, dpose.p, dcost.p,
-                                                  max_iterations > 0 ? max_iterations : 30);
+    const int iters = max_iterations > 0 ? max_iterations : 30;
+    if (lens == LENS_EQUIDISTANT)
+      pnp_kernel<LENS_EQUIDISTANT><<<ceil_div(n, 128), 128, 0, s>>>(n, dsh.p, dsz.p, dpx.p, dpose.p, dcost.p, iters);
+    else
+      pnp_kernel<LENS_RADTAN><<<ceil_div(n, 128), 128, 0, s>>>(n, dsh.p, dsz.p, dpx.p, dpose.p, dcost.p, iters);
     RCC_CUDA(cudaGetLastError());
     dpose.download(cam_T_tag, (size_t)n * 6, s);
     if (final_cost) dcost.download(final_cost, (size_t)n, s);
@@ -233,4 +260,10 @@ extern "C" int rcc_pnp_batch(int32_t device, int64_t n, const double* shared9, c
     return e.status;
   }
   return RCC_OK;
+}
+
+extern "C" int rcc_pnp_batch(int32_t device, int64_t n, const double* shared9, const double* sizes,
+                             const double* pixels, double* cam_T_tag, double* final_cost, int32_t max_iterations) {
+  return rcc_pnp_batch_lens(device, rcc::LENS_RADTAN, n, shared9, sizes, pixels, cam_T_tag, final_cost,
+                            max_iterations);
 }

@@ -504,6 +504,7 @@ static void refresh_constants(P_t* P) {
     const int b = 6 * P->n_f + c * P->sp;
     if (P->c_intr[c]) for (int k = 0; k < 4; ++k) idx.push_back(b + k);
     if (P->c_dist[c]) for (int k = 4; k < 9; ++k) idx.push_back(b + k);
+    else if (P->lens == LENS_EQUIDISTANT) idx.push_back(b + 8);   // the reserved distortion slot
     if (P->rig && P->c_ext[c]) for (int k = 9; k < 15; ++k) idx.push_back(b + k);
   }
   P->n_const = (int)idx.size();
@@ -566,7 +567,7 @@ static void do_linearize(P_t* P) {
         ak.chunks = P->e_chunks.p + c0;
         ak.n_chunks = c1 - c0;
         ak.partials = P->part_e.p + (size_t)c0 * part;
-        launch_assemble(P->rig, true, P->elim_view, ak, P->stream);
+        launch_assemble(P->rig, true, P->elim_view, P->lens, ak, P->stream);
         P->launch_count += 1;
         if (!f_done) continue;
         AssembleArgs af = a;
@@ -577,11 +578,11 @@ static void do_linearize(P_t* P) {
         af.n_chunks = P->f_piece_ptr[k + 1] - P->f_piece_ptr[k];
         af.partials = P->part_f.p;
         af.W = nullptr;
-        launch_assemble(P->rig, false, !P->elim_view, af, P->stream);
+        launch_assemble(P->rig, false, !P->elim_view, P->lens, af, P->stream);
         P->launch_count += 1;
       }
     } else {
-      launch_assemble(P->rig, true, P->elim_view, a, P->stream);
+      launch_assemble(P->rig, true, P->elim_view, P->lens, a, P->stream);
     }
   }
   ensure_pixels(P);
@@ -593,7 +594,7 @@ static void do_linearize(P_t* P) {
     a.n_chunks = P->n_chunks_f;
     a.partials = P->part_f.p;
     a.W = nullptr;
-    launch_assemble(P->rig, false, !P->elim_view, a, P->stream);
+    launch_assemble(P->rig, false, !P->elim_view, P->lens, a, P->stream);
   }
   {
     Scoped t(P, ST_FINALIZE, 1);
@@ -1112,7 +1113,7 @@ static void do_candidate_cost(P_t* P) {
     EvalArgs a = eval_args(P, true);
     a.fail_flag = P->fail_flag.p + 1;   // slot 1: candidate point (slot 0 keeps the linearisation point's flag)
     RCC_CUDA(cudaMemsetAsync(a.fail_flag, 0, sizeof(int32_t), P->stream));
-    launch_cost(P->rig, a, P->stream);
+    launch_cost(P->rig, P->lens, a, P->stream);
     launch_sum(P->cost_partials.p, eval_grid(P->n_obs), P->stats.p + SX_CAND2, 1.0, P->stream);
   }
   if (P->comm) {
@@ -1601,6 +1602,15 @@ int rcc_ba_set_loss(rcc_ba_problem* P, int32_t loss, double scale) {
   API_END(P)
 }
 
+int rcc_ba_set_lens(rcc_ba_problem* P, int32_t lens) {
+  API_BEGIN(P)
+  RCC_REQUIRE(lens == RCC_LENS_RADTAN || lens == RCC_LENS_EQUIDISTANT, RCC_BAD_ARG, "unknown lens");
+  P->lens = lens;
+  P->const_dirty = true;   // the reserved slot of the equidistant lens is held constant
+  P->linearized = P->schur_done = P->step_ready = P->cand_ready = false;
+  API_END(P)
+}
+
 int rcc_ba_get_intrinsics(rcc_ba_problem* P, double* intr, double* dist) {
   API_BEGIN(P)
   std::vector<double> h((size_t)P->n_shared);
@@ -1660,7 +1670,7 @@ static int evaluate_impl(P_t* P, int want_j, double* cost, bool to_host, double*
   RCC_CUDA(cudaMemsetAsync(a.fail_flag, 0, sizeof(int32_t), P->stream));
   {
     Scoped t(P, ST_EVALUATE, 2);
-    launch_evaluate(P->rig, want_j != 0, a, P->stream);
+    launch_evaluate(P->rig, want_j != 0, P->lens, a, P->stream);
     launch_sum(P->cost_partials.p, eval_partials(want_j != 0, a), P->scalar.p, 0.5, P->stream);
   }
   int fail = 0;

@@ -137,6 +137,7 @@ struct rcc_ba_problem {
   int jacobi = 0;                    // Jacobi column scaling of the LM diagonal
   int loss = 0;
   double loss_scale = 1.0;
+  int lens = 0;                      // rcc::Lens of every camera (rcc_ba_set_lens)
   rcc::StageTimer timer;
   rcc::DBuf<double> flush_buf;
 

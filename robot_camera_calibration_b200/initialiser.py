@@ -19,17 +19,22 @@ from . import _lib as L
 from .scenes import Scene, compose, invert
 
 
-def pnp_batch(intr, dist, sizes, pixels, guess=None, device=0, max_iterations=100):
-    """cam_T_tag (n,6) and final cost (n,) for n tags (4 corners each) on the GPU."""
+def pnp_batch(intr, dist, sizes, pixels, guess=None, device=0, max_iterations=100, lens="radtan"):
+    """cam_T_tag (n,6) and final cost (n,) for n tags (4 corners each) on the GPU.  lens "radtan" (dist = k1 k2 p1 p2
+    k3) or "equidistant" (dist = k1 k2 k3 k4); missing trailing coefficients are zero."""
     lib = L.load()
+    if lens not in L.LENSES:
+        raise ValueError(f"unknown lens {lens!r}: expected one of {sorted(L.LENSES)}")
     sizes = np.ascontiguousarray(sizes, np.float64)
     pixels = np.ascontiguousarray(pixels, np.float64).reshape(-1, 8)
     n = len(sizes)
-    sh = np.ascontiguousarray(np.concatenate([np.asarray(intr, float).ravel()[:4], np.asarray(dist, float).ravel()[:5]]))
+    d = np.asarray(dist, float).ravel()[:5]
+    sh = np.ascontiguousarray(np.concatenate([np.asarray(intr, float).ravel()[:4], d, np.zeros(5 - len(d))]))
     poses = np.zeros((n, 6)) if guess is None else np.ascontiguousarray(guess, np.float64).reshape(n, 6).copy()
     cost = np.empty(n)
     dp = lambda a: a.ctypes.data_as(L.c_double_p)
-    rc = lib.rcc_pnp_batch(int(device), n, dp(sh), dp(sizes), dp(pixels), dp(poses), dp(cost), int(max_iterations))
+    rc = lib.rcc_pnp_batch_lens(int(device), L.LENSES[lens], n, dp(sh), dp(sizes), dp(pixels), dp(poses), dp(cost),
+                                int(max_iterations))
     if rc != L.RCC_OK:
         raise L.RccError(rc, "rcc_pnp_batch failed (no CPU fallback)")
     return poses, cost
@@ -86,14 +91,14 @@ def chain_poses(frames, cam_T_tag):
     return ids, sizes, np.array(poses).reshape(-1, 6), w_T_cam
 
 
-def initialise(frames_pixels, intr, dist, device=0):
+def initialise(frames_pixels, intr, dist, device=0, lens="radtan"):
     """frames_pixels: list (per frame) of lists of (tag_id, size, pixels8).
     Returns a Scene holding the initial guesses (frames never referenced are dropped,
     like the reference leaves them without a world_T_camera stanza), the tag ids and
     the frame numbers kept."""
     flat_sizes = [sz for fr in frames_pixels for (_, sz, _) in fr]
     flat_pix = [px for fr in frames_pixels for (_, _, px) in fr]
-    poses, _ = pnp_batch(intr, dist, flat_sizes, np.array(flat_pix).reshape(-1, 8), device=device)
+    poses, _ = pnp_batch(intr, dist, flat_sizes, np.array(flat_pix).reshape(-1, 8), device=device, lens=lens)
     per_frame, o = [], 0
     for fr in frames_pixels:
         per_frame.append(poses[o:o + len(fr)])
@@ -107,7 +112,9 @@ def initialise(frames_pixels, intr, dist, device=0):
         for (t, _, p) in frames_pixels[n]:
             if t in index_of:
                 vi.append(v); mi.append(index_of[t]); px.append(p)
-    scene = Scene(model="single", intr=np.asarray(intr, float).reshape(1, 4), dist=np.asarray(dist, float).reshape(1, 5),
+    d = np.asarray(dist, float).ravel()
+    scene = Scene(model="single", intr=np.asarray(intr, float).reshape(1, 4),
+                  dist=np.concatenate([d, np.zeros(5 - len(d))]).reshape(1, 5), lens=lens,
                   ext=np.zeros((1, 6)), views=np.array([w_T_cam[n] for n in keep]).reshape(-1, 6), markers=w_T_tag,
                   sizes=np.array(sizes, float), view_idx=np.array(vi, np.int32), marker_idx=np.array(mi, np.int32),
                   cam_idx=np.zeros(len(vi), np.int32), pixels=np.array(px, float).reshape(-1, 8))

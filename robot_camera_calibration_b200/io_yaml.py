@@ -4,7 +4,8 @@
                       `world_T_camera:` stanza camera_pose.cpp:95-99 appends
   targets.yaml        camera_pose.cpp:103-129
   camera.yaml         ROS camera_calibration output that `rosparam load` feeds to
-                      camera_pose.cpp:59-64 (/camera_matrix/data, /distortion_coefficients/data)
+                      camera_pose.cpp:59-64 (/camera_matrix/data, /distortion_coefficients/data);
+                      distortion_model plumb_bob (k1 k2 p1 p2 k3) or equidistant / fisheye (k1 k2 k3 k4)
 
 Writers reproduce the reference's `fout <<` statements byte for byte
 (`std::to_string(double)` == "%f", 6 decimals).  `optimise_directory` is the
@@ -72,14 +73,22 @@ def targets_text(tag_ids, sizes, poses, precision=None):
     return "".join(out)
 
 
-def camera_yaml_text(intr, dist, image_size=(640, 480), name="camera"):
+def camera_yaml_text(intr, dist, image_size=(640, 480), name="camera", lens="radtan"):
+    """ROS camera_info YAML: distortion_model plumb_bob with 5 coefficients, or equidistant with k1 k2 k3 k4 (the
+    reserved fifth slot of the library's dist[5] is not written)."""
     fx, fy, cx, cy = (float(v) for v in intr)
-    d = ", ".join(repr(float(v)) for v in dist)
+    if lens not in _LENS_MODEL:
+        raise ValueError(f"unknown lens {lens!r}")
+    coeffs = list(dist)[:4] if lens == "equidistant" else list(dist)
+    d = ", ".join(repr(float(v)) for v in coeffs)
     return (f"image_width: {int(image_size[0])}\nimage_height: {int(image_size[1])}\ncamera_name: {name}\n"
             "camera_matrix:\n  rows: 3\n  cols: 3\n"
             f"  data: [{fx!r}, 0.0, {cx!r}, 0.0, {fy!r}, {cy!r}, 0.0, 0.0, 1.0]\n"
-            "distortion_model: plumb_bob\ndistortion_coefficients:\n  rows: 1\n  cols: 5\n"
+            f"distortion_model: {_LENS_MODEL[lens]}\ndistortion_coefficients:\n  rows: 1\n  cols: {len(coeffs)}\n"
             f"  data: [{d}]\n")
+
+
+_LENS_MODEL = {"radtan": "plumb_bob", "equidistant": "equidistant"}     # library lens -> ROS distortion_model
 
 
 def write_dataset(directory, scene, tag_ids=None, with_poses=True, precision=None):
@@ -110,23 +119,46 @@ def write_dataset(directory, scene, tag_ids=None, with_poses=True, precision=Non
     with open(os.path.join(directory, "targets.yaml"), "w") as f:
         f.write(targets_text(tag_ids, scene.sizes, scene.markers, precision))
     with open(os.path.join(directory, "camera.yaml"), "w") as f:
-        f.write(camera_yaml_text(scene.intr[0], scene.dist[0], scene.image_size))
+        f.write(camera_yaml_text(scene.intr[0], scene.dist[0], scene.image_size, lens=scene.lens))
 
 
 # ------------------------------------------------------------------ readers
-def read_camera_yaml(path):
-    """-> (intr[4], dist[5]) with fx=K[0] fy=K[4] cx=K[2] cy=K[5] (camera_pose.cpp:61-64)."""
+def read_camera(path):
+    """-> (intr[4], dist[5], lens) with fx=K[0] fy=K[4] cx=K[2] cy=K[5] (camera_pose.cpp:61-64).
+    distortion_model equidistant or fisheye (ROS camera_info, Kalibr, cv::fisheye): lens "equidistant", dist =
+    k1 k2 k3 k4 and the reserved slot 0.  Any other model (plumb_bob, or none given): lens "radtan", dist = the first
+    five coefficients k1 k2 p1 p2 k3 (missing trailing ones 0)."""
     with open(path) as f:
         y = yaml.safe_load(f)
     K = [float(v) for v in y["camera_matrix"]["data"]]
-    d = [float(v) for v in y["distortion_coefficients"]["data"]][:5]
+    model = str(y.get("distortion_model", "plumb_bob")).strip().lower()
+    lens = "equidistant" if model in ("equidistant", "fisheye") else "radtan"
+    d = [float(v) for v in y["distortion_coefficients"]["data"]]
+    if lens == "equidistant":
+        if len(d) != 4:
+            raise ValueError(f"{path}: an equidistant camera has 4 distortion coefficients, found {len(d)}")
+    else:
+        d = d[:5]
     d += [0.0] * (5 - len(d))
-    return np.array([K[0], K[4], K[2], K[5]]), np.array(d)
+    return np.array([K[0], K[4], K[2], K[5]]), np.array(d), lens
 
 
-def read_dataset(directory, intr=None, dist=None):
+def read_camera_yaml(path):
+    """-> (intr[4], dist[5]) of a radial-tangential camera (camera_pose.cpp:61-64).  An equidistant (fisheye) file
+    raises ValueError: its k1 k2 k3 k4 are not k1 k2 p1 p2, so read it with read_camera, which returns the lens."""
+    intr, dist, lens = read_camera(path)
+    if lens != "radtan":
+        raise ValueError(f"{path} describes an {lens} lens: read it with io_yaml.read_camera, which returns "
+                         "(intr, dist, lens)")
+    return intr, dist
+
+
+def read_dataset(directory, intr=None, dist=None, lens=None):
     """Read targets.yaml + detections_*.yaml (+ camera.yaml) into a Scene.
-    The intrinsics come from camera.yaml unless `intr` (fx fy cx cy) and `dist` (k1 k2 p1 p2 k3) are given;
+    The intrinsics come from camera.yaml unless `intr` (fx fy cx cy) and `dist` (k1 k2 p1 p2 k3, or k1 k2 k3 k4 with
+    lens="equidistant") are given.  The lens is camera.yaml's distortion_model whenever camera.yaml exists, also with
+    explicit intrinsics, so that a fisheye directory is never optimised as a radial-tangential camera; `lens` overrides
+    it only for explicit intrinsics (with intrinsics from camera.yaml it must agree); "radtan" when there is neither;
     a dataset with neither is an error (the reference logs ROS_ERROR when the intrinsics are not loaded,
     camera_pose.cpp:66-67 -- optimising from made-up intrinsics would silently overwrite good files).
     Frames without a `world_T_camera` stanza (never referenced by
@@ -134,6 +166,8 @@ def read_dataset(directory, intr=None, dist=None):
     are skipped.  Returns (scene, tag_ids, frame_numbers)."""
     with open(os.path.join(directory, "targets.yaml")) as f:
         targets = (yaml.safe_load(f) or {}).get("targets") or []
+    if lens is not None and lens not in _LENS_MODEL:
+        raise ValueError(f"unknown lens {lens!r}: expected one of {sorted(_LENS_MODEL)}")
     if not targets:
         raise ValueError(f"{directory}/targets.yaml lists no targets: nothing defines the world frame "
                          "(camera_pose.cpp:71-80 makes the first tag of frame 0 the world tag)")
@@ -164,16 +198,22 @@ def read_dataset(directory, intr=None, dist=None):
             px.append([c[k][a] for k in range(4) for a in range(2)])
     cam = os.path.join(directory, "camera.yaml")
     if intr is not None and dist is not None:
-        intr, dist = np.asarray(intr, dtype=np.float64), np.asarray(dist, dtype=np.float64)
+        intr, dist = np.asarray(intr, dtype=np.float64), np.asarray(dist, dtype=np.float64).ravel()
+        dist = np.concatenate([dist, np.zeros(5 - len(dist))])
+        if lens is None:
+            lens = read_camera(cam)[2] if os.path.exists(cam) else "radtan"
     elif os.path.exists(cam):
-        intr, dist = read_camera_yaml(cam)
+        intr, dist, cam_lens = read_camera(cam)
+        if lens is not None and lens != cam_lens:
+            raise ValueError(f"{cam} describes an {cam_lens} lens, not {lens}: its coefficients are that model's")
+        lens = cam_lens
     else:
         raise FileNotFoundError(f"{cam} not found and no intr/dist given: the camera intrinsics are required "
                                 "(camera_pose.cpp:59-67)")
     scene = Scene(model="single", intr=intr.reshape(1, 4), dist=dist.reshape(1, 5), ext=np.zeros((1, 6)),
                   views=np.array(views, dtype=np.float64).reshape(-1, 6), markers=markers, sizes=sizes,
                   view_idx=np.array(vi, dtype=np.int32), marker_idx=np.array(mi, dtype=np.int32),
-                  cam_idx=np.zeros(len(vi), dtype=np.int32), pixels=_pixel_array(px))
+                  cam_idx=np.zeros(len(vi), dtype=np.int32), pixels=_pixel_array(px), lens=lens)
     return scene, tag_ids, np.array(frames)
 
 
@@ -204,10 +244,11 @@ def write_results(directory, scene, tag_ids, frames, precision=None):
 
 
 def optimise_directory(directory, device=0, refine_intrinsics=True, precision=None, intr=None, dist=None,
-                       **lm_options):
-    """Milestone 3: detections/ -> GPU bundle adjustment -> detections/ (same formats)."""
+                       lens=None, **lm_options):
+    """Milestone 3: detections/ -> GPU bundle adjustment -> detections/ (same formats).  The lens is camera.yaml's
+    distortion_model (plumb_bob, or equidistant / fisheye), and camera_refined.yaml is written in the same model."""
     from .problem import BAProblem
-    scene, tag_ids, frames = read_dataset(directory, intr=intr, dist=dist)
+    scene, tag_ids, frames = read_dataset(directory, intr=intr, dist=dist, lens=lens)
     scene.const_intr[:] = not refine_intrinsics
     scene.const_dist[:] = not refine_intrinsics
     with BAProblem.from_scene(scene, device=device) as p:
@@ -218,5 +259,5 @@ def optimise_directory(directory, device=0, refine_intrinsics=True, precision=No
     write_results(directory, scene, tag_ids, frames, precision)
     if refine_intrinsics:
         with open(os.path.join(directory, "camera_refined.yaml"), "w") as f:
-            f.write(camera_yaml_text(intr[0], dist[0], scene.image_size))
+            f.write(camera_yaml_text(intr[0], dist[0], scene.image_size, lens=scene.lens))
     return summary

@@ -38,10 +38,12 @@ class BAProblem:
 
     model "single": views are world_T_camera (camera_pose.cpp:88-98);
     model "rig":    views are world_T_body and ext[c] is body_T_cam_c.
+    lens "radtan" (dist = k1 k2 p1 p2 k3) or "equidistant" (dist = k1 k2 k3 k4 + a reserved slot held constant),
+    the same for every camera (rcc_ba_set_lens).
     """
 
     def __init__(self, n_views, n_markers, n_cameras=1, n_obs_blocks=0, model="single", device=0,
-                 eliminate="auto"):
+                 eliminate="auto", lens="radtan"):
         self.lib = L.load()
         self.model = model
         self.n_views, self.n_markers, self.n_cameras = int(n_views), int(n_markers), int(n_cameras)
@@ -58,6 +60,9 @@ class BAProblem:
         d = L.Dims()
         self._check(self.lib.rcc_ba_get_dims(self.h, C.byref(d)))
         self.dims = d
+        self.lens = "radtan"
+        if lens != "radtan":
+            self.set_lens(lens)
 
     # ------------------------------------------------------------------ plumbing
     def _check(self, rc):
@@ -85,7 +90,7 @@ class BAProblem:
     @classmethod
     def from_scene(cls, scene, device=0, eliminate="auto"):
         p = cls(len(scene.views), len(scene.markers), len(scene.intr), scene.n_blocks, scene.model,
-                device=device, eliminate=eliminate)
+                device=device, eliminate=eliminate, lens=scene.lens)
         p.set_intrinsics(scene.intr, scene.dist)
         if scene.model == "rig":
             p.set_rig_extrinsics(scene.ext)
@@ -159,6 +164,13 @@ class BAProblem:
         """loss: 'trivial' | 'huber' | 'cauchy' on each tag's 8-residual block (scale in pixels)."""
         code = {"trivial": 0, "huber": 1, "cauchy": 2}[loss] if isinstance(loss, str) else int(loss)
         self._check(self.lib.rcc_ba_set_loss(self.h, code, float(scale)))
+
+    def set_lens(self, lens):
+        """lens: 'radtan' | 'equidistant' for every camera; invalidates the linearisation like set_loss."""
+        if lens not in L.LENSES:
+            raise ValueError(f"unknown lens {lens!r}: expected one of {sorted(L.LENSES)}")
+        self._check(self.lib.rcc_ba_set_lens(self.h, L.LENSES[lens]))
+        self.lens = lens
 
     # ------------------------------------------------------------------ getters
     def get_intrinsics(self):

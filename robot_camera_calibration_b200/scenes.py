@@ -68,9 +68,9 @@ def obj_points(size):
                      np.stack([s, s, z], -1), np.stack([-s, s, z], -1)], -2)
 
 
-def project(model, intr, dist, ext, view, marker, size):
-    """Pinhole + radial-tangential projection of the 4 tag corners (numpy;
-    used only to synthesise pixels).  Returns (uv (N,4,2), depth (N,4))."""
+def project(model, intr, dist, ext, view, marker, size, lens="radtan"):
+    """Projection of the 4 tag corners through a pinhole + radial-tangential lens or an equidistant fisheye lens
+    (numpy; used only to synthesise pixels).  Returns (uv (N,4,2), depth (N,4))."""
     o = obj_points(size)
     Rm = rodrigues_np(marker[:, 0:3])
     Pw = np.einsum('nij,nkj->nki', Rm, o) + marker[:, None, 3:6]
@@ -80,13 +80,23 @@ def project(model, intr, dist, ext, view, marker, size):
         Rx = rodrigues_np(ext[:, 0:3])
         q = np.einsum('nji,nkj->nki', Rx, q - ext[:, None, 3:6])
     Z = q[..., 2]
-    Zs = np.where(np.abs(Z) < 1e-9, 1e-9, Z)
-    x, y = q[..., 0] / Zs, q[..., 1] / Zs
-    r2 = x * x + y * y
-    k1, k2, p1, p2, k3 = (dist[:, i:i + 1] for i in range(5))
-    rad = 1 + r2 * (k1 + r2 * (k2 + r2 * k3))
-    xd = x * rad + 2 * p1 * x * y + p2 * (r2 + 2 * x * x)
-    yd = y * rad + p1 * (r2 + 2 * y * y) + 2 * p2 * x * y
+    if lens == "equidistant":
+        # th = atan2(rho, Z), th_d = th (1 + k1 th^2 + k2 th^4 + k3 th^6 + k4 th^8), (xd, yd) = th_d (X, Y) / rho
+        rho = np.hypot(q[..., 0], q[..., 1])
+        th = np.arctan2(rho, Z)
+        t2 = th * th
+        k1, k2, k3, k4 = (dist[:, i:i + 1] for i in range(4))
+        thd = th * (1 + t2 * (k1 + t2 * (k2 + t2 * (k3 + t2 * k4))))
+        s = np.where(rho > 1e-12, thd / np.where(rho > 1e-12, rho, 1.0), 1.0 / np.where(Z > 1e-9, Z, 1e-9))
+        xd, yd = s * q[..., 0], s * q[..., 1]
+    else:
+        Zs = np.where(np.abs(Z) < 1e-9, 1e-9, Z)
+        x, y = q[..., 0] / Zs, q[..., 1] / Zs
+        r2 = x * x + y * y
+        k1, k2, p1, p2, k3 = (dist[:, i:i + 1] for i in range(5))
+        rad = 1 + r2 * (k1 + r2 * (k2 + r2 * k3))
+        xd = x * rad + 2 * p1 * x * y + p2 * (r2 + 2 * x * x)
+        yd = y * rad + p1 * (r2 + 2 * y * y) + 2 * p2 * x * y
     u = intr[:, 0:1] * xd + intr[:, 2:3]
     v = intr[:, 1:2] * yd + intr[:, 3:4]
     return np.stack([u, v], -1), Z
@@ -98,7 +108,7 @@ class Scene:
     """Inputs of one bundle-adjustment problem (numpy, host)."""
     model: str                      # "single" | "rig"
     intr: np.ndarray                # (n_cam,4) fx fy cx cy         (initial guess)
-    dist: np.ndarray                # (n_cam,5) k1 k2 p1 p2 k3
+    dist: np.ndarray                # (n_cam,5) k1 k2 p1 p2 k3 | equidistant: k1 k2 k3 k4 + reserved slot
     ext: np.ndarray                 # (n_cam,6) body_T_cam (rig) else zeros
     views: np.ndarray               # (n_views,6) world_T_camera | world_T_body
     markers: np.ndarray             # (n_markers,6) world_T_target
@@ -115,6 +125,7 @@ class Scene:
     truth: dict = field(default_factory=dict)   # ground-truth parameter arrays
     image_size: tuple = (640, 480)
     name: str = ""
+    lens: str = "radtan"            # "radtan" | "equidistant", every camera
 
     def __post_init__(self):
         nv, nm, nc = len(self.views), len(self.markers), len(self.intr)
@@ -157,9 +168,11 @@ def _look_at(cam_pos, target, roll):
     return R @ Rz
 
 
-def _wall_views(rng, n, wall_w, wall_h, d_mean, T0inv):
+def _wall_views(rng, n, wall_w, wall_h, d_mean, T0inv, tilt=0.0):
     """n views looking at random points of the wall from d in [0.7, 1.3] d_mean (tags face -z of the wall
-    frame towards the cameras: wall normal is +z, the camera sits at negative z looking towards +z)."""
+    frame towards the cameras: wall normal is +z, the camera sits at negative z looking towards +z).
+    tilt > 0 then turns each camera about its x and y axes by up to +-tilt rad (wide-angle lenses: the tags
+    land far off the optical axis)."""
     tgt = np.stack([rng.uniform(-0.5, 0.5, n) * wall_w * 0.9,
                     rng.uniform(-0.5, 0.5, n) * wall_h * 0.9,
                     np.zeros(n)], -1)
@@ -169,13 +182,17 @@ def _wall_views(rng, n, wall_w, wall_h, d_mean, T0inv):
                               -dist_cam * np.sqrt(np.maximum(0.2, 1 - (off ** 2).sum(-1)))], -1)
     Rwc = _look_at(cam_pos, tgt, rng.normal(0, 0.2, n))
     views_wall = np.concatenate([rotation_to_rvec(Rwc), cam_pos], -1)
+    if tilt > 0:
+        turn = np.concatenate([rng.uniform(-tilt, tilt, (n, 2)), np.zeros((n, 4))], -1)
+        views_wall = compose(views_wall, turn)
     return compose(np.broadcast_to(T0inv, views_wall.shape), views_wall)
 
 
 def _chunk_observations(rng, v0, views_c, markers_t, sizes, intr_t, dist_t, ext_t, model, n_cam, visibility,
-                        W, Himg, tag_size, dtype_idx):
+                        W, Himg, tag_size, dtype_idx, lens="radtan"):
     """Observation blocks of the views views_c (global view numbers v0, v0+1, ...): every tag whose 4 corners
-    project inside the image with positive depth, thinned at random to the requested visibility."""
+    project inside the image with positive depth (equidistant: less than 85 degrees off the optical axis), thinned
+    at random to the requested visibility."""
     n_markers = len(markers_t)
     nv = len(views_c)
     m_all = np.arange(n_markers)
@@ -189,17 +206,24 @@ def _chunk_observations(rng, v0, views_c, markers_t, sizes, intr_t, dist_t, ext_
             Rx = rodrigues_np(ext_t[c, 0:3])
             pc = (ctr - ext_t[c, 3:6]) @ Rx                                   # Rx^T (p - t_x)
         zc = np.maximum(pc[..., 2], 1e-9)
-        margin = 0.35 * max(W, Himg) + intr_t[c, 0] * tag_size / zc          # distortion + tag extent
-        cand = ((pc[..., 2] > 0.05)
-                & (np.abs(intr_t[c, 0] * pc[..., 0] / zc + intr_t[c, 2] - W / 2) < W / 2 + margin)
-                & (np.abs(intr_t[c, 1] * pc[..., 1] / zc + intr_t[c, 3] - Himg / 2) < Himg / 2 + margin))
+        if lens == "equidistant":
+            cand = (pc[..., 2] > 0.05) & (np.arctan2(np.hypot(pc[..., 0], pc[..., 1]), pc[..., 2]) < np.deg2rad(88))
+        else:
+            margin = 0.35 * max(W, Himg) + intr_t[c, 0] * tag_size / zc          # distortion + tag extent
+            cand = ((pc[..., 2] > 0.05)
+                    & (np.abs(intr_t[c, 0] * pc[..., 0] / zc + intr_t[c, 2] - W / 2) < W / 2 + margin)
+                    & (np.abs(intr_t[c, 1] * pc[..., 1] / zc + intr_t[c, 3] - Himg / 2) < Himg / 2 + margin))
         cv_, cm_ = np.nonzero(cand)
         uv_c, Z_c = project(model, np.broadcast_to(intr_t[c], (len(cv_), 4)),
                             np.broadcast_to(dist_t[c], (len(cv_), 5)),
                             np.broadcast_to(ext_t[c], (len(cv_), 6)),
-                            views_c[cv_], markers_t[cm_], sizes[cm_])
+                            views_c[cv_], markers_t[cm_], sizes[cm_], lens)
         ok_c = ((Z_c > 0.1).all(-1) & (uv_c[..., 0] >= 0).all(-1) & (uv_c[..., 0] < W).all(-1)
                 & (uv_c[..., 1] >= 0).all(-1) & (uv_c[..., 1] < Himg).all(-1))
+        if lens == "equidistant":
+            # the corner itself, not only the tag centre, within 85 degrees of the optical axis
+            Pq = _corners_in_camera(model, ext_t[c], views_c[cv_], markers_t[cm_], sizes[cm_])
+            ok_c &= (np.arctan2(np.hypot(Pq[..., 0], Pq[..., 1]), Pq[..., 2]) < np.deg2rad(85)).all(-1)
         # scatter back to the dense (view, marker) grid the thinning below works on
         vv = np.repeat(np.arange(v0, v0 + nv), n_markers)
         mm = np.tile(m_all, nv)
@@ -226,10 +250,21 @@ def _chunk_observations(rng, v0, views_c, markers_t, sizes, intr_t, dist_t, ext_
     return np.concatenate(vi_l), np.concatenate(mi_l), np.concatenate(ci_l), np.concatenate(px_l)
 
 
+def _corners_in_camera(model, ext, view, marker, size):
+    """(N,4,3) tag corners in the camera frame."""
+    o = obj_points(size)
+    Pw = np.einsum('nij,nkj->nki', rodrigues_np(marker[:, 0:3]), o) + marker[:, None, 3:6]
+    q = np.einsum('nji,nkj->nki', rodrigues_np(view[:, 0:3]), Pw - view[:, None, 3:6])
+    if model == "rig":
+        q = (q - ext[3:6]) @ rodrigues_np(ext[0:3])
+    return q
+
+
 def make_scene(n_markers, n_views, visibility, n_cam=1, model="single", seed=0,
-               tag_size=0.1, pixel_noise=0.3, image_size=(640, 480),
+               tag_size=0.1, pixel_noise=0.3, image_size=None,
                perturb=(0.02, 0.02, 0.01), round_pixels=False, chunk_views=256,
-               name="", dtype_idx=np.int32, view_seed=None, blocked=False, view_range=None, threads=None):
+               name="", dtype_idx=np.int32, view_seed=None, blocked=False, view_range=None, threads=None,
+               lens="radtan"):
     """Generate a synthetic marker scene.
 
     visibility : target fraction of tags seen per view (per camera); the wall
@@ -239,21 +274,34 @@ def make_scene(n_markers, n_views, visibility, n_cam=1, model="single", seed=0,
                  generator seeded (seed, view_seed) while cameras and tags only
                  depend on `seed` -- weak-scaling shards share one tag cloud.
     round_pixels: truncate pixels to int like corner_detections.cpp:53-54.
+    lens       : "radtan" (640 x 480, f ~ 600 px) or "equidistant": a wide-angle fisheye camera (1280 x 1024,
+                 f ~ 330 px, k1..k4, reserved slot 0) whose views are turned by up to +-1.2 rad so that tags are
+                 seen up to 85 degrees off the optical axis.  image_size overrides the default size.
     blocked    : every chunk of `chunk_views` views draws from its own random stream
                  (seed, chunk number): chunks are generated by `threads` host threads, and
                  `view_range=(lo, hi)` (multiples of chunk_views) yields exactly the views lo..hi-1 of the
                  full scene, renumbered from 0 -- the strong-scaling shards of one fixed problem.
                  The default (False) keeps the single sequential stream.
     """
+    if lens not in ("radtan", "equidistant"):
+        raise ValueError(f"unknown lens {lens!r}")
+    fisheye = lens == "equidistant"
+    if image_size is None:
+        image_size = (1280, 1024) if fisheye else (640, 480)
     rng = np.random.default_rng(seed)
     W, Himg = image_size
     # ---- cameras (truth): SURVEY 8(d2)
-    intr_t = np.stack([rng.uniform(550, 650, n_cam), rng.uniform(550, 650, n_cam),
+    f_lo, f_hi = (320, 340) if fisheye else (550, 650)
+    intr_t = np.stack([rng.uniform(f_lo, f_hi, n_cam), rng.uniform(f_lo, f_hi, n_cam),
                        W / 2 + rng.uniform(-10, 10, n_cam),
                        Himg / 2 + rng.uniform(-10, 10, n_cam)], -1)
-    dist_t = np.stack([rng.normal(0, 0.1, n_cam), rng.normal(0, 0.05, n_cam),
-                       rng.normal(0, 2e-3, n_cam), rng.normal(0, 2e-3, n_cam),
-                       rng.normal(0, 0.01, n_cam)], -1)
+    if fisheye:
+        dist_t = np.stack([rng.normal(0, 0.02, n_cam), rng.normal(0, 0.01, n_cam),
+                           rng.normal(0, 2e-3, n_cam), rng.normal(0, 5e-4, n_cam), np.zeros(n_cam)], -1)
+    else:
+        dist_t = np.stack([rng.normal(0, 0.1, n_cam), rng.normal(0, 0.05, n_cam),
+                           rng.normal(0, 2e-3, n_cam), rng.normal(0, 2e-3, n_cam),
+                           rng.normal(0, 0.01, n_cam)], -1)
     ext_t = np.zeros((n_cam, 6))
     if model == "rig":
         # cameras fan out around the body's optical axis
@@ -288,7 +336,8 @@ def make_scene(n_markers, n_views, visibility, n_cam=1, model="single", seed=0,
     markers_t[0] = 0.0
     sizes = np.full(n_markers, tag_size)
     s_r, s_t, s_i = perturb
-    obs_args = (markers_t, sizes, intr_t, dist_t, ext_t, model, n_cam, visibility, W, Himg, tag_size, dtype_idx)
+    obs_args = (markers_t, sizes, intr_t, dist_t, ext_t, model, n_cam, visibility, W, Himg, tag_size, dtype_idx, lens)
+    tilt = 1.2 if fisheye else 0.0
 
     if blocked:
         # ---- one random stream per chunk of views: parallel, and any aligned view range on its own
@@ -301,7 +350,7 @@ def make_scene(n_markers, n_views, visibility, n_cam=1, model="single", seed=0,
         def one(v0):
             r = np.random.default_rng([seed, 104729, v0 // chunk_views] + vs)
             v1 = min(hi, v0 + chunk_views, n_views)
-            vt = _wall_views(r, v1 - v0, wall_w, wall_h, d_mean, T0inv)
+            vt = _wall_views(r, v1 - v0, wall_w, wall_h, d_mean, T0inv, tilt)
             vi, mi, ci, px = _chunk_observations(r, v0 - lo, vt, *obs_args)
             px = px + r.normal(0, pixel_noise, px.shape)
             v0g = vt + np.concatenate([r.normal(0, s_r, (v1 - v0, 3)), r.normal(0, s_t, (v1 - v0, 3))], -1)
@@ -331,7 +380,7 @@ def make_scene(n_markers, n_views, visibility, n_cam=1, model="single", seed=0,
             rng = np.random.default_rng([seed, int(view_seed)])
         else:
             rng_shared = None
-        views_t = _wall_views(rng, n_views, wall_w, wall_h, d_mean, T0inv)
+        views_t = _wall_views(rng, n_views, wall_w, wall_h, d_mean, T0inv, tilt)
         # ---- observations (chunked over views so 10k x 5k scenes stay in memory)
         parts = [_chunk_observations(rng, v0, views_t[v0:min(n_views, v0 + chunk_views)], *obs_args)
                  for v0 in range(0, n_views, chunk_views)]
@@ -349,6 +398,8 @@ def make_scene(n_markers, n_views, visibility, n_cam=1, model="single", seed=0,
     markers0[0] = 0.0
     intr0 = intr_t * (1 + rs.normal(0, s_i, intr_t.shape))
     dist0 = dist_t + rs.normal(0, s_i, dist_t.shape) * 0.1
+    if fisheye:
+        dist0[:, 4] = 0.0                       # the reserved slot
     ext0 = ext_t.copy()
     if model == "rig" and n_cam > 1:
         ext0[1:] += np.concatenate([rs.normal(0, s_r, (n_cam - 1, 3)),
@@ -358,7 +409,7 @@ def make_scene(n_markers, n_views, visibility, n_cam=1, model="single", seed=0,
                  cam_idx=cam_idx, pixels=pixels,
                  truth=dict(intr=intr_t, dist=dist_t, ext=ext_t, views=views_t,
                             markers=markers_t),
-                 image_size=image_size, name=name)
+                 image_size=image_size, name=name, lens=lens)
 
 
 # ---------------------------------------------------------------- the BASELINE.json configs
