@@ -22,7 +22,7 @@
  * Parameter blocks (FP64), conventions cited to camera_pose.cpp:
  *   intr[4] = fx fy cx cy   (K[0] K[4] K[2] K[5], :61-62)
  *   dist[5] = k1 k2 p1 p2 k3 (:39,63-64)        [radial-tangential lens, the default]
- *           = k1 k2 k3 k4 -                       [equidistant lens, rcc_ba_set_lens]
+ *           = k1 k2 k3 k4 -                       [equidistant lens, rcc_ba_set_lens / rcc_ba_set_camera_lenses]
  *   view[6] = Rodrigues rvec, t of world_T_camera (:88-98)   [rig: world_T_body]
  *   marker[6] = rvec, t of world_T_target (:111-121)
  *   ext[6]  = rvec, t of body_T_cam   (rig model only; not in the reference)
@@ -55,7 +55,7 @@ enum rcc_model { RCC_MODEL_SINGLE = 0, RCC_MODEL_RIG = 1 };
 enum rcc_eliminate { RCC_ELIM_AUTO = 0, RCC_ELIM_VIEWS = 1, RCC_ELIM_MARKERS = 2 };
 enum rcc_loss { RCC_LOSS_TRIVIAL = 0, RCC_LOSS_HUBER = 1, RCC_LOSS_CAUCHY = 2 };
 enum rcc_block_kind { RCC_BLOCK_VIEW = 0, RCC_BLOCK_MARKER = 1, RCC_BLOCK_INTR = 2, RCC_BLOCK_DIST = 3, RCC_BLOCK_EXT = 4 };
-/* Lens model of every camera of a handle.  For the corner Pc = (X, Y, Z) in the camera frame:
+/* Lens model of a camera; each camera of a handle has its own (rcc_ba_set_camera_lenses).  For the corner Pc = (X, Y, Z) in the camera frame:
  *   RCC_LENS_RADTAN       pinhole + radial-tangential (cv::projectPoints): x = X/Z, y = Y/Z, r2 = x^2 + y^2,
  *                         x' = x (1 + k1 r2 + k2 r2^2 + k3 r2^3) + 2 p1 x y + p2 (r2 + 2 x^2), y' likewise
  *   RCC_LENS_EQUIDISTANT  equidistant fisheye, Kannala-Brandt with 4 coefficients (cv::fisheye with skew 0, ROS
@@ -65,7 +65,8 @@ enum rcc_block_kind { RCC_BLOCK_VIEW = 0, RCC_BLOCK_MARKER = 1, RCC_BLOCK_INTR =
  * then u = fx x' + cx, v = fy y' + cy for both.  Under the equidistant lens dist[5] = k1 k2 k3 k4 and a reserved
  * slot 4: the projection ignores it, its jac_dist column is exactly 0, the library always holds it constant (whatever
  * rcc_ba_set_constant says), so its step and its covariance rows and columns are exactly 0 and
- * rcc_ba_get_intrinsics returns it as it was set.  A corner with Z <= 0 fails the evaluation (RCC_EVAL_FAILED) under
+ * rcc_ba_get_intrinsics returns it as it was set.  This holds camera by camera: the slot 4 (k3) of a
+ * radial-tangential camera stays free in a handle whose other cameras are equidistant.  A corner with Z <= 0 fails the evaluation (RCC_EVAL_FAILED) under
  * either lens: the equidistant field of view is below 180 degrees. */
 enum rcc_lens { RCC_LENS_RADTAN = 0, RCC_LENS_EQUIDISTANT = 1 };
 
@@ -156,6 +157,12 @@ int rcc_ba_set_loss(rcc_ba_problem* p, int32_t loss, double scale);
 /* lens model of every camera (rcc_lens; default RCC_LENS_RADTAN).  May be called at any time; like rcc_ba_set_loss it
  * invalidates the linearisation.  RCC_BAD_ARG for an unknown lens. */
 int rcc_ba_set_lens(rcc_ba_problem* p, int32_t lens);
+/* lens model of each camera: lenses[n_cameras] (rcc_lens), for both models, so that one rig can mix pinhole and
+ * fisheye cameras and still share its body poses and markers.  The whole array is checked first: RCC_BAD_ARG for a
+ * NULL handle or array or an unknown lens, and then nothing changes.  Otherwise like rcc_ba_set_lens: may be called at
+ * any time and invalidates the linearisation; whichever of the two calls came last sets the lenses.  With a
+ * communicator attached (rcc_ba_comm_init) every rank must set the same lenses. */
+int rcc_ba_set_camera_lenses(rcc_ba_problem* p, const int32_t* lenses);
 
 int rcc_ba_get_intrinsics(rcc_ba_problem* p, double* intr, double* dist);
 int rcc_ba_get_rig_extrinsics(rcc_ba_problem* p, double* ext);
@@ -166,7 +173,7 @@ int rcc_ba_get_marker_poses(rcc_ba_problem* p, double* markers);
  * Outputs are in the caller's observation order.  Any pointer may be NULL.
  *   residuals   : n_obs_blocks x 8
  *   jac_intr    : n_obs_blocks x 8 x 4   row-major per block  (= jacobians[0])
- *   jac_dist    : n_obs_blocks x 8 x 5                        (= jacobians[1]; column 4 is 0 under the equidistant lens)
+ *   jac_dist    : n_obs_blocks x 8 x 5                        (= jacobians[1]; column 4 is 0 for an equidistant camera)
  *   jac_view    : n_obs_blocks x 8 x 6                        (= jacobians[2])
  *   jac_marker  : n_obs_blocks x 8 x 6                        (= jacobians[3])
  *   jac_ext     : n_obs_blocks x 8 x 6   (rig only)           (= jacobians[4])

@@ -172,16 +172,12 @@ class Problem:
         if not self._blocks:
             raise ValueError("problem has no residual blocks")
         rig = self._blocks[0][0].rig
-        lens = self._blocks[0][0].lens
-        views, markers, cams = {}, {}, {}
+        views, markers, cams, lenses = {}, {}, {}, {}
         vi, mi, ci, px, sizes = [], [], [], [], {}
         seen = {}     # id(array) -> camera key: one Ceres parameter block must belong to exactly one GPU camera
         for cost, intr, dist, view, marker, ext in self._blocks:
             if cost.rig != rig:
                 raise NotImplementedError("rig and single-camera cost functions cannot be mixed in one problem")
-            if cost.lens != lens:
-                raise NotImplementedError("cost functions of different lenses cannot be mixed in one problem: the "
-                                          "lens applies to every camera of the GPU problem")
             v = views.setdefault(id(view), (len(views), view))[0]
             m = markers.setdefault(id(marker), (len(markers), marker))[0]
             key = (id(intr), id(dist), id(ext) if ext is not None else 0)
@@ -192,6 +188,8 @@ class Problem:
                         "camera blocks differ: the GPU camera record is (intr, dist, ext) as a unit, so the shared "
                         "array would be optimised as several independent copies")
             c = cams.setdefault(key, (len(cams), intr, dist, ext))[0]
+            if lenses.setdefault(c, cost.lens) != cost.lens:
+                raise ValueError("one camera (intr, dist, ext) is used by cost functions of different lenses")
             if sizes.setdefault(m, cost.tag_size) != cost.tag_size:
                 raise ValueError("one marker was given two different tag sizes")
             vi.append(v); mi.append(m); ci.append(c); px.append(cost.pixels)
@@ -199,7 +197,7 @@ class Problem:
         mlist = [a for _, a in sorted(markers.values(), key=lambda t: t[0])]
         clist = sorted(cams.values(), key=lambda t: t[0])
         gp = BAProblem(len(vlist), len(mlist), len(clist), len(vi), model="rig" if rig else "single",
-                       device=self.device, eliminate=self.eliminate, lens=lens)
+                       device=self.device, eliminate=self.eliminate, lens=[lenses[c] for c in range(len(clist))])
         gp.set_intrinsics(np.stack([c[1] for c in clist]), np.stack([c[2] for c in clist]))
         if rig:
             gp.set_rig_extrinsics(np.stack([c[3] for c in clist]))

@@ -112,7 +112,16 @@ __global__ void __launch_bounds__(EVAL_THREADS, EVAL_CTAS_PER_SM) evaluate_kerne
       double ox, oy;
       corner_xy(t, mx[PX_HS], ox, oy);
       CornerRows<RIG> c;
-      eval_corner<RIG, false, L>(geo, a.shared + (size_t)cur.cam * SP, ox, oy, cur.px.x, cur.px.y, c);
+      const double* sh = a.shared + (size_t)cur.cam * SP;
+      if constexpr (L == LENS_PER_CAMERA) {
+        // the 4 corner lanes of a block share its camera: a warp takes at most both branches
+        if ((a.cam_equidistant >> cur.cam) & 1u)
+          eval_corner<RIG, false, LENS_EQUIDISTANT>(geo, sh, ox, oy, cur.px.x, cur.px.y, c);
+        else
+          eval_corner<RIG, false, LENS_RADTAN>(geo, sh, ox, oy, cur.px.x, cur.px.y, c);
+      } else {
+        eval_corner<RIG, false, L>(geo, sh, ox, oy, cur.px.x, cur.px.y, c);
+      }
       if (!(c.depth > 0.0) || !isfinite(c.r[0]) || !isfinite(c.r[1])) *a.fail_flag = 1;
       r2 = c.r[0] * c.r[0] + c.r[1] * c.r[1];
       if (a.residuals)
@@ -293,7 +302,11 @@ static void launch_evaluate_l(bool rig, bool want_jac, const EvalArgs& a, cudaSt
 
 void launch_evaluate(bool rig, bool want_jac, int lens, const EvalArgs& a, cudaStream_t s) {
   if (a.n == 0) return;
-  if (lens == LENS_EQUIDISTANT) launch_evaluate_l<LENS_EQUIDISTANT>(rig, want_jac, a, s);
+  if (lens == LENS_PER_CAMERA) {
+    if (want_jac) throw Error(RCC_BAD_ARG, "K1 takes one lens per launch");
+    if (rig) launch_evaluate_t<true, LENS_PER_CAMERA>(a, s);
+    else launch_evaluate_t<false, LENS_PER_CAMERA>(a, s);
+  } else if (lens == LENS_EQUIDISTANT) launch_evaluate_l<LENS_EQUIDISTANT>(rig, want_jac, a, s);
   else launch_evaluate_l<LENS_RADTAN>(rig, want_jac, a, s);
 }
 

@@ -73,8 +73,10 @@ struct AssembleArgs {
 };
 
 // K2: fused residual + Jacobian + J^T J tiles.  own_is_view tells which pose
-// table the segment owner indexes; lens is a Lens (model.cuh).  Under the equidistant lens tile B holds
-// [cx cy k1 k2 k3 k4 0 | r]: the reserved slot's column is zero.
+// table the segment owner indexes; lens is a Lens (model.cuh) other than LENS_PER_CAMERA: with mixed lenses the
+// caller launches once per lens, each launch covering that lens's chunks through chunk_list.  Under the equidistant
+// lens tile B holds [cx cy k1 k2 k3 k4 0 | r]: the reserved slot's column is zero.
+constexpr int N_LENSES = 2;   // LENS_RADTAN, LENS_EQUIDISTANT
 void launch_assemble(bool rig, bool epass, bool own_is_view, int lens, const AssembleArgs& a, cudaStream_t s);
 // the equidistant instantiations (assemble_equidistant.cu)
 void launch_assemble_equidistant(bool rig, bool epass, bool own_is_view, const AssembleArgs& a, cudaStream_t s);
@@ -152,8 +154,11 @@ struct EvalArgs {
   int32_t n_chunks;
   const int32_t* oth;       // [n] other 6-dof block of each sorted block (own block comes from the chunk)
   int32_t own_is_view;
+  uint32_t cam_equidistant; // lens LENS_PER_CAMERA: bit c set = camera c has the equidistant lens
 };
 int eval_grid(int64_t n);   // CTAs launch_evaluate / launch_cost will use
+// lens is a Lens; LENS_PER_CAMERA only without Jacobians (K6).  K1 takes one lens per launch: with mixed lenses the
+// caller launches it once per lens over that lens's chunks.
 void launch_evaluate(bool rig, bool want_jac, int lens, const EvalArgs& a, cudaStream_t s);
 // number of cost partials launch_evaluate writes (want_jac: one per chunk; else one per CTA)
 int eval_partials(bool want_jac, const EvalArgs& a);

@@ -31,11 +31,13 @@ constexpr int PX_R = 0, PX_JR = 9, PX_T = 18;
 constexpr int PX_RJ = PX_JR;   // marker records
 constexpr int PX_HS = 21;  // marker records: half tag size (filled by expand_poses_kernel)
 
-// Lens model of a camera (the same for every camera of a problem):
+// Lens model of a camera (each camera of a problem has its own):
 //   LENS_RADTAN       pinhole + radial-tangential, dist = k1 k2 p1 p2 k3 (cv::projectPoints)
 //   LENS_EQUIDISTANT  equidistant fisheye (Kannala-Brandt), dist = k1 k2 k3 k4 + one reserved slot that the
 //                     projection ignores (cv::fisheye::projectPoints with skew 0)
-enum Lens : int { LENS_RADTAN = 0, LENS_EQUIDISTANT = 1 };
+//   LENS_PER_CAMERA   not a lens: the cost-only kernel K6 picks one of the two per observation block from its
+//                     camera (EvalArgs::cam_equidistant); eval_corner never takes it
+enum Lens : int { LENS_RADTAN = 0, LENS_EQUIDISTANT = 1, LENS_PER_CAMERA = 2 };
 
 // sin(t)/t, accurate for all t >= 0
 RCC_HD double sinc_d(double t2, double t) {
@@ -257,6 +259,7 @@ struct CornerRows {
 template <bool RIG, bool WANT_J, Lens L = LENS_RADTAN, class Sink>
 RCC_HD double eval_corner(const BlockGeom<RIG>& g, const double* __restrict__ sh, double ox, double oy, double pu,
                           double pv, Sink& sink, double& r0, double& r1) {
+  static_assert(L == LENS_RADTAN || L == LENS_EQUIDISTANT, "eval_corner takes one lens");
   const double fx = sh[0], fy = sh[1], cx = sh[2], cy = sh[3];
   const double k1 = sh[4], k2 = sh[5], p1 = sh[6], p2 = sh[7], k3 = sh[8];
   double d[3], P[3];

@@ -237,6 +237,48 @@ static int env_int(const char* name, int dflt) {
   return (v && *v) ? atoi(v) : dflt;
 }
 
+// the per-lens chunk lists of a handle whose cameras mix lenses (problem.h: lens_chunks_e ...), from the chunk
+// records and the cameras' lenses; nothing to do when every camera has the same lens
+static void build_lens_lists(P_t* P) {
+  if (!P->lens_mixed || !P->have_obs) return;
+  cudaStream_t s = P->stream;
+  auto by_lens = [&](const std::vector<Chunk>& chunks, std::vector<int32_t>& list, int* ptr) {
+    list.clear();
+    for (int l = 0; l < N_LENSES; ++l) {
+      ptr[l] = (int)list.size();
+      for (size_t c = 0; c < chunks.size(); ++c)
+        if (P->cam_lens[chunks[c].cam] == l) list.push_back((int32_t)c);
+    }
+    ptr[N_LENSES] = (int)list.size();
+  };
+  std::vector<int32_t> le, lf, fp;
+  by_lens(P->e_chunks_h, le, P->lens_ptr_e);
+  by_lens(P->f_chunks_h, lf, P->lens_ptr_f);
+  std::vector<Chunk> recs(le.size());
+  for (size_t i = 0; i < le.size(); ++i) recs[i] = P->e_chunks_h[le[i]];
+  // E piece k is the chunk range [piece_chunk[k], piece_chunk[k+1]): its part of each ascending lens list
+  for (int l = 0; l < N_LENSES; ++l)
+    for (int k = 0; k <= rcc_ba_problem::PIX_PIECES; ++k)
+      P->lens_piece_e[l][k] = (int)(std::lower_bound(le.begin() + P->lens_ptr_e[l], le.begin() + P->lens_ptr_e[l + 1],
+                                                     P->piece_chunk[k]) - le.begin());
+  // F piece k is f_piece_list[f_piece_ptr[k] .. f_piece_ptr[k+1]): regrouped by lens
+  for (int k = 0; k < rcc_ba_problem::PIX_PIECES; ++k)
+    for (int l = 0; l < N_LENSES; ++l) {
+      P->f_piece_lens_ptr[k * N_LENSES + l] = (int)fp.size();
+      for (int i = P->f_piece_ptr[k]; i < P->f_piece_ptr[k + 1]; ++i)
+        if (P->cam_lens[P->f_chunks_h[P->f_piece_list_h[i]].cam] == l) fp.push_back(P->f_piece_list_h[i]);
+    }
+  P->f_piece_lens_ptr[rcc_ba_problem::PIX_PIECES * N_LENSES] = (int)fp.size();
+  for (auto* v : {&le, &lf, &fp})
+    if (v->empty()) v->push_back(0);
+  if (recs.empty()) recs.push_back(Chunk{0, 0, 0, 0});
+  P->lens_chunks_e.upload(le, s);
+  P->lens_chunks_f.upload(lf, s);
+  P->f_piece_lens.upload(fp, s);
+  P->lens_recs_e.upload(recs, s);
+  RCC_CUDA(cudaStreamSynchronize(s));
+}
+
 static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker_idx, const int32_t* cam_idx) {
   const int64_t n = P->n_obs;
   RCC_REQUIRE(n < (int64_t)2000000000 / 36 * 8, RCC_BAD_ARG, "too many observation blocks for 32-bit indexing");
@@ -267,6 +309,7 @@ static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker
   make_chunks(perm_e, seg_e, cam_idx, P->n_e, bpw, ch_max, chunks, chunk_ptr);
   P->n_chunks_e = (int)chunks.size();
   P->e_chunks.upload(chunks, s);
+  P->e_chunks_h = chunks;
   P->e_chunk_ptr.upload(chunk_ptr, s);
   cam_lists(chunks, P->n_cam, list, ptr);
   P->cam_chunks_e.upload(list, s);
@@ -335,11 +378,13 @@ static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker
           if (group[chunks[c].start] == k) plist.push_back((int32_t)c);
     }
     P->f_piece_ptr[rcc_ba_problem::PIX_PIECES] = (int)plist.size();
+    P->f_piece_list_h = plist;
     if (plist.empty()) plist.push_back(0);
     P->f_piece_list.upload(plist, s);
   }
   P->n_chunks_f = (int)chunks.size();
   P->f_chunks.upload(chunks, s);
+  P->f_chunks_h = chunks;
   P->f_chunk_ptr.upload(chunk_ptr, s);
   cam_lists(chunks, P->n_cam, list, ptr);
   P->cam_chunks_f.upload(list, s);
@@ -489,6 +534,7 @@ static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker
   RCC_CUDA(cudaStreamSynchronize(s));
   P->have_obs = true;
   P->linearized = P->schur_done = P->step_ready = P->cand_ready = false;
+  build_lens_lists(P);
 }
 
 static void refresh_constants(P_t* P) {
@@ -504,7 +550,7 @@ static void refresh_constants(P_t* P) {
     const int b = 6 * P->n_f + c * P->sp;
     if (P->c_intr[c]) for (int k = 0; k < 4; ++k) idx.push_back(b + k);
     if (P->c_dist[c]) for (int k = 4; k < 9; ++k) idx.push_back(b + k);
-    else if (P->lens == LENS_EQUIDISTANT) idx.push_back(b + 8);   // the reserved distortion slot
+    else if (P->cam_lens[c] == LENS_EQUIDISTANT) idx.push_back(b + 8);   // the reserved distortion slot
     if (P->rig && P->c_ext[c]) for (int k = 9; k < 15; ++k) idx.push_back(b + k);
   }
   P->n_const = (int)idx.size();
@@ -532,12 +578,28 @@ static void ensure_pixels(P_t* P) {
   P->pix_pending = false;
 }
 
+// K2 over the chunks of a handle whose cameras mix lenses: one launch per lens l, covering list[lo[l] .. hi[l]).
+// a.chunks and a.partials are the whole pass's (the list holds chunk ids).  Returns the launches issued.
+static int assemble_by_lens(P_t* P, bool epass, AssembleArgs a, const int32_t* list, const int* lo, const int* hi) {
+  int n = 0;
+  for (int l = 0; l < N_LENSES; ++l) {
+    if (hi[l] <= lo[l]) continue;
+    a.chunk_list = list + lo[l];
+    a.n_chunks = hi[l] - lo[l];
+    launch_assemble(P->rig, epass, epass ? P->elim_view : !P->elim_view, l, a, P->stream);
+    ++n;
+  }
+  return n;
+}
+
 static void do_linearize(P_t* P) {
   RCC_REQUIRE(P->have_obs, RCC_NOT_READY, "set_observations has not been called");
   ensure_expanded(P);
   RCC_CUDA(cudaMemsetAsync(P->fail_flag.p, 0, sizeof(int32_t), P->stream));
   AssembleArgs a{};
   bool f_done = false;
+  const int* lp_e = P->lens_ptr_e;
+  const int* lp_f = P->lens_ptr_f;
   a.view_x = P->view_x.p;
   a.marker_x = P->marker_x.p;
   a.ext_x = P->ext_x.p;
@@ -563,6 +625,21 @@ static void do_linearize(P_t* P) {
         const int c0 = P->piece_chunk[k], c1 = P->piece_chunk[k + 1];
         RCC_CUDA(cudaStreamWaitEvent(P->stream, P->ev_piece[k], 0));
         if (c1 <= c0) continue;
+        if (P->lens_mixed) {
+          const int lo[N_LENSES] = {P->lens_piece_e[0][k], P->lens_piece_e[1][k]};
+          const int hi[N_LENSES] = {P->lens_piece_e[0][k + 1], P->lens_piece_e[1][k + 1]};
+          P->launch_count += assemble_by_lens(P, true, a, P->lens_chunks_e.p, lo, hi);
+          if (!f_done) continue;
+          AssembleArgs af = a;
+          af.oth = P->f_oth.p;
+          af.pix = P->f_pix.p;
+          af.chunks = P->f_chunks.p;
+          af.partials = P->part_f.p;
+          af.W = nullptr;
+          const int* fp = P->f_piece_lens_ptr + k * N_LENSES;
+          P->launch_count += assemble_by_lens(P, false, af, P->f_piece_lens.p, fp, fp + 1);
+          continue;
+        }
         AssembleArgs ak = a;
         ak.chunks = P->e_chunks.p + c0;
         ak.n_chunks = c1 - c0;
@@ -581,6 +658,8 @@ static void do_linearize(P_t* P) {
         launch_assemble(P->rig, false, !P->elim_view, P->lens, af, P->stream);
         P->launch_count += 1;
       }
+    } else if (P->lens_mixed) {
+      P->launch_count += assemble_by_lens(P, true, a, P->lens_chunks_e.p, lp_e, lp_e + 1) - 1;
     } else {
       launch_assemble(P->rig, true, P->elim_view, P->lens, a, P->stream);
     }
@@ -594,7 +673,8 @@ static void do_linearize(P_t* P) {
     a.n_chunks = P->n_chunks_f;
     a.partials = P->part_f.p;
     a.W = nullptr;
-    launch_assemble(P->rig, false, !P->elim_view, P->lens, a, P->stream);
+    if (P->lens_mixed) P->launch_count += assemble_by_lens(P, false, a, P->lens_chunks_f.p, lp_f, lp_f + 1) - 1;
+    else launch_assemble(P->rig, false, !P->elim_view, P->lens, a, P->stream);
   }
   {
     Scoped t(P, ST_FINALIZE, 1);
@@ -1097,8 +1177,12 @@ static EvalArgs eval_args(P_t* P, bool cand) {
   a.fail_flag = P->fail_flag.p;
   a.loss = P->loss;
   a.loss_a2 = P->loss_scale * P->loss_scale;
+  a.cam_equidistant = P->cam_equidistant;
   return a;
 }
+
+// the lens argument of launch_evaluate / launch_cost without Jacobians (K6 picks the lens per block when mixed)
+static int cost_lens(const P_t* P) { return P->lens_mixed ? LENS_PER_CAMERA : P->lens; }
 
 static void do_candidate_cost(P_t* P) {
   RCC_REQUIRE(P->step_ready, RCC_NOT_READY, "solve_step has not been called");
@@ -1113,7 +1197,7 @@ static void do_candidate_cost(P_t* P) {
     EvalArgs a = eval_args(P, true);
     a.fail_flag = P->fail_flag.p + 1;   // slot 1: candidate point (slot 0 keeps the linearisation point's flag)
     RCC_CUDA(cudaMemsetAsync(a.fail_flag, 0, sizeof(int32_t), P->stream));
-    launch_cost(P->rig, P->lens, a, P->stream);
+    launch_cost(P->rig, cost_lens(P), a, P->stream);
     launch_sum(P->cost_partials.p, eval_grid(P->n_obs), P->stats.p + SX_CAND2, 1.0, P->stream);
   }
   if (P->comm) {
@@ -1419,6 +1503,7 @@ int rcc_ba_create(const rcc_ba_options* opt, rcc_ba_problem** out) {
     P->ext_x.alloc((size_t)P->n_cam * POSEX); P->ext_xc.alloc((size_t)P->n_cam * POSEX);
     P->c_view.assign(P->n_views, 0); P->c_marker.assign(P->n_markers, 0);
     P->c_intr.assign(P->n_cam, 0); P->c_dist.assign(P->n_cam, 0); P->c_ext.assign(P->n_cam, 0);
+    P->cam_lens.assign(P->n_cam, LENS_RADTAN);
     P->Hee.alloc((size_t)P->n_e * 36); P->ge.alloc((size_t)P->n_e * 6); P->Hes.alloc((size_t)P->n_e * 6 * P->n_shared);
     P->Hff.alloc((size_t)P->n_f * 36); P->gf.alloc((size_t)P->n_f * 6); P->Hfs.alloc((size_t)P->n_f * 6 * P->n_shared);
     P->fin_scratch.alloc((size_t)P->n_cam * P->fin_slices * PassGeom<true>::PART_E);
@@ -1602,12 +1687,34 @@ int rcc_ba_set_loss(rcc_ba_problem* P, int32_t loss, double scale) {
   API_END(P)
 }
 
+// every check first: a refused call changes nothing
+static void set_camera_lenses(P_t* P, const int32_t* lenses) {
+  RCC_REQUIRE(lenses, RCC_BAD_ARG, "null pointer");
+  for (int c = 0; c < P->n_cam; ++c)
+    RCC_REQUIRE(lenses[c] == RCC_LENS_RADTAN || lenses[c] == RCC_LENS_EQUIDISTANT, RCC_BAD_ARG, "unknown lens");
+  P->cam_lens.assign(lenses, lenses + P->n_cam);
+  P->lens = lenses[0];
+  P->lens_mixed = false;
+  P->cam_equidistant = 0;
+  for (int c = 0; c < P->n_cam; ++c) {
+    P->lens_mixed |= lenses[c] != lenses[0];
+    if (lenses[c] == RCC_LENS_EQUIDISTANT) P->cam_equidistant |= 1u << c;
+  }
+  build_lens_lists(P);
+  P->const_dirty = true;   // the reserved slot of an equidistant camera is held constant
+  P->linearized = P->schur_done = P->step_ready = P->cand_ready = false;
+}
+
 int rcc_ba_set_lens(rcc_ba_problem* P, int32_t lens) {
   API_BEGIN(P)
   RCC_REQUIRE(lens == RCC_LENS_RADTAN || lens == RCC_LENS_EQUIDISTANT, RCC_BAD_ARG, "unknown lens");
-  P->lens = lens;
-  P->const_dirty = true;   // the reserved slot of the equidistant lens is held constant
-  P->linearized = P->schur_done = P->step_ready = P->cand_ready = false;
+  set_camera_lenses(P, std::vector<int32_t>((size_t)P->n_cam, lens).data());
+  API_END(P)
+}
+
+int rcc_ba_set_camera_lenses(rcc_ba_problem* P, const int32_t* lenses) {
+  API_BEGIN(P)
+  set_camera_lenses(P, lenses);
   API_END(P)
 }
 
@@ -1670,7 +1777,24 @@ static int evaluate_impl(P_t* P, int want_j, double* cost, bool to_host, double*
   RCC_CUDA(cudaMemsetAsync(a.fail_flag, 0, sizeof(int32_t), P->stream));
   {
     Scoped t(P, ST_EVALUATE, 2);
-    launch_evaluate(P->rig, want_j != 0, P->lens, a, P->stream);
+    if (P->lens_mixed && want_j) {
+      // K1 once per lens over a lens-major copy of the E chunk records; outputs go to caller positions and the cost
+      // partials stay one per chunk, so the launches are independent
+      int n = 0;
+      for (int l = 0; l < N_LENSES; ++l) {
+        const int c0 = P->lens_ptr_e[l], c1 = P->lens_ptr_e[l + 1];
+        if (c1 <= c0) continue;
+        EvalArgs b = a;
+        b.chunks = P->lens_recs_e.p + c0;
+        b.n_chunks = c1 - c0;
+        b.cost2_partials = a.cost2_partials + c0;
+        launch_evaluate(P->rig, true, l, b, P->stream);
+        ++n;
+      }
+      P->launch_count += n - 1;
+    } else {
+      launch_evaluate(P->rig, want_j != 0, want_j ? P->lens : cost_lens(P), a, P->stream);
+    }
     launch_sum(P->cost_partials.p, eval_partials(want_j != 0, a), P->scalar.p, 0.5, P->stream);
   }
   int fail = 0;

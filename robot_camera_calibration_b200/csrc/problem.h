@@ -137,7 +137,23 @@ struct rcc_ba_problem {
   int jacobi = 0;                    // Jacobi column scaling of the LM diagonal
   int loss = 0;
   double loss_scale = 1.0;
-  int lens = 0;                      // rcc::Lens of every camera (rcc_ba_set_lens)
+  // lenses (rcc_ba_set_lens, rcc_ba_set_camera_lenses).  With a communicator attached every rank sets the same lenses;
+  // nothing in the multi-rank path depends on them.
+  std::vector<int32_t> cam_lens;     // rcc::Lens of each camera
+  bool lens_mixed = false;           // the cameras do not all have the same lens
+  int lens = 0;                      // !lens_mixed: the lens of every camera
+  uint32_t cam_equidistant = 0;      // bit c: camera c is equidistant (K6 under LENS_PER_CAMERA)
+  // lens_mixed: K2 and K1 run once per lens.  lens_chunks_e/f hold the chunk ids of lens l in ascending order at
+  // [lens_ptr_e/f[l], lens_ptr_e/f[l+1]); lens_recs_e the E chunk records in that order (K1's chunk array).  Upload
+  // piece k of E covers positions [lens_piece_e[l][k], lens_piece_e[l][k+1]) of lens_chunks_e, and of F the positions
+  // [f_piece_lens_ptr[2k+l], f_piece_lens_ptr[2k+l+1]) of f_piece_lens (f_piece_list regrouped by lens in each piece).
+  rcc::DBuf<int32_t> lens_chunks_e, lens_chunks_f, f_piece_lens;
+  rcc::DBuf<rcc::Chunk> lens_recs_e;
+  int lens_ptr_e[rcc::N_LENSES + 1] = {0}, lens_ptr_f[rcc::N_LENSES + 1] = {0};
+  int lens_piece_e[rcc::N_LENSES][PIX_PIECES + 1] = {{0}};
+  int f_piece_lens_ptr[PIX_PIECES * rcc::N_LENSES + 1] = {0};
+  std::vector<rcc::Chunk> e_chunks_h, f_chunks_h;   // host copies of the chunk records (the lens lists come from them)
+  std::vector<int32_t> f_piece_list_h;
   rcc::StageTimer timer;
   rcc::DBuf<double> flush_buf;
 

@@ -38,8 +38,9 @@ class BAProblem:
 
     model "single": views are world_T_camera (camera_pose.cpp:88-98);
     model "rig":    views are world_T_body and ext[c] is body_T_cam_c.
-    lens "radtan" (dist = k1 k2 p1 p2 k3) or "equidistant" (dist = k1 k2 k3 k4 + a reserved slot held constant),
-    the same for every camera (rcc_ba_set_lens).
+    lens "radtan" (dist = k1 k2 p1 p2 k3) or "equidistant" (dist = k1 k2 k3 k4 + a reserved slot held constant)
+    for every camera (rcc_ba_set_lens), or a sequence of n_cameras such names, one per camera
+    (rcc_ba_set_camera_lenses): a rig may mix pinhole and fisheye cameras.
     """
 
     def __init__(self, n_views, n_markers, n_cameras=1, n_obs_blocks=0, model="single", device=0,
@@ -166,11 +167,21 @@ class BAProblem:
         self._check(self.lib.rcc_ba_set_loss(self.h, code, float(scale)))
 
     def set_lens(self, lens):
-        """lens: 'radtan' | 'equidistant' for every camera; invalidates the linearisation like set_loss."""
-        if lens not in L.LENSES:
-            raise ValueError(f"unknown lens {lens!r}: expected one of {sorted(L.LENSES)}")
-        self._check(self.lib.rcc_ba_set_lens(self.h, L.LENSES[lens]))
-        self.lens = lens
+        """lens: 'radtan' | 'equidistant' for every camera, or a sequence of n_cameras such names (one per camera);
+        invalidates the linearisation like set_loss.  Afterwards .lens is the name when every camera has the same
+        lens and the tuple of names otherwise."""
+        names = (lens,) if isinstance(lens, str) else tuple(lens)
+        for n in names:
+            if n not in L.LENSES:
+                raise ValueError(f"unknown lens {n!r}: expected one of {sorted(L.LENSES)}")
+        if isinstance(lens, str):
+            self._check(self.lib.rcc_ba_set_lens(self.h, L.LENSES[lens]))
+        else:
+            if len(names) != self.n_cameras:
+                raise ValueError(f"{len(names)} lenses for {self.n_cameras} cameras")
+            codes = np.array([L.LENSES[n] for n in names], dtype=np.int32)
+            self._check(self.lib.rcc_ba_set_camera_lenses(self.h, _ip(codes)))
+        self.lens = names[0] if len(set(names)) == 1 else names
 
     # ------------------------------------------------------------------ getters
     def get_intrinsics(self):

@@ -123,9 +123,9 @@ class Scene:
     const_dist: np.ndarray = None
     const_ext: np.ndarray = None
     truth: dict = field(default_factory=dict)   # ground-truth parameter arrays
-    image_size: tuple = (640, 480)
+    image_size: tuple = (640, 480)  # mixed lenses: one (width, height) per camera
     name: str = ""
-    lens: str = "radtan"            # "radtan" | "equidistant", every camera
+    lens: str = "radtan"            # "radtan" | "equidistant" for every camera, or a tuple of one per camera
 
     def __post_init__(self):
         nv, nm, nc = len(self.views), len(self.markers), len(self.intr)
@@ -201,26 +201,29 @@ def _chunk_observations(rng, v0, views_c, markers_t, sizes, intr_t, dist_t, ext_
     # marker centres in the view/body frame: R^T (t_m - t_v)   (cheap conservative prefilter)
     ctr = np.einsum('vji,vmj->vmi', Rv, markers_t[None, :, 3:6] - views_c[:, None, 3:6])
     for c in range(n_cam):
+        # mixed lenses: one lens and image size per camera
+        lens_c = lens if isinstance(lens, str) else lens[c]
+        W_c, H_c = (W, Himg) if np.ndim(W) == 0 else (W[c], Himg[c])
         pc = ctr
         if model == "rig":
             Rx = rodrigues_np(ext_t[c, 0:3])
             pc = (ctr - ext_t[c, 3:6]) @ Rx                                   # Rx^T (p - t_x)
         zc = np.maximum(pc[..., 2], 1e-9)
-        if lens == "equidistant":
+        if lens_c == "equidistant":
             cand = (pc[..., 2] > 0.05) & (np.arctan2(np.hypot(pc[..., 0], pc[..., 1]), pc[..., 2]) < np.deg2rad(88))
         else:
-            margin = 0.35 * max(W, Himg) + intr_t[c, 0] * tag_size / zc          # distortion + tag extent
+            margin = 0.35 * max(W_c, H_c) + intr_t[c, 0] * tag_size / zc          # distortion + tag extent
             cand = ((pc[..., 2] > 0.05)
-                    & (np.abs(intr_t[c, 0] * pc[..., 0] / zc + intr_t[c, 2] - W / 2) < W / 2 + margin)
-                    & (np.abs(intr_t[c, 1] * pc[..., 1] / zc + intr_t[c, 3] - Himg / 2) < Himg / 2 + margin))
+                    & (np.abs(intr_t[c, 0] * pc[..., 0] / zc + intr_t[c, 2] - W_c / 2) < W_c / 2 + margin)
+                    & (np.abs(intr_t[c, 1] * pc[..., 1] / zc + intr_t[c, 3] - H_c / 2) < H_c / 2 + margin))
         cv_, cm_ = np.nonzero(cand)
         uv_c, Z_c = project(model, np.broadcast_to(intr_t[c], (len(cv_), 4)),
                             np.broadcast_to(dist_t[c], (len(cv_), 5)),
                             np.broadcast_to(ext_t[c], (len(cv_), 6)),
-                            views_c[cv_], markers_t[cm_], sizes[cm_], lens)
-        ok_c = ((Z_c > 0.1).all(-1) & (uv_c[..., 0] >= 0).all(-1) & (uv_c[..., 0] < W).all(-1)
-                & (uv_c[..., 1] >= 0).all(-1) & (uv_c[..., 1] < Himg).all(-1))
-        if lens == "equidistant":
+                            views_c[cv_], markers_t[cm_], sizes[cm_], lens_c)
+        ok_c = ((Z_c > 0.1).all(-1) & (uv_c[..., 0] >= 0).all(-1) & (uv_c[..., 0] < W_c).all(-1)
+                & (uv_c[..., 1] >= 0).all(-1) & (uv_c[..., 1] < H_c).all(-1))
+        if lens_c == "equidistant":
             # the corner itself, not only the tag centre, within 85 degrees of the optical axis
             Pq = _corners_in_camera(model, ext_t[c], views_c[cv_], markers_t[cm_], sizes[cm_])
             ok_c &= (np.arctan2(np.hypot(Pq[..., 0], Pq[..., 1]), Pq[..., 2]) < np.deg2rad(85)).all(-1)
@@ -277,31 +280,63 @@ def make_scene(n_markers, n_views, visibility, n_cam=1, model="single", seed=0,
     lens       : "radtan" (640 x 480, f ~ 600 px) or "equidistant": a wide-angle fisheye camera (1280 x 1024,
                  f ~ 330 px, k1..k4, reserved slot 0) whose views are turned by up to +-1.2 rad so that tags are
                  seen up to 85 degrees off the optical axis.  image_size overrides the default size.
+                 A sequence of n_cam such names gives each camera its own lens, image size and intrinsics range
+                 (Scene.image_size is then one size per camera).  In a rig the equidistant cameras other than
+                 camera 0 are yawed a further 1 rad away from the body axis, so that they see the tags the body
+                 looks at far off their own axis; the views are turned by up to +-0.6 rad when there is no such
+                 camera to yaw (single model, or camera 0 equidistant).
     blocked    : every chunk of `chunk_views` views draws from its own random stream
                  (seed, chunk number): chunks are generated by `threads` host threads, and
                  `view_range=(lo, hi)` (multiples of chunk_views) yields exactly the views lo..hi-1 of the
                  full scene, renumbered from 0 -- the strong-scaling shards of one fixed problem.
                  The default (False) keeps the single sequential stream.
     """
-    if lens not in ("radtan", "equidistant"):
-        raise ValueError(f"unknown lens {lens!r}")
+    lenses = (lens,) if isinstance(lens, str) else tuple(lens)
+    for name_ in lenses:
+        if name_ not in ("radtan", "equidistant"):
+            raise ValueError(f"unknown lens {name_!r}")
+    if not isinstance(lens, str):
+        if len(lenses) != n_cam:
+            raise ValueError(f"{len(lenses)} lenses for {n_cam} cameras")
+        if len(set(lenses)) == 1:
+            lens = lenses[0]                    # one lens after all: the same scene as the name gives
+    mixed = not isinstance(lens, str)
     fisheye = lens == "equidistant"
-    if image_size is None:
-        image_size = (1280, 1024) if fisheye else (640, 480)
     rng = np.random.default_rng(seed)
-    W, Himg = image_size
-    # ---- cameras (truth): SURVEY 8(d2)
-    f_lo, f_hi = (320, 340) if fisheye else (550, 650)
-    intr_t = np.stack([rng.uniform(f_lo, f_hi, n_cam), rng.uniform(f_lo, f_hi, n_cam),
-                       W / 2 + rng.uniform(-10, 10, n_cam),
-                       Himg / 2 + rng.uniform(-10, 10, n_cam)], -1)
-    if fisheye:
-        dist_t = np.stack([rng.normal(0, 0.02, n_cam), rng.normal(0, 0.01, n_cam),
-                           rng.normal(0, 2e-3, n_cam), rng.normal(0, 5e-4, n_cam), np.zeros(n_cam)], -1)
+    if not mixed:
+        if image_size is None:
+            image_size = (1280, 1024) if fisheye else (640, 480)
+        W, Himg = image_size
+        # ---- cameras (truth): SURVEY 8(d2)
+        f_lo, f_hi = (320, 340) if fisheye else (550, 650)
+        intr_t = np.stack([rng.uniform(f_lo, f_hi, n_cam), rng.uniform(f_lo, f_hi, n_cam),
+                           W / 2 + rng.uniform(-10, 10, n_cam),
+                           Himg / 2 + rng.uniform(-10, 10, n_cam)], -1)
+        if fisheye:
+            dist_t = np.stack([rng.normal(0, 0.02, n_cam), rng.normal(0, 0.01, n_cam),
+                               rng.normal(0, 2e-3, n_cam), rng.normal(0, 5e-4, n_cam), np.zeros(n_cam)], -1)
+        else:
+            dist_t = np.stack([rng.normal(0, 0.1, n_cam), rng.normal(0, 0.05, n_cam),
+                               rng.normal(0, 2e-3, n_cam), rng.normal(0, 2e-3, n_cam),
+                               rng.normal(0, 0.01, n_cam)], -1)
     else:
-        dist_t = np.stack([rng.normal(0, 0.1, n_cam), rng.normal(0, 0.05, n_cam),
+        # each camera from its own lens's ranges; the wall below is sized for the radial-tangential default
+        fish = np.array([name_ == "equidistant" for name_ in lenses])
+        image_size = tuple(tuple(image_size) if image_size is not None else ((1280, 1024) if f_ else (640, 480))
+                           for f_ in fish)
+        W_cam = np.array([sz[0] for sz in image_size], dtype=np.float64)
+        H_cam = np.array([sz[1] for sz in image_size], dtype=np.float64)
+        f_lo, f_hi = np.where(fish, 320.0, 550.0), np.where(fish, 340.0, 650.0)
+        intr_t = np.stack([rng.uniform(f_lo, f_hi), rng.uniform(f_lo, f_hi),
+                           W_cam / 2 + rng.uniform(-10, 10, n_cam),
+                           H_cam / 2 + rng.uniform(-10, 10, n_cam)], -1)
+        dist_f = np.stack([rng.normal(0, 0.02, n_cam), rng.normal(0, 0.01, n_cam),
+                           rng.normal(0, 2e-3, n_cam), rng.normal(0, 5e-4, n_cam), np.zeros(n_cam)], -1)
+        dist_r = np.stack([rng.normal(0, 0.1, n_cam), rng.normal(0, 0.05, n_cam),
                            rng.normal(0, 2e-3, n_cam), rng.normal(0, 2e-3, n_cam),
                            rng.normal(0, 0.01, n_cam)], -1)
+        dist_t = np.where(fish[:, None], dist_f, dist_r)
+        W, Himg = (640, 480)
     ext_t = np.zeros((n_cam, 6))
     if model == "rig":
         # cameras fan out around the body's optical axis
@@ -311,6 +346,10 @@ def make_scene(n_markers, n_views, visibility, n_cam=1, model="single", seed=0,
         ext_t[1:, 0:3] += rng.normal(0, 0.02, (n_cam - 1, 3))
         ext_t[1:, 3:6] += rng.normal(0, 0.01, (n_cam - 1, 3))
         ext_t[0] = 0.0                          # body frame == camera 0 (gauge)
+        if mixed:
+            # fisheye cameras look 1 rad further out: the tags the body looks at land far off their axis
+            yaw_out = fish & (np.arange(n_cam) > 0)
+            ext_t[yaw_out, 1] += np.where(ang[yaw_out] < 0, -1.0, 1.0)
 
     # ---- wall of tags: area so that footprint/area ~ visibility
     d_mean = 2.0
@@ -336,8 +375,14 @@ def make_scene(n_markers, n_views, visibility, n_cam=1, model="single", seed=0,
     markers_t[0] = 0.0
     sizes = np.full(n_markers, tag_size)
     s_r, s_t, s_i = perturb
-    obs_args = (markers_t, sizes, intr_t, dist_t, ext_t, model, n_cam, visibility, W, Himg, tag_size, dtype_idx, lens)
-    tilt = 1.2 if fisheye else 0.0
+    if mixed:
+        obs_args = (markers_t, sizes, intr_t, dist_t, ext_t, model, n_cam, visibility, W_cam, H_cam, tag_size,
+                    dtype_idx, lenses)
+        tilt = 0.6 if (model != "rig" or fish[0]) else 0.0
+    else:
+        obs_args = (markers_t, sizes, intr_t, dist_t, ext_t, model, n_cam, visibility, W, Himg, tag_size, dtype_idx,
+                    lens)
+        tilt = 1.2 if fisheye else 0.0
 
     if blocked:
         # ---- one random stream per chunk of views: parallel, and any aligned view range on its own
@@ -400,6 +445,8 @@ def make_scene(n_markers, n_views, visibility, n_cam=1, model="single", seed=0,
     dist0 = dist_t + rs.normal(0, s_i, dist_t.shape) * 0.1
     if fisheye:
         dist0[:, 4] = 0.0                       # the reserved slot
+    elif mixed:
+        dist0[fish, 4] = 0.0
     ext0 = ext_t.copy()
     if model == "rig" and n_cam > 1:
         ext0[1:] += np.concatenate([rs.normal(0, s_r, (n_cam - 1, 3)),
