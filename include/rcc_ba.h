@@ -164,6 +164,33 @@ int rcc_ba_set_lens(rcc_ba_problem* p, int32_t lens);
  * communicator attached (rcc_ba_comm_init) every rank must set the same lenses. */
 int rcc_ba_set_camera_lenses(rcc_ba_problem* p, const int32_t* lenses);
 
+/* Gaussian priors (ceres::NormalPrior) on the blocks of one kind: n priors, index[n] (view, marker or camera),
+ * mean[n x k], sqrt_information[n x k x k] row-major (A_i), k = size of the kind (view / marker / ext 6, intr 4,
+ * dist 5).  Replaces every earlier prior of that kind; n == 0 clears them (the arrays may then be NULL).
+ * A prior on block x_i is the residual block r_i = A_i (x_i - mu_i), A_i the square root of the information matrix
+ * and mu_i the mean, exactly as ceres::NormalPrior(A_i, mu_i).  It is linear in the stored parameters: a Rodrigues
+ * vector is differenced as a plain 3-vector, as Ceres does for a NormalPrior on an rvec block.  A prior is never
+ * robustified, whatever rcc_ba_set_loss says (a NormalPrior added with a NULL loss).  Wherever the library uses the
+ * tag cost it uses the total  1/2 sum rho(||r_tag||^2) + 1/2 sum ||r_i||^2:
+ *   - rcc_ba_linearize adds A^T A to the block's diagonal block (H_ee, H_ff or the camera's block of H_ss) and
+ *     A^T A (x - mu) to its gradient; W, H_es and H_fs do not change.  rcc_ba_get_normal_blocks returns the sums.
+ *   - the LM damping and the Jacobi scaling read diag(J^T J), prior rows included (they are columns of J like any
+ *     other, as in Ceres); the model cost change and the gradient-tolerance test use the same gradient.
+ *   - the costs of rcc_ba_linearize, rcc_ba_evaluate, rcc_ba_evaluate_device, rcc_ba_candidate_cost and the
+ *     initial_cost / final_cost of rcc_lm_summary include the prior cost.  The residual and Jacobian arrays of
+ *     rcc_ba_evaluate stay the tag blocks only.
+ *   - rcc_ba_covariance and rcc_ba_covariance_blocks invert the undamped system with the priors in it: a prior on a
+ *     gauge block (the world tag near identity) makes J^T J positive definite without holding a block constant.
+ *   - a prior on a constant block adds its cost only: the block's step and covariance rows stay exactly 0.  So does
+ *     column 4 of a dist prior on an equidistant camera: it adds cost and never moves the reserved slot.
+ * RCC_BAD_ARG, checked before anything changes, for an unknown kind, RCC_BLOCK_EXT on the single-camera model,
+ * n < 0, a NULL array with n > 0, an index out of range, the same index twice in one call, or a non-finite mean or
+ * A.  Like rcc_ba_set_loss it may be called at any time and invalidates the linearisation; like the parameter setters
+ * it copies the caller's arrays and returns without a stream synchronisation.  A handle without priors issues no
+ * launch for them.  With a communicator attached each rank adds the priors it was given (see rcc_ba_comm_init). */
+int rcc_ba_set_priors(rcc_ba_problem* p, int32_t block_kind, int64_t n, const int32_t* index, const double* mean,
+                      const double* sqrt_information);
+
 int rcc_ba_get_intrinsics(rcc_ba_problem* p, double* intr, double* dist);
 int rcc_ba_get_rig_extrinsics(rcc_ba_problem* p, double* ext);
 int rcc_ba_get_view_poses(rcc_ba_problem* p, double* views);
@@ -263,6 +290,10 @@ int rcc_ba_get_step(rcc_ba_problem* p, double* d_e, double* d_f, double* d_share
  * owner, one all-reduce of the reduced system per LM iteration ------------- */
 #define RCC_COMM_ID_BYTES 128
 int rcc_comm_get_unique_id(char id[RCC_COMM_ID_BYTES]);             /* rank 0 calls, then broadcasts */
+/* Priors (rcc_ba_set_priors) on several ranks: each rank adds exactly the priors it was given, and the all-reduce of
+ * the reduced system and of the costs sums them like everything else.  So give each prior to exactly one rank: priors
+ * on kept blocks and on the shared intr / dist / ext blocks to rank 0, priors on eliminated blocks to the rank that
+ * owns the block's observations. */
 int rcc_ba_comm_init(rcc_ba_problem* p, const char id[RCC_COMM_ID_BYTES], int32_t rank, int32_t n_ranks);
 
 /* ---- measurement -------------------------------------------------------- */

@@ -4,7 +4,7 @@ detections_N.yaml with initial world_T_camera / world_T_target guesses, camera_p
 run the GPU bundle adjustment, and write the refined poses back in the same formats, where opt_vis_node
 (opt_visualization.cpp:162-220) picks them up.
 
-    python -m robot_camera_calibration_b200 <detections directory> [--fix-intrinsics] [--device 0] ...
+    python -m robot_camera_calibration_b200 <detections directory> [--fix-intrinsics | --intrinsics-sigma F C D] ...
 """
 from __future__ import annotations
 
@@ -21,9 +21,14 @@ def parser():
     ap = argparse.ArgumentParser(prog="python -m robot_camera_calibration_b200", description=__doc__.split("\n\n")[0])
     ap.add_argument("directory", help="the detections directory (camera_pose.cpp:41-51: <package>/detections)")
     ap.add_argument("--device", type=int, default=0, help="CUDA device")
-    ap.add_argument("--fix-intrinsics", action="store_true",
-                    help="keep camera.yaml's intrinsics and distortion constant (default: refined, written to "
-                         "camera_refined.yaml)")
+    intr = ap.add_mutually_exclusive_group()
+    intr.add_argument("--fix-intrinsics", action="store_true",
+                      help="keep camera.yaml's intrinsics and distortion constant (default: refined, written to "
+                           "camera_refined.yaml)")
+    intr.add_argument("--intrinsics-sigma", type=float, nargs=3, metavar=("FOCAL_PX", "PRINCIPAL_PX", "DIST"),
+                      default=None,
+                      help="refine the intrinsics under a Gaussian prior centred on camera.yaml: standard deviations "
+                           "of fx fy, of cx cy (pixels) and of every distortion coefficient")
     ap.add_argument("--max-iterations", type=int, default=50)
     ap.add_argument("--function-tolerance", type=float, default=None)
     ap.add_argument("--gradient-tolerance", type=float, default=None)
@@ -35,7 +40,10 @@ def parser():
 
 
 def main(argv=None):
-    args = parser().parse_args(argv)
+    ap = parser()
+    args = ap.parse_args(argv)
+    if args.intrinsics_sigma is not None and not all(0 < s < float("inf") for s in args.intrinsics_sigma):
+        ap.error("--intrinsics-sigma: every sigma must be positive and finite")
     from . import io_yaml
     opts = {"max_iterations": args.max_iterations, "verbose": int(args.verbose)}
     for k in ("function_tolerance", "gradient_tolerance", "parameter_tolerance"):
@@ -43,7 +51,8 @@ def main(argv=None):
             opts[k] = getattr(args, k)
     try:
         summary = io_yaml.optimise_directory(args.directory, device=args.device,
-                                             refine_intrinsics=not args.fix_intrinsics, precision=args.precision, **opts)
+                                             refine_intrinsics=not args.fix_intrinsics, precision=args.precision,
+                                             intrinsics_sigma=args.intrinsics_sigma, **opts)
     except (FileNotFoundError, ValueError) as e:          # missing camera.yaml / targets.yaml, empty dataset
         print(f"error: {e}", file=sys.stderr)
         return 2

@@ -6,6 +6,7 @@ Same names, argument meaning and error behaviour as the published Ceres API
     problem = Problem()
     problem.AddResidualBlock(TagReprojectionCost(pixels8, tag_size), None, intr, dist, view, marker)
     problem.SetParameterBlockConstant(marker0)              # gauge, camera_pose.cpp:71-80
+    problem.AddResidualBlock(NormalPrior(A, b), None, intr)  # soft knowledge: intr stays near b
     summary = Solve(SolverOptions(max_num_iterations=50), problem)   # refines the arrays in place
 
 Parameter blocks are numpy float64 arrays that the caller owns (Ceres: `double*`);
@@ -65,6 +66,54 @@ class TagReprojectionCost:
         return not out["failed"]
 
 
+class NormalPrior:
+    """ceres::NormalPrior(A, b): the residual A (x - b) on one parameter block of size b.size, A m x b.size.  Linear in
+    the stored parameters (a Rodrigues vector is differenced as a plain 3-vector).  On the GPU path a prior takes no
+    loss function, and A is handed to rcc_ba_set_priors as a k x k matrix: an m x k A (m != k), and several priors
+    on one block stacked, are reduced by QR, which keeps A^T A and ||A (x - b)||."""
+
+    def __init__(self, A, b):
+        self.b = np.array(b, dtype=np.float64).reshape(-1)
+        self.A = np.array(A, dtype=np.float64).reshape(-1, self.b.size)
+
+    def num_residuals(self):
+        return self.A.shape[0]
+
+    def parameter_block_sizes(self):
+        return [self.b.size]
+
+    def residual(self, x):
+        return self.A @ (np.asarray(x, dtype=np.float64).reshape(-1) - self.b)
+
+    def Evaluate(self, parameters, residuals, jacobians):
+        """bool Evaluate(parameters, residuals, jacobians): r = A (x - b), dr/dx = A (row-major m x k)."""
+        residuals[:] = self.residual(parameters[0])
+        if jacobians is not None and jacobians[0] is not None:
+            np.asarray(jacobians[0]).reshape(-1)[:] = self.A.reshape(-1)
+        return True
+
+
+def reduce_normal_priors(priors):
+    """Priors [(A_j, b_j)] on one block of size k -> (A, mu, c) with A k x k and
+    sum_j ||A_j (x - b_j)||^2 = ||A (x - mu)||^2 + c for every x.  One k x k prior comes back unchanged; otherwise A is
+    the R factor of the stacked A_j (zero rows appended when there are fewer than k rows).  mu is the common b_j, or
+    the least-squares point of the stacked system when the b_j differ (then c > 0 is its residual)."""
+    k = priors[0][1].size
+    if len(priors) == 1 and priors[0][0].shape[0] == k:
+        return priors[0][0], priors[0][1], 0.0
+    M = np.vstack([A for A, _ in priors])
+    if all(np.array_equal(b, priors[0][1]) for _, b in priors):
+        mu, c = priors[0][1], 0.0
+    else:
+        rhs = np.concatenate([A @ b for A, b in priors])
+        mu = np.linalg.lstsq(M, rhs, rcond=None)[0]
+        c = float(np.sum((M @ mu - rhs) ** 2))
+    R = np.linalg.qr(M, mode="r")
+    A = np.zeros((k, k))
+    A[:R.shape[0]] = R
+    return A, mu, c
+
+
 class HuberLoss:
     """ceres::HuberLoss(a): rho(s) = s for s <= a^2, 2 a sqrt(s) - a^2 beyond."""
     kind = "huber"
@@ -106,11 +155,13 @@ class Summary:
 
 
 class Problem:
-    """ceres::Problem for tag-reprojection residual blocks."""
+    """ceres::Problem for tag-reprojection and NormalPrior residual blocks."""
 
     def __init__(self, device=0, eliminate="auto"):
         self.device, self.eliminate = device, eliminate
         self._blocks = []            # (cost, intr, dist, view, marker, ext)
+        self._priors = []            # (NormalPrior, block)
+        self._order = []             # ("tag" | "prior", position in _blocks | _priors): Ceres residual block order
         self._const = set()
         self._known = {}
         self._loss = None
@@ -122,6 +173,16 @@ class Problem:
         return a
 
     def AddResidualBlock(self, cost_function, loss_function, *parameter_blocks):
+        if isinstance(cost_function, NormalPrior):
+            if loss_function is not None:
+                raise NotImplementedError("a NormalPrior takes no loss function on this path")
+            if len(parameter_blocks) != 1:
+                raise ValueError(f"expected 1 parameter block, got {len(parameter_blocks)}")
+            block = self._check_block(parameter_blocks[0], cost_function.b.size)
+            self._known[id(block)] = block
+            self._priors.append((cost_function, block))
+            self._order.append(("prior", len(self._priors) - 1))
+            return len(self._order) - 1
         key = None if loss_function is None else (loss_function.kind, loss_function.a)
         if self._blocks and key != self._loss:
             raise NotImplementedError("all residual blocks must share one loss function on this path")
@@ -133,7 +194,8 @@ class Problem:
         for b in blocks:
             self._known[id(b)] = b
         self._blocks.append((cost_function, *blocks, *([None] if len(blocks) == 4 else [])))
-        return len(self._blocks) - 1
+        self._order.append(("tag", len(self._blocks) - 1))
+        return len(self._order) - 1
 
     def SetParameterBlockConstant(self, values):
         if id(values) not in self._known:
@@ -144,20 +206,24 @@ class Problem:
         self._const.discard(id(values))
 
     def NumResidualBlocks(self):
-        return len(self._blocks)
+        return len(self._order)
 
     def NumResiduals(self):
-        return 8 * len(self._blocks)
+        return 8 * len(self._blocks) + sum(c.num_residuals() for c, _ in self._priors)
 
     def NumParameterBlocks(self):
         return len(self._known)
 
     def Evaluate(self):
-        """-> (cost, residuals (8N,), jacobian blocks dict) like Problem::Evaluate."""
+        """-> (cost, residuals, jacobian blocks dict) like Problem::Evaluate: the residuals of every block in the order
+        the blocks were added, the tag blocks' from the GPU and the priors' A (x - b) formed here; the jacobian blocks
+        are the tag blocks'.  The cost is the library's, priors included."""
         gp, maps = self._build()
         with gp:
             out = gp.evaluate()
-        return out["cost"], out["residuals"].reshape(-1), out["jacobians"]
+        tags = out["residuals"]
+        res = [tags[j] if kind == "tag" else self._priors[j][0].residual(self._priors[j][1]) for kind, j in self._order]
+        return out["cost"] + self._prior_const, np.concatenate(res), out["jacobians"]
 
     # -- batching -----------------------------------------------------------
     @staticmethod
@@ -220,7 +286,34 @@ class Problem:
                 gp.set_constant("dist", i)
             if rig and id(ext) in self._const:
                 gp.set_constant("ext", i)
+        self._prior_const = self._set_priors(gp, vlist, mlist, clist, rig)
         return gp, (vlist, mlist, clist, rig)
+
+    def _set_priors(self, gp, vlist, mlist, clist, rig):
+        """The NormalPrior blocks, reduced to one k x k prior per parameter block, into gp.  Returns the cost the
+        reduction leaves out (nonzero only for stacked priors with different means)."""
+        where = {}
+        for i, a in enumerate(vlist):
+            where[id(a)] = ("view", i)
+        for i, a in enumerate(mlist):
+            where[id(a)] = ("marker", i)
+        for c, (_, intr, dist, ext) in enumerate(clist):
+            where[id(intr)], where[id(dist)] = ("intr", c), ("dist", c)
+            if rig:
+                where[id(ext)] = ("ext", c)
+        groups = {}
+        for cost, block in self._priors:
+            if id(block) not in where:
+                raise NotImplementedError("a NormalPrior's parameter block is not used by any tag residual block")
+            groups.setdefault(where[id(block)], []).append((cost.A, cost.b))
+        per_kind, const = {}, 0.0
+        for (kind, i), priors in groups.items():
+            A, mu, c = reduce_normal_priors(priors)
+            per_kind.setdefault(kind, []).append((i, mu, A))
+            const += 0.5 * c
+        for kind, lst in per_kind.items():
+            gp.set_priors(kind, [i for i, _, _ in lst], np.stack([m for _, m, _ in lst]), np.stack([a for _, _, a in lst]))
+        return const
 
 
 def Solve(options, problem):
@@ -234,6 +327,8 @@ def Solve(options, problem):
                      parameter_tolerance=o.parameter_tolerance, min_diagonal=o.min_lm_diagonal,
                      max_diagonal=o.max_lm_diagonal, verbose=int(o.minimizer_progress_to_stdout),
                      jacobi_scaling=int(o.jacobi_scaling))
+        s["initial_cost"] += problem._prior_const
+        s["final_cost"] += problem._prior_const
         views, markers = gp.get_view_poses(), gp.get_marker_poses()
         intr, dist = gp.get_intrinsics()
         ext = gp.get_rig_extrinsics() if rig else None

@@ -6,6 +6,8 @@
 #include <math.h>
 #include <stdint.h>
 
+#include "../../include/rcc_ba.h"
+
 namespace rcc {
 
 // ---------------------------------------------------------------------------
@@ -118,6 +120,36 @@ inline int fin_slices(int n_sm, int n_cam) {
 // E side, F side and both stages of the shared reduction in one launch
 void launch_finalize(bool rig, const FinalizeSideArgs& e, const FinalizeSideArgs& f, const FinalizeSharedArgs& sh,
                      cudaStream_t s);
+
+// ---------------------------------------------------------------------------
+// Gaussian priors (prior.cu): r_i = A_i (x_i - mu_i) on one parameter block each (ceres::NormalPrior)
+// ---------------------------------------------------------------------------
+constexpr int PRIOR_KINDS = 5;   // rcc_block_kind: view, marker, intr, dist, ext
+__host__ __device__ inline int prior_block_size(int kind) {
+  return kind == RCC_BLOCK_INTR ? 4 : kind == RCC_BLOCK_DIST ? 5 : 6;
+}
+struct PriorArgs {
+  int32_t off[PRIOR_KINDS + 1];  // the priors of kind t are [off[t], off[t+1]), kinds back to back in rcc_block_kind order
+  const int32_t* index;          // [n] view, marker or camera
+  const double* mean;            // [n*6]   mu, first k used
+  const double* A;               // [n*36]  row-major 6 x 6, the k x k square root of the information, zero padded
+  const double* AtA;             // [n*36]  A^T A (launch_prior_gram)
+  const double* views;           // parameters the priors are evaluated at (current or candidate)
+  const double* markers;
+  const double* shared;
+  int32_t sp, n_shared, elim_view;
+  double* Hee;                   // linearisation only: A^T A into the block's diagonal block, A^T A (x - mu) into g
+  double* ge;
+  double* Hff;
+  double* gf;
+  double* Hss;
+  double* gs;
+  double* cost2;                 // [prior_grid(n)] sum ||A (x - mu)||^2 per CTA
+};
+int prior_grid(int n);           // CTAs (= cost partials) of launch_prior over n priors; 0 for none
+void launch_prior_gram(int n, const double* A, double* AtA, cudaStream_t s);
+// linearize: add the priors to H and g (after launch_finalize) and write the cost partials; else the cost partials only
+void launch_prior(bool linearize, const PriorArgs& a, cudaStream_t s);
 
 // pose expansion: rvec,t -> R, Jr, t
 void launch_expand_poses(const double* views, int n_views, double* view_x, const double* markers,
@@ -249,7 +281,7 @@ struct ReducedTailArgs {
   const double* gf;
   const double* Hss;
   const double* gs;
-  const double* cost2_cam;  // [n_cam]
+  const double* cost2_cam;  // [n_cam]: summed in order (the caller passes the prior cost partials after the cameras')
   int32_t n_cam;
   double* S;                // tail starts at S + n*ld
 };

@@ -530,7 +530,7 @@ static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker
   P->part_f.alloc((size_t)P->n_chunks_f * (P->rig ? PassGeom<true>::PART_F : PassGeom<false>::PART_F));
   P->W.alloc((size_t)n * 36);
   P->Y.alloc((size_t)std::max<int64_t>(P->n_pairs, 1) * 36);
-  P->cost_partials.alloc((size_t)std::max(std::max(1, eval_grid(n)), P->n_chunks_e));
+  P->cost_partials.alloc((size_t)std::max(std::max(1, eval_grid(n)), P->n_chunks_e) + P->n_prior_parts);
   RCC_CUDA(cudaStreamSynchronize(s));
   P->have_obs = true;
   P->linearized = P->schur_done = P->step_ready = P->cand_ready = false;
@@ -590,6 +590,21 @@ static int assemble_by_lens(P_t* P, bool epass, AssembleArgs a, const int32_t* l
     ++n;
   }
   return n;
+}
+
+// the priors evaluated at the current or the candidate parameters; H and g are the linearisation's blocks (used by
+// launch_prior(true, ...) only)
+static PriorArgs prior_args(P_t* P, bool cand, double* cost2) {
+  PriorArgs a{};
+  for (int t = 0; t <= PRIOR_KINDS; ++t) a.off[t] = P->prior_off[t];
+  a.index = P->prior_index.p; a.mean = P->prior_mean.p; a.A = P->prior_A.p; a.AtA = P->prior_AtA.p;
+  a.views = cand ? P->views_c.p : P->views.p;
+  a.markers = cand ? P->markers_c.p : P->markers.p;
+  a.shared = cand ? P->shared_c.p : P->shared.p;
+  a.sp = P->sp; a.n_shared = P->n_shared; a.elim_view = P->elim_view ? 1 : 0;
+  a.Hee = P->Hee.p; a.ge = P->ge.p; a.Hff = P->Hff.p; a.gf = P->gf.p; a.Hss = P->Hss.p; a.gs = P->gs.p;
+  a.cost2 = cost2;
+  return a;
 }
 
 static void do_linearize(P_t* P) {
@@ -677,12 +692,14 @@ static void do_linearize(P_t* P) {
     else launch_assemble(P->rig, false, !P->elim_view, P->lens, a, P->stream);
   }
   {
-    Scoped t(P, ST_FINALIZE, 1);
+    Scoped t(P, ST_FINALIZE, P->n_prior_parts > 0 ? 2 : 1);
     FinalizeSideArgs fe{P->part_e.p, P->e_chunks.p, P->e_chunk_ptr.p, P->n_e, P->n_shared, P->Hee.p, P->ge.p, P->Hes.p};
     FinalizeSideArgs ff{P->part_f.p, P->f_chunks.p, P->f_chunk_ptr.p, P->n_f, P->n_shared, P->Hff.p, P->gf.p, P->Hfs.p};
     FinalizeSharedArgs fs{P->part_e.p, P->cam_chunks_e.p, P->cam_ptr_e.p, P->n_cam, P->n_shared, P->Hss.p, P->gs.p,
                           P->cost2_cam.p, P->fin_scratch.p, P->fin_done.p, P->loss != 0 ? 1 : 0, P->fin_slices};
     launch_finalize(P->rig, fe, ff, fs, P->stream);
+    // the priors add into the finalized blocks; their cost partials follow the cameras' in cost2_cam
+    if (P->n_prior_parts > 0) launch_prior(true, prior_args(P, false, P->cost2_cam.p + P->n_cam), P->stream);
   }
   P->linearized = true;
   P->schur_done = P->step_ready = P->cand_ready = false;
@@ -723,8 +740,8 @@ static void do_schur(P_t* P, double radius, int32_t* pivot_fail = nullptr) {
     SchurSharedArgs sh{P->n_e, P->n_f, P->n_shared, P->n_bb, P->ld, P->Yb.p, P->Hss.p, P->gs.p, P->shared_scratch.p,
                        P->S.p};
     launch_schur_shared(sh, P->side_stream);
-    ReducedTailArgs r{P->n_f, P->n_shared, P->ld, P->Hff.p, P->gf.p, P->Hss.p, P->gs.p, P->cost2_cam.p, P->n_cam,
-                      P->S.p};
+    ReducedTailArgs r{P->n_f, P->n_shared, P->ld, P->Hff.p, P->gf.p, P->Hss.p, P->gs.p, P->cost2_cam.p,
+                      P->n_cam + P->n_prior_parts, P->S.p};
     launch_reduced_tail(r, P->side_stream);
     RCC_CUDA(cudaEventRecord(P->ev_join, P->side_stream));
     eager = P->comm != nullptr && P->n_ranks > 1;
@@ -1193,12 +1210,14 @@ static void do_candidate_cost(P_t* P) {
                         P->shared_c.p, P->n_cam, P->sp, P->ext_xc.p, P->stream);
   }
   {
-    Scoped t(P, ST_COST, 2);
+    Scoped t(P, ST_COST, P->n_prior_parts > 0 ? 3 : 2);
     EvalArgs a = eval_args(P, true);
     a.fail_flag = P->fail_flag.p + 1;   // slot 1: candidate point (slot 0 keeps the linearisation point's flag)
     RCC_CUDA(cudaMemsetAsync(a.fail_flag, 0, sizeof(int32_t), P->stream));
     launch_cost(P->rig, cost_lens(P), a, P->stream);
-    launch_sum(P->cost_partials.p, eval_grid(P->n_obs), P->stats.p + SX_CAND2, 1.0, P->stream);
+    const int np = eval_grid(P->n_obs);
+    if (P->n_prior_parts > 0) launch_prior(false, prior_args(P, true, P->cost_partials.p + np), P->stream);
+    launch_sum(P->cost_partials.p, np + P->n_prior_parts, P->stats.p + SX_CAND2, 1.0, P->stream);
   }
   if (P->comm) {
     Scoped t(P, ST_ALLREDUCE, 2);
@@ -1718,6 +1737,77 @@ int rcc_ba_set_camera_lenses(rcc_ba_problem* P, const int32_t* lenses) {
   API_END(P)
 }
 
+// every check first: a refused call changes nothing
+static void set_priors(P_t* P, int32_t kind, int64_t n, const int32_t* index, const double* mean, const double* sqrt_info) {
+  int count = 0;
+  switch (kind) {
+    case RCC_BLOCK_VIEW: count = P->n_views; break;
+    case RCC_BLOCK_MARKER: count = P->n_markers; break;
+    case RCC_BLOCK_INTR: case RCC_BLOCK_DIST: count = P->n_cam; break;
+    case RCC_BLOCK_EXT:
+      RCC_REQUIRE(P->rig, RCC_BAD_ARG, "RCC_BLOCK_EXT needs the rig model");
+      count = P->n_cam;
+      break;
+    default: throw Error(RCC_BAD_ARG, "unknown block kind " + std::to_string(kind));
+  }
+  RCC_REQUIRE(n >= 0, RCC_BAD_ARG, "n must not be negative");
+  RCC_REQUIRE(n <= count, RCC_BAD_ARG, "more priors than blocks: an index out of range or repeated");
+  RCC_REQUIRE(n == 0 || (index && mean && sqrt_info), RCC_BAD_ARG, "null pointer");
+  const int k = prior_block_size(kind);
+  std::vector<uint8_t> seen((size_t)count, 0);
+  for (int64_t i = 0; i < n; ++i) {
+    RCC_REQUIRE(index[i] >= 0 && index[i] < count, RCC_BAD_ARG, "prior block index out of range");
+    RCC_REQUIRE(!seen[index[i]], RCC_BAD_ARG, "block " + std::to_string(index[i]) + " has two priors in one call");
+    seen[index[i]] = 1;
+    for (int j = 0; j < k; ++j) RCC_REQUIRE(std::isfinite(mean[i * k + j]), RCC_BAD_ARG, "non-finite prior mean");
+    for (int j = 0; j < k * k; ++j)
+      RCC_REQUIRE(std::isfinite(sqrt_info[i * k * k + j]), RCC_BAD_ARG, "non-finite prior sqrt_information");
+  }
+  std::vector<int32_t>& hi = P->prior_index_h[kind];
+  std::vector<double>& hm = P->prior_mean_h[kind];
+  std::vector<double>& ha = P->prior_A_h[kind];
+  hi.assign(index, index + n);
+  hm.assign((size_t)n * 6, 0.0);
+  ha.assign((size_t)n * 36, 0.0);
+  for (int64_t i = 0; i < n; ++i)
+    for (int r = 0; r < k; ++r) {
+      hm[i * 6 + r] = mean[i * k + r];
+      for (int c = 0; c < k; ++c) ha[i * 36 + r * 6 + c] = sqrt_info[i * k * k + r * k + c];
+    }
+  std::vector<int32_t> idx;
+  std::vector<double> mu, A;
+  for (int t = 0; t < PRIOR_KINDS; ++t) {
+    P->prior_off[t] = (int)idx.size();
+    idx.insert(idx.end(), P->prior_index_h[t].begin(), P->prior_index_h[t].end());
+    mu.insert(mu.end(), P->prior_mean_h[t].begin(), P->prior_mean_h[t].end());
+    A.insert(A.end(), P->prior_A_h[t].begin(), P->prior_A_h[t].end());
+  }
+  const int total = (int)idx.size();
+  P->prior_off[PRIOR_KINDS] = total;
+  P->n_prior_parts = prior_grid(total);
+  if (total > 0) {
+    cudaStream_t s = P->stream;
+    P->prior_index.upload(idx, s);
+    P->prior_mean.upload(mu, s);
+    P->prior_A.upload(A, s);
+    P->prior_AtA.ensure((size_t)total * 36);
+    Scoped t(P, ST_H2D, 1);
+    launch_prior_gram(total, P->prior_A.p, P->prior_AtA.p, s);
+  }
+  // the cost partials of the priors follow the cameras' (linearisation) and K1's / K6's (evaluation, candidate cost)
+  P->cost2_cam.ensure((size_t)P->n_cam + P->n_prior_parts);
+  if (P->have_obs)
+    P->cost_partials.ensure((size_t)std::max(std::max(1, eval_grid(P->n_obs)), P->n_chunks_e) + P->n_prior_parts);
+  P->linearized = P->schur_done = P->step_ready = P->cand_ready = false;
+}
+
+int rcc_ba_set_priors(rcc_ba_problem* P, int32_t block_kind, int64_t n, const int32_t* index, const double* mean,
+                      const double* sqrt_information) {
+  API_BEGIN(P)
+  set_priors(P, block_kind, n, index, mean, sqrt_information);
+  API_END(P)
+}
+
 int rcc_ba_get_intrinsics(rcc_ba_problem* P, double* intr, double* dist) {
   API_BEGIN(P)
   std::vector<double> h((size_t)P->n_shared);
@@ -1776,7 +1866,7 @@ static int evaluate_impl(P_t* P, int want_j, double* cost, bool to_host, double*
   a.fail_flag = P->fail_flag.p + 2;   // slot 2: materialised evaluation
   RCC_CUDA(cudaMemsetAsync(a.fail_flag, 0, sizeof(int32_t), P->stream));
   {
-    Scoped t(P, ST_EVALUATE, 2);
+    Scoped t(P, ST_EVALUATE, P->n_prior_parts > 0 ? 3 : 2);
     if (P->lens_mixed && want_j) {
       // K1 once per lens over a lens-major copy of the E chunk records; outputs go to caller positions and the cost
       // partials stay one per chunk, so the launches are independent
@@ -1795,7 +1885,9 @@ static int evaluate_impl(P_t* P, int want_j, double* cost, bool to_host, double*
     } else {
       launch_evaluate(P->rig, want_j != 0, want_j ? P->lens : cost_lens(P), a, P->stream);
     }
-    launch_sum(P->cost_partials.p, eval_partials(want_j != 0, a), P->scalar.p, 0.5, P->stream);
+    const int np = eval_partials(want_j != 0, a);
+    if (P->n_prior_parts > 0) launch_prior(false, prior_args(P, false, P->cost_partials.p + np), P->stream);
+    launch_sum(P->cost_partials.p, np + P->n_prior_parts, P->scalar.p, 0.5, P->stream);
   }
   int fail = 0;
   if (to_host) {
@@ -1840,7 +1932,7 @@ int rcc_ba_linearize(rcc_ba_problem* P, double* cost) {
   API_BEGIN(P)
   do_linearize(P);
   if (cost) {
-    std::vector<double> c2((size_t)P->n_cam);
+    std::vector<double> c2((size_t)P->n_cam + P->n_prior_parts);   // the cameras', then the priors' cost
     int32_t fail = 0;
     P->cost2_cam.download(c2.data(), c2.size(), P->stream);
     RCC_CUDA(cudaMemcpyAsync(&fail, P->fail_flag.p, sizeof(int32_t), cudaMemcpyDeviceToHost, P->stream));

@@ -154,6 +154,15 @@ struct rcc_ba_problem {
   int f_piece_lens_ptr[PIX_PIECES * rcc::N_LENSES + 1] = {0};
   std::vector<rcc::Chunk> e_chunks_h, f_chunks_h;   // host copies of the chunk records (the lens lists come from them)
   std::vector<int32_t> f_piece_list_h;
+  // Gaussian priors (rcc_ba_set_priors), per rcc_block_kind on the host: index, mean (6 doubles per prior) and A
+  // (36: row-major 6 x 6 holding the k x k matrix, zero padded).  On the device the kinds lie back to back in kind
+  // order, the priors of kind t at [prior_off[t], prior_off[t+1]).
+  std::vector<int32_t> prior_index_h[rcc::PRIOR_KINDS];
+  std::vector<double> prior_mean_h[rcc::PRIOR_KINDS], prior_A_h[rcc::PRIOR_KINDS];
+  int prior_off[rcc::PRIOR_KINDS + 1] = {0};
+  int n_prior_parts = 0;             // cost partials of launch_prior (0: no priors, and no prior launches)
+  rcc::DBuf<int32_t> prior_index;
+  rcc::DBuf<double> prior_mean, prior_A, prior_AtA;
   rcc::StageTimer timer;
   rcc::DBuf<double> flush_buf;
 

@@ -53,15 +53,34 @@ def shard_scene(scene, rank, world, eliminate="auto"):
     return s, (lo, hi)
 
 
+def shard_priors(priors, elim_view, rank, owned):
+    """The priors rank `rank`, owner of the eliminated blocks owned = (lo, hi), adds (rcc_ba_comm_init): priors on
+    kept blocks and on the shared intr / dist / ext blocks go to rank 0, priors on an eliminated block to the rank
+    that owns it.  priors: {kind: (index, mean, sqrt_information)}, kind "view" | "marker" | "intr" | "dist" | "ext";
+    returns the same for this rank."""
+    out = {}
+    for kind, (index, mean, A) in priors.items():
+        index = np.asarray(index, dtype=np.int64).reshape(-1)
+        if kind in ("view", "marker") and (kind == "view") == elim_view:
+            lo, hi = owned
+            keep = (index >= lo) & (index < hi)
+        else:
+            keep = np.full(len(index), rank == 0)
+        out[kind] = (index[keep], np.asarray(mean)[keep], np.asarray(A)[keep])
+    return out
+
+
 class DistributedBA:
     """One rank of a multi-GPU bundle adjustment.  Usage (under torchrun):
 
         dba = DistributedBA(scene, device=local_rank)      # scene = the FULL problem on every rank
+        # priors={kind: (index, mean, sqrt_information)} (BAProblem.set_priors), the same full set on every rank:
+        # each prior is added on exactly one rank (shard_priors)
         summary = dba.solve(max_iterations=30)
         views, markers, intr, dist = dba.gather_parameters()
     """
 
-    def __init__(self, scene, device=0, eliminate="auto", rank=None, world=None, process_group=None):
+    def __init__(self, scene, device=0, eliminate="auto", rank=None, world=None, process_group=None, priors=None):
         import torch.distributed as dist
         from .problem import BAProblem
         self.dist = dist
@@ -73,6 +92,9 @@ class DistributedBA:
         self.local, self.range = shard_scene(scene, self.rank, self.world, eliminate)
         self.problem = BAProblem.from_scene(self.local, device=device,
                                             eliminate="views" if self.elim_view else "markers")
+        if priors:
+            for kind, (index, mean, A) in shard_priors(priors, self.elim_view, self.rank, self.range).items():
+                self.problem.set_priors(kind, index, mean, A)
         if self.world > 1:
             ids = [BAProblem.comm_unique_id() if self.rank == 0 else None]
             dist.broadcast_object_list(ids, src=0, group=process_group)

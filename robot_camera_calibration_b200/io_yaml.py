@@ -243,15 +243,37 @@ def write_results(directory, scene, tag_ids, frames, precision=None):
             f.write(head + world_T_camera_text(scene.views[v, 0:3], scene.views[v, 3:6], precision))
 
 
+def intrinsics_priors(intr, dist, sigma):
+    """Diagonal priors that keep every camera's intr and dist near (intr, dist): sigma = (focal px, principal point
+    px, distortion coefficient), the standard deviations of fx fy, of cx cy and of every distortion entry.  Returns
+    {kind: (index, mean, sqrt_information)} for BAProblem.set_priors."""
+    f, c, d = (float(x) for x in sigma)
+    if not (f > 0 and c > 0 and d > 0 and np.isfinite([f, c, d]).all()):
+        raise ValueError(f"intrinsics sigmas must be positive and finite, got {sigma}")
+    intr, dist = np.asarray(intr, dtype=np.float64), np.asarray(dist, dtype=np.float64)
+    n = len(intr)
+    a_intr = np.diag([1 / f, 1 / f, 1 / c, 1 / c])
+    a_dist = np.eye(5) / d
+    return {"intr": (np.arange(n), intr, np.broadcast_to(a_intr, (n, 4, 4))),
+            "dist": (np.arange(n), dist, np.broadcast_to(a_dist, (n, 5, 5)))}
+
+
 def optimise_directory(directory, device=0, refine_intrinsics=True, precision=None, intr=None, dist=None,
-                       lens=None, **lm_options):
+                       lens=None, intrinsics_sigma=None, **lm_options):
     """Milestone 3: detections/ -> GPU bundle adjustment -> detections/ (same formats).  The lens is camera.yaml's
-    distortion_model (plumb_bob, or equidistant / fisheye), and camera_refined.yaml is written in the same model."""
+    distortion_model (plumb_bob, or equidistant / fisheye), and camera_refined.yaml is written in the same model.
+    intrinsics_sigma = (focal px, principal point px, distortion): refine the intrinsics under a diagonal Gaussian
+    prior centred on camera.yaml (intrinsics_priors) instead of freely; it needs refine_intrinsics."""
     from .problem import BAProblem
+    if intrinsics_sigma is not None and not refine_intrinsics:
+        raise ValueError("intrinsics_sigma puts a prior on refined intrinsics: it cannot be combined with fixed ones")
     scene, tag_ids, frames = read_dataset(directory, intr=intr, dist=dist, lens=lens)
     scene.const_intr[:] = not refine_intrinsics
     scene.const_dist[:] = not refine_intrinsics
     with BAProblem.from_scene(scene, device=device) as p:
+        if intrinsics_sigma is not None:
+            for kind, args in intrinsics_priors(scene.intr, scene.dist, intrinsics_sigma).items():
+                p.set_priors(kind, *args)
         summary = p.solve(**lm_options)
         scene.views, scene.markers = p.get_view_poses(), p.get_marker_poses()
         intr, dist = p.get_intrinsics()

@@ -26,6 +26,13 @@ _BLOCK_KINDS = {"view": L.BLOCK_VIEW, "marker": L.BLOCK_MARKER, "intr": L.BLOCK_
 _BLOCK_SIZES = {L.BLOCK_VIEW: 6, L.BLOCK_MARKER: 6, L.BLOCK_INTR: 4, L.BLOCK_DIST: 5, L.BLOCK_EXT: 6}
 
 
+def sqrt_information(cov):
+    """The sqrt_information A of a Gaussian prior whose covariance is cov: A = L^-1 for cov = L L^T (Cholesky), so
+    that ||A (x - mu)||^2 = (x - mu)^T cov^-1 (x - mu).  cov is one k x k matrix or a stack (..., k, k)."""
+    L_ = np.linalg.cholesky(np.asarray(cov, dtype=np.float64))
+    return np.linalg.solve(L_, np.broadcast_to(np.eye(L_.shape[-1]), L_.shape))
+
+
 def _f64(a, shape=None):
     a = np.ascontiguousarray(a, dtype=np.float64)
     if shape is not None:
@@ -182,6 +189,26 @@ class BAProblem:
             codes = np.array([L.LENSES[n] for n in names], dtype=np.int32)
             self._check(self.lib.rcc_ba_set_camera_lenses(self.h, _ip(codes)))
         self.lens = names[0] if len(set(names)) == 1 else names
+
+    def set_priors(self, kind, index, mean, sqrt_information):
+        """Gaussian priors (ceres::NormalPrior) on the blocks of one kind: the residual block A_i (x_i - mu_i) on block
+        index[i], mean (n, k), sqrt_information (n, k, k) with k the kind's block size (view / marker / ext 6, intr 4,
+        dist 5).  Replaces every earlier prior of that kind; an empty index clears them (rcc_ba_set_priors).  For a
+        covariance Sigma use sqrt_information(Sigma)."""
+        kind = _BLOCK_KINDS[kind] if isinstance(kind, str) else int(kind)
+        k = _BLOCK_SIZES.get(kind, 6)
+        idx = np.ascontiguousarray(index, dtype=np.int32).reshape(-1)
+        n = len(idx)
+        mu = _f64(mean, (n, k))
+        A = _f64(sqrt_information, (n, k, k))
+        self._check(self.lib.rcc_ba_set_priors(self.h, kind, n, _ip(idx), _dp(mu), _dp(A)))
+
+    def clear_priors(self, kind=None):
+        """Remove the priors of one kind, or of every kind (kind=None)."""
+        kinds = [kind] if kind is not None else ["view", "marker", "intr", "dist"] + (["ext"] if self.model == "rig" else [])
+        for k in kinds:
+            k = _BLOCK_KINDS[k] if isinstance(k, str) else int(k)
+            self._check(self.lib.rcc_ba_set_priors(self.h, k, 0, None, None, None))
 
     # ------------------------------------------------------------------ getters
     def get_intrinsics(self):
