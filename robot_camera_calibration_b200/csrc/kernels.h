@@ -76,7 +76,7 @@ struct AssembleArgs {
 
 // K2: fused residual + Jacobian + J^T J tiles.  own_is_view tells which pose
 // table the segment owner indexes; lens is a Lens (model.cuh) other than LENS_PER_CAMERA: with mixed lenses the
-// caller launches once per lens, each launch covering that lens's chunks through chunk_list.  Under the equidistant
+// caller launches once per lens, over that lens's chunks (problem.cu: plan_launches).  Under the equidistant
 // lens tile B holds [cx cy k1 k2 k3 k4 0 | r]: the reserved slot's column is zero.
 constexpr int N_LENSES = 2;   // LENS_RADTAN, LENS_EQUIDISTANT
 void launch_assemble(bool rig, bool epass, bool own_is_view, int lens, const AssembleArgs& a, cudaStream_t s);
@@ -190,7 +190,7 @@ struct EvalArgs {
 };
 int eval_grid(int64_t n);   // CTAs launch_evaluate / launch_cost will use
 // lens is a Lens; LENS_PER_CAMERA only without Jacobians (K6).  K1 takes one lens per launch: with mixed lenses the
-// caller launches it once per lens over that lens's chunks.
+// caller launches it once per lens over a lens-ordered copy of the chunk records (problem.cu: plan_launches).
 void launch_evaluate(bool rig, bool want_jac, int lens, const EvalArgs& a, cudaStream_t s);
 // number of cost partials launch_evaluate writes (want_jac: one per chunk; else one per CTA)
 int eval_partials(bool want_jac, const EvalArgs& a);

@@ -117,6 +117,7 @@ rcc_ba_problem::~rcc_ba_problem() {
 }
 
 typedef rcc_ba_problem P_t;
+typedef rcc_ba_problem::Run Run;
 
 #define RCC_NCCL(expr)                                                                                         \
   do {                                                                                                         \
@@ -222,14 +223,20 @@ static void make_chunks(const std::vector<int32_t>& perm, const std::vector<int3
   }
 }
 
+// counting sort of the ids 0 .. n by key(id) < n_groups: group g is list[ptr[g] .. ptr[g+1]), ascending
+template <typename Key>
+static void group_by(size_t n, int n_groups, Key key, std::vector<int32_t>& list, std::vector<int32_t>& ptr) {
+  ptr.assign((size_t)n_groups + 1, 0);
+  for (size_t i = 0; i < n; ++i) ptr[key(i) + 1]++;
+  for (int g = 0; g < n_groups; ++g) ptr[g + 1] += ptr[g];
+  list.resize(n);
+  std::vector<int32_t> cur(ptr.begin(), ptr.end() - 1);
+  for (size_t i = 0; i < n; ++i) list[cur[key(i)]++] = (int32_t)i;
+}
+
 static void cam_lists(const std::vector<Chunk>& chunks, int n_cam, std::vector<int32_t>& list,
                       std::vector<int32_t>& ptr) {
-  ptr.assign((size_t)n_cam + 1, 0);
-  for (auto& c : chunks) ptr[c.cam + 1]++;
-  for (int i = 0; i < n_cam; ++i) ptr[i + 1] += ptr[i];
-  list.resize(chunks.size());
-  std::vector<int32_t> cur(ptr.begin(), ptr.end() - 1);
-  for (size_t i = 0; i < chunks.size(); ++i) list[cur[chunks[i].cam]++] = (int32_t)i;
+  group_by(chunks.size(), n_cam, [&](size_t c) { return chunks[c].cam; }, list, ptr);
 }
 
 static int env_int(const char* name, int dflt) {
@@ -237,45 +244,69 @@ static int env_int(const char* name, int dflt) {
   return (v && *v) ? atoi(v) : dflt;
 }
 
-// the per-lens chunk lists of a handle whose cameras mix lenses (problem.h: lens_chunks_e ...), from the chunk
-// records and the cameras' lenses; nothing to do when every camera has the same lens
-static void build_lens_lists(P_t* P) {
-  if (!P->lens_mixed || !P->have_obs) return;
-  cudaStream_t s = P->stream;
-  auto by_lens = [&](const std::vector<Chunk>& chunks, std::vector<int32_t>& list, int* ptr) {
-    list.clear();
-    for (int l = 0; l < N_LENSES; ++l) {
-      ptr[l] = (int)list.size();
-      for (size_t c = 0; c < chunks.size(); ++c)
-        if (P->cam_lens[chunks[c].cam] == l) list.push_back((int32_t)c);
+// the lens every camera has, or LENS_PER_CAMERA when they differ
+static int handle_lens(const P_t* P) {
+  for (int32_t l : P->cam_lens)
+    if (l != P->cam_lens[0]) return LENS_PER_CAMERA;
+  return P->cam_lens[0];
+}
+
+// The K2 and K1 runs (problem.h: Run) from the chunk records, the upload pieces and the cameras' lenses.  A pass, or
+// each upload piece of it, is launched once per lens among its chunks, in lens order, the ids ascending; a run whose
+// ids form a contiguous range needs no id list.  With one lens for every camera a pass or a piece is one run, even
+// without chunks (launch_assemble then returns at once; the run still counts as a launch); an upload piece without E
+// chunks has no runs, and neither has any piece unless the caller order is the E-sorted order (pix_identity).
+static void plan_launches(P_t* P) {
+  if (!P->have_obs) return;
+  const int common = handle_lens(P);
+  std::vector<int32_t> ids, list, ptr;
+  auto plan = [&](const std::vector<Chunk>& chunks, int n_groups, auto group_of, std::vector<Run>* runs) {
+    group_by(chunks.size(), n_groups * N_LENSES,
+             [&](size_t c) { return group_of(c) * N_LENSES + P->cam_lens[chunks[c].cam]; }, list, ptr);
+    for (int g = 0; g < n_groups; ++g) {
+      runs[g].clear();
+      for (int l = 0; l < N_LENSES; ++l) {
+        const int lo = ptr[g * N_LENSES + l], n = ptr[g * N_LENSES + l + 1] - lo;
+        if (n == 0 && l != common) continue;
+        const bool listed = n > 0 && list[lo + n - 1] - list[lo] != n - 1;
+        runs[g].push_back(Run{l, listed ? (int)ids.size() : n > 0 ? list[lo] : 0, n, listed});
+        if (listed) ids.insert(ids.end(), list.begin() + lo, list.begin() + lo + n);
+      }
     }
-    ptr[N_LENSES] = (int)list.size();
   };
-  std::vector<int32_t> le, lf, fp;
-  by_lens(P->e_chunks_h, le, P->lens_ptr_e);
-  by_lens(P->f_chunks_h, lf, P->lens_ptr_f);
-  std::vector<Chunk> recs(le.size());
-  for (size_t i = 0; i < le.size(); ++i) recs[i] = P->e_chunks_h[le[i]];
-  // E piece k is the chunk range [piece_chunk[k], piece_chunk[k+1]): its part of each ascending lens list
-  for (int l = 0; l < N_LENSES; ++l)
-    for (int k = 0; k <= rcc_ba_problem::PIX_PIECES; ++k)
-      P->lens_piece_e[l][k] = (int)(std::lower_bound(le.begin() + P->lens_ptr_e[l], le.begin() + P->lens_ptr_e[l + 1],
-                                                     P->piece_chunk[k]) - le.begin());
-  // F piece k is f_piece_list[f_piece_ptr[k] .. f_piece_ptr[k+1]): regrouped by lens
-  for (int k = 0; k < rcc_ba_problem::PIX_PIECES; ++k)
-    for (int l = 0; l < N_LENSES; ++l) {
-      P->f_piece_lens_ptr[k * N_LENSES + l] = (int)fp.size();
-      for (int i = P->f_piece_ptr[k]; i < P->f_piece_ptr[k + 1]; ++i)
-        if (P->cam_lens[P->f_chunks_h[P->f_piece_list_h[i]].cam] == l) fp.push_back(P->f_piece_list_h[i]);
+  constexpr int NP = rcc_ba_problem::PIX_PIECES;
+  if (P->pix_identity) {
+    std::vector<int32_t> e_piece(P->e_chunks_h.size());
+    for (int k = 0; k < NP; ++k)
+      for (int c = P->piece_chunk[k]; c < P->piece_chunk[k + 1]; ++c) e_piece[c] = k;
+    plan(P->e_chunks_h, NP, [&](size_t c) { return e_piece[c]; }, P->piece_runs_e);
+    plan(P->f_chunks_h, NP, [&](size_t c) { return P->f_chunk_piece_h[c]; }, P->piece_runs_f);
+  }
+  for (int k = 0; k < NP; ++k)
+    if (!P->pix_identity || P->piece_chunk[k + 1] <= P->piece_chunk[k]) {
+      P->piece_runs_e[k].clear();
+      P->piece_runs_f[k].clear();
     }
-  P->f_piece_lens_ptr[rcc_ba_problem::PIX_PIECES * N_LENSES] = (int)fp.size();
-  for (auto* v : {&le, &lf, &fp})
-    if (v->empty()) v->push_back(0);
-  if (recs.empty()) recs.push_back(Chunk{0, 0, 0, 0});
-  P->lens_chunks_e.upload(le, s);
-  P->lens_chunks_f.upload(lf, s);
-  P->f_piece_lens.upload(fp, s);
-  P->lens_recs_e.upload(recs, s);
+  plan(P->f_chunks_h, 1, [](size_t) { return 0; }, &P->runs_f);
+  plan(P->e_chunks_h, 1, [](size_t) { return 0; }, &P->runs_e);
+  // K1: the E runs as positions of `list` (the E chunk ids in lens order); a copy of the records unless that order
+  // is the chunk order
+  bool copy = false;
+  for (size_t i = 0; i < list.size(); ++i) copy |= list[i] != (int32_t)i;
+  P->runs_k1 = P->runs_e;
+  for (int i = 0, pos = 0; i < (int)P->runs_k1.size(); pos += P->runs_k1[i++].count) {
+    P->runs_k1[i].first = pos;
+    P->runs_k1[i].listed = copy;
+  }
+  cudaStream_t s = P->stream;
+  if (copy) {
+    std::vector<Chunk> recs(list.size());
+    for (size_t i = 0; i < list.size(); ++i) recs[i] = P->e_chunks_h[list[i]];
+    P->k1_chunks.upload(recs, s);
+  } else {
+    P->k1_chunks.release();
+  }
+  P->run_ids.upload(ids, s);
   RCC_CUDA(cudaStreamSynchronize(s));
 }
 
@@ -369,18 +400,8 @@ static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker
       for (int64_t i = 0; i < n; ++i) group[i] = piece_of_e[e_of[perm_f[i]]];
     }
     make_chunks(perm_f, seg_f, cam_idx, P->n_f, bpw, ch_max, chunks, chunk_ptr, P->pix_identity ? &group : nullptr);
-    std::vector<int32_t> plist;
-    plist.reserve(chunks.size());
-    for (int k = 0; k < rcc_ba_problem::PIX_PIECES; ++k) {
-      P->f_piece_ptr[k] = (int)plist.size();
-      if (P->pix_identity)
-        for (size_t c = 0; c < chunks.size(); ++c)
-          if (group[chunks[c].start] == k) plist.push_back((int32_t)c);
-    }
-    P->f_piece_ptr[rcc_ba_problem::PIX_PIECES] = (int)plist.size();
-    P->f_piece_list_h = plist;
-    if (plist.empty()) plist.push_back(0);
-    P->f_piece_list.upload(plist, s);
+    P->f_chunk_piece_h.resize(chunks.size());
+    for (size_t c = 0; c < chunks.size(); ++c) P->f_chunk_piece_h[c] = group[chunks[c].start];
   }
   P->n_chunks_f = (int)chunks.size();
   P->f_chunks.upload(chunks, s);
@@ -534,7 +555,7 @@ static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker
   RCC_CUDA(cudaStreamSynchronize(s));
   P->have_obs = true;
   P->linearized = P->schur_done = P->step_ready = P->cand_ready = false;
-  build_lens_lists(P);
+  plan_launches(P);
 }
 
 static void refresh_constants(P_t* P) {
@@ -578,18 +599,19 @@ static void ensure_pixels(P_t* P) {
   P->pix_pending = false;
 }
 
-// K2 over the chunks of a handle whose cameras mix lenses: one launch per lens l, covering list[lo[l] .. hi[l]).
-// a.chunks and a.partials are the whole pass's (the list holds chunk ids).  Returns the launches issued.
-static int assemble_by_lens(P_t* P, bool epass, AssembleArgs a, const int32_t* list, const int* lo, const int* hi) {
-  int n = 0;
-  for (int l = 0; l < N_LENSES; ++l) {
-    if (hi[l] <= lo[l]) continue;
-    a.chunk_list = list + lo[l];
-    a.n_chunks = hi[l] - lo[l];
-    launch_assemble(P->rig, epass, epass ? P->elim_view : !P->elim_view, l, a, P->stream);
-    ++n;
+// K2 over one run of a pass; a.chunks and a.partials are the whole pass's
+static void assemble_run(P_t* P, bool epass, AssembleArgs a, const Run& r) {
+  const int part = epass ? (P->rig ? PassGeom<true>::PART_E : PassGeom<false>::PART_E)
+                         : (P->rig ? PassGeom<true>::PART_F : PassGeom<false>::PART_F);
+  if (r.listed) {
+    a.chunk_list = P->run_ids.p + r.first;
+  } else {
+    a.chunks += r.first;
+    a.partials += (size_t)r.first * part;
   }
-  return n;
+  a.n_chunks = r.count;
+  launch_assemble(P->rig, epass, epass ? P->elim_view : !P->elim_view, r.lens, a, P->stream);
+  P->launch_count += 1;
 }
 
 // the priors evaluated at the current or the candidate parameters; H and g are the linearisation's blocks (used by
@@ -611,85 +633,46 @@ static void do_linearize(P_t* P) {
   RCC_REQUIRE(P->have_obs, RCC_NOT_READY, "set_observations has not been called");
   ensure_expanded(P);
   RCC_CUDA(cudaMemsetAsync(P->fail_flag.p, 0, sizeof(int32_t), P->stream));
-  AssembleArgs a{};
+  AssembleArgs e{};
+  e.view_x = P->view_x.p;
+  e.marker_x = P->marker_x.p;
+  e.ext_x = P->ext_x.p;
+  e.shared = P->shared.p;
+  e.fail_flag = P->fail_flag.p;
+  e.loss = P->loss;
+  e.loss_a2 = P->loss_scale * P->loss_scale;
+  AssembleArgs f = e;
+  e.oth = P->e_oth.p;
+  e.pix = P->e_pix.p;
+  e.chunks = P->e_chunks.p;
+  e.partials = P->part_e.p;
+  e.W = P->W.p;
+  f.oth = P->f_oth.p;
+  f.pix = P->f_pix.p;
+  f.chunks = P->f_chunks.p;
+  f.partials = P->part_f.p;
   bool f_done = false;
-  const int* lp_e = P->lens_ptr_e;
-  const int* lp_f = P->lens_ptr_f;
-  a.view_x = P->view_x.p;
-  a.marker_x = P->marker_x.p;
-  a.ext_x = P->ext_x.p;
-  a.shared = P->shared.p;
-  a.fail_flag = P->fail_flag.p;
-  a.loss = P->loss;
-  a.loss_a2 = P->loss_scale * P->loss_scale;
   {
-    Scoped t(P, ST_ASSEMBLE_E, P->pix_pending ? 0 : 1);
-    a.oth = P->e_oth.p;
-    a.pix = P->e_pix.p;
-    a.chunks = P->e_chunks.p;
-    a.n_chunks = P->n_chunks_e;
-    a.partials = P->part_e.p;
-    a.W = P->W.p;
+    Scoped t(P, ST_ASSEMBLE_E, 0);
     if (P->pix_pending) {
       // pixels are still arriving on the side stream: the E pass of a piece starts when the piece has landed,
       // and so does its F pass on large uploads (the piece scattered itself into f_pix, and no F chunk straddles
       // pieces)
-      const int part = P->rig ? PassGeom<true>::PART_E : PassGeom<false>::PART_E;
       f_done = P->n_obs >= rcc_ba_problem::LARGE_UPLOAD_BLOCKS;
       for (int k = 0; k < rcc_ba_problem::PIX_PIECES; ++k) {
-        const int c0 = P->piece_chunk[k], c1 = P->piece_chunk[k + 1];
         RCC_CUDA(cudaStreamWaitEvent(P->stream, P->ev_piece[k], 0));
-        if (c1 <= c0) continue;
-        if (P->lens_mixed) {
-          const int lo[N_LENSES] = {P->lens_piece_e[0][k], P->lens_piece_e[1][k]};
-          const int hi[N_LENSES] = {P->lens_piece_e[0][k + 1], P->lens_piece_e[1][k + 1]};
-          P->launch_count += assemble_by_lens(P, true, a, P->lens_chunks_e.p, lo, hi);
-          if (!f_done) continue;
-          AssembleArgs af = a;
-          af.oth = P->f_oth.p;
-          af.pix = P->f_pix.p;
-          af.chunks = P->f_chunks.p;
-          af.partials = P->part_f.p;
-          af.W = nullptr;
-          const int* fp = P->f_piece_lens_ptr + k * N_LENSES;
-          P->launch_count += assemble_by_lens(P, false, af, P->f_piece_lens.p, fp, fp + 1);
-          continue;
-        }
-        AssembleArgs ak = a;
-        ak.chunks = P->e_chunks.p + c0;
-        ak.n_chunks = c1 - c0;
-        ak.partials = P->part_e.p + (size_t)c0 * part;
-        launch_assemble(P->rig, true, P->elim_view, P->lens, ak, P->stream);
-        P->launch_count += 1;
-        if (!f_done) continue;
-        AssembleArgs af = a;
-        af.oth = P->f_oth.p;
-        af.pix = P->f_pix.p;
-        af.chunks = P->f_chunks.p;
-        af.chunk_list = P->f_piece_list.p + P->f_piece_ptr[k];
-        af.n_chunks = P->f_piece_ptr[k + 1] - P->f_piece_ptr[k];
-        af.partials = P->part_f.p;
-        af.W = nullptr;
-        launch_assemble(P->rig, false, !P->elim_view, P->lens, af, P->stream);
-        P->launch_count += 1;
+        for (const Run& r : P->piece_runs_e[k]) assemble_run(P, true, e, r);
+        if (f_done)
+          for (const Run& r : P->piece_runs_f[k]) assemble_run(P, false, f, r);
       }
-    } else if (P->lens_mixed) {
-      P->launch_count += assemble_by_lens(P, true, a, P->lens_chunks_e.p, lp_e, lp_e + 1) - 1;
     } else {
-      launch_assemble(P->rig, true, P->elim_view, P->lens, a, P->stream);
+      for (const Run& r : P->runs_e) assemble_run(P, true, e, r);
     }
   }
   ensure_pixels(P);
   if (!f_done) {
-    Scoped t(P, ST_ASSEMBLE_F, 1);
-    a.oth = P->f_oth.p;
-    a.pix = P->f_pix.p;
-    a.chunks = P->f_chunks.p;
-    a.n_chunks = P->n_chunks_f;
-    a.partials = P->part_f.p;
-    a.W = nullptr;
-    if (P->lens_mixed) P->launch_count += assemble_by_lens(P, false, a, P->lens_chunks_f.p, lp_f, lp_f + 1) - 1;
-    else launch_assemble(P->rig, false, !P->elim_view, P->lens, a, P->stream);
+    Scoped t(P, ST_ASSEMBLE_F, 0);
+    for (const Run& r : P->runs_f) assemble_run(P, false, f, r);
   }
   {
     Scoped t(P, ST_FINALIZE, P->n_prior_parts > 0 ? 2 : 1);
@@ -1198,9 +1181,6 @@ static EvalArgs eval_args(P_t* P, bool cand) {
   return a;
 }
 
-// the lens argument of launch_evaluate / launch_cost without Jacobians (K6 picks the lens per block when mixed)
-static int cost_lens(const P_t* P) { return P->lens_mixed ? LENS_PER_CAMERA : P->lens; }
-
 static void do_candidate_cost(P_t* P) {
   RCC_REQUIRE(P->step_ready, RCC_NOT_READY, "solve_step has not been called");
   ensure_pixels(P);
@@ -1214,7 +1194,7 @@ static void do_candidate_cost(P_t* P) {
     EvalArgs a = eval_args(P, true);
     a.fail_flag = P->fail_flag.p + 1;   // slot 1: candidate point (slot 0 keeps the linearisation point's flag)
     RCC_CUDA(cudaMemsetAsync(a.fail_flag, 0, sizeof(int32_t), P->stream));
-    launch_cost(P->rig, cost_lens(P), a, P->stream);
+    launch_cost(P->rig, handle_lens(P), a, P->stream);
     const int np = eval_grid(P->n_obs);
     if (P->n_prior_parts > 0) launch_prior(false, prior_args(P, true, P->cost_partials.p + np), P->stream);
     launch_sum(P->cost_partials.p, np + P->n_prior_parts, P->stats.p + SX_CAND2, 1.0, P->stream);
@@ -1712,14 +1692,10 @@ static void set_camera_lenses(P_t* P, const int32_t* lenses) {
   for (int c = 0; c < P->n_cam; ++c)
     RCC_REQUIRE(lenses[c] == RCC_LENS_RADTAN || lenses[c] == RCC_LENS_EQUIDISTANT, RCC_BAD_ARG, "unknown lens");
   P->cam_lens.assign(lenses, lenses + P->n_cam);
-  P->lens = lenses[0];
-  P->lens_mixed = false;
   P->cam_equidistant = 0;
-  for (int c = 0; c < P->n_cam; ++c) {
-    P->lens_mixed |= lenses[c] != lenses[0];
+  for (int c = 0; c < P->n_cam; ++c)
     if (lenses[c] == RCC_LENS_EQUIDISTANT) P->cam_equidistant |= 1u << c;
-  }
-  build_lens_lists(P);
+  plan_launches(P);
   P->const_dirty = true;   // the reserved slot of an equidistant camera is held constant
   P->linearized = P->schur_done = P->step_ready = P->cand_ready = false;
 }
@@ -1866,24 +1842,21 @@ static int evaluate_impl(P_t* P, int want_j, double* cost, bool to_host, double*
   a.fail_flag = P->fail_flag.p + 2;   // slot 2: materialised evaluation
   RCC_CUDA(cudaMemsetAsync(a.fail_flag, 0, sizeof(int32_t), P->stream));
   {
-    Scoped t(P, ST_EVALUATE, P->n_prior_parts > 0 ? 3 : 2);
-    if (P->lens_mixed && want_j) {
-      // K1 once per lens over a lens-major copy of the E chunk records; outputs go to caller positions and the cost
-      // partials stay one per chunk, so the launches are independent
-      int n = 0;
-      for (int l = 0; l < N_LENSES; ++l) {
-        const int c0 = P->lens_ptr_e[l], c1 = P->lens_ptr_e[l + 1];
-        if (c1 <= c0) continue;
+    Scoped t(P, ST_EVALUATE, P->n_prior_parts > 0 ? 2 : 1);
+    if (want_j) {
+      // K1 once per run; outputs go to caller positions and the cost partials stay one per chunk, so the launches
+      // are independent
+      for (const Run& r : P->runs_k1) {
         EvalArgs b = a;
-        b.chunks = P->lens_recs_e.p + c0;
-        b.n_chunks = c1 - c0;
-        b.cost2_partials = a.cost2_partials + c0;
-        launch_evaluate(P->rig, true, l, b, P->stream);
-        ++n;
+        b.chunks = (r.listed ? P->k1_chunks.p : P->e_chunks.p) + r.first;
+        b.n_chunks = r.count;
+        b.cost2_partials = a.cost2_partials + r.first;
+        launch_evaluate(P->rig, true, r.lens, b, P->stream);
+        P->launch_count += 1;
       }
-      P->launch_count += n - 1;
     } else {
-      launch_evaluate(P->rig, want_j != 0, want_j ? P->lens : cost_lens(P), a, P->stream);
+      launch_evaluate(P->rig, false, handle_lens(P), a, P->stream);
+      P->launch_count += 1;
     }
     const int np = eval_partials(want_j != 0, a);
     if (P->n_prior_parts > 0) launch_prior(false, prior_args(P, false, P->cost_partials.p + np), P->stream);

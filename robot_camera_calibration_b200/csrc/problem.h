@@ -92,8 +92,8 @@ struct rcc_ba_problem {
   rcc::DBuf<char> staging;           // caller's pixels on the device, of any element type, before launch_load_pixels
   rcc::DBuf<rcc::Chunk> e_chunks, f_chunks;
   rcc::DBuf<int32_t> cam_chunks_e, cam_ptr_e, cam_chunks_f, cam_ptr_f;
-  rcc::DBuf<int32_t> f_piece_list;   // F-pass chunk ids grouped by upload piece
-  int f_piece_ptr[PIX_PIECES + 1] = {0};
+  std::vector<rcc::Chunk> e_chunks_h, f_chunks_h;   // host copies of the chunk records (plan_launches)
+  std::vector<int32_t> f_chunk_piece_h;             // the upload piece of each F chunk (pix_identity)
   std::vector<int32_t> row_ptr_h;    // row_ptr on the host (rcc_ba_covariance_blocks plans its work from it)
   rcc::DBuf<int32_t> row_ptr, pair_e, pair_f, pair_mptr, pair_members, row_pos0, col_ptr, col_pair, tile_ptr, syrk_ctas, e_count;
   rcc::DBuf<uint8_t> e_const;
@@ -140,20 +140,15 @@ struct rcc_ba_problem {
   // lenses (rcc_ba_set_lens, rcc_ba_set_camera_lenses).  With a communicator attached every rank sets the same lenses;
   // nothing in the multi-rank path depends on them.
   std::vector<int32_t> cam_lens;     // rcc::Lens of each camera
-  bool lens_mixed = false;           // the cameras do not all have the same lens
-  int lens = 0;                      // !lens_mixed: the lens of every camera
   uint32_t cam_equidistant = 0;      // bit c: camera c is equidistant (K6 under LENS_PER_CAMERA)
-  // lens_mixed: K2 and K1 run once per lens.  lens_chunks_e/f hold the chunk ids of lens l in ascending order at
-  // [lens_ptr_e/f[l], lens_ptr_e/f[l+1]); lens_recs_e the E chunk records in that order (K1's chunk array).  Upload
-  // piece k of E covers positions [lens_piece_e[l][k], lens_piece_e[l][k+1]) of lens_chunks_e, and of F the positions
-  // [f_piece_lens_ptr[2k+l], f_piece_lens_ptr[2k+l+1]) of f_piece_lens (f_piece_list regrouped by lens in each piece).
-  rcc::DBuf<int32_t> lens_chunks_e, lens_chunks_f, f_piece_lens;
-  rcc::DBuf<rcc::Chunk> lens_recs_e;
-  int lens_ptr_e[rcc::N_LENSES + 1] = {0}, lens_ptr_f[rcc::N_LENSES + 1] = {0};
-  int lens_piece_e[rcc::N_LENSES][PIX_PIECES + 1] = {{0}};
-  int f_piece_lens_ptr[PIX_PIECES * rcc::N_LENSES + 1] = {0};
-  std::vector<rcc::Chunk> e_chunks_h, f_chunks_h;   // host copies of the chunk records (the lens lists come from them)
-  std::vector<int32_t> f_piece_list_h;
+  // The K2 and K1 launches (plan_launches): one run per lens, and per upload piece for the piecewise path.  A run
+  // covers `count` chunks of its pass: the chunk ids [first, first + count), or with `listed` the ids at
+  // run_ids.p + first.  K1 has no id list: its runs are positions [first, first + count) of the E chunks in lens order,
+  // read from k1_chunks (that order's copy of the records) when `listed`, else from e_chunks.
+  struct Run { int lens, first, count; bool listed; };
+  std::vector<Run> runs_e, runs_f, runs_k1, piece_runs_e[PIX_PIECES], piece_runs_f[PIX_PIECES];
+  rcc::DBuf<int32_t> run_ids;
+  rcc::DBuf<rcc::Chunk> k1_chunks;
   // Gaussian priors (rcc_ba_set_priors), per rcc_block_kind on the host: index, mean (6 doubles per prior) and A
   // (36: row-major 6 x 6 holding the k x k matrix, zero padded).  On the device the kinds lie back to back in kind
   // order, the priors of kind t at [prior_off[t], prior_off[t+1]).

@@ -202,21 +202,33 @@ def test_update_pixels_matches_a_fresh_problem(shuffled):
     rng = np.random.default_rng(7)
     pix2 = np.ascontiguousarray(s.pixels + rng.normal(0.0, 0.5, s.pixels.shape))
     pix3 = np.ascontiguousarray(s.pixels + rng.normal(0.0, 0.5, s.pixels.shape))
-    with BAProblem.from_scene(s) as gp:
+    launches = []
+
+    def linearize(gp):
+        n0 = gp.launch_count()
+        c = gp.linearize()
+        launches.append(gp.launch_count() - n0)
+        return c
+
+    # views are eliminated: make_scene's view-major caller order is then the E-sorted order
+    with BAProblem.from_scene(s, eliminate="views") as gp:
         gp.linearize()
         gp.update_pixels(pix2)
-        c2 = gp.linearize()
+        c2 = linearize(gp)
         nb2 = gp.normal_blocks()
         gp.update_pixels(pix3)
         gp.update_pixels(pix2)                       # overwritten before anything consumed it
         e2 = gp.evaluate(want_jacobians=False)
         gp.update_pixels(pix3)
-        c3 = gp.linearize()
+        c3 = linearize(gp)
+    # the poses stay expanded; K2's E pass runs once per upload piece (4 below LARGE_UPLOAD_BLOCKS) or once, then
+    # the F pass and finalize
+    assert launches == [(1 if shuffled else 4) + 2] * 2
     ref = make_scene(60, 40, 0.7, seed=58)
     ref.view_idx, ref.marker_idx, ref.cam_idx = s.view_idx, s.marker_idx, s.cam_idx
     for pix, cost, nb in ((pix2, c2, nb2), (pix3, c3, None)):
         ref.pixels = pix
-        with BAProblem.from_scene(ref) as gq:
+        with BAProblem.from_scene(ref, eliminate="views") as gq:
             assert gq.linearize() == cost
             if nb is not None:
                 nq = gq.normal_blocks()
@@ -239,7 +251,9 @@ def test_update_pixels_in_pieces_at_size_matches_a_fresh_problem():
         gp.linearize()
         for pix, dt in zip(new_pixels, (np.float64, np.int16)):
             gp.update_pixels(pix.astype(dt))
+            n0 = gp.launch_count()
             cost = gp.linearize()
+            assert gp.launch_count() - n0 == 8 * 2 + 1      # K2's E and F pass of each of the 8 pieces, finalize
             nb = gp.normal_blocks()
             s.pixels = pix
             with BAProblem.from_scene(s, eliminate="views") as gq:

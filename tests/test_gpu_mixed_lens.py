@@ -186,16 +186,29 @@ def _sorted_by_view(s):
     return s
 
 
+def _lenses_per_piece(s, n_pieces):
+    """How many lenses the blocks of each upload piece of a view-sorted scene have.  Piece k ends at the first view
+    that starts at or after k / n_pieces of the blocks (problem.cu: build_indices)."""
+    starts = np.append(np.flatnonzero(np.diff(s.view_idx, prepend=-1)), s.n_blocks)
+    ends = starts[np.searchsorted(starts, s.n_blocks * np.arange(1, n_pieces + 1) // n_pieces)]
+    fish = _fish(s)[s.cam_idx]
+    return np.array([len(np.unique(fish[a:b])) for a, b in zip(np.append(0, ends[:-1]), ends)])
+
+
 @pytest.mark.parametrize("name", list(SCENES))
 def test_piecewise_update_pixels_is_bitwise_set_observations(name):
     s = _sorted_by_view(_scene(name))
     pix2 = np.ascontiguousarray(s.pixels + np.random.default_rng(7).normal(0.0, 0.5, s.pixels.shape))
+    # K2's E pass once per lens of each of the 4 pieces, the F pass once per lens, finalize
+    want = _lenses_per_piece(s, 4).sum() + len(np.unique(_fish(s)[s.cam_idx])) + 1
     runs = []
     for _ in range(2):
         with BAProblem.from_scene(s, eliminate="views") as gp:
             gp.linearize()
             gp.update_pixels(pix2)
+            n0 = gp.launch_count()
             c = gp.linearize()
+            assert gp.launch_count() - n0 == want
             runs.append((c, gp.normal_blocks(), gp.evaluate(want_jacobians=False)["residuals"]))
     s.pixels = pix2
     with BAProblem.from_scene(s, eliminate="views") as gq:
@@ -219,7 +232,9 @@ def test_piecewise_update_pixels_in_pieces_at_size_is_bitwise_set_observations()
     with BAProblem.from_scene(s, eliminate="views") as gp:
         gp.linearize()
         gp.update_pixels(pix)
+        n0 = gp.launch_count()
         cost = gp.linearize()
+        assert gp.launch_count() - n0 == 2 * _lenses_per_piece(s, 8).sum() + 1    # E and F of each piece, finalize
         nb = gp.normal_blocks(want_W=False)
     s.pixels = pix
     with BAProblem.from_scene(s, eliminate="views") as gq:
