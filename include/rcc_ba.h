@@ -24,7 +24,7 @@
  *   dist[5] = k1 k2 p1 p2 k3 (:39,63-64)        [radial-tangential lens, the default]
  *           = k1 k2 k3 k4 -                       [equidistant lens, rcc_ba_set_lens / rcc_ba_set_camera_lenses]
  *   view[6] = Rodrigues rvec, t of world_T_camera (:88-98)   [rig: world_T_body]
- *   marker[6] = rvec, t of world_T_target (:111-121)
+ *   marker[6] = rvec, t of world_T_target (:111-121) or world_T_board (rcc_ba_set_corner_layout)
  *   ext[6]  = rvec, t of body_T_cam   (rig model only; not in the reference)
  * Observation block = one tag in one frame = 4 corners (bl br tr tl,
  * :123-126) = 8 residuals  u0 v0 u1 v1 u2 v2 u3 v3  (corner_detections.cpp:34-37).
@@ -190,6 +190,22 @@ int rcc_ba_set_camera_lenses(rcc_ba_problem* p, const int32_t* lenses);
  * launch for them.  With a communicator attached each rank adds the priors it was given (see rcc_ba_comm_init). */
 int rcc_ba_set_priors(rcc_ba_problem* p, int32_t block_kind, int64_t n, const int32_t* index, const double* mean,
                       const double* sqrt_information);
+
+/* Corner layout: the corners of observation block i are corners[slot[i]][k] = (x, y), k = bl br tr tl, in the frame
+ * of the block's marker (z = 0), instead of (-+s/2, -+s/2, 0) from rcc_ba_set_marker_sizes.  A marker whose blocks
+ * point at different slots is one rigid planar target (a tag board) with one 6-dof pose; slot[i] = -1 keeps the
+ * square of the marker's size for that block.  corners: n_slots x 4 x 2; slot: n_obs_blocks, caller order.
+ * n_slots == 0 clears the layout (slot may then be NULL).
+ *   - Errors, all checked before anything changes: RCC_BAD_ARG for n_slots < 0, a NULL array with n_slots > 0, a slot
+ *     outside [-1, n_slots) or a non-finite corner; then RCC_NOT_READY before rcc_ba_set_observations.
+ *   - Lifetime: rcc_ba_set_observations[_i16|_i32] clears the layout; rcc_ba_update_pixels[_i16] keeps it.  Like
+ *     rcc_ba_set_loss it invalidates the linearisation.  The call copies the caller's arrays and returns without a
+ *     stream synchronisation.
+ *   - The marker block is the target's pose: rcc_ba_get_marker_poses, jac_marker, priors, rcc_ba_set_constant and the
+ *     covariance all refer to it, as for a single tag.
+ *   - With a communicator attached every rank passes the same corners and the slots of its own blocks.
+ *   - A handle without a layout, or with its layout cleared, issues exactly the launches it issues without this call. */
+int rcc_ba_set_corner_layout(rcc_ba_problem* p, int32_t n_slots, const double* corners, const int32_t* slot);
 
 int rcc_ba_get_intrinsics(rcc_ba_problem* p, double* intr, double* dist);
 int rcc_ba_get_rig_extrinsics(rcc_ba_problem* p, double* ext);

@@ -29,6 +29,10 @@ def parser():
                       default=None,
                       help="refine the intrinsics under a Gaussian prior centred on camera.yaml: standard deviations "
                            "of fx fy, of cx cy (pixels) and of every distortion coefficient")
+    ap.add_argument("--target", action="append", default=None, metavar="FILE",
+                    help="a rigid tag board in Kalibr's AprilGrid format (target_type: aprilgrid, tagRows, tagCols, "
+                         "tagSize, tagSpacing, optional firstTagId); repeatable.  Its detected tags are solved with "
+                         "one pose per board; a tag id on two targets is an error")
     ap.add_argument("--max-iterations", type=int, default=50)
     ap.add_argument("--function-tolerance", type=float, default=None)
     ap.add_argument("--gradient-tolerance", type=float, default=None)
@@ -52,8 +56,8 @@ def main(argv=None):
     try:
         summary = io_yaml.optimise_directory(args.directory, device=args.device,
                                              refine_intrinsics=not args.fix_intrinsics, precision=args.precision,
-                                             intrinsics_sigma=args.intrinsics_sigma, **opts)
-    except (FileNotFoundError, ValueError) as e:          # missing camera.yaml / targets.yaml, empty dataset
+                                             intrinsics_sigma=args.intrinsics_sigma, targets=args.target, **opts)
+    except (FileNotFoundError, ValueError) as e:          # missing camera.yaml / targets.yaml, empty dataset, bad target
         print(f"error: {e}", file=sys.stderr)
         return 2
     summary["termination_name"] = TERMINATION.get(summary["termination"], "?")

@@ -13,8 +13,8 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "librcc_ba.so")
-SOURCES = ["assemble.cu", "assemble_equidistant.cu", "evaluate.cu", "schur.cu", "dense.cu", "problem.cu",
-           "pnp.cu", "prior.cu"]
+SOURCES = ["assemble.cu", "assemble_equidistant.cu", "assemble_target.cu", "assemble_target_equidistant.cu",
+           "evaluate.cu", "evaluate_target.cu", "schur.cu", "dense.cu", "problem.cu", "pnp.cu", "prior.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 CFLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC,-fopenmp,-O3", "-Xptxas", "-v",

@@ -78,6 +78,7 @@ SIGNATURES = {
     "rcc_ba_set_loss": (C.c_int, [_H, C.c_int32, C.c_double]),
     "rcc_ba_set_lens": (C.c_int, [_H, C.c_int32]),
     "rcc_ba_set_camera_lenses": (C.c_int, [_H, c_int32_p]),
+    "rcc_ba_set_corner_layout": (C.c_int, [_H, C.c_int32, c_double_p, c_int32_p]),
     "rcc_ba_set_priors": (C.c_int, [_H, C.c_int32, C.c_int64, c_int32_p, c_double_p, c_double_p]),
     "rcc_ba_get_intrinsics": (C.c_int, [_H, c_double_p, c_double_p]),
     "rcc_ba_get_rig_extrinsics": (C.c_int, [_H, c_double_p]),

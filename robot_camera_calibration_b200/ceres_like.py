@@ -26,13 +26,21 @@ from .problem import BAProblem
 class TagReprojectionCost:
     """CostFunction of one detected tag: 8 residuals (4 corners x (u,v)), parameter
     blocks intr[4], dist[5], view[6], marker[6] (+ ext[6] in a rig).  lens "radtan" (dist = k1 k2 p1 p2 k3) or
-    "equidistant" (dist = k1 k2 k3 k4 + a reserved slot that is held constant)."""
+    "equidistant" (dist = k1 k2 k3 k4 + a reserved slot that is held constant).
 
-    def __init__(self, pixels, tag_size, rig=False, lens="radtan"):
+    The tag's corners are the square (-+s/2, -+s/2, 0) of tag_size s, or `corners` (4 x 2: bl br tr tl, z = 0) in the
+    frame of the marker parameter block.  A marker array shared by residual blocks with different corners is one rigid
+    board (its pose is world_T_board), as a Ceres user would write it; Problem gives each distinct corner set one slot
+    of the corner layout (rcc_ba_set_corner_layout)."""
+
+    def __init__(self, pixels, tag_size=None, rig=False, lens="radtan", corners=None):
         if lens not in L.LENSES:
             raise ValueError(f"unknown lens {lens!r}: expected one of {sorted(L.LENSES)}")
+        if (tag_size is None) == (corners is None):
+            raise ValueError("give exactly one of tag_size and corners")
         self.pixels = np.ascontiguousarray(pixels, dtype=np.float64).reshape(8)
-        self.tag_size = float(tag_size)
+        self.tag_size = None if tag_size is None else float(tag_size)
+        self.corners = None if corners is None else np.ascontiguousarray(corners, dtype=np.float64).reshape(4, 2)
         self.rig = bool(rig)
         self.lens = lens
 
@@ -54,8 +62,10 @@ class TagReprojectionCost:
                 p.set_rig_extrinsics(ext)
             p.set_view_poses(view)
             p.set_marker_poses(marker)
-            p.set_marker_sizes([self.tag_size])
+            p.set_marker_sizes([self.tag_size if self.corners is None else 1.0])
             p.set_observations([0], [0], [0], self.pixels)
+            if self.corners is not None:
+                p.set_corner_layout(self.corners[None], [0])
             out = p.evaluate(want_jacobians=jacobians is not None, allow_failure=True)
         residuals[:] = out["residuals"].reshape(8)
         if jacobians is not None:
@@ -64,6 +74,18 @@ class TagReprojectionCost:
                 if j is not None:
                     np.asarray(j).reshape(-1)[:] = out["jacobians"][n].reshape(-1)
         return not out["failed"]
+
+
+def corner_layout(corners):
+    """The corner layout of residual blocks whose corners are `corners` (one 4 x 2 array, or None for the square of
+    the tag size, per block): (table (n_slots, 4, 2), slot (n,) int32), one slot per distinct corner set in order of
+    first use, slot -1 for None."""
+    slots, slot = {}, np.full(len(corners), -1, dtype=np.int32)
+    for i, c in enumerate(corners):
+        if c is not None:
+            slot[i] = slots.setdefault(np.ascontiguousarray(c, dtype=np.float64).tobytes(), len(slots))
+    table = np.array([np.frombuffer(k, dtype=np.float64).reshape(4, 2) for k in slots]).reshape(-1, 4, 2)
+    return table, slot
 
 
 class NormalPrior:
@@ -256,8 +278,9 @@ class Problem:
             c = cams.setdefault(key, (len(cams), intr, dist, ext))[0]
             if lenses.setdefault(c, cost.lens) != cost.lens:
                 raise ValueError("one camera (intr, dist, ext) is used by cost functions of different lenses")
-            if sizes.setdefault(m, cost.tag_size) != cost.tag_size:
-                raise ValueError("one marker was given two different tag sizes")
+            if cost.corners is None:
+                if sizes.setdefault(m, cost.tag_size) != cost.tag_size:
+                    raise ValueError("one marker was given two different tag sizes")
             vi.append(v); mi.append(m); ci.append(c); px.append(cost.pixels)
         vlist = [a for _, a in sorted(views.values(), key=lambda t: t[0])]
         mlist = [a for _, a in sorted(markers.values(), key=lambda t: t[0])]
@@ -269,8 +292,11 @@ class Problem:
             gp.set_rig_extrinsics(np.stack([c[3] for c in clist]))
         gp.set_view_poses(np.stack(vlist))
         gp.set_marker_poses(np.stack(mlist))
-        gp.set_marker_sizes([sizes[m] for m in range(len(mlist))])
+        gp.set_marker_sizes([sizes.get(m, 1.0) for m in range(len(mlist))])   # 1.0: a marker with layout corners only
         gp.set_observations(vi, mi, ci, np.stack(px))
+        table, slot = corner_layout([b[0].corners for b in self._blocks])
+        if len(table):
+            gp.set_corner_layout(table, slot)
         if self._loss is not None:
             gp.set_loss(*self._loss)
         for i, a in enumerate(vlist):

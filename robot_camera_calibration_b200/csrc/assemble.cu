@@ -28,7 +28,10 @@
 namespace rcc {
 
 void launch_assemble(bool rig, bool epass, bool own_is_view, int lens, const AssembleArgs& a, cudaStream_t s) {
-  if (lens == LENS_EQUIDISTANT) launch_assemble_equidistant(rig, epass, own_is_view, a, s);
+  if (a.corners) {
+    if (lens == LENS_EQUIDISTANT) launch_assemble_target_equidistant(rig, epass, own_is_view, a, s);
+    else launch_assemble_target(rig, epass, own_is_view, a, s);
+  } else if (lens == LENS_EQUIDISTANT) launch_assemble_equidistant(rig, epass, own_is_view, a, s);
   else if (a.loss != 0) launch_assemble_l<true, LENS_RADTAN>(rig, epass, own_is_view, a, s);
   else launch_assemble_l<false, LENS_RADTAN>(rig, epass, own_is_view, a, s);
 }

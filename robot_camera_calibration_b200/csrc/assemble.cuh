@@ -1,6 +1,8 @@
 // K2 kernel template (see assemble.cu for the design).  Included by assemble.cu, which instantiates the
-// radial-tangential lens, and by assemble_equidistant.cu, which instantiates the equidistant lens, so that the two
-// sets of 16 kernels compile in parallel.
+// radial-tangential lens, by assemble_equidistant.cu, which instantiates the equidistant lens, and by
+// assemble_target.cu and assemble_target_equidistant.cu, which instantiate both lenses with the corners of a corner
+// layout, so that the four sets of 16 kernels compile in parallel.  One body, assemble_body, serves both entry points:
+// assemble_kernel (the square of the marker's size) and assemble_target_kernel (chunk.cuh: TARGET).
 #pragma once
 
 #include "chunk.cuh"
@@ -65,16 +67,18 @@ struct WarpSmem {
   static constexpr int TOTAL = STAGE + CHUNK_POSE_SMEM<RIG>;
 };
 
-template <bool RIG, bool EPASS, bool OWN_IS_VIEW, bool LOSS, Lens L>
-__global__ void __launch_bounds__(PassGeom<RIG>::WARPS * 32,
-                                  (RIG && EPASS) ? 2 : ((!RIG && !EPASS) ? RCC_K2_MIN_CTAS_F : RCC_K2_MIN_CTAS))   // rig E pass: 89 KB smem per CTA
-assemble_kernel(const AssembleArgs a) {
+template <bool RIG, bool EPASS>
+constexpr int K2_MIN_CTAS = (RIG && EPASS) ? 2 : ((!RIG && !EPASS) ? RCC_K2_MIN_CTAS_F : RCC_K2_MIN_CTAS);   // rig E pass: 89 KB smem per CTA
+
+// tid = threadIdx.x, read by the __global__ entry point: there the compiler knows its range from the launch bounds
+template <bool RIG, bool EPASS, bool OWN_IS_VIEW, bool LOSS, Lens L, bool TARGET>
+__device__ __forceinline__ void assemble_body(const AssembleArgs& a, unsigned tid) {
   using PG = PassGeom<RIG>;
   using WS = WarpSmem<RIG, EPASS>;
   constexpr int BPW = PG::BPW, RS = WS::RS, BS = WS::BS;
   constexpr int PART = EPASS ? PG::PART_E : PG::PART_F;
   extern __shared__ __align__(16) double smem[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int warp = tid >> 5, lane = tid & 31;
   const int launch_pos = blockIdx.x * PG::WARPS + warp;
   if (launch_pos >= a.n_chunks) return;  // whole warp leaves together
   const int chunk_id = a.chunk_list ? a.chunk_list[launch_pos] : launch_pos;
@@ -87,7 +91,7 @@ assemble_kernel(const AssembleArgs a) {
 
   // chunk constants -> shared memory; pad columns of the staged rows (never read back as results, but they do enter
   // the MMAs) are cleared once; then the first group's poses and pixels are set in flight
-  ChunkPoses<RIG, OWN_IS_VIEW, AssembleArgs> poses(a, ch, wsm + WS::STAGE, lane);
+  ChunkPoses<RIG, OWN_IS_VIEW, AssembleArgs, TARGET> poses(a, ch, wsm + WS::STAGE, lane);
   for (int k = lane; k < BPW * BS; k += 32) rows[k] = 0.0;
   poses.start();
 
@@ -193,11 +197,26 @@ assemble_kernel(const AssembleArgs a) {
 }
 
 template <bool RIG, bool EPASS, bool OWN_IS_VIEW, bool LOSS, Lens L>
+__global__ void __launch_bounds__(PassGeom<RIG>::WARPS * 32, K2_MIN_CTAS<RIG, EPASS>)
+assemble_kernel(const AssembleArgs a) {
+  assemble_body<RIG, EPASS, OWN_IS_VIEW, LOSS, L, false>(a, threadIdx.x);
+}
+
+// the same with the corners of the corner layout
+template <bool RIG, bool EPASS, bool OWN_IS_VIEW, bool LOSS, Lens L>
+__global__ void __launch_bounds__(PassGeom<RIG>::WARPS * 32, K2_MIN_CTAS<RIG, EPASS>)
+assemble_target_kernel(const AssembleArgs a) {
+  assemble_body<RIG, EPASS, OWN_IS_VIEW, LOSS, L, true>(a, threadIdx.x);
+}
+
+template <bool RIG, bool EPASS, bool OWN_IS_VIEW, bool LOSS, Lens L, bool TARGET>
 static void launch_assemble_t(const AssembleArgs& a, cudaStream_t s) {
   using PG = PassGeom<RIG>;
   if (a.n_chunks == 0) return;
   const size_t smem = PG::WARPS * WarpSmem<RIG, EPASS>::TOTAL * sizeof(double);
-  auto k = assemble_kernel<RIG, EPASS, OWN_IS_VIEW, LOSS, L>;
+  void (*k)(AssembleArgs);
+  if constexpr (TARGET) k = assemble_target_kernel<RIG, EPASS, OWN_IS_VIEW, LOSS, L>;
+  else k = assemble_kernel<RIG, EPASS, OWN_IS_VIEW, LOSS, L>;
   static SmemOptIn optin;   // one per template instantiation
   optin.ensure(k, smem);
   const int grid = ceil_div(a.n_chunks, PG::WARPS);
@@ -205,18 +224,18 @@ static void launch_assemble_t(const AssembleArgs& a, cudaStream_t s) {
   RCC_CUDA(cudaGetLastError());
 }
 
-template <bool LOSS, Lens L>
+template <bool LOSS, Lens L, bool TARGET = false>
 static void launch_assemble_l(bool rig, bool epass, bool own_is_view, const AssembleArgs& a, cudaStream_t s) {
   const int sel = (rig ? 4 : 0) | (epass ? 2 : 0) | (own_is_view ? 1 : 0);
   switch (sel) {
-    case 0: launch_assemble_t<false, false, false, LOSS, L>(a, s); break;
-    case 1: launch_assemble_t<false, false, true, LOSS, L>(a, s); break;
-    case 2: launch_assemble_t<false, true, false, LOSS, L>(a, s); break;
-    case 3: launch_assemble_t<false, true, true, LOSS, L>(a, s); break;
-    case 4: launch_assemble_t<true, false, false, LOSS, L>(a, s); break;
-    case 5: launch_assemble_t<true, false, true, LOSS, L>(a, s); break;
-    case 6: launch_assemble_t<true, true, false, LOSS, L>(a, s); break;
-    default: launch_assemble_t<true, true, true, LOSS, L>(a, s); break;
+    case 0: launch_assemble_t<false, false, false, LOSS, L, TARGET>(a, s); break;
+    case 1: launch_assemble_t<false, false, true, LOSS, L, TARGET>(a, s); break;
+    case 2: launch_assemble_t<false, true, false, LOSS, L, TARGET>(a, s); break;
+    case 3: launch_assemble_t<false, true, true, LOSS, L, TARGET>(a, s); break;
+    case 4: launch_assemble_t<true, false, false, LOSS, L, TARGET>(a, s); break;
+    case 5: launch_assemble_t<true, false, true, LOSS, L, TARGET>(a, s); break;
+    case 6: launch_assemble_t<true, true, false, LOSS, L, TARGET>(a, s); break;
+    default: launch_assemble_t<true, true, true, LOSS, L, TARGET>(a, s); break;
   }
 }
 

@@ -72,16 +72,23 @@ struct AssembleArgs {
   int32_t* fail_flag;     // set to 1 on depth <= 0 / non-finite residual
   int32_t loss;           // 0 trivial, 1 Huber, 2 Cauchy (per tag residual block)
   double loss_a2;         // squared loss scale
+  // corner layout (rcc_ba_set_corner_layout; both null without one): the target instantiations read them
+  const int32_t* slot;    // [n] layout slot of each sorted block of this pass, -1: the square of the marker's size
+  const double* corners;  // [n_slots*8] corners bl br tr tl (x, y) of each slot
 };
 
 // K2: fused residual + Jacobian + J^T J tiles.  own_is_view tells which pose
 // table the segment owner indexes; lens is a Lens (model.cuh) other than LENS_PER_CAMERA: with mixed lenses the
 // caller launches once per lens, over that lens's chunks (problem.cu: plan_launches).  Under the equidistant
-// lens tile B holds [cx cy k1 k2 k3 k4 0 | r]: the reserved slot's column is zero.
+// lens tile B holds [cx cy k1 k2 k3 k4 0 | r]: the reserved slot's column is zero.  With a corner layout
+// (a.corners set) the target instantiations run (assemble_target_kernel), otherwise assemble_kernel.
 constexpr int N_LENSES = 2;   // LENS_RADTAN, LENS_EQUIDISTANT
 void launch_assemble(bool rig, bool epass, bool own_is_view, int lens, const AssembleArgs& a, cudaStream_t s);
-// the equidistant instantiations (assemble_equidistant.cu)
+// the equidistant instantiations (assemble_equidistant.cu) and the target ones (assemble_target.cu,
+// assemble_target_equidistant.cu)
 void launch_assemble_equidistant(bool rig, bool epass, bool own_is_view, const AssembleArgs& a, cudaStream_t s);
+void launch_assemble_target(bool rig, bool epass, bool own_is_view, const AssembleArgs& a, cudaStream_t s);
+void launch_assemble_target_equidistant(bool rig, bool epass, bool own_is_view, const AssembleArgs& a, cudaStream_t s);
 
 // per-own-block reduction of the chunk partials
 struct FinalizeSideArgs {
@@ -187,11 +194,20 @@ struct EvalArgs {
   const int32_t* oth;       // [n] other 6-dof block of each sorted block (own block comes from the chunk)
   int32_t own_is_view;
   uint32_t cam_equidistant; // lens LENS_PER_CAMERA: bit c set = camera c has the equidistant lens
+  // corner layout (AssembleArgs::slot, corners), the slots in the E-sorted order
+  const int32_t* slot;
+  const double* corners;
 };
 int eval_grid(int64_t n);   // CTAs launch_evaluate / launch_cost will use
 // lens is a Lens; LENS_PER_CAMERA only without Jacobians (K6).  K1 takes one lens per launch: with mixed lenses the
 // caller launches it once per lens over a lens-ordered copy of the chunk records (problem.cu: plan_launches).
+// With a corner layout (a.corners set) the target instantiations run (materialise_target_kernel,
+// evaluate_target_kernel: evaluate_target.cu).
 void launch_evaluate(bool rig, bool want_jac, int lens, const EvalArgs& a, cudaStream_t s);
+void launch_evaluate_target(bool rig, bool want_jac, int lens, const EvalArgs& a, cudaStream_t s);
+// caller-order layout slots -> both sorted orders: e_slot[g] = slot[orig[g]], f_slot[f_inv[g]] = e_slot[g]
+void launch_sort_slots(const int32_t* slot, const int32_t* orig, const int32_t* f_inv, int32_t* e_slot, int32_t* f_slot,
+                       int64_t n, cudaStream_t s);
 // number of cost partials launch_evaluate writes (want_jac: one per chunk; else one per CTA)
 int eval_partials(bool want_jac, const EvalArgs& a);
 void launch_cost(bool rig, int lens, const EvalArgs& a, cudaStream_t s);

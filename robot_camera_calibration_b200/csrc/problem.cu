@@ -554,6 +554,7 @@ static void build_indices(P_t* P, const int32_t* view_idx, const int32_t* marker
   P->cost_partials.alloc((size_t)std::max(std::max(1, eval_grid(n)), P->n_chunks_e) + P->n_prior_parts);
   RCC_CUDA(cudaStreamSynchronize(s));
   P->have_obs = true;
+  P->n_slots = 0;   // new observations clear the corner layout
   P->linearized = P->schur_done = P->step_ready = P->cand_ready = false;
   plan_launches(P);
 }
@@ -651,6 +652,11 @@ static void do_linearize(P_t* P) {
   f.pix = P->f_pix.p;
   f.chunks = P->f_chunks.p;
   f.partials = P->part_f.p;
+  if (P->n_slots > 0) {   // the target instantiations, for every run of plan_launches
+    e.corners = f.corners = P->corners.p;
+    e.slot = P->e_slot.p;
+    f.slot = P->f_slot.p;
+  }
   bool f_done = false;
   {
     Scoped t(P, ST_ASSEMBLE_E, 0);
@@ -1178,6 +1184,10 @@ static EvalArgs eval_args(P_t* P, bool cand) {
   a.loss = P->loss;
   a.loss_a2 = P->loss_scale * P->loss_scale;
   a.cam_equidistant = P->cam_equidistant;
+  if (P->n_slots > 0) {   // the target instantiations of K1 and K6
+    a.slot = P->e_slot.p;
+    a.corners = P->corners.p;
+  }
   return a;
 }
 
@@ -1781,6 +1791,36 @@ int rcc_ba_set_priors(rcc_ba_problem* P, int32_t block_kind, int64_t n, const in
                       const double* sqrt_information) {
   API_BEGIN(P)
   set_priors(P, block_kind, n, index, mean, sqrt_information);
+  API_END(P)
+}
+
+// every check first: a refused call changes nothing
+static void set_corner_layout(P_t* P, int32_t n_slots, const double* corners, const int32_t* slot) {
+  RCC_REQUIRE(n_slots >= 0, RCC_BAD_ARG, "n_slots must not be negative");
+  RCC_REQUIRE(n_slots == 0 || (corners && slot), RCC_BAD_ARG, "null pointer");
+  RCC_REQUIRE(P->have_obs, RCC_NOT_READY, "set_observations has not been called");
+  const int64_t n = P->n_obs;
+  if (n_slots > 0) {
+    for (int64_t i = 0; i < (int64_t)n_slots * 8; ++i)
+      RCC_REQUIRE(std::isfinite(corners[i]), RCC_BAD_ARG, "non-finite layout corner");
+    for (int64_t i = 0; i < n; ++i)
+      RCC_REQUIRE(slot[i] >= -1 && slot[i] < n_slots, RCC_BAD_ARG,
+                  "layout slot " + std::to_string(slot[i]) + " of block " + std::to_string(i) + " out of range");
+    cudaStream_t s = P->stream;
+    P->corners.upload(corners, (size_t)n_slots * 8, s);
+    P->slot_in.upload(slot, (size_t)n, s);
+    P->e_slot.ensure((size_t)n);
+    P->f_slot.ensure((size_t)n);
+    Scoped t(P, ST_H2D, n > 0 ? 1 : 0);
+    launch_sort_slots(P->slot_in.p, P->e_orig.p, P->f_inv.p, P->e_slot.p, P->f_slot.p, n, s);
+  }
+  P->n_slots = n_slots;
+  P->linearized = P->schur_done = P->step_ready = P->cand_ready = false;
+}
+
+int rcc_ba_set_corner_layout(rcc_ba_problem* P, int32_t n_slots, const double* corners, const int32_t* slot) {
+  API_BEGIN(P)
+  set_corner_layout(P, n_slots, corners, slot);
   API_END(P)
 }
 

@@ -152,6 +152,11 @@ struct rcc_ba_problem {
   // Gaussian priors (rcc_ba_set_priors), per rcc_block_kind on the host: index, mean (6 doubles per prior) and A
   // (36: row-major 6 x 6 holding the k x k matrix, zero padded).  On the device the kinds lie back to back in kind
   // order, the priors of kind t at [prior_off[t], prior_off[t+1]).
+  // corner layout (rcc_ba_set_corner_layout): the slot records and each block's slot in the E- and F-sorted orders.
+  // n_slots == 0: no layout (the buffers may stay allocated), and the kernels take the square of the marker's size.
+  int n_slots = 0;
+  rcc::DBuf<double> corners;
+  rcc::DBuf<int32_t> slot_in, e_slot, f_slot;
   std::vector<int32_t> prior_index_h[rcc::PRIOR_KINDS];
   std::vector<double> prior_mean_h[rcc::PRIOR_KINDS], prior_A_h[rcc::PRIOR_KINDS];
   int prior_off[rcc::PRIOR_KINDS + 1] = {0};

@@ -40,7 +40,8 @@ def shard_scene(scene, rank, world, eliminate="auto"):
     """The observations whose eliminated block this rank owns.  Parameter arrays
     keep their global size and indexing (kept blocks and shared parameters are
     replicated; eliminated blocks this rank does not own simply have no
-    observations here and stay untouched).  Returns (sub_scene, (lo, hi))."""
+    observations here and stay untouched).  A corner layout (Scene.corners) is replicated and its slots go with their
+    blocks.  Returns (sub_scene, (lo, hi))."""
     ev = eliminated_is_view(scene, eliminate)
     e_idx = scene.view_idx if ev else scene.marker_idx
     n_e = len(scene.views) if ev else len(scene.markers)
@@ -50,6 +51,8 @@ def shard_scene(scene, rank, world, eliminate="auto"):
     s = copy.copy(scene)
     s.view_idx, s.marker_idx = scene.view_idx[keep], scene.marker_idx[keep]
     s.cam_idx, s.pixels = scene.cam_idx[keep], scene.pixels[keep]
+    if getattr(scene, "corner_slot", None) is not None:
+        s.corner_slot = scene.corner_slot[keep]
     return s, (lo, hi)
 
 

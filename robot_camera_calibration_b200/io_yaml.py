@@ -22,7 +22,7 @@ import re
 import numpy as np
 import yaml
 
-from .scenes import Scene
+from .scenes import Scene, board_layout, compose, invert
 
 
 def _ts(x, precision=None):
@@ -217,6 +217,104 @@ def read_dataset(directory, intr=None, dist=None, lens=None):
     return scene, tag_ids, np.array(frames)
 
 
+def read_target(path):
+    """A rigid tag board in Kalibr's AprilGrid format -> (tag ids (n,), corners (n, 4, 2)): keys target_type:
+    aprilgrid, tagCols, tagRows, tagSize (m), tagSpacing (the gap between tags over tagSize), and firstTagId (ours,
+    default 0).  Convention: tag (r, c) has id firstTagId + r tagCols + c; the board origin is the bottom-left corner
+    of tag firstTagId, the tag axes are the board axes, and tag (r, c) is centred at (c (1 + spacing) s + s/2,
+    r (1 + spacing) s + s/2) for s = tagSize (scenes.board_layout); the corners are bl br tr tl in the board frame.
+    Agreement with Kalibr's own id numbering and board origin has not been verified against Kalibr."""
+    with open(path) as f:
+        y = yaml.safe_load(f) or {}
+    if str(y.get("target_type", "")).strip().lower() != "aprilgrid":
+        raise ValueError(f"{path}: target_type must be aprilgrid, got {y.get('target_type')!r}")
+    try:
+        rows, cols = int(y["tagRows"]), int(y["tagCols"])
+        size, spacing = float(y["tagSize"]), float(y["tagSpacing"])
+    except KeyError as e:
+        raise ValueError(f"{path}: missing key {e.args[0]}") from None
+    first = int(y.get("firstTagId", 0))
+    if rows < 1 or cols < 1 or not 0 < size < np.inf or not 0 <= spacing < np.inf or first < 0:
+        raise ValueError(f"{path}: tagRows and tagCols must be positive, tagSize positive, tagSpacing and firstTagId "
+                         "not negative")
+    return first + np.arange(rows * cols), board_layout(rows, cols, size, spacing)
+
+
+def read_targets(paths):
+    """read_target of every file; a tag id on two targets is an error."""
+    out, owner = [], {}
+    for k, path in enumerate(paths):
+        ids, corners = read_target(path)
+        for i in ids.tolist():
+            if owner.setdefault(i, k) != k:
+                raise ValueError(f"tag id {i} is on two targets: {paths[owner[i]]} and {path}")
+        out.append((ids, corners))
+    return out
+
+
+def board_scene(scene, tag_ids, targets):
+    """Map the tags of a per-tag scene (read_dataset) onto rigid boards: targets = read_targets(...).  Every board
+    with a detected tag becomes one marker block, first the boards in target order, then the tags on no board (free,
+    slot -1).  A board's initial pose is world_T_tag o (board_T_tag)^-1 of its most-detected tag; a board carrying
+    the world tag (marker 0 of the scene, camera_pose.cpp:71-80) is the gauge and held constant.  Returns
+    (board_scene, tag_pose) with tag_pose(markers) -> the world_T_tag of every tag of `scene` (tag_ids order) from
+    the board scene's markers."""
+    where = {}                                                  # tag id -> (target, slot)
+    for b, (ids, _) in enumerate(targets):
+        for k, i in enumerate(ids.tolist()):
+            where[i] = (b, k)
+    n_tags = len(tag_ids)
+    counts = np.bincount(scene.marker_idx, minlength=n_tags)
+    on = [where.get(int(t)) for t in tag_ids]
+    used = sorted({w[0] for w, c in zip(on, counts) if w is not None and c > 0})
+    new_of_board = {b: j for j, b in enumerate(used)}
+    free = [m for m in range(n_tags) if on[m] is None or on[m][0] not in new_of_board]
+    new_of_tag = np.empty(n_tags, dtype=np.int64)
+    slot_of_tag = np.full(n_tags, -1, dtype=np.int32)
+    offset = np.zeros(len(targets) + 1, dtype=np.int64)         # slots of target b: [offset[b], offset[b + 1])
+    offset[1:] = np.cumsum([len(ids) for ids, _ in targets])
+    for m in range(n_tags):
+        if on[m] is not None and on[m][0] in new_of_board:
+            new_of_tag[m] = new_of_board[on[m][0]]
+            slot_of_tag[m] = offset[on[m][0]] + on[m][1]
+    for j, m in enumerate(free):
+        new_of_tag[m] = len(used) + j
+    corners = np.concatenate([c for _, c in targets]).reshape(-1, 4, 2)
+
+    def board_T_tag(slot):                                      # the tag frame: centred on the tag, board axes
+        ctr = corners[slot].mean(0)
+        return np.array([0.0, 0.0, 0.0, ctr[0], ctr[1], 0.0])
+
+    markers = np.zeros((len(used) + len(free), 6))
+    sizes = np.zeros(len(markers))
+    const = np.zeros(len(markers), bool)
+    for b in used:
+        tags = [m for m in range(n_tags) if on[m] is not None and on[m][0] == b]
+        best = max(tags, key=lambda m: counts[m])
+        markers[new_of_board[b]] = compose(scene.markers[best], invert(board_T_tag(slot_of_tag[best])))
+        sizes[new_of_board[b]] = scene.sizes[best]
+        const[new_of_board[b]] = any(scene.const_markers[m] for m in tags)
+    for j, m in enumerate(free):
+        markers[len(used) + j] = scene.markers[m]
+        sizes[len(used) + j] = scene.sizes[m]
+        const[len(used) + j] = scene.const_markers[m]
+    s = Scene(model=scene.model, intr=scene.intr, dist=scene.dist, ext=scene.ext, views=scene.views, markers=markers,
+              sizes=sizes, view_idx=scene.view_idx, marker_idx=new_of_tag[scene.marker_idx].astype(np.int32),
+              cam_idx=scene.cam_idx, pixels=scene.pixels, const_views=scene.const_views, const_markers=const,
+              const_intr=scene.const_intr, const_dist=scene.const_dist, image_size=scene.image_size,
+              lens=scene.lens, corners=corners, corner_slot=slot_of_tag[scene.marker_idx])
+
+    def tag_pose(new_markers):
+        out = np.empty((n_tags, 6))
+        for m in range(n_tags):
+            j = new_of_tag[m]
+            out[m] = new_markers[j] if slot_of_tag[m] < 0 else compose(new_markers[j], board_T_tag(slot_of_tag[m]))
+        return out
+
+    boards = [(int(targets[b][0][0]), new_of_board[b]) for b in used]   # (first tag id, marker block)
+    return s, tag_pose, boards
+
+
 def _pixel_array(px):
     """Corner lists -> (N,8) array.  corner_detections.cpp:53-54 writes integer corners: those stay integers
     (int16 when they fit) so that BAProblem ships 16 bytes per tag to the GPU; anything else is FP64."""
@@ -259,17 +357,23 @@ def intrinsics_priors(intr, dist, sigma):
 
 
 def optimise_directory(directory, device=0, refine_intrinsics=True, precision=None, intr=None, dist=None,
-                       lens=None, intrinsics_sigma=None, **lm_options):
+                       lens=None, intrinsics_sigma=None, targets=None, **lm_options):
     """Milestone 3: detections/ -> GPU bundle adjustment -> detections/ (same formats).  The lens is camera.yaml's
     distortion_model (plumb_bob, or equidistant / fisheye), and camera_refined.yaml is written in the same model.
     intrinsics_sigma = (focal px, principal point px, distortion): refine the intrinsics under a diagonal Gaussian
-    prior centred on camera.yaml (intrinsics_priors) instead of freely; it needs refine_intrinsics."""
+    prior centred on camera.yaml (intrinsics_priors) instead of freely; it needs refine_intrinsics.
+    targets: AprilGrid target files (read_target).  Their detected tags are solved as rigid boards, one pose each
+    (board_scene); targets.yaml is still written per tag (world_T_board o board_T_tag), and the summary gains
+    "boards": [{"first_tag_id", "world_T_board": rvec + t}] per board."""
     from .problem import BAProblem
     if intrinsics_sigma is not None and not refine_intrinsics:
         raise ValueError("intrinsics_sigma puts a prior on refined intrinsics: it cannot be combined with fixed ones")
     scene, tag_ids, frames = read_dataset(directory, intr=intr, dist=dist, lens=lens)
     scene.const_intr[:] = not refine_intrinsics
     scene.const_dist[:] = not refine_intrinsics
+    tags = scene
+    if targets:
+        scene, tag_pose, boards = board_scene(tags, tag_ids, read_targets(list(targets)))
     with BAProblem.from_scene(scene, device=device) as p:
         if intrinsics_sigma is not None:
             for kind, args in intrinsics_priors(scene.intr, scene.dist, intrinsics_sigma).items():
@@ -278,6 +382,10 @@ def optimise_directory(directory, device=0, refine_intrinsics=True, precision=No
         scene.views, scene.markers = p.get_view_poses(), p.get_marker_poses()
         intr, dist = p.get_intrinsics()
         scene.intr, scene.dist = intr, dist
+    if targets:
+        summary["boards"] = [{"first_tag_id": i, "world_T_board": scene.markers[j].tolist()} for i, j in boards]
+        tags.views, tags.markers = scene.views, tag_pose(scene.markers)
+        scene = tags
     write_results(directory, scene, tag_ids, frames, precision)
     if refine_intrinsics:
         with open(os.path.join(directory, "camera_refined.yaml"), "w") as f:

@@ -113,6 +113,8 @@ class BAProblem:
         if scene.model == "rig":
             for i in np.nonzero(scene.const_ext)[0]:
                 p.set_constant(L.BLOCK_EXT, int(i), True)
+        if getattr(scene, "corners", None) is not None:
+            p.set_corner_layout(scene.corners, scene.corner_slot)
         return p
 
     def set_intrinsics(self, intr, dist):
@@ -163,6 +165,23 @@ class BAProblem:
             return
         px = _f64(pixels, (self.n_obs, 8))
         self._check(self.lib.rcc_ba_update_pixels(self.h, _dp(px)))
+
+    def set_corner_layout(self, corners, slot):
+        """Rigid planar targets (rcc_ba_set_corner_layout): corners (n_slots, 4, 2) bl br tr tl in the frame of the
+        block's marker, slot (n_obs_blocks,) in caller order, -1 for the square of the marker's size.  A marker whose
+        blocks use different slots is one tag board with one pose.  An empty corners array clears the layout;
+        set_observations clears it too, update_pixels keeps it."""
+        c = _f64(corners).reshape(-1, 4, 2)
+        if len(c) == 0:
+            self.clear_corner_layout()
+            return
+        sl = np.ascontiguousarray(slot, dtype=np.int32).reshape(-1)
+        if len(sl) != self.n_obs:
+            raise ValueError(f"{len(sl)} slots for {self.n_obs} observation blocks")
+        self._check(self.lib.rcc_ba_set_corner_layout(self.h, len(c), _dp(c), _ip(sl)))
+
+    def clear_corner_layout(self):
+        self._check(self.lib.rcc_ba_set_corner_layout(self.h, 0, None, None))
 
     def set_constant(self, kind, index, is_constant=True):
         kind = _BLOCK_KINDS[kind] if isinstance(kind, str) else kind

@@ -71,7 +71,11 @@ def obj_points(size):
 def project(model, intr, dist, ext, view, marker, size, lens="radtan"):
     """Projection of the 4 tag corners through a pinhole + radial-tangential lens or an equidistant fisheye lens
     (numpy; used only to synthesise pixels).  Returns (uv (N,4,2), depth (N,4))."""
-    o = obj_points(size)
+    return project_points(model, intr, dist, ext, view, marker, obj_points(size), lens)
+
+
+def project_points(model, intr, dist, ext, view, marker, o, lens="radtan"):
+    """project() of the object points o (N,4,3) in the marker frame instead of the square of a tag size."""
     Rm = rodrigues_np(marker[:, 0:3])
     Pw = np.einsum('nij,nkj->nki', Rm, o) + marker[:, None, 3:6]
     Rv = rodrigues_np(view[:, 0:3])
@@ -126,6 +130,8 @@ class Scene:
     image_size: tuple = (640, 480)  # mixed lenses: one (width, height) per camera
     name: str = ""
     lens: str = "radtan"            # "radtan" | "equidistant" for every camera, or a tuple of one per camera
+    corners: np.ndarray = None      # (n_slots,4,2) corner layout (rcc_ba_set_corner_layout) or None
+    corner_slot: np.ndarray = None  # (N,) int32 layout slot of each block, -1: the square of the marker's size
 
     def __post_init__(self):
         nv, nm, nc = len(self.views), len(self.markers), len(self.intr)
@@ -457,6 +463,120 @@ def make_scene(n_markers, n_views, visibility, n_cam=1, model="single", seed=0,
                  truth=dict(intr=intr_t, dist=dist_t, ext=ext_t, views=views_t,
                             markers=markers_t),
                  image_size=image_size, name=name, lens=lens)
+
+
+# ---------------------------------------------------------------- rigid multi-tag targets
+def board_layout(rows, cols, tag_size, spacing):
+    """(rows*cols, 4, 2) corners bl br tr tl of the tags of a rows x cols board in the board frame, slot r*cols + c
+    for tag (r, c): the origin is the bottom-left corner of tag 0, the tag axes are the board axes, and tag (r, c) is
+    centred at (c (1 + spacing) s + s/2, r (1 + spacing) s + s/2) for s = tag_size (Kalibr AprilGrid: tagSpacing is
+    the gap over the tag size)."""
+    r, c = np.divmod(np.arange(rows * cols), cols)
+    pitch = (1 + spacing) * tag_size
+    ctr = np.stack([c * pitch + tag_size / 2, r * pitch + tag_size / 2], -1)
+    h = tag_size / 2
+    return ctr[:, None, :] + np.array([[-h, -h], [h, -h], [h, h], [-h, h]])
+
+
+def make_target_scene(rows, cols, n_views, n_boards=1, n_free=0, n_cam=1, model="single", seed=0, tag_size=0.1,
+                      spacing=0.3, distance=2.5, pixel_noise=0.3, perturb=(0.02, 0.02, 0.01), lens="radtan",
+                      image_size=None, name=""):
+    """A scene of rigid tag boards (Scene.corners / corner_slot): n_boards boards of rows x cols tags (board_layout,
+    one marker block each, slot = tag number, shared by the boards) side by side on a wall, plus n_free free tags
+    (slot -1) between them; marker 0 is board 0 at the world origin (the gauge).  Each of the n_views views (body
+    poses of a rig) looks at a random point of the wall from about `distance` and sees every tag whose four corners
+    project inside the image with positive depth (equidistant: within 85 degrees of the optical axis).  Cameras and
+    lenses as make_scene, which this does not call and whose random streams it leaves alone."""
+    lenses = (lens,) * n_cam if isinstance(lens, str) else tuple(lens)
+    if len(lenses) != n_cam or any(x not in ("radtan", "equidistant") for x in lenses):
+        raise ValueError(f"lens must be 'radtan', 'equidistant' or one of them per camera, got {lens!r}")
+    rng = np.random.default_rng([seed, 52361])
+    fish = np.array([x == "equidistant" for x in lenses])
+    sizes_img = [tuple(image_size) if image_size is not None else ((1280, 1024) if f_ else (640, 480)) for f_ in fish]
+    W = np.array([sz[0] for sz in sizes_img], dtype=np.float64)
+    H = np.array([sz[1] for sz in sizes_img], dtype=np.float64)
+    f_lo, f_hi = np.where(fish, 320.0, 550.0), np.where(fish, 340.0, 650.0)
+    intr_t = np.stack([rng.uniform(f_lo, f_hi), rng.uniform(f_lo, f_hi), W / 2 + rng.uniform(-10, 10, n_cam),
+                       H / 2 + rng.uniform(-10, 10, n_cam)], -1)
+    dist_f = np.stack([rng.normal(0, 0.02, n_cam), rng.normal(0, 0.01, n_cam), rng.normal(0, 2e-3, n_cam),
+                       rng.normal(0, 5e-4, n_cam), np.zeros(n_cam)], -1)
+    dist_r = np.stack([rng.normal(0, 0.1, n_cam), rng.normal(0, 0.05, n_cam), rng.normal(0, 2e-3, n_cam),
+                       rng.normal(0, 2e-3, n_cam), rng.normal(0, 0.01, n_cam)], -1)
+    dist_t = np.where(fish[:, None], dist_f, dist_r)
+    ext_t = np.zeros((n_cam, 6))
+    if model == "rig" and n_cam > 1:
+        ext_t[:, 1] = np.linspace(-0.3, 0.3, n_cam)
+        ext_t[:, 3] = np.linspace(-0.1, 0.1, n_cam)
+        ext_t[1:, 0:3] += rng.normal(0, 0.02, (n_cam - 1, 3))
+        ext_t[1:, 3:6] += rng.normal(0, 0.01, (n_cam - 1, 3))
+        ext_t[0] = 0.0
+    # boards in a row along x with a gap of two tags, free tags in the gaps and below the boards
+    layout = board_layout(rows, cols, tag_size, spacing)
+    pitch = (1 + spacing) * tag_size
+    bw, bh = cols * pitch, rows * pitch
+    boards = np.zeros((n_boards, 6))
+    boards[:, 3] = np.arange(n_boards) * (bw + 2 * pitch)
+    boards[1:, 0:3] = rng.normal(0, 0.05, (n_boards - 1, 3))
+    free = np.zeros((n_free, 6))
+    free[:, 0:3] = rng.normal(0, 0.2, (n_free, 3))
+    free[:, 3] = rng.uniform(-pitch, n_boards * (bw + 2 * pitch) - pitch, n_free)
+    free[:, 4] = rng.uniform(-1.5 * pitch, bh + 0.5 * pitch, n_free)
+    free[:, 5] = rng.uniform(-0.05, 0.05, n_free)
+    markers_t = np.concatenate([boards, free])
+    sizes = np.full(len(markers_t), tag_size)
+    # every tag of the scene: (marker, slot, object points)
+    tag_marker = np.concatenate([np.repeat(np.arange(n_boards), rows * cols), n_boards + np.arange(n_free)])
+    tag_slot = np.concatenate([np.tile(np.arange(rows * cols), n_boards), np.full(n_free, -1)]).astype(np.int32)
+    obj = np.concatenate([np.broadcast_to(np.concatenate([layout, np.zeros((rows * cols, 4, 1))], -1),
+                                          (n_boards, rows * cols, 4, 3)).reshape(-1, 4, 3),
+                          obj_points(np.full(n_free, tag_size))])
+    # views: cameras at -z looking at random points of the wall (the tags face -z)
+    wall_c = np.array([(n_boards * (bw + 2 * pitch) - 2 * pitch) / 2, bh / 2, 0.0])
+    wall_w, wall_h = n_boards * (bw + 2 * pitch), bh
+    tgt = wall_c + np.stack([rng.uniform(-0.4, 0.4, n_views) * wall_w, rng.uniform(-0.4, 0.4, n_views) * wall_h,
+                             np.zeros(n_views)], -1)
+    d = rng.uniform(0.8, 1.2, n_views) * distance
+    off = rng.normal(0, 0.25, (n_views, 2))
+    cam_pos = tgt + np.stack([off[:, 0] * d, off[:, 1] * d, -d * np.sqrt(np.maximum(0.2, 1 - (off ** 2).sum(-1)))], -1)
+    Rwc = _look_at(cam_pos, tgt, rng.normal(0, 0.2, n_views))
+    views_t = np.concatenate([rotation_to_rvec(Rwc), cam_pos], -1)
+    vi_l, mi_l, ci_l, sl_l, px_l = [], [], [], [], []
+    n_tags = len(tag_marker)
+    for c in range(n_cam):
+        vv, tt = np.repeat(np.arange(n_views), n_tags), np.tile(np.arange(n_tags), n_views)
+        uv, Z = project_points(model, np.broadcast_to(intr_t[c], (len(vv), 4)), np.broadcast_to(dist_t[c], (len(vv), 5)),
+                               np.broadcast_to(ext_t[c], (len(vv), 6)), views_t[vv], markers_t[tag_marker[tt]],
+                               obj[tt], lenses[c])
+        ok = ((Z > 0.1).all(-1) & (uv[..., 0] >= 0).all(-1) & (uv[..., 0] < W[c]).all(-1)
+              & (uv[..., 1] >= 0).all(-1) & (uv[..., 1] < H[c]).all(-1))
+        if fish[c]:
+            Rm = rodrigues_np(markers_t[tag_marker[tt], 0:3])
+            Pw = np.einsum('nij,nkj->nki', Rm, obj[tt]) + markers_t[tag_marker[tt], None, 3:6]
+            q = np.einsum('nji,nkj->nki', rodrigues_np(views_t[vv, 0:3]), Pw - views_t[vv, None, 3:6])
+            if model == "rig":
+                q = (q - ext_t[c, 3:6]) @ rodrigues_np(ext_t[c, 0:3])
+            ok &= (np.arctan2(np.hypot(q[..., 0], q[..., 1]), q[..., 2]) < np.deg2rad(85)).all(-1)
+        vi_l.append(vv[ok]); mi_l.append(tag_marker[tt[ok]]); ci_l.append(np.full(ok.sum(), c))
+        sl_l.append(tag_slot[tt[ok]]); px_l.append(uv[ok].reshape(-1, 8))
+    view_idx, marker_idx, cam_idx, slot = (np.concatenate(x).astype(np.int32) for x in (vi_l, mi_l, ci_l, sl_l))
+    pixels = np.concatenate(px_l) + rng.normal(0, pixel_noise, (len(view_idx), 8))
+    s_r, s_t, s_i = perturb
+    n_m = len(markers_t)
+    views0 = views_t + np.concatenate([rng.normal(0, s_r, (n_views, 3)), rng.normal(0, s_t, (n_views, 3))], -1)
+    markers0 = markers_t + np.concatenate([rng.normal(0, s_r, (n_m, 3)), rng.normal(0, s_t, (n_m, 3))], -1)
+    markers0[0] = markers_t[0]
+    intr0 = intr_t * (1 + rng.normal(0, s_i, intr_t.shape))
+    dist0 = dist_t + rng.normal(0, s_i, dist_t.shape) * 0.1
+    dist0[fish, 4] = 0.0
+    ext0 = ext_t.copy()
+    if model == "rig" and n_cam > 1:
+        ext0[1:] += np.concatenate([rng.normal(0, s_r, (n_cam - 1, 3)), rng.normal(0, s_t, (n_cam - 1, 3))], -1)
+    one = lenses[0] if len(set(lenses)) == 1 else lenses
+    return Scene(model=model, intr=intr0, dist=dist0, ext=ext0, views=views0, markers=markers0, sizes=sizes,
+                 view_idx=view_idx, marker_idx=marker_idx, cam_idx=cam_idx, pixels=pixels,
+                 truth=dict(intr=intr_t, dist=dist_t, ext=ext_t, views=views_t, markers=markers_t),
+                 image_size=sizes_img[0] if isinstance(one, str) else tuple(sizes_img), name=name, lens=one,
+                 corners=layout, corner_slot=slot)
 
 
 # ---------------------------------------------------------------- the BASELINE.json configs
