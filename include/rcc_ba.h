@@ -352,6 +352,20 @@ int rcc_pnp_batch(int32_t device, int64_t n, const double* shared9, const double
  * takes tan(th) along the distorted direction.  RCC_BAD_ARG for an unknown lens. */
 int rcc_pnp_batch_lens(int32_t device, int32_t lens, int64_t n, const double* shared9, const double* sizes,
                        const double* pixels, double* cam_T_tag, double* final_cost, int32_t max_iterations);
+/* Batched PnP of rigid targets (what cv::calibrateCamera's per-view solvePnP does for a board): one problem per
+ * (frame, target), minimising the reprojection error of every corner of the target's detected tags over
+ * cam_T_target (6 dof).  Problem p owns tags [start[p], start[p + 1]); tag t's corners are corners[slot[t]], the
+ * 64-byte records of rcc_ba_set_corner_layout (bl br tr tl, x y in the target frame, z = 0), its pixels
+ * pixels[8 t .. 8 t + 7].  lens and shared9 as in rcc_pnp_batch_lens.  cam_T_target (in/out) n_problems x 6: a guess
+ * of all zeros starts from the DLT homography of all the problem's corners, anything else is refined from there.
+ * final_cost n_problems (may be NULL): the cost 0.5 |r|^2, or -1 when a corner has depth <= 0 or a residual is not
+ * finite.  max_iterations <= 0 means 30.  One warp solves one problem; a problem's result depends only on its own
+ * inputs, bitwise, whatever the batch.  RCC_BAD_ARG, before any device is touched, for an unknown lens,
+ * n_problems < 0, a NULL array (n_problems > 0), start[0] != 0 or a problem without tags, n_slots < 1, a slot
+ * outside [0, n_slots) or a non-finite corner; n_problems == 0 is RCC_OK.  Free tags keep rcc_pnp_batch_lens. */
+int rcc_pnp_target_batch(int32_t device, int32_t lens, const double* shared9, int32_t n_slots, const double* corners,
+                         int64_t n_problems, const int64_t* start, const int32_t* slot, const double* pixels,
+                         double* cam_T_target, double* final_cost, int32_t max_iterations);
 
 #ifdef __cplusplus
 }

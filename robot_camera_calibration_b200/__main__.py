@@ -5,6 +5,9 @@ run the GPU bundle adjustment, and write the refined poses back in the same form
 (opt_visualization.cpp:162-220) picks them up.
 
     python -m robot_camera_calibration_b200 <detections directory> [--fix-intrinsics | --intrinsics-sigma F C D] ...
+
+With --initialise the directory needs only the detections and camera.yaml: the initial poses come from a batched
+GPU PnP per tag, or per (frame, board) with --target, chained the way camera_pose_node chains tags.
 """
 from __future__ import annotations
 
@@ -33,6 +36,10 @@ def parser():
                     help="a rigid tag board in Kalibr's AprilGrid format (target_type: aprilgrid, tagRows, tagCols, "
                          "tagSize, tagSpacing, optional firstTagId); repeatable.  Its detected tags are solved with "
                          "one pose per board; a tag id on two targets is an error")
+    ap.add_argument("--initialise", action="store_true",
+                    help="start from detections_N.yaml and camera.yaml alone: targets.yaml and any world_T_camera "
+                         "stanzas are ignored, the initial poses come from PnP on the GPU (one per (frame, board) "
+                         "with --target), and every frame that could not be chained loses its stanza")
     ap.add_argument("--max-iterations", type=int, default=50)
     ap.add_argument("--function-tolerance", type=float, default=None)
     ap.add_argument("--gradient-tolerance", type=float, default=None)
@@ -56,7 +63,8 @@ def main(argv=None):
     try:
         summary = io_yaml.optimise_directory(args.directory, device=args.device,
                                              refine_intrinsics=not args.fix_intrinsics, precision=args.precision,
-                                             intrinsics_sigma=args.intrinsics_sigma, targets=args.target, **opts)
+                                             intrinsics_sigma=args.intrinsics_sigma, targets=args.target,
+                                             initialise=args.initialise, **opts)
     except (FileNotFoundError, ValueError) as e:          # missing camera.yaml / targets.yaml, empty dataset, bad target
         print(f"error: {e}", file=sys.stderr)
         return 2

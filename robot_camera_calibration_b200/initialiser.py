@@ -8,6 +8,10 @@ Mirrors PoseSystem in /root/reference/real_preprocessing/src/camera_pose.cpp:
   tagCalc   :176-203  w_T_cam = w_T_tag * tag_T_cam ; new tags: w_T_tag = w_T_cam * cam_T_tag
   unknownFilepoll :249-263 / fileStream :267-285  deferred frames are retried, last first
 The pose chaining itself is a few 4x4 products per frame and stays on the host.
+
+initialise_targets does the same for rigid tag boards (io_yaml.read_targets): one PnP per (frame, board) over all
+of the board's detected corners (rcc_pnp_target_batch), as cv::calibrateCamera and Kalibr start a board, and the
+same chaining with a board or a free tag in place of each tag.
 """
 from __future__ import annotations
 
@@ -37,6 +41,36 @@ def pnp_batch(intr, dist, sizes, pixels, guess=None, device=0, max_iterations=10
                                 int(max_iterations))
     if rc != L.RCC_OK:
         raise L.RccError(rc, "rcc_pnp_batch failed (no CPU fallback)")
+    return poses, cost
+
+
+def pnp_targets(intr, dist, corners, start, slot, pixels, guess=None, device=0, max_iterations=100, lens="radtan"):
+    """cam_T_target (n,6) and final cost (n,) of n rigid-target problems on the GPU.  corners (n_slots,4,2): the
+    corners bl br tr tl of each layout slot in the target frame; problem p owns the tags [start[p], start[p + 1]) of
+    slot (tag's layout slot) and pixels (tag's 8 pixels).  A zero guess row starts from the DLT homography of the
+    problem's corners.  Cost -1: a corner behind the camera or a non-finite residual.  lens and dist as in
+    pnp_batch."""
+    lib = L.load()
+    if lens not in L.LENSES:
+        raise ValueError(f"unknown lens {lens!r}: expected one of {sorted(L.LENSES)}")
+    corners = np.ascontiguousarray(corners, np.float64).reshape(-1, 8)
+    start = np.ascontiguousarray(start, np.int64).ravel()
+    slot = np.ascontiguousarray(slot, np.int32).ravel()
+    pixels = np.ascontiguousarray(pixels, np.float64).reshape(-1, 8)
+    n = max(len(start) - 1, 0)
+    if len(start) == 0 or len(slot) != start[-1] or len(pixels) != len(slot):
+        raise ValueError(f"start ({len(start)}) must end at the number of tags: slot has {len(slot)}, "
+                         f"pixels {len(pixels)}")
+    d = np.asarray(dist, float).ravel()[:5]
+    sh = np.ascontiguousarray(np.concatenate([np.asarray(intr, float).ravel()[:4], d, np.zeros(5 - len(d))]))
+    poses = np.zeros((n, 6)) if guess is None else np.ascontiguousarray(guess, np.float64).reshape(n, 6).copy()
+    cost = np.empty(n)
+    dp = lambda a: a.ctypes.data_as(L.c_double_p)
+    rc = lib.rcc_pnp_target_batch(int(device), L.LENSES[lens], dp(sh), len(corners), dp(corners), n,
+                                  start.ctypes.data_as(L.c_int64_p), slot.ctypes.data_as(L.c_int32_p), dp(pixels),
+                                  dp(poses), dp(cost), int(max_iterations))
+    if rc != L.RCC_OK:
+        raise L.RccError(rc, "rcc_pnp_target_batch failed (no CPU fallback)")
     return poses, cost
 
 
@@ -119,3 +153,112 @@ def initialise(frames_pixels, intr, dist, device=0, lens="radtan"):
                   sizes=np.array(sizes, float), view_idx=np.array(vi, np.int32), marker_idx=np.array(mi, np.int32),
                   cam_idx=np.zeros(len(vi), np.int32), pixels=np.array(px, float).reshape(-1, 8))
     return scene, np.array(ids), np.array(keep)
+
+
+def board_T_tag(corners):
+    """The frame of a tag on a board: centred on its corners (4,2), with the board's axes."""
+    ctr = np.asarray(corners, float).reshape(4, 2).mean(0)
+    return np.array([0.0, 0.0, 0.0, ctr[0], ctr[1], 0.0])
+
+
+def group_entities(frame, where):
+    """The entities of one frame's detections [(tag_id, size, pixels8)]: one per target with a detected tag, keyed
+    ("target", b), and one per free tag, keyed ("tag", id), in the order of their first detection.  where: tag id ->
+    (target, slot).  Returns [(key, [detection index, ..])]."""
+    order, members = [], {}
+    for k, (t, _, _) in enumerate(frame):
+        w = where.get(int(t))
+        key = ("target", w[0]) if w is not None else ("tag", int(t))
+        if key not in members:
+            members[key] = []
+            order.append(key)
+        members[key].append(k)
+    return [(key, members[key]) for key in order]
+
+
+def initialise_targets(frames_pixels, intr, dist, targets, device=0, lens="radtan"):
+    """initialise() with rigid targets: targets = io_yaml.read_targets(...) [(tag ids, corners (n,4,2))].
+    Each frame's detections are grouped into entities (group_entities): a target's cam_T_target comes from one
+    pnp_targets problem over all its detected corners in the frame, a free tag's from pnp_batch.  The entities are
+    chained by chain_poses exactly as tags are (camera_pose.cpp: the world entity first, the last known entity wins,
+    deferred frames retried).  The world is the frame of the first tag of frame 0 (camera_pose.cpp:71-80): when
+    that tag is on a target, the target's pose is invert(board_T_tag) of it, and the target is held constant.
+    Returns (scene, tag_ids, kept_frames, tag_pose, boards) as io_yaml.board_scene: the scene (marker 0 the world
+    entity, then the entities in the order they were chained) carries the corner layout; tag_ids are the detected
+    tags of the chained entities, the world tag first; tag_pose(markers) -> world_T_tag of every tag of tag_ids;
+    boards = [(first tag id of the target, marker block)] in target order."""
+    where, offset = {}, 0
+    for b, (ids, _) in enumerate(targets):
+        for k, i in enumerate(np.asarray(ids).tolist()):
+            where[int(i)] = (b, offset + k)
+        offset += len(ids)
+    corners = (np.concatenate([np.asarray(c, float).reshape(-1, 4, 2) for _, c in targets]) if targets
+               else np.zeros((0, 4, 2)))
+    grouped = [group_entities(fr, where) for fr in frames_pixels]
+    # one target problem per (frame, target entity), one pnp_batch row per free tag
+    t_start, t_slot, t_pix, f_size, f_pix = [0], [], [], [], []
+    for fr, ents in zip(frames_pixels, grouped):
+        for key, ks in ents:
+            if key[0] == "target":
+                t_slot += [where[int(fr[k][0])][1] for k in ks]
+                t_pix += [fr[k][2] for k in ks]
+                t_start.append(len(t_slot))
+            else:
+                f_size.append(fr[ks[0]][1])
+                f_pix.append(fr[ks[0]][2])
+    t_pose = (pnp_targets(intr, dist, corners, t_start, t_slot, np.array(t_pix, float).reshape(-1, 8),
+                          device=device, lens=lens)[0] if len(t_start) > 1 else np.zeros((0, 6)))
+    f_pose = (pnp_batch(intr, dist, f_size, np.array(f_pix, float).reshape(-1, 8), device=device, lens=lens)[0]
+              if f_size else np.zeros((0, 6)))
+    frames, cTe, it, jf = [], [], 0, 0
+    for fr, ents in zip(frames_pixels, grouped):
+        poses = []
+        for key, ks in ents:
+            if key[0] == "target":
+                poses.append(t_pose[it]); it += 1
+            else:
+                poses.append(f_pose[jf]); jf += 1
+        frames.append([(key, fr[ks[0]][1]) for key, ks in ents])
+        cTe.append(np.array(poses).reshape(-1, 6))
+    keys, _, w_T_e, w_T_cam = chain_poses(frames, cTe)
+    if keys and keys[0][0] == "target":
+        # the chain's world is the target's frame: move it to the world tag's, world_T_target = invert(board_T_tag)
+        w_T_b = invert(board_T_tag(corners[where[int(frames_pixels[0][0][0])][1]]))
+        w_T_e = compose(np.broadcast_to(w_T_b, w_T_e.shape), w_T_e)
+        w_T_cam = [None if x is None else compose(w_T_b, x) for x in w_T_cam]
+    keep = [n for n in range(len(frames)) if w_T_cam[n] is not None]
+    marker_of = {key: m for m, key in enumerate(keys)}
+    vi, mi, sl, px, tags, sizes = [], [], [], [], {}, np.zeros(len(keys))
+    for v, n in enumerate(keep):
+        for key, ks in grouped[n]:
+            for k in ks:
+                t, sz, p = frames_pixels[n][k]
+                vi.append(v); mi.append(marker_of[key]); px.append(p)
+                sl.append(where[int(t)][1] if key[0] == "target" else -1)
+                tags.setdefault(int(t), (marker_of[key], sl[-1]))
+                if sizes[marker_of[key]] == 0:
+                    sizes[marker_of[key]] = sz
+    world_tag = int(frames_pixels[0][0][0]) if keys else None
+    tag_ids = sorted(tags, key=lambda t: (t != world_tag, tags[t][0], tags[t][1]))
+    pix = np.array(px).reshape(-1, 8)
+    if not np.issubdtype(pix.dtype, np.integer):
+        pix = pix.astype(np.float64)
+    elif pix.size and pix.min() >= -32768 and pix.max() <= 32767:
+        pix = pix.astype(np.int16)
+    d = np.asarray(dist, float).ravel()
+    scene = Scene(model="single", intr=np.asarray(intr, float).reshape(1, 4),
+                  dist=np.concatenate([d, np.zeros(5 - len(d))]).reshape(1, 5), lens=lens,
+                  ext=np.zeros((1, 6)), views=np.array([w_T_cam[n] for n in keep]).reshape(-1, 6),
+                  markers=np.asarray(w_T_e, float).reshape(-1, 6), sizes=sizes, view_idx=np.array(vi, np.int32),
+                  marker_idx=np.array(mi, np.int32), cam_idx=np.zeros(len(vi), np.int32), pixels=pix,
+                  corners=corners, corner_slot=np.array(sl, np.int32))
+
+    def tag_pose(markers):
+        out = np.empty((len(tag_ids), 6))
+        for j, t in enumerate(tag_ids):
+            m, s = tags[t]
+            out[j] = markers[m] if s < 0 else compose(markers[m], board_T_tag(corners[s]))
+        return out
+
+    boards = [(int(targets[key[1]][0][0]), marker_of[key]) for key in sorted(k for k in keys if k[0] == "target")]
+    return scene, np.array(tag_ids, dtype=np.int64), np.array(keep, dtype=np.int64), tag_pose, boards

@@ -196,6 +196,38 @@ def read_dataset(directory, intr=None, dist=None, lens=None):
             vi.append(v)
             mi.append(index_of[tid])
             px.append([c[k][a] for k in range(4) for a in range(2)])
+    intr, dist, lens = _dataset_camera(directory, intr, dist, lens)
+    scene = Scene(model="single", intr=intr.reshape(1, 4), dist=dist.reshape(1, 5), ext=np.zeros((1, 6)),
+                  views=np.array(views, dtype=np.float64).reshape(-1, 6), markers=markers, sizes=sizes,
+                  view_idx=np.array(vi, dtype=np.int32), marker_idx=np.array(mi, dtype=np.int32),
+                  cam_idx=np.zeros(len(vi), dtype=np.int32), pixels=_pixel_array(px), lens=lens)
+    return scene, tag_ids, np.array(frames)
+
+
+def read_detections(directory):
+    """detections_N.yaml of a directory in numeric order of N -> (frame numbers, frames_pixels), frames_pixels in the
+    format initialiser.initialise takes: per frame [(tag_id, size, pixels8)], the size from the file's `size` entry
+    (corner_detections.cpp:18-39) and the pixels as the corners' own numbers (integers stay integers, so that the
+    scene keeps the int16 pixel path).  Any world_T_camera stanza is ignored."""
+    files = glob.glob(os.path.join(directory, "detections_*.yaml"))
+    numbered = sorted((int(re.search(r"detections_(\d+)\.yaml$", p).group(1)), p) for p in files)
+    frames, out = [], []
+    for n, path in numbered:
+        with open(path) as f:
+            y = yaml.safe_load(f) or {}
+        fr = []
+        for det in y.get("detections") or []:
+            c = det["corners"]
+            px = [c[k][a] for k in range(4) for a in range(2)]
+            px = np.array(px, dtype=np.int64 if all(isinstance(v, int) for v in px) else np.float64)
+            fr.append((int(det["targetID"]), float(det["size"][0]), px))
+        frames.append(n)
+        out.append(fr)
+    return np.array(frames, dtype=np.int64), out
+
+
+def _dataset_camera(directory, intr, dist, lens):
+    """The camera of a dataset as read_dataset documents it -> (intr, dist[5], lens)."""
     cam = os.path.join(directory, "camera.yaml")
     if intr is not None and dist is not None:
         intr, dist = np.asarray(intr, dtype=np.float64), np.asarray(dist, dtype=np.float64).ravel()
@@ -210,11 +242,7 @@ def read_dataset(directory, intr=None, dist=None, lens=None):
     else:
         raise FileNotFoundError(f"{cam} not found and no intr/dist given: the camera intrinsics are required "
                                 "(camera_pose.cpp:59-67)")
-    scene = Scene(model="single", intr=intr.reshape(1, 4), dist=dist.reshape(1, 5), ext=np.zeros((1, 6)),
-                  views=np.array(views, dtype=np.float64).reshape(-1, 6), markers=markers, sizes=sizes,
-                  view_idx=np.array(vi, dtype=np.int32), marker_idx=np.array(mi, dtype=np.int32),
-                  cam_idx=np.zeros(len(vi), dtype=np.int32), pixels=_pixel_array(px), lens=lens)
-    return scene, tag_ids, np.array(frames)
+    return intr, dist, lens
 
 
 def read_target(path):
@@ -329,8 +357,12 @@ def _pixel_array(px):
 def write_results(directory, scene, tag_ids, frames, precision=None):
     """Write refined poses back: targets.yaml is rewritten (camera_pose.cpp:103-129)
     and the world_T_camera stanza of every frame is replaced (:95-99)."""
+    _write_poses(directory, tag_ids, scene.sizes, scene.markers, scene.views, frames, precision)
+
+
+def _write_poses(directory, tag_ids, sizes, markers, views, frames, precision=None):
     with open(os.path.join(directory, "targets.yaml"), "w") as f:
-        f.write(targets_text(tag_ids, scene.sizes, scene.markers, precision))
+        f.write(targets_text(tag_ids, sizes, markers, precision))
     for v, n in enumerate(frames):
         path = os.path.join(directory, f"detections_{int(n)}.yaml")
         with open(path) as f:
@@ -338,7 +370,46 @@ def write_results(directory, scene, tag_ids, frames, precision=None):
         k = txt.find("world_T_camera:")
         head = txt[:k] if k >= 0 else txt
         with open(path, "w") as f:
-            f.write(head + world_T_camera_text(scene.views[v, 0:3], scene.views[v, 3:6], precision))
+            f.write(head + world_T_camera_text(views[v, 0:3], views[v, 3:6], precision))
+
+
+def _remove_stanza(path):
+    """Drop the world_T_camera stanza of a detections file, if it has one."""
+    with open(path) as f:
+        txt = f.read()
+    k = txt.find("world_T_camera:")
+    if k >= 0:
+        with open(path, "w") as f:
+            f.write(txt[:k])
+
+
+def _initialise_directory(directory, intr, dist, lens, targets):
+    """The start of optimise_directory(initialise=True): the camera as read_dataset reads it, the poses from the
+    detections alone.  Returns (scene, tag_ids, kept frame numbers, (all frame numbers, frames_pixels), tag_pose,
+    boards); tag_pose and boards as board_scene's (per tag and empty without targets)."""
+    from . import initialiser
+    if lens is not None and lens not in _LENS_MODEL:
+        raise ValueError(f"unknown lens {lens!r}: expected one of {sorted(_LENS_MODEL)}")
+    intr, dist, lens = _dataset_camera(directory, intr, dist, lens)
+    numbers, frames_pixels = read_detections(directory)
+    if not frames_pixels or not frames_pixels[0]:
+        raise ValueError(f"{directory}: the first detections file has no detection: nothing defines the world frame "
+                         "(camera_pose.cpp:71-80 makes the first tag of frame 0 the world tag)")
+    if targets:
+        scene, tag_ids, keep, tag_pose, boards = initialiser.initialise_targets(
+            frames_pixels, intr, dist, read_targets(list(targets)), lens=lens)
+    else:
+        scene, tag_ids, keep = initialiser.initialise(frames_pixels, intr, dist, lens=lens)
+        scene.pixels = _integer_pixels(scene.pixels, frames_pixels)
+        tag_pose, boards = (lambda markers: markers), []
+    return scene, tag_ids, numbers[keep], (numbers, frames_pixels), tag_pose, boards
+
+
+def _integer_pixels(pixels, frames_pixels):
+    """initialiser.initialise returns FP64 pixels: give integer detections their integer type back (_pixel_array)."""
+    if all(np.issubdtype(np.asarray(p).dtype, np.integer) for fr in frames_pixels for (_, _, p) in fr):
+        return _pixel_array(np.asarray(pixels).astype(np.int64).tolist())
+    return pixels
 
 
 def intrinsics_priors(intr, dist, sigma):
@@ -357,22 +428,31 @@ def intrinsics_priors(intr, dist, sigma):
 
 
 def optimise_directory(directory, device=0, refine_intrinsics=True, precision=None, intr=None, dist=None,
-                       lens=None, intrinsics_sigma=None, targets=None, **lm_options):
+                       lens=None, intrinsics_sigma=None, targets=None, initialise=False, **lm_options):
     """Milestone 3: detections/ -> GPU bundle adjustment -> detections/ (same formats).  The lens is camera.yaml's
     distortion_model (plumb_bob, or equidistant / fisheye), and camera_refined.yaml is written in the same model.
     intrinsics_sigma = (focal px, principal point px, distortion): refine the intrinsics under a diagonal Gaussian
     prior centred on camera.yaml (intrinsics_priors) instead of freely; it needs refine_intrinsics.
     targets: AprilGrid target files (read_target).  Their detected tags are solved as rigid boards, one pose each
     (board_scene); targets.yaml is still written per tag (world_T_board o board_T_tag), and the summary gains
-    "boards": [{"first_tag_id", "world_T_board": rvec + t}] per board."""
+    "boards": [{"first_tag_id", "world_T_board": rvec + t}] per board.
+    initialise: start from the detections alone instead of camera_pose_node's output.  targets.yaml and any
+    world_T_camera stanzas are ignored; the camera comes from camera.yaml or intr / dist as in read_dataset; the
+    poses come from initialiser.initialise_targets (with targets) or initialiser.initialise (without).  After the
+    solve targets.yaml is written per tag, every chained frame gets a world_T_camera stanza, and the stanza of a frame
+    that could not be chained is removed, so that no stale pose is left behind."""
     from .problem import BAProblem
     if intrinsics_sigma is not None and not refine_intrinsics:
         raise ValueError("intrinsics_sigma puts a prior on refined intrinsics: it cannot be combined with fixed ones")
-    scene, tag_ids, frames = read_dataset(directory, intr=intr, dist=dist, lens=lens)
+    if initialise:
+        scene, tag_ids, frames, all_frames, tag_pose, boards = _initialise_directory(directory, intr, dist, lens,
+                                                                                     targets)
+    else:
+        scene, tag_ids, frames = read_dataset(directory, intr=intr, dist=dist, lens=lens)
     scene.const_intr[:] = not refine_intrinsics
     scene.const_dist[:] = not refine_intrinsics
     tags = scene
-    if targets:
+    if targets and not initialise:
         scene, tag_pose, boards = board_scene(tags, tag_ids, read_targets(list(targets)))
     with BAProblem.from_scene(scene, device=device) as p:
         if intrinsics_sigma is not None:
@@ -384,9 +464,19 @@ def optimise_directory(directory, device=0, refine_intrinsics=True, precision=No
         scene.intr, scene.dist = intr, dist
     if targets:
         summary["boards"] = [{"first_tag_id": i, "world_T_board": scene.markers[j].tolist()} for i, j in boards]
-        tags.views, tags.markers = scene.views, tag_pose(scene.markers)
-        scene = tags
-    write_results(directory, scene, tag_ids, frames, precision)
+    if initialise:
+        size_of = {int(t): float(sz) for fr in all_frames[1] for (t, sz, _) in fr}
+        _write_poses(directory, tag_ids, [size_of[int(t)] for t in tag_ids], tag_pose(scene.markers), scene.views,
+                     frames, precision)
+        kept = set(frames.tolist())
+        for n in all_frames[0].tolist():
+            if n not in kept:
+                _remove_stanza(os.path.join(directory, f"detections_{n}.yaml"))
+    else:
+        if targets:
+            tags.views, tags.markers = scene.views, tag_pose(scene.markers)
+            scene = tags
+        write_results(directory, scene, tag_ids, frames, precision)
     if refine_intrinsics:
         with open(os.path.join(directory, "camera_refined.yaml"), "w") as f:
             f.write(camera_yaml_text(intr[0], dist[0], scene.image_size, lens=scene.lens))
