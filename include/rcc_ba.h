@@ -366,6 +366,19 @@ int rcc_pnp_batch_lens(int32_t device, int32_t lens, int64_t n, const double* sh
 int rcc_pnp_target_batch(int32_t device, int32_t lens, const double* shared9, int32_t n_slots, const double* corners,
                          int64_t n_problems, const int64_t* start, const int32_t* slot, const double* pixels,
                          double* cam_T_target, double* final_cost, int32_t max_iterations);
+/* Batched plane homographies of rigid targets (what cv::findHomography, method 0, does per view before
+ * cv::initCameraMatrix2D): problems, start, slot, corners and pixels as in rcc_pnp_target_batch; no lens and no
+ * intrinsics.  H n_problems x 9 (out): row-major, maps (X, Y, 1) in the target frame to (u, v, 1) in raw pixels and
+ * is scaled to H[8] = 1.  It minimises the pixel reprojection error 0.5 sum |u - H(X)|^2 (cv::findHomography's
+ * refinement cost, run to convergence) from a DLT start with both sides Hartley-normalised.  final_cost n_problems
+ * (may be NULL): that cost in px^2, or -1 (and H all zero) when the DLT is singular, a residual is not finite or a
+ * corner has w = h31 X + h32 Y + h33 <= 0 at the result.  max_iterations <= 0 means 30.  One warp solves one
+ * problem; a problem's result depends only on its own inputs, bitwise, whatever the batch.  RCC_BAD_ARG, before
+ * any device is touched, for n_problems < 0, a NULL array (n_problems > 0), start[0] != 0 or a problem without
+ * tags, n_slots < 1, a slot outside [0, n_slots) or a non-finite corner; n_problems == 0 is RCC_OK. */
+int rcc_homography_target_batch(int32_t device, int32_t n_slots, const double* corners, int64_t n_problems,
+                                const int64_t* start, const int32_t* slot, const double* pixels, double* H,
+                                double* final_cost, int32_t max_iterations);
 
 #ifdef __cplusplus
 }

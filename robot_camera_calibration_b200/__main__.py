@@ -7,7 +7,8 @@ run the GPU bundle adjustment, and write the refined poses back in the same form
     python -m robot_camera_calibration_b200 <detections directory> [--fix-intrinsics | --intrinsics-sigma F C D] ...
 
 With --initialise the directory needs only the detections and camera.yaml: the initial poses come from a batched
-GPU PnP per tag, or per (frame, board) with --target, chained the way camera_pose_node chains tags.
+GPU PnP per tag, or per (frame, board) with --target, chained the way camera_pose_node chains tags.  Adding
+--image-size W H calibrates a camera without camera.yaml: its intrinsics start from the board detections.
 """
 from __future__ import annotations
 
@@ -40,6 +41,13 @@ def parser():
                     help="start from detections_N.yaml and camera.yaml alone: targets.yaml and any world_T_camera "
                          "stanzas are ignored, the initial poses come from PnP on the GPU (one per (frame, board) "
                          "with --target), and every frame that could not be chained loses its stanza")
+    ap.add_argument("--image-size", type=int, nargs=2, metavar=("W", "H"), default=None,
+                    help="with --initialise and --target: calibrate the camera from the board detections alone.  The "
+                         "start comes from one homography per (frame, board) and OpenCV's closed form with the "
+                         "principal point at the image centre, with zero distortion; camera.yaml is neither read nor "
+                         "written, and camera_refined.yaml gets this size")
+    ap.add_argument("--lens", choices=("radtan", "equidistant"), default=None,
+                    help="with --image-size: the lens model to calibrate (default radtan)")
     ap.add_argument("--max-iterations", type=int, default=50)
     ap.add_argument("--function-tolerance", type=float, default=None)
     ap.add_argument("--gradient-tolerance", type=float, default=None)
@@ -55,6 +63,15 @@ def main(argv=None):
     args = ap.parse_args(argv)
     if args.intrinsics_sigma is not None and not all(0 < s < float("inf") for s in args.intrinsics_sigma):
         ap.error("--intrinsics-sigma: every sigma must be positive and finite")
+    if args.lens is not None and args.image_size is None:
+        ap.error("--lens names the model to calibrate: it needs --image-size")
+    if args.image_size is not None:
+        if not args.initialise or not args.target:
+            ap.error("--image-size estimates the intrinsics from board detections: it needs --initialise and --target")
+        if args.fix_intrinsics or args.intrinsics_sigma is not None:
+            ap.error("--image-size calibrates the intrinsics: it excludes --fix-intrinsics and --intrinsics-sigma")
+        if not all(0 < v for v in args.image_size):
+            ap.error("--image-size: width and height must be positive")
     from . import io_yaml
     opts = {"max_iterations": args.max_iterations, "verbose": int(args.verbose)}
     for k in ("function_tolerance", "gradient_tolerance", "parameter_tolerance"):
@@ -64,7 +81,8 @@ def main(argv=None):
         summary = io_yaml.optimise_directory(args.directory, device=args.device,
                                              refine_intrinsics=not args.fix_intrinsics, precision=args.precision,
                                              intrinsics_sigma=args.intrinsics_sigma, targets=args.target,
-                                             initialise=args.initialise, **opts)
+                                             initialise=args.initialise, image_size=args.image_size, lens=args.lens,
+                                             **opts)
     except (FileNotFoundError, ValueError) as e:          # missing camera.yaml / targets.yaml, empty dataset, bad target
         print(f"error: {e}", file=sys.stderr)
         return 2

@@ -118,6 +118,8 @@ SIGNATURES = {
                                      c_double_p, C.c_int32]),
     "rcc_pnp_target_batch": (C.c_int, [C.c_int32, C.c_int32, c_double_p, C.c_int32, c_double_p, C.c_int64, c_int64_p,
                                        c_int32_p, c_double_p, c_double_p, c_double_p, C.c_int32]),
+    "rcc_homography_target_batch": (C.c_int, [C.c_int32, C.c_int32, c_double_p, C.c_int64, c_int64_p, c_int32_p,
+                                              c_double_p, c_double_p, c_double_p, C.c_int32]),
 }
 
 _lib = None

@@ -457,6 +457,194 @@ __global__ void __launch_bounds__(128) pnp_target_kernel(int64_t n, const double
   }
 }
 
+// ---- plane homographies of rigid-target problems (cv::findHomography, method 0), one warp per problem
+//
+// Both sides are Hartley-normalised, board points (X', Y') = sb (X - mX, Y - mY) and pixels (x', y') = sp (u - mu,
+// v - mv), and the 8 free entries h of the normalised homography Hn (h33 = 1) are solved for there: the DLT start and
+// the Levenberg-Marquardt refinement both stay well conditioned although raw pixels are ~1e3 and board points ~1e-1.
+// The residual is the pixel residual of H = Tp^-1 Hn Tb: (x'_pred - x') / sp == u_pred - u, so the minimiser is the
+// one of cv::findHomography's HomographyRefineCallback cost.  pnp_target_kernel keeps its own inline copy of the
+// board-side normalisation and DLT accumulation (it undistorts the image side and normalises only the board side).
+
+// cost (normalised units: times 1 / sp^2 for px^2) of the problem at h and, with WANT_J, the upper triangle of J^T J
+// (36 values, row by row) and J^T r, all summed over the warp.  ok: every corner has w' > 0 and finite residuals.
+template <bool WANT_J>
+__device__ double homography_cost(const double* h, const TargetProblem& q, int lane, const double* nrm, double* H,
+                                  double* g, bool* ok) {
+  constexpr int NS = WANT_J ? 45 : 1;   // [cost, J^T J (36), J^T r (8)]
+  double acc[NS];
+#pragma unroll
+  for (int i = 0; i < NS; ++i) acc[i] = 0.0;
+  bool good = true;
+  for (int c = lane; c < q.n; c += 32) {
+    double X, Y, u, v;
+    target_corner(q, c, X, Y, u, v);
+    X = (X - nrm[0]) * nrm[2];
+    Y = (Y - nrm[1]) * nrm[2];
+    const double x = (u - nrm[3]) * nrm[5], y = (v - nrm[4]) * nrm[5];
+    const double wv = h[6] * X + h[7] * Y + 1.0;
+    const double iw = 1.0 / wv;
+    const double px = (h[0] * X + h[1] * Y + h[2]) * iw, py = (h[3] * X + h[4] * Y + h[5]) * iw;
+    const double r[2] = {px - x, py - y};
+    if (!(wv > 0.0) || !isfinite(r[0]) || !isfinite(r[1])) good = false;
+    acc[0] += r[0] * r[0] + r[1] * r[1];
+    if (WANT_J) {
+      const double j[2][8] = {{X * iw, Y * iw, iw, 0, 0, 0, -px * X * iw, -px * Y * iw},
+                              {0, 0, 0, X * iw, Y * iw, iw, -py * X * iw, -py * Y * iw}};
+#pragma unroll
+      for (int i = 0; i < 2; ++i) {
+        int m = 1;
+#pragma unroll
+        for (int a = 0; a < 8; ++a)
+#pragma unroll
+          for (int b = a; b < 8; ++b) acc[m++] += j[i][a] * j[i][b];
+#pragma unroll
+        for (int a = 0; a < 8; ++a) acc[37 + a] += j[i][a] * r[i];
+      }
+    }
+  }
+  warp_sum(acc);
+  *ok = __all_sync(0xffffffffu, good);
+  if (WANT_J) {
+#pragma unroll
+    for (int i = 0; i < 36; ++i) H[i] = acc[1 + i];
+#pragma unroll
+    for (int a = 0; a < 8; ++a) g[a] = acc[37 + a];
+  }
+  return 0.5 * acc[0];
+}
+
+__global__ void __launch_bounds__(128) homography_target_kernel(int64_t n, const double* __restrict__ corners,
+                                                                const int64_t* __restrict__ start,
+                                                                const int32_t* __restrict__ slot,
+                                                                const double* __restrict__ pixels,
+                                                                double* __restrict__ Hout,
+                                                                double* __restrict__ final_cost, int max_iter) {
+  const int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (w >= n) return;   // whole warps leave together: blockDim is a multiple of 32
+  const int64_t t0 = start[w];
+  const TargetProblem q{corners, slot + t0, pixels + 8 * t0, (int)(4 * (start[w + 1] - t0))};
+
+  // ---- Hartley normalisation of both sides: nrm = {mX, mY, sb, mu, mv, sp}
+  double m[4] = {0.0, 0.0, 0.0, 0.0};
+  for (int c = lane; c < q.n; c += 32) {
+    double X, Y, u, v;
+    target_corner(q, c, X, Y, u, v);
+    m[0] += X; m[1] += Y; m[2] += u; m[3] += v;
+  }
+  warp_sum(m);
+  double nrm[6] = {m[0] / q.n, m[1] / q.n, 1.0, m[2] / q.n, m[3] / q.n, 1.0};
+  double dsum[2] = {0.0, 0.0};
+  for (int c = lane; c < q.n; c += 32) {
+    double X, Y, u, v;
+    target_corner(q, c, X, Y, u, v);
+    dsum[0] += sqrt((X - nrm[0]) * (X - nrm[0]) + (Y - nrm[1]) * (Y - nrm[1]));
+    dsum[1] += sqrt((u - nrm[3]) * (u - nrm[3]) + (v - nrm[4]) * (v - nrm[4]));
+  }
+  warp_sum(dsum);
+  if (dsum[0] > 0.0) nrm[2] = sqrt(2.0) * q.n / dsum[0];
+  if (dsum[1] > 0.0) nrm[5] = sqrt(2.0) * q.n / dsum[1];
+
+  // ---- DLT start, h33 = 1, least squares over all corners: the normal equations, upper triangle of A^T A (36) and
+  // A^T b (8), accumulated per lane and summed over the warp
+  double ne[44];
+#pragma unroll
+  for (int i = 0; i < 44; ++i) ne[i] = 0.0;
+  for (int c = lane; c < q.n; c += 32) {
+    double X, Y, u, v;
+    target_corner(q, c, X, Y, u, v);
+    X = (X - nrm[0]) * nrm[2];
+    Y = (Y - nrm[1]) * nrm[2];
+    const double x = (u - nrm[3]) * nrm[5], y = (v - nrm[4]) * nrm[5];
+    const double r0[8] = {X, Y, 1, 0, 0, 0, -x * X, -x * Y};
+    const double r1[8] = {0, 0, 0, X, Y, 1, -y * X, -y * Y};
+    int k = 0;
+#pragma unroll
+    for (int a = 0; a < 8; ++a)
+#pragma unroll
+      for (int b = a; b < 8; ++b) ne[k++] += r0[a] * r0[b] + r1[a] * r1[b];
+#pragma unroll
+    for (int a = 0; a < 8; ++a) ne[36 + a] += r0[a] * x + r1[a] * y;
+  }
+  warp_sum(ne);
+  double h[8];
+  bool ok;
+  {
+    double A[8][8];
+    int k = 0;
+    for (int a = 0; a < 8; ++a)
+      for (int c = a; c < 8; ++c) { A[a][c] = ne[k]; A[c][a] = ne[k]; ++k; }
+    for (int a = 0; a < 8; ++a) h[a] = ne[36 + a];
+    ok = solve_dense<8>(A, h);
+  }
+
+  double cost = -1.0;
+  if (ok) {
+    // ---- Levenberg-Marquardt on the normalised entries: pnp_target_kernel's acceptance, damping and stopping rules
+    double H[36], g[8];
+    cost = homography_cost<true>(h, q, lane, nrm, H, g, &ok);
+    double lambda = 1e-3;
+    for (int it = 0; it < max_iter; ++it) {
+      double A8[8][8], rhs[8];
+      {
+        int k = 0;
+        for (int a = 0; a < 8; ++a)
+          for (int c = a; c < 8; ++c) { A8[a][c] = H[k]; A8[c][a] = H[k]; ++k; }
+      }
+      for (int a = 0; a < 8; ++a) {
+        A8[a][a] += lambda * fmax(A8[a][a], 1e-12);
+        rhs[a] = -g[a];
+      }
+      if (!solve_dense<8>(A8, rhs)) { lambda *= 10.0; continue; }
+      double hq[8];
+      double dn = 0.0, pn = 0.0;
+      for (int a = 0; a < 8; ++a) { hq[a] = h[a] + rhs[a]; dn += rhs[a] * rhs[a]; pn += h[a] * h[a]; }
+      bool ok2;
+      const double c2 = homography_cost<false>(hq, q, lane, nrm, nullptr, nullptr, &ok2);
+      // steps below 1e-5 relative are taken on trust (see pnp_kernel)
+      const bool tiny = dn <= 1e-10 * (pn + 1e-10);
+      if (ok2 && (tiny || c2 <= cost * (1.0 + 4e-16))) {
+        for (int a = 0; a < 8; ++a) h[a] = hq[a];
+        cost = homography_cost<true>(h, q, lane, nrm, H, g, &ok);
+        lambda = fmax(lambda * 0.1, 1e-12);
+        if (dn <= 1e-26 * (pn + 1e-26)) break;
+      } else {
+        lambda *= 10.0;
+        if (lambda > 1e12) break;
+      }
+    }
+  }
+
+  // ---- back to the board frame and raw pixels: H = Tp^-1 Hn Tb with Tb = [sb 0 -sb mX; 0 sb -sb mY; 0 0 1] and
+  // Tp^-1 = [1/sp 0 mu; 0 1/sp mv; 0 0 1], then scaled to H[8] = 1.  Tp^-1 keeps the third row, so w at a corner is
+  // w' / H[8] before the scaling: every corner has w > 0 at the result when all w' > 0 and H[8] > 0.
+  double R[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+  if (ok) {
+    const double hn[9] = {h[0], h[1], h[2], h[3], h[4], h[5], h[6], h[7], 1.0};
+    double M[9];   // Hn Tb
+    for (int r = 0; r < 3; ++r) {
+      M[3 * r + 0] = nrm[2] * hn[3 * r + 0];
+      M[3 * r + 1] = nrm[2] * hn[3 * r + 1];
+      M[3 * r + 2] = hn[3 * r + 2] - nrm[2] * (nrm[0] * hn[3 * r + 0] + nrm[1] * hn[3 * r + 1]);
+    }
+    for (int c = 0; c < 3; ++c) {
+      R[c] = M[c] / nrm[5] + nrm[3] * M[6 + c];
+      R[3 + c] = M[3 + c] / nrm[5] + nrm[4] * M[6 + c];
+      R[6 + c] = M[6 + c];
+    }
+    const double s = R[8];
+    ok = s > 0.0 && isfinite(s);
+    for (int k = 0; k < 9; ++k) R[k] /= s;
+    R[8] = 1.0;
+    for (int k = 0; k < 9; ++k) ok = ok && isfinite(R[k]);
+  }
+  if (lane == 0) {
+    for (int k = 0; k < 9; ++k) Hout[w * 9 + k] = ok ? R[k] : 0.0;
+    if (final_cost) final_cost[w] = ok ? cost / (nrm[5] * nrm[5]) : -1.0;
+  }
+}
+
 }  // namespace rcc
 
 extern "C" int rcc_pnp_batch_lens(int32_t device, int32_t lens, int64_t n, const double* shared9, const double* sizes,
@@ -552,6 +740,55 @@ extern "C" int rcc_pnp_target_batch(int32_t device, int32_t lens, const double* 
   } catch (const Error& e) {
     if (s) cudaStreamDestroy(s);
     fprintf(stderr, "[rcc_pnp_target_batch] %s\n", e.what());
+    return e.status;
+  }
+  return RCC_OK;
+}
+
+extern "C" int rcc_homography_target_batch(int32_t device, int32_t n_slots, const double* corners, int64_t n_problems,
+                                           const int64_t* start, const int32_t* slot, const double* pixels, double* H,
+                                           double* final_cost, int32_t max_iterations) {
+  using namespace rcc;
+  if (n_problems < 0) return RCC_BAD_ARG;
+  if (n_problems == 0) return RCC_OK;
+  if (!corners || !start || !slot || !pixels || !H) return RCC_BAD_ARG;
+  if (n_slots < 1) return RCC_BAD_ARG;
+  if (start[0] != 0) return RCC_BAD_ARG;
+  for (int64_t p = 0; p < n_problems; ++p)   // every problem has a tag, and no more corners than an int counts
+    if (!(start[p + 1] > start[p]) || start[p + 1] - start[p] > (int64_t)(INT32_MAX / 4)) return RCC_BAD_ARG;
+  const int64_t n_tags = start[n_problems];
+  for (int64_t t = 0; t < n_tags; ++t)
+    if (slot[t] < 0 || slot[t] >= n_slots) return RCC_BAD_ARG;
+  for (int64_t i = 0; i < (int64_t)n_slots * 8; ++i)
+    if (!std::isfinite(corners[i])) return RCC_BAD_ARG;
+  cudaStream_t s = nullptr;
+  try {
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
+      throw Error(RCC_CUDA_ERROR, "no CUDA device (this library has no CPU fallback)");
+    RCC_CUDA(cudaSetDevice(device));
+    DBuf<double> dcorn, dpx, dH, dcost;
+    DBuf<int64_t> dstart;
+    DBuf<int32_t> dslot;
+    RCC_CUDA(cudaStreamCreate(&s));
+    dcorn.upload(corners, (size_t)n_slots * 8, s);
+    dstart.upload(start, (size_t)n_problems + 1, s);
+    dslot.upload(slot, (size_t)n_tags, s);
+    dpx.upload(pixels, (size_t)n_tags * 8, s);
+    dH.alloc((size_t)n_problems * 9);
+    dcost.alloc((size_t)n_problems);
+    const int iters = max_iterations > 0 ? max_iterations : 30;
+    const int blocks = ceil_div(n_problems, 4);   // 4 warps of 128 threads, one problem each
+    homography_target_kernel<<<blocks, 128, 0, s>>>(n_problems, dcorn.p, dstart.p, dslot.p, dpx.p, dH.p, dcost.p,
+                                                    iters);
+    RCC_CUDA(cudaGetLastError());
+    dH.download(H, (size_t)n_problems * 9, s);
+    if (final_cost) dcost.download(final_cost, (size_t)n_problems, s);
+    RCC_CUDA(cudaStreamSynchronize(s));
+    cudaStreamDestroy(s);
+  } catch (const Error& e) {
+    if (s) cudaStreamDestroy(s);
+    fprintf(stderr, "[rcc_homography_target_batch] %s\n", e.what());
     return e.status;
   }
   return RCC_OK;

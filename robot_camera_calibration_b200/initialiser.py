@@ -12,6 +12,10 @@ The pose chaining itself is a few 4x4 products per frame and stays on the host.
 initialise_targets does the same for rigid tag boards (io_yaml.read_targets): one PnP per (frame, board) over all
 of the board's detected corners (rcc_pnp_target_batch), as cv::calibrateCamera and Kalibr start a board, and the
 same chaining with a board or a free tag in place of each tag.
+
+initialise_intrinsics gives a camera without known intrinsics its start, as cv::initCameraMatrix2D does for
+cv::calibrateCamera: one plane homography per (frame, board) on the GPU (rcc_homography_target_batch) and
+OpenCV's closed form for fx and fy with the principal point at the image centre.
 """
 from __future__ import annotations
 
@@ -176,17 +180,10 @@ def group_entities(frame, where):
     return [(key, members[key]) for key in order]
 
 
-def initialise_targets(frames_pixels, intr, dist, targets, device=0, lens="radtan"):
-    """initialise() with rigid targets: targets = io_yaml.read_targets(...) [(tag ids, corners (n,4,2))].
-    Each frame's detections are grouped into entities (group_entities): a target's cam_T_target comes from one
-    pnp_targets problem over all its detected corners in the frame, a free tag's from pnp_batch.  The entities are
-    chained by chain_poses exactly as tags are (camera_pose.cpp: the world entity first, the last known entity wins,
-    deferred frames retried).  The world is the frame of the first tag of frame 0 (camera_pose.cpp:71-80): when
-    that tag is on a target, the target's pose is invert(board_T_tag) of it, and the target is held constant.
-    Returns (scene, tag_ids, kept_frames, tag_pose, boards) as io_yaml.board_scene: the scene (marker 0 the world
-    entity, then the entities in the order they were chained) carries the corner layout; tag_ids are the detected
-    tags of the chained entities, the world tag first; tag_pose(markers) -> world_T_tag of every tag of tag_ids;
-    boards = [(first tag id of the target, marker block)] in target order."""
+def _entity_problems(frames_pixels, targets):
+    """The problems of initialise_targets: where (tag id -> (target, slot)), the corner layout (n_slots,4,2), each
+    frame's group_entities, the target problems (start, slot, pixels) in the order of the frames and their entities,
+    and the free tags (sizes, pixels) in the same order."""
     where, offset = {}, 0
     for b, (ids, _) in enumerate(targets):
         for k, i in enumerate(np.asarray(ids).tolist()):
@@ -206,6 +203,109 @@ def initialise_targets(frames_pixels, intr, dist, targets, device=0, lens="radta
             else:
                 f_size.append(fr[ks[0]][1])
                 f_pix.append(fr[ks[0]][2])
+    return where, corners, grouped, (t_start, t_slot, t_pix), (f_size, f_pix)
+
+
+def homographies(corners, start, slot, pixels, device=0, max_iterations=100):
+    """H (n,3,3) and final cost (n,) of n rigid-target problems on the GPU (rcc_homography_target_batch): the plane
+    homography (X, Y, 1) in the target frame -> (u, v, 1) in raw pixels, scaled to H[2,2] = 1, that minimises the
+    pixel reprojection error of the problem's corners (cv2.findHomography, method 0, refined to convergence).
+    corners, start, slot and pixels as in pnp_targets.  Cost -1 (and H zero): a singular DLT, a non-finite residual
+    or a corner on or behind the horizon of the plane (w <= 0)."""
+    lib = L.load()
+    corners = np.ascontiguousarray(corners, np.float64).reshape(-1, 8)
+    start = np.ascontiguousarray(start, np.int64).ravel()
+    slot = np.ascontiguousarray(slot, np.int32).ravel()
+    pixels = np.ascontiguousarray(pixels, np.float64).reshape(-1, 8)
+    n = max(len(start) - 1, 0)
+    if len(start) == 0 or len(slot) != start[-1] or len(pixels) != len(slot):
+        raise ValueError(f"start ({len(start)}) must end at the number of tags: slot has {len(slot)}, "
+                         f"pixels {len(pixels)}")
+    H = np.zeros((n, 9))
+    cost = np.empty(n)
+    dp = lambda a: a.ctypes.data_as(L.c_double_p)
+    rc = lib.rcc_homography_target_batch(int(device), len(corners), dp(corners), n, start.ctypes.data_as(L.c_int64_p),
+                                         slot.ctypes.data_as(L.c_int32_p), dp(pixels), dp(H), dp(cost),
+                                         int(max_iterations))
+    if rc != L.RCC_OK:
+        raise L.RccError(rc, "rcc_homography_target_batch failed (no CPU fallback)")
+    return H.reshape(n, 3, 3), cost
+
+
+_UNCONSTRAINED = "the views do not constrain the focal length -- tilt the board"
+
+
+def intrinsics_from_homographies(H, image_size):
+    """intr = (fx, fy, cx, cy) from plane homographies H (n,3,3) of views of a plane and the image size (W, H): the
+    closed form of OpenCV's initIntrinsicParams2D (cv2.initCameraMatrix2D with aspectRatio = 0), restated.  The
+    principal point is the image centre ((W - 1)/2, (H - 1)/2); with it subtracted, each homography's columns h, v
+    and d1 = (h + v)/2, d2 = (h - v)/2 (of the columns before normalisation, each then normalised) give Zhang's two
+    orthogonality rows in (1/fx^2, 1/fy^2), solved by least squares over all views.
+    One intended difference from OpenCV: where OpenCV takes the absolute value of a solution that is not positive,
+    this raises ValueError, as it does when the 2x2 normal matrix is singular or has a condition number above 1e12 --
+    views that do not constrain the focal length (all fronto-parallel, say) give no start at all rather than a wrong
+    one."""
+    H = np.asarray(H, np.float64).reshape(-1, 3, 3)
+    cx, cy = (float(image_size[0]) - 1) * 0.5, (float(image_size[1]) - 1) * 0.5
+    A, b = np.empty((2 * len(H), 2)), np.empty(2 * len(H))
+    for i, h in enumerate(H):
+        h = h.copy()
+        h[0] -= h[2] * cx
+        h[1] -= h[2] * cy
+        t0, t1 = h[:, 0], h[:, 1]
+        d1, d2 = (t0 + t1) * 0.5, (t0 - t1) * 0.5
+        t0, t1, d1, d2 = (x / np.sqrt(x @ x) for x in (t0, t1, d1, d2))
+        A[2 * i] = t0[0] * t1[0], t0[1] * t1[1]
+        A[2 * i + 1] = d1[0] * d2[0], d1[1] * d2[1]
+        b[2 * i], b[2 * i + 1] = -t0[2] * t1[2], -d1[2] * d2[2]
+    N = A.T @ A
+    if not len(H) or not np.isfinite(N).all() or not np.linalg.cond(N) <= 1e12:
+        raise ValueError(_UNCONSTRAINED)
+    f = np.linalg.solve(N, A.T @ b)
+    if not (f > 0).all():
+        raise ValueError(_UNCONSTRAINED)
+    return np.array([np.sqrt(1.0 / f[0]), np.sqrt(1.0 / f[1]), cx, cy])
+
+
+def initialise_intrinsics(frames_pixels, targets, image_size, device=0, min_tags=4):
+    """A pinhole start (fx, fy, cx, cy) for a camera from board detections alone, as cv2.initCameraMatrix2D gives
+    cv2.calibrateCamera's: one homography per (frame, target) problem of initialise_targets with at least min_tags
+    detected tags of the target (homographies, on the GPU), then intrinsics_from_homographies.  Free tags never
+    contribute: the homography of one small tag's 4 corners is too noisy to constrain the focal length.  Returns
+    (intr, number of problems used).  ValueError when no problem qualifies or the views do not constrain the focal
+    length.
+    The start is meant for initialise_targets(frames_pixels, intr, zeros(5), targets, lens=...) with either lens,
+    distortion starting at zero as in OpenCV.  For the equidistant lens the pinhole start is an approximation that
+    holds for boards seen within a moderate field of view; boards seen near 90 degrees off the optical axis have not
+    been verified."""
+    where, corners, grouped, (t_start, t_slot, t_pix), _ = _entity_problems(frames_pixels, targets)
+    n_tags = np.diff(t_start)
+    use = np.nonzero(n_tags >= min_tags)[0]
+    if len(use) == 0:
+        raise ValueError(f"no (frame, board) problem has {min_tags} or more detected tags of a board: the intrinsics "
+                         "are estimated from board views only (free tags are too small to constrain them)")
+    start = np.concatenate([[0], np.cumsum(n_tags[use])])
+    sel = np.concatenate([np.arange(t_start[p], t_start[p + 1]) for p in use])
+    H, cost = homographies(corners, start, np.asarray(t_slot, np.int32)[sel],
+                           np.array(t_pix, float).reshape(-1, 8)[sel], device=device)
+    good = cost >= 0
+    if not good.any():
+        raise ValueError("no board view gave a homography")
+    return intrinsics_from_homographies(H[good], image_size), int(good.sum())
+
+
+def initialise_targets(frames_pixels, intr, dist, targets, device=0, lens="radtan"):
+    """initialise() with rigid targets: targets = io_yaml.read_targets(...) [(tag ids, corners (n,4,2))].
+    Each frame's detections are grouped into entities (group_entities): a target's cam_T_target comes from one
+    pnp_targets problem over all its detected corners in the frame, a free tag's from pnp_batch.  The entities are
+    chained by chain_poses exactly as tags are (camera_pose.cpp: the world entity first, the last known entity wins,
+    deferred frames retried).  The world is the frame of the first tag of frame 0 (camera_pose.cpp:71-80): when
+    that tag is on a target, the target's pose is invert(board_T_tag) of it, and the target is held constant.
+    Returns (scene, tag_ids, kept_frames, tag_pose, boards) as io_yaml.board_scene: the scene (marker 0 the world
+    entity, then the entities in the order they were chained) carries the corner layout; tag_ids are the detected
+    tags of the chained entities, the world tag first; tag_pose(markers) -> world_T_tag of every tag of tag_ids;
+    boards = [(first tag id of the target, marker block)] in target order."""
+    where, corners, grouped, (t_start, t_slot, t_pix), (f_size, f_pix) = _entity_problems(frames_pixels, targets)
     t_pose = (pnp_targets(intr, dist, corners, t_start, t_slot, np.array(t_pix, float).reshape(-1, 8),
                           device=device, lens=lens)[0] if len(t_start) > 1 else np.zeros((0, 6)))
     f_pose = (pnp_batch(intr, dist, f_size, np.array(f_pix, float).reshape(-1, 8), device=device, lens=lens)[0]

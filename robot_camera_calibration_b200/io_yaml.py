@@ -383,26 +383,37 @@ def _remove_stanza(path):
             f.write(txt[:k])
 
 
-def _initialise_directory(directory, intr, dist, lens, targets):
-    """The start of optimise_directory(initialise=True): the camera as read_dataset reads it, the poses from the
-    detections alone.  Returns (scene, tag_ids, kept frame numbers, (all frame numbers, frames_pixels), tag_pose,
-    boards); tag_pose and boards as board_scene's (per tag and empty without targets)."""
+def _initialise_directory(directory, intr, dist, lens, targets, image_size=None, device=0):
+    """The start of optimise_directory(initialise=True): the camera as read_dataset reads it, or, with image_size,
+    initialiser.initialise_intrinsics from the board detections and zero distortion; the poses from the detections
+    alone.  Returns (scene, tag_ids, kept frame numbers, (all frame numbers, frames_pixels), tag_pose, boards,
+    initial intrinsics summary or None); tag_pose and boards as board_scene's (per tag and empty without targets)."""
     from . import initialiser
     if lens is not None and lens not in _LENS_MODEL:
         raise ValueError(f"unknown lens {lens!r}: expected one of {sorted(_LENS_MODEL)}")
-    intr, dist, lens = _dataset_camera(directory, intr, dist, lens)
+    if image_size is None:
+        intr, dist, lens = _dataset_camera(directory, intr, dist, lens)
     numbers, frames_pixels = read_detections(directory)
     if not frames_pixels or not frames_pixels[0]:
         raise ValueError(f"{directory}: the first detections file has no detection: nothing defines the world frame "
                          "(camera_pose.cpp:71-80 makes the first tag of frame 0 the world tag)")
+    boards_read = read_targets(list(targets)) if targets else None
+    initial = None
+    if image_size is not None:
+        lens = lens or "radtan"
+        intr, used = initialiser.initialise_intrinsics(frames_pixels, boards_read, image_size, device=device)
+        dist = np.zeros(5)
+        initial = {"intr": intr.tolist(), "problems_used": used}
     if targets:
         scene, tag_ids, keep, tag_pose, boards = initialiser.initialise_targets(
-            frames_pixels, intr, dist, read_targets(list(targets)), lens=lens)
+            frames_pixels, intr, dist, boards_read, lens=lens)
+        if image_size is not None:
+            scene.image_size = (int(image_size[0]), int(image_size[1]))
     else:
         scene, tag_ids, keep = initialiser.initialise(frames_pixels, intr, dist, lens=lens)
         scene.pixels = _integer_pixels(scene.pixels, frames_pixels)
         tag_pose, boards = (lambda markers: markers), []
-    return scene, tag_ids, numbers[keep], (numbers, frames_pixels), tag_pose, boards
+    return scene, tag_ids, numbers[keep], (numbers, frames_pixels), tag_pose, boards, initial
 
 
 def _integer_pixels(pixels, frames_pixels):
@@ -428,7 +439,8 @@ def intrinsics_priors(intr, dist, sigma):
 
 
 def optimise_directory(directory, device=0, refine_intrinsics=True, precision=None, intr=None, dist=None,
-                       lens=None, intrinsics_sigma=None, targets=None, initialise=False, **lm_options):
+                       lens=None, intrinsics_sigma=None, targets=None, initialise=False, image_size=None,
+                       **lm_options):
     """Milestone 3: detections/ -> GPU bundle adjustment -> detections/ (same formats).  The lens is camera.yaml's
     distortion_model (plumb_bob, or equidistant / fisheye), and camera_refined.yaml is written in the same model.
     intrinsics_sigma = (focal px, principal point px, distortion): refine the intrinsics under a diagonal Gaussian
@@ -440,13 +452,22 @@ def optimise_directory(directory, device=0, refine_intrinsics=True, precision=No
     world_T_camera stanzas are ignored; the camera comes from camera.yaml or intr / dist as in read_dataset; the
     poses come from initialiser.initialise_targets (with targets) or initialiser.initialise (without).  After the
     solve targets.yaml is written per tag, every chained frame gets a world_T_camera stanza, and the stanza of a frame
-    that could not be chained is removed, so that no stale pose is left behind."""
+    that could not be chained is removed, so that no stale pose is left behind.
+    image_size = (width, height): calibrate the camera from the detections alone (needs initialise and targets, and
+    excludes intr / dist, fixed intrinsics and intrinsics_sigma).  camera.yaml is neither read nor written; the start
+    is initialiser.initialise_intrinsics with zero distortion, lens (default "radtan") is the model calibrated, and
+    camera_refined.yaml carries image_size.  The summary gains "initial_intrinsics": {"intr", "problems_used"}."""
     from .problem import BAProblem
     if intrinsics_sigma is not None and not refine_intrinsics:
         raise ValueError("intrinsics_sigma puts a prior on refined intrinsics: it cannot be combined with fixed ones")
+    if image_size is not None and (not initialise or not targets or intr is not None or dist is not None
+                                   or not refine_intrinsics or intrinsics_sigma is not None):
+        raise ValueError("image_size estimates the intrinsics from board detections: it needs initialise and targets "
+                         "and excludes intr, dist, fixed intrinsics and intrinsics_sigma")
+    initial = None
     if initialise:
-        scene, tag_ids, frames, all_frames, tag_pose, boards = _initialise_directory(directory, intr, dist, lens,
-                                                                                     targets)
+        scene, tag_ids, frames, all_frames, tag_pose, boards, initial = _initialise_directory(
+            directory, intr, dist, lens, targets, image_size, device)
     else:
         scene, tag_ids, frames = read_dataset(directory, intr=intr, dist=dist, lens=lens)
     scene.const_intr[:] = not refine_intrinsics
@@ -464,6 +485,8 @@ def optimise_directory(directory, device=0, refine_intrinsics=True, precision=No
         scene.intr, scene.dist = intr, dist
     if targets:
         summary["boards"] = [{"first_tag_id": i, "world_T_board": scene.markers[j].tolist()} for i, j in boards]
+    if initial is not None:
+        summary["initial_intrinsics"] = initial
     if initialise:
         size_of = {int(t): float(sz) for fr in all_frames[1] for (t, sz, _) in fr}
         _write_poses(directory, tag_ids, [size_of[int(t)] for t in tag_ids], tag_pose(scene.markers), scene.views,
